@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this implementation (B200)
     python bench.py --impl reference --gpus N --steps K ...  # CPU restatement of the reference path
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # + DIR/scores.npy of the last timed step
 
 A step = one pass of the hot path over one batch: the model call the reference makes per
 batch (/root/reference/src/models/basic.py:61-63: full-graph propagation, embedding lookup,
@@ -62,7 +63,15 @@ def parse():
     ap.add_argument("--catalog-users", type=int, default=4736,
                     help="users per rank scored against the whole catalog (4736 = 148 SMs x 2 CTAs x 16 users: one full wave of "
                          "the fp32 kernel; the bf16 kernel gets 4x as many)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the scores the model call returned in the last one as "
+                         "DIR/scores.npy (float32, one per pair of the seeded batch; DIR/scores_rank<r>.npy per rank when N > 1)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return args
 
 
 # ----------------------------------------------------------------------------- CPU arm
@@ -413,11 +422,20 @@ def run_b200(args):
     ops.PROFILE_ON = True
     ops.LAUNCHES = 0
     nvl0 = nvlink_counters(local) if world > 1 else None
-    ms, t0, t1 = timed(lambda: model((u_dev, i_dev)), args.steps, 0)
+    last = {}
+
+    def step():
+        last["scores"] = model((u_dev, i_dev))
+    ms, t0, t1 = timed(step, args.steps, 0)
     nvl1 = nvlink_counters(local) if world > 1 else None
     launches = ops.LAUNCHES
     ops.PROFILE_ON = False
     clocks = sampler.stop(t0, t1) if sampler else None
+    if args.dump_outputs:
+        # copied out before anything else runs the model: two builds compare their scores for the same seeded inputs
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        fname = "scores.npy" if world == 1 else "scores_rank%d.npy" % rank
+        np.save(os.path.join(args.dump_outputs, fname), last["scores"].float().cpu().numpy())
     spmm_ms = [a.elapsed_time(b) for (name, a, b, _) in ops.PROFILE if name == "spmm"]
     spmm_meta = [meta for (name, _, _, meta) in ops.PROFILE if name == "spmm"]
     breakdown = {}
