@@ -60,6 +60,8 @@ _SIGS = {
     "cbrs_score_hybrid_topk_bf16_workspace_bytes": (c_size_t, []),
     "cbrs_score_hybrid_topk_bf16": (c_int, [P, P, P, P, c_int64, c_int32, c_int32, P, P, P, P, P, P, P, P, P, P, c_int32, P, P, P,
                                             c_size_t, P]),
+    "cbrs_score_hybrid_topk_bf16_ex": (c_int, [P, P, P, P, c_int64, c_int32, c_int32, P, P, P, P, P, P, P, P, P, P, c_int32, P, P,
+                                               P, P, P, c_size_t, P]),
     "cbrs_dense_grouped": (c_int, [P, c_int64, P, c_int64, c_int32, c_int32, c_int32, P, c_int64, c_int64, c_int,
                                    POINTER(c_void_p), c_int, P]),
     "cbrs_dense_tf32x3_eligible": (c_int, [c_int32, c_int32]),
@@ -74,17 +76,24 @@ _SIGS = {
                                    c_int64, c_int32, P, c_int64, P]),
     "cbrs_gather_rows": (c_int, [P, c_int64, P, c_int64, c_int32, P, c_int64, P]),
     "cbrs_topk_rows": (c_int, [P, c_int64, c_int64, c_int32, c_int32, P, P, P]),
+    "cbrs_exclude_cols": (c_int, [P, c_int64, c_int64, c_int32, c_int32, P, P, P]),
     "cbrs_topk_pairs_workspace_bytes": (c_size_t, [c_int64]),
     "cbrs_topk_pairs": (c_int, [P, P, c_int64, c_int64, P, P, P, c_size_t, P]),
     "cbrs_score_catalog_topk": (c_int, [P, c_int64, P, c_int64, c_int64, c_int32, c_int32, P, P, c_int32, P, P, c_int32,
                                         P, P, P]),
+    "cbrs_score_catalog_topk_ex": (c_int, [P, c_int64, P, c_int64, c_int64, c_int32, c_int32, P, P, c_int32, P, P, c_int32,
+                                           P, P, P, P, P]),
     "cbrs_score_catalog_topk_tf32x3_eligible": (c_int, [c_int32, c_int32]),
     "cbrs_score_catalog_topk_tf32x3_workspace_bytes": (c_size_t, [c_int32, c_int32]),
     "cbrs_score_catalog_topk_tf32x3": (c_int, [P, c_int64, P, c_int64, c_int64, c_int32, c_int32, P, P, c_int32, P, P, c_int32,
                                                P, P, P, c_size_t, P]),
+    "cbrs_score_catalog_topk_tf32x3_ex": (c_int, [P, c_int64, P, c_int64, c_int64, c_int32, c_int32, P, P, c_int32, P, P,
+                                                  c_int32, P, P, P, P, P, c_size_t, P]),
     "cbrs_score_catalog_topk_bf16_workspace_bytes": (c_size_t, [c_int32, c_int32, c_int32]),
     "cbrs_score_catalog_topk_bf16": (c_int, [P, c_int64, P, c_int64, c_int64, c_int32, c_int32, P, P, c_int32, P, P,
                                              c_int32, P, P, P, c_size_t, P]),
+    "cbrs_score_catalog_topk_bf16_ex": (c_int, [P, c_int64, P, c_int64, c_int64, c_int32, c_int32, P, P, c_int32, P, P,
+                                                c_int32, P, P, P, P, P, c_size_t, P]),
     "cbrs_peer_alloc": (c_int, [c_size_t, POINTER(c_void_p)]),
     "cbrs_peer_free": (c_int, [P]),
     "cbrs_peer_export": (c_int, [P, P]),

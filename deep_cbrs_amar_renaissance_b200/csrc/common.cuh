@@ -77,4 +77,22 @@ __device__ __forceinline__ float ld_stream_f32(const float *p) {
     return v;
 }
 
+// Catalog exclusion lists (CSR; contract in include/cbrs_b200.h): is `item` in row `row`'s list?  A lower-bound binary
+// search over [rowptr[row], rowptr[row + 1]): at most log2(len) + 1 probes, never a read outside that range, so an
+// unsorted row can only miss some of its own items.  Null lists exclude nothing.  The fused scorers call it only for
+// a candidate that beats the user's current k-th key, so the search runs rarely; they are instantiated twice
+// (template flag kExcl) so that a call without lists runs the kernel without the check at all.
+__device__ __forceinline__ bool excluded_item(const int64_t *__restrict__ rowptr, const int32_t *__restrict__ items,
+                                              int64_t row, int32_t item) {
+    if (rowptr == nullptr) return false;
+    int64_t lo = __ldg(rowptr + row);
+    const int64_t end = __ldg(rowptr + row + 1);
+    int64_t hi = end;
+    while (lo < hi) {
+        const int64_t mid = lo + ((hi - lo) >> 1);
+        if (__ldg(items + mid) < item) lo = mid + 1; else hi = mid;
+    }
+    return lo < end && __ldg(items + lo) == item;
+}
+
 }  // namespace cbrs

@@ -29,6 +29,7 @@ struct ScoreParams {
     const float *w2, *b2, *w3, *b3;
     int32_t k;
     int32_t *ids_out; float *scores_out;
+    const int64_t *excl_rowptr; const int32_t *excl_items;   // exclusion lists (both null: none)
 };
 
 constexpr int kScThreads = 256;
@@ -74,7 +75,8 @@ __device__ void sc_compact(unsigned long long *c, int *cnt, unsigned long long *
     __syncwarp();
 }
 
-template <int CT>  // threads across the classifier's second-layer columns: 8 (c2 <= 64) or 16 (c2 <= 128)
+// CT: threads across the classifier's second-layer columns: 8 (c2 <= 64) or 16 (c2 <= 128); kExcl: exclusion lists given
+template <int CT, bool kExcl>
 __global__ void __launch_bounds__(kScThreads, 2) score_catalog_kernel(const ScoreParams p) {
     constexpr int PG = kScThreads / CT;  // pair groups (1 user x 8 items each)
     constexpr int UPP = PG / 4;          // users per pass (a user's 32 items = 4 groups)
@@ -176,7 +178,7 @@ __global__ void __launch_bounds__(kScThreads, 2) score_catalog_kernel(const Scor
                     const float score = 1.f / (1.f + expf(-(mine + b3)));
                     const unsigned long long key =
                         ((unsigned long long)sc_orderable(score) << 32) | (unsigned long long)(0xffffffffu - (uint32_t)item);
-                    if (key > thr[ul]) {
+                    if (key > thr[ul] && !(kExcl && excluded_item(p.excl_rowptr, p.excl_items, user, item))) {
                         const int pos = atomicAdd(cnt + ul, 1);
                         cand[ul * cap + pos] = key;  // pos < cap: lists above cap-32 were compacted before this tile
                     }
@@ -217,9 +219,10 @@ template <int CT>
 static int launch_score(const ScoreParams &p, cudaStream_t s) {
     const size_t smem = score_smem_bytes<CT>(p.c1, p.k);
     CBRS_REQUIRE(smem <= 200 * 1024, CBRS_E_UNSUPPORTED, "score_catalog: needs %zu bytes of shared memory", smem);
-    cudaError_t e = cudaFuncSetAttribute(score_catalog_kernel<CT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    auto kernel = p.excl_rowptr ? score_catalog_kernel<CT, true> : score_catalog_kernel<CT, false>;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     CBRS_REQUIRE(e == cudaSuccess, CBRS_E_CUDA, "score_catalog: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    score_catalog_kernel<CT><<<(unsigned)cdiv(p.n_users, kScTU), kScThreads, smem, s>>>(p);
+    kernel<<<(unsigned)cdiv(p.n_users, kScTU), kScThreads, smem, s>>>(p);
     CBRS_CHECK_LAUNCH("score_catalog");
     return CBRS_OK;
 }
@@ -232,7 +235,17 @@ extern "C" int cbrs_score_catalog_topk(const float *P, int64_t ldp, const float 
                                        int32_t n_items, int32_t c1, const float *w2, const float *b2, int32_t c2,
                                        const float *w3, const float *b3, int32_t k, int32_t *ids_out, float *scores_out,
                                        void *stream) {
+    return cbrs_score_catalog_topk_ex(P, ldp, Q, ldq, n_users, n_items, c1, w2, b2, c2, w3, b3, k, ids_out, scores_out,
+                                      nullptr, nullptr, stream);
+}
+
+extern "C" int cbrs_score_catalog_topk_ex(const float *P, int64_t ldp, const float *Q, int64_t ldq, int64_t n_users,
+                                          int32_t n_items, int32_t c1, const float *w2, const float *b2, int32_t c2,
+                                          const float *w3, const float *b3, int32_t k, int32_t *ids_out, float *scores_out,
+                                          const int64_t *excl_rowptr, const int32_t *excl_items, void *stream) {
     CBRS_REQUIRE(P && Q && w2 && b2 && w3 && b3 && ids_out && scores_out, CBRS_E_INVALID, "score_catalog: null argument");
+    CBRS_REQUIRE(!excl_rowptr == !excl_items, CBRS_E_INVALID, "score_catalog: %s is null but %s is not",
+                 excl_rowptr ? "excl_items" : "excl_rowptr", excl_rowptr ? "excl_rowptr" : "excl_items");
     CBRS_REQUIRE(n_users >= 0 && n_items > 0 && k > 0 && k <= 128, CBRS_E_INVALID, "score_catalog: n_users=%lld n_items=%d k=%d",
                  (long long)n_users, n_items, k);
     CBRS_REQUIRE(c1 > 0 && c1 % 4 == 0 && c1 <= 256 && c2 > 0 && c2 <= 128, CBRS_E_UNSUPPORTED,
@@ -240,6 +253,6 @@ extern "C" int cbrs_score_catalog_topk(const float *P, int64_t ldp, const float 
     CBRS_REQUIRE(ldp >= c1 && ldq >= c1 && ldq % 4 == 0 && ((uintptr_t)Q % 16) == 0, CBRS_E_INVALID,
                  "score_catalog: Q must be 16-byte aligned with ldq %% 4 == 0");
     if (n_users == 0) return CBRS_OK;
-    ScoreParams p{P, ldp, Q, ldq, n_users, n_items, c1, c2, w2, b2, w3, b3, k, ids_out, scores_out};
+    ScoreParams p{P, ldp, Q, ldq, n_users, n_items, c1, c2, w2, b2, w3, b3, k, ids_out, scores_out, excl_rowptr, excl_items};
     return c2 <= 64 ? launch_score<8>(p, (cudaStream_t)stream) : launch_score<16>(p, (cudaStream_t)stream);
 }

@@ -41,6 +41,8 @@ struct HybridTcParams {
     int32_t k;
     int32_t *ids_out;
     float *scores_out;
+    const int64_t *excl_rowptr;          // exclusion lists (both null: none)
+    const int32_t *excl_items;
 };
 
 __device__ __forceinline__ uint32_t hy_orderable(float f) {
@@ -112,7 +114,7 @@ __device__ __forceinline__ void hy_store_row(unsigned char *tile, int tid, bool 
 
 constexpr int kHyQLd = kHyC + 4;   // padded row of the staged Q tile: 8 consecutive lanes hit 8 distinct 16-byte bank groups
 
-template <int TU>
+template <int TU, bool kExcl>   // kExcl: exclusion lists given
 __global__ void __launch_bounds__(kHyThreads, 2) score_hybrid_tc_kernel(const HybridTcParams p) {
     extern __shared__ __align__(1024) unsigned char hy_smem[];
     const int cap = 2 * p.k + kHyTI;
@@ -299,7 +301,7 @@ __global__ void __launch_bounds__(kHyThreads, 2) score_hybrid_tc_kernel(const Hy
                 // ranked by the logit (sigmoid is monotonic); the sigmoid is applied to the k winners
                 const unsigned long long key =
                     ((unsigned long long)hy_orderable(logit + bc3) << 32) | (unsigned long long)(0xffffffffu - (uint32_t)item);
-                if (key > thr[ul]) {
+                if (key > thr[ul] && !(kExcl && excluded_item(p.excl_rowptr, p.excl_items, user, item))) {
                     const int pos = atomicAdd(cnt + ul, 1);
                     cand[ul * cap + pos] = key;
                 }
@@ -341,13 +343,15 @@ template <int TU>
 static int hy_launch(const HybridTcParams &p, cudaStream_t s) {
     const size_t smem = hy_smem_bytes(p.k, TU);
     CBRS_REQUIRE(smem <= 227 * 1024, CBRS_E_UNSUPPORTED, "score_hybrid_topk_bf16: needs %zu bytes of shared memory", smem);
-    static size_t configured = 0;
-    if (smem > configured) {
-        cudaError_t e = cudaFuncSetAttribute(score_hybrid_tc_kernel<TU>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    static size_t configured[2] = {0, 0};
+    const int x = p.excl_rowptr ? 1 : 0;
+    auto kernel = x ? score_hybrid_tc_kernel<TU, true> : score_hybrid_tc_kernel<TU, false>;
+    if (smem > configured[x]) {
+        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         CBRS_REQUIRE(e == cudaSuccess, CBRS_E_CUDA, "score_hybrid_topk_bf16: %s", cudaGetErrorString(e));
-        configured = smem;
+        configured[x] = smem;
     }
-    score_hybrid_tc_kernel<TU><<<(unsigned)cdiv(p.n_users, TU), kHyThreads, smem, s>>>(p);
+    kernel<<<(unsigned)cdiv(p.n_users, TU), kHyThreads, smem, s>>>(p);
     CBRS_CHECK_LAUNCH("score_hybrid_topk_bf16");
     return CBRS_OK;
 }
@@ -363,9 +367,22 @@ extern "C" int cbrs_score_hybrid_topk_bf16(const float *P1, const float *Q1, con
                                            const float *b3b2, const float *wc1, const float *bc1, const float *wc2,
                                            const float *bc2, const float *wc3, const float *bc3, int32_t k, int32_t *ids_out,
                                            float *scores_out, void *workspace, size_t workspace_bytes, void *stream) {
+    return cbrs_score_hybrid_topk_bf16_ex(P1, Q1, P2, Q2, n_users, n_items, c, w3a2, b3a2, w3b2, b3b2, wc1, bc1, wc2, bc2, wc3,
+                                          bc3, k, ids_out, scores_out, nullptr, nullptr, workspace, workspace_bytes, stream);
+}
+
+extern "C" int cbrs_score_hybrid_topk_bf16_ex(const float *P1, const float *Q1, const float *P2, const float *Q2,
+                                              int64_t n_users, int32_t n_items, int32_t c, const float *w3a2,
+                                              const float *b3a2, const float *w3b2, const float *b3b2, const float *wc1,
+                                              const float *bc1, const float *wc2, const float *bc2, const float *wc3,
+                                              const float *bc3, int32_t k, int32_t *ids_out, float *scores_out,
+                                              const int64_t *excl_rowptr, const int32_t *excl_items, void *workspace,
+                                              size_t workspace_bytes, void *stream) {
     CBRS_REQUIRE(P1 && Q1 && P2 && Q2 && w3a2 && b3a2 && w3b2 && b3b2 && wc1 && bc1 && wc2 && bc2 && wc3 && bc3 && ids_out &&
                      scores_out && workspace,
                  CBRS_E_INVALID, "score_hybrid_topk_bf16: null argument");
+    CBRS_REQUIRE(!excl_rowptr == !excl_items, CBRS_E_INVALID, "score_hybrid_topk_bf16: %s is null but %s is not",
+                 excl_rowptr ? "excl_items" : "excl_rowptr", excl_rowptr ? "excl_rowptr" : "excl_items");
     CBRS_REQUIRE(c == kHyC, CBRS_E_UNSUPPORTED, "score_hybrid_topk_bf16: built for %d-wide hidden layers (every hybrid grid of the "
                  "reference), got %d", kHyC, c);
     CBRS_REQUIRE(n_users >= 0 && n_items > 0 && k > 0 && k <= 128 && k <= n_items, CBRS_E_INVALID,
@@ -381,6 +398,7 @@ extern "C" int cbrs_score_hybrid_topk_bf16(const float *P1, const float *Q1, con
     p.w_images = (const uint8_t *)workspace;
     p.b3a2 = b3a2; p.b3b2 = b3b2; p.bc1 = bc1; p.bc2 = bc2; p.wc3 = wc3; p.bc3 = bc3;
     p.k = k; p.ids_out = ids_out; p.scores_out = scores_out;
+    p.excl_rowptr = excl_rowptr; p.excl_items = excl_items;
     // users per CTA: 16, unless 24 or 32 bring the grid down to one wave (2 CTAs per SM) - a second, part-filled wave
     // costs as much as a full one
     const int64_t slots = 2 * kSMs;

@@ -33,6 +33,7 @@ struct ScoreTcParams {
     const float *b2, *w3, *b3;
     int32_t k;
     int32_t *ids_out; float *scores_out;
+    const int64_t *excl_rowptr; const int32_t *excl_items;   // exclusion lists (both null: none)
 };
 
 constexpr int kTcThreads = 128;
@@ -93,7 +94,7 @@ __global__ void score_tc_prep_kernel(const float *__restrict__ w2, int c1, int c
 // QREG: the classifier's first width fits one 64-wide K block, so a thread keeps its item's Q row
 // (64 floats) in registers for all passes of a tile and refills it while the last pass's MMA and
 // epilogue are in flight; otherwise Q chunks are re-read (L1) in every pass.
-template <bool QREG>
+template <bool QREG, bool kExcl>   // kExcl: exclusion lists given
 __global__ void __launch_bounds__(kTcThreads, QREG ? 4 : 3) score_tc_kernel(const ScoreTcParams p) {
     extern __shared__ __align__(1024) unsigned char smem_raw[];  // SWIZZLE_128B tiles need 1024-byte alignment
     const int c1 = p.c1;
@@ -249,7 +250,7 @@ __global__ void __launch_bounds__(kTcThreads, QREG ? 4 : 3) score_tc_kernel(cons
                 // candidates are ranked by the logit (sigmoid is monotonic); the sigmoid is applied to the k winners
                 const unsigned long long key =
                     ((unsigned long long)tcs_orderable(logit + b3) << 32) | (unsigned long long)(0xffffffffu - (uint32_t)item);
-                if (key > thr[ul]) {
+                if (key > thr[ul] && !(kExcl && excluded_item(p.excl_rowptr, p.excl_items, user, item))) {
                     const int pos = atomicAdd(cnt + ul, 1);
                     cand[ul * cap + pos] = key;
                 }
@@ -299,6 +300,7 @@ struct ScoreTc2Params {
     const float *b2, *w3, *b3;
     int32_t k;
     int32_t *ids_out; float *scores_out;
+    const int64_t *excl_rowptr; const int32_t *excl_items;   // exclusion lists (both null: none)
 };
 
 // bias and output-layer weights in constant memory: the fully unrolled epilogue (NP > 0) reads them as
@@ -343,7 +345,7 @@ __device__ __forceinline__ unsigned long long f32x2_fma(unsigned long long a, un
     return d;
 }
 
-template <bool kPackedEpilogue, int NP>
+template <bool kPackedEpilogue, int NP, bool kExcl>   // kExcl: exclusion lists given
 __global__ void __launch_bounds__(kTcThreads, 4) score_tc2_kernel(const __grid_constant__ ScoreTc2Params p) {
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     const int c1 = p.c1;
@@ -530,7 +532,7 @@ __global__ void __launch_bounds__(kTcThreads, 4) score_tc2_kernel(const __grid_c
         if (item < p.n_items && user < p.n_users) {
             const unsigned long long key =
                 ((unsigned long long)tcs_orderable(logit + b3) << 32) | (unsigned long long)(0xffffffffu - (uint32_t)item);
-            if (key > thr[ul]) {
+            if (key > thr[ul] && !(kExcl && excluded_item(p.excl_rowptr, p.excl_items, user, item))) {
                 const int pos = atomicAdd(cnt + ul, 1);
                 cand[ul * cap + pos] = key;
             }
@@ -594,6 +596,7 @@ struct ScoreTc3Params {
     const float *b3;
     int32_t k;
     int32_t *ids_out; float *scores_out;
+    const int64_t *excl_rowptr; const int32_t *excl_items;   // exclusion lists (both null: none)
 };
 
 __global__ void score_tc3_prep_kernel(const float *__restrict__ w2, const float *__restrict__ b2, const float *__restrict__ w3,
@@ -659,6 +662,7 @@ __device__ __forceinline__ uint32_t w3_pack_relu(float lo, float hi) {
     return d;
 }
 
+template <bool kExcl>   // exclusion lists given
 __global__ void __launch_bounds__(kW3Threads, 1) score_tc3_kernel(const __grid_constant__ ScoreTc3Params p) {
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     const int cap = 2 * p.k + kTcTI;
@@ -789,6 +793,12 @@ __global__ void __launch_bounds__(kW3Threads, 1) score_tc3_kernel(const __grid_c
         }
     } else if (warp < 12) {
         // ---------------- final: logit column -> candidate list of the row's user ----------------
+        // Exclusion lists (kExcl): a binary search of the user's list per candidate above the threshold (excluded_item).
+        // It costs these warps, the pipeline's last stage, +15 % / +21 % kernel time with MovieLens-like / Zipf lists at
+        // 4,736 x 200,000 on a B200.  The rival - a bitmask of the tile's listed items, filled by this warp from a per-user
+        // cursor before it waits for the logit (no synchronisation with the producer / MMA warps needed) - measured worse:
+        // +42 % / +40 %, and +25 % with empty lists, the per-step ballot + reduction on this critical stage costing more
+        // than the rare searches (profiles/r03_score_bench_exclusion.jsonl, README there).
         const int quad = warp & 3;
         const float b3 = __ldg(p.b3);
         int step = 0;
@@ -811,7 +821,7 @@ __global__ void __launch_bounds__(kW3Threads, 1) score_tc3_kernel(const __grid_c
                 if (item < p.n_items && user < p.n_users) {
                     const unsigned long long key =
                         ((unsigned long long)tcs_orderable(logit + b3) << 32) | (unsigned long long)(0xffffffffu - (uint32_t)item);
-                    if (key > thr[ul]) {
+                    if (key > thr[ul] && !(kExcl && excluded_item(p.excl_rowptr, p.excl_items, user, item))) {
                         const int pos = atomicAdd(cnt + ul, 1);
                         cand[ul * cap + pos] = key;
                     }
@@ -919,7 +929,18 @@ extern "C" int cbrs_score_catalog_topk_bf16(const float *P, int64_t ldp, const f
                                             int32_t n_items, int32_t c1, const float *w2, const float *b2, int32_t c2,
                                             const float *w3, const float *b3, int32_t k, int32_t *ids_out,
                                             float *scores_out, void *workspace, size_t workspace_bytes, void *stream) {
+    return cbrs_score_catalog_topk_bf16_ex(P, ldp, Q, ldq, n_users, n_items, c1, w2, b2, c2, w3, b3, k, ids_out, scores_out,
+                                           nullptr, nullptr, workspace, workspace_bytes, stream);
+}
+
+extern "C" int cbrs_score_catalog_topk_bf16_ex(const float *P, int64_t ldp, const float *Q, int64_t ldq, int64_t n_users,
+                                               int32_t n_items, int32_t c1, const float *w2, const float *b2, int32_t c2,
+                                               const float *w3, const float *b3, int32_t k, int32_t *ids_out,
+                                               float *scores_out, const int64_t *excl_rowptr, const int32_t *excl_items,
+                                               void *workspace, size_t workspace_bytes, void *stream) {
     CBRS_REQUIRE(P && Q && w2 && b2 && w3 && b3 && ids_out && scores_out, CBRS_E_INVALID, "score_catalog_bf16: null argument");
+    CBRS_REQUIRE(!excl_rowptr == !excl_items, CBRS_E_INVALID, "score_catalog_bf16: %s is null but %s is not",
+                 excl_rowptr ? "excl_items" : "excl_rowptr", excl_rowptr ? "excl_rowptr" : "excl_items");
     CBRS_REQUIRE(n_users >= 0 && n_items > 0 && k > 0 && k <= 128, CBRS_E_INVALID, "score_catalog_bf16: n_users=%lld n_items=%d k=%d",
                  (long long)n_users, n_items, k);
     CBRS_REQUIRE(c1 >= 8 && c1 % 8 == 0 && c1 <= 256 && c2 > 0 && c2 <= 256, CBRS_E_UNSUPPORTED,
@@ -945,17 +966,20 @@ extern "C" int cbrs_score_catalog_topk_bf16(const float *P, int64_t ldp, const f
             CBRS_CHECK_LAUNCH("score_tc3_prep");
             const size_t smem3 = score_tc3_smem(k);
             CBRS_REQUIRE(smem3 <= 200 * 1024, CBRS_E_UNSUPPORTED, "score_catalog_bf16: needs %zu bytes of shared memory", smem3);
-            cudaError_t e3 = cudaFuncSetAttribute(score_tc3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem3);
+            auto k3 = excl_rowptr ? score_tc3_kernel<true> : score_tc3_kernel<false>;
+            cudaError_t e3 = cudaFuncSetAttribute(k3, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem3);
             CBRS_REQUIRE(e3 == cudaSuccess, CBRS_E_CUDA, "score_catalog_bf16: cudaFuncSetAttribute: %s", cudaGetErrorString(e3));
-            ScoreTc3Params p3{P, ldp, Qb, n_users, n_items, c1, c2, img, img + 2 * 8192, b3, k, ids_out, scores_out};
-            score_tc3_kernel<<<(unsigned)cdiv(n_users, kTcTU), kW3Threads, smem3, s>>>(p3);
+            ScoreTc3Params p3{P, ldp, Qb, n_users, n_items, c1, c2, img, img + 2 * 8192, b3, k, ids_out, scores_out,
+                               excl_rowptr, excl_items};
+            k3<<<(unsigned)cdiv(n_users, kTcTU), kW3Threads, smem3, s>>>(p3);
             CBRS_CHECK_LAUNCH("score_tc3");
             return CBRS_OK;
         }
         const size_t smem2 = score_tc2_smem(c2, k);
         CBRS_REQUIRE(smem2 <= 220 * 1024, CBRS_E_UNSUPPORTED, "score_catalog_bf16: needs %zu bytes of shared memory", smem2);
         static const int mode = getenv("CBRS_SCORE_EPILOGUE") ? atoi(getenv("CBRS_SCORE_EPILOGUE")) : 0;  // tuning knob
-        ScoreTc2Params p2{P, ldp, Qb, n_users, n_items, c1, c2, (const uint8_t *)workspace, b2, w3, b3, k, ids_out, scores_out};
+        ScoreTc2Params p2{P, ldp, Qb, n_users, n_items, c1, c2, (const uint8_t *)workspace, b2, w3, b3, k, ids_out, scores_out,
+                          excl_rowptr, excl_items};
         const unsigned grid = (unsigned)cdiv(n_users, kTcTU);
         // mode 0: n_pad == 64 -> constant-bank epilogue (b2/w3 copied to constant memory);
         // mode 1: shared-memory scalar epilogue; mode 2: shared-memory packed fp32x2 epilogue
@@ -964,32 +988,34 @@ extern "C" int cbrs_score_catalog_topk_bf16(const float *P, int64_t ldp, const f
             cudaError_t ec = cudaMemcpyToSymbolAsync(g_score_b2, b2, sizeof(float) * c2, 0, cudaMemcpyDeviceToDevice, s);
             if (ec == cudaSuccess) ec = cudaMemcpyToSymbolAsync(g_score_w3, w3, sizeof(float) * c2, 0, cudaMemcpyDeviceToDevice, s);
             CBRS_REQUIRE(ec == cudaSuccess, CBRS_E_CUDA, "score_catalog_bf16: staging b2/w3: %s", cudaGetErrorString(ec));
-            cudaError_t e2 = cudaFuncSetAttribute(score_tc2_kernel<false, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
+            auto k2 = excl_rowptr ? score_tc2_kernel<false, 64, true> : score_tc2_kernel<false, 64, false>;
+            cudaError_t e2 = cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
             CBRS_REQUIRE(e2 == cudaSuccess, CBRS_E_CUDA, "score_catalog_bf16: cudaFuncSetAttribute: %s", cudaGetErrorString(e2));
-            score_tc2_kernel<false, 64><<<grid, kTcThreads, smem2, s>>>(p2);
+            k2<<<grid, kTcThreads, smem2, s>>>(p2);
         } else if (mode == 2) {
-            cudaError_t e2 = cudaFuncSetAttribute(score_tc2_kernel<true, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
+            auto k2 = excl_rowptr ? score_tc2_kernel<true, 0, true> : score_tc2_kernel<true, 0, false>;
+            cudaError_t e2 = cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
             CBRS_REQUIRE(e2 == cudaSuccess, CBRS_E_CUDA, "score_catalog_bf16: cudaFuncSetAttribute: %s", cudaGetErrorString(e2));
-            score_tc2_kernel<true, 0><<<grid, kTcThreads, smem2, s>>>(p2);
+            k2<<<grid, kTcThreads, smem2, s>>>(p2);
         } else {
-            cudaError_t e2 = cudaFuncSetAttribute(score_tc2_kernel<false, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
+            auto k2 = excl_rowptr ? score_tc2_kernel<false, 0, true> : score_tc2_kernel<false, 0, false>;
+            cudaError_t e2 = cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
             CBRS_REQUIRE(e2 == cudaSuccess, CBRS_E_CUDA, "score_catalog_bf16: cudaFuncSetAttribute: %s", cudaGetErrorString(e2));
-            score_tc2_kernel<false, 0><<<grid, kTcThreads, smem2, s>>>(p2);
+            k2<<<grid, kTcThreads, smem2, s>>>(p2);
         }
         CBRS_CHECK_LAUNCH("score_tc2");
         return CBRS_OK;
     }
     const size_t smem = score_tc_smem(c1, c2, k);
     CBRS_REQUIRE(smem <= 220 * 1024, CBRS_E_UNSUPPORTED, "score_catalog_bf16: needs %zu bytes of shared memory", smem);
-    ScoreTcParams p{P, ldp, Q, ldq, n_users, n_items, c1, c2, (const uint8_t *)workspace, b2, w3, b3, k, ids_out, scores_out};
+    ScoreTcParams p{P, ldp, Q, ldq, n_users, n_items, c1, c2, (const uint8_t *)workspace, b2, w3, b3, k, ids_out, scores_out,
+                     excl_rowptr, excl_items};
     const bool qreg = c1 <= 64;
-    cudaError_t e = qreg ? cudaFuncSetAttribute(score_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
-                         : cudaFuncSetAttribute(score_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    auto k1 = qreg ? (excl_rowptr ? score_tc_kernel<true, true> : score_tc_kernel<true, false>)
+                   : (excl_rowptr ? score_tc_kernel<false, true> : score_tc_kernel<false, false>);
+    cudaError_t e = cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     CBRS_REQUIRE(e == cudaSuccess, CBRS_E_CUDA, "score_catalog_bf16: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    if (qreg)
-        score_tc_kernel<true><<<(unsigned)cdiv(n_users, kTcTU), kTcThreads, smem, s>>>(p);
-    else
-        score_tc_kernel<false><<<(unsigned)cdiv(n_users, kTcTU), kTcThreads, smem, s>>>(p);
+    k1<<<(unsigned)cdiv(n_users, kTcTU), kTcThreads, smem, s>>>(p);
     CBRS_CHECK_LAUNCH("score_tc");
     return CBRS_OK;
 }

@@ -38,6 +38,7 @@ struct ScoreT3Params {
     const float *b2, *w3, *b3;
     int32_t k;
     int32_t *ids_out; float *scores_out;
+    const int64_t *excl_rowptr; const int32_t *excl_items;   // exclusion lists (both null: none)
 };
 
 constexpr int kS3TU = 16;   // users per CTA (4 passes of 4 users per item tile)
@@ -141,7 +142,7 @@ __device__ __forceinline__ void s3_tmem_st16(uint32_t taddr, const uint32_t (&v)
 //               output layer, candidate list of the row's user (user u is only ever touched by warp 9 + u % 4).  (Eight
 //               epilogue warps - two per quadrant, partial logits combined through shared memory - measured slower:
 //               50.8 vs 47.4 ms at 4736 x 200k.)
-template <int C1, int NP>
+template <int C1, int NP, bool kExcl>   // kExcl: exclusion lists given
 __global__ void __launch_bounds__(kS3WsThreads, 1) score_tf32x3_ws_kernel(const __grid_constant__ ScoreT3Params p) {
     extern __shared__ __align__(1024) unsigned char s3_smem[];
     constexpr int kAtoms = C1 / 32;
@@ -282,6 +283,10 @@ __global__ void __launch_bounds__(kS3WsThreads, 1) score_tf32x3_ws_kernel(const 
         }
     } else {
         // ---------------- epilogue (warps 9..12: TMEM lane quadrant = warp & 3) ----------------
+        // Exclusion lists (kExcl): a binary search of the user's list per candidate above the threshold (excluded_item):
+        // +7 % / +10 % kernel time with MovieLens-like / Zipf lists at 4,736 x 200,000 on a B200.  A per-tile bitmask filled
+        // by these warps from a per-user cursor measured worse (+12 % / +11 %, +9 % with empty lists;
+        // profiles/r03_score_bench_exclusion.jsonl, README there).
         const int quad = warp & 3;
         const float b3 = __ldg(p.b3);
         int step = 0;
@@ -317,7 +322,7 @@ __global__ void __launch_bounds__(kS3WsThreads, 1) score_tf32x3_ws_kernel(const 
                     // candidates are ranked by the logit (sigmoid is monotonic); the sigmoid is applied to the k winners
                     const unsigned long long key = ((unsigned long long)s3_orderable(logit + b3) << 32) |
                                                    (unsigned long long)(0xffffffffu - (uint32_t)item);
-                    if (key > thr[ul]) {
+                    if (key > thr[ul] && !(kExcl && excluded_item(p.excl_rowptr, p.excl_items, user, item))) {
                         const int pos = atomicAdd(cnt + ul, 1);
                         cand[ul * cap + pos] = key;
                     }
@@ -360,9 +365,10 @@ template <int C1, int NP>
 static int s3_launch_ws(const ScoreT3Params &p, cudaStream_t s) {
     const size_t smem = s3_smem_bytes(C1, NP, p.k);
     CBRS_REQUIRE(smem <= 200 * 1024, CBRS_E_UNSUPPORTED, "score_catalog_tf32x3: needs %zu bytes of shared memory", smem);
-    cudaError_t e = cudaFuncSetAttribute(score_tf32x3_ws_kernel<C1, NP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    auto kernel = p.excl_rowptr ? score_tf32x3_ws_kernel<C1, NP, true> : score_tf32x3_ws_kernel<C1, NP, false>;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     CBRS_REQUIRE(e == cudaSuccess, CBRS_E_CUDA, "score_catalog_tf32x3: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    score_tf32x3_ws_kernel<C1, NP><<<(unsigned)cdiv(p.n_users, kS3TU), kS3WsThreads, smem, s>>>(p);
+    kernel<<<(unsigned)cdiv(p.n_users, kS3TU), kS3WsThreads, smem, s>>>(p);
     CBRS_CHECK_LAUNCH("score_catalog_tf32x3");
     return CBRS_OK;
 }
@@ -384,7 +390,18 @@ extern "C" int cbrs_score_catalog_topk_tf32x3(const float *P, int64_t ldp, const
                                               int32_t n_items, int32_t c1, const float *w2, const float *b2, int32_t c2,
                                               const float *w3, const float *b3, int32_t k, int32_t *ids_out, float *scores_out,
                                               void *workspace, size_t workspace_bytes, void *stream) {
+    return cbrs_score_catalog_topk_tf32x3_ex(P, ldp, Q, ldq, n_users, n_items, c1, w2, b2, c2, w3, b3, k, ids_out, scores_out,
+                                             nullptr, nullptr, workspace, workspace_bytes, stream);
+}
+
+extern "C" int cbrs_score_catalog_topk_tf32x3_ex(const float *P, int64_t ldp, const float *Q, int64_t ldq, int64_t n_users,
+                                                 int32_t n_items, int32_t c1, const float *w2, const float *b2, int32_t c2,
+                                                 const float *w3, const float *b3, int32_t k, int32_t *ids_out,
+                                                 float *scores_out, const int64_t *excl_rowptr, const int32_t *excl_items,
+                                                 void *workspace, size_t workspace_bytes, void *stream) {
     CBRS_REQUIRE(P && Q && w2 && b2 && w3 && b3 && ids_out && scores_out, CBRS_E_INVALID, "score_catalog_tf32x3: null argument");
+    CBRS_REQUIRE(!excl_rowptr == !excl_items, CBRS_E_INVALID, "score_catalog_tf32x3: %s is null but %s is not",
+                 excl_rowptr ? "excl_items" : "excl_rowptr", excl_rowptr ? "excl_rowptr" : "excl_items");
     CBRS_REQUIRE(n_users >= 0 && n_items > 0 && k > 0 && k <= 128, CBRS_E_INVALID, "score_catalog_tf32x3: n_users=%lld n_items=%d k=%d",
                  (long long)n_users, n_items, k);
     CBRS_REQUIRE(cbrs_score_catalog_topk_tf32x3_eligible(c1, c2), CBRS_E_UNSUPPORTED,
@@ -410,7 +427,7 @@ extern "C" int cbrs_score_catalog_topk_tf32x3(const float *P, int64_t ldp, const
     }
     int rc = cbrs_dense_tf32x3_prepare(w_src, c1, np, image, stream);
     if (rc != CBRS_OK) return rc;
-    ScoreT3Params p{P, ldp, Q, ldq, n_users, n_items, c1, c2, image, b2, w3, b3, k, ids_out, scores_out};
+    ScoreT3Params p{P, ldp, Q, ldq, n_users, n_items, c1, c2, image, b2, w3, b3, k, ids_out, scores_out, excl_rowptr, excl_items};
     if (c1 == 64) return np == 64 ? s3_launch_ws<64, 64>(p, s) : s3_launch_ws<64, 32>(p, s);
     return np == 64 ? s3_launch_ws<32, 64>(p, s) : s3_launch_ws<32, 32>(p, s);
 }

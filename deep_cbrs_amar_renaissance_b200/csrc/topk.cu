@@ -86,9 +86,47 @@ __global__ void pair_rank_kernel(const uint64_t *__restrict__ keys, const uint32
     }
 }
 
+// Generic catalog path: one warp per row writes -inf over the listed items that fall in the row's column block
+// [col_base, col_base + n_cols).  A binary search finds the first entry >= col_base; the lanes then walk the entries
+// inside the block only, so a row costs log2(len) + (its items in the block) / 32 reads.
+constexpr int kExclThreads = 256;
+__global__ void __launch_bounds__(kExclThreads) exclude_cols_kernel(float *__restrict__ scores, int64_t ld, int64_t n_rows,
+                                                                   int32_t n_cols, int32_t col_base,
+                                                                   const int64_t *__restrict__ rowptr,
+                                                                   const int32_t *__restrict__ items) {
+    const int64_t r = (int64_t)blockIdx.x * (kExclThreads / 32) + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (r >= n_rows) return;
+    const int64_t end = __ldg(rowptr + r + 1);
+    int64_t lo = __ldg(rowptr + r), hi = end;
+    while (lo < hi) {
+        const int64_t mid = lo + ((hi - lo) >> 1);
+        if (__ldg(items + mid) < col_base) lo = mid + 1; else hi = mid;
+    }
+    for (int64_t j = lo + lane; j < end; j += 32) {
+        const int64_t c = (int64_t)__ldg(items + j) - col_base;
+        if (c >= n_cols) break;   // sorted row: every later entry of this lane is past the block too
+        if (c >= 0) scores[r * ld + c] = -INFINITY;
+    }
+}
+
 }  // namespace cbrs
 
 using namespace cbrs;
+
+extern "C" int cbrs_exclude_cols(float *scores, int64_t ld, int64_t n_rows, int32_t n_cols, int32_t col_base,
+                                 const int64_t *excl_rowptr, const int32_t *excl_items, void *stream) {
+    CBRS_REQUIRE(scores, CBRS_E_INVALID, "exclude_cols: null scores");
+    CBRS_REQUIRE(!excl_rowptr == !excl_items, CBRS_E_INVALID, "exclude_cols: %s is null but %s is not",
+                 excl_rowptr ? "excl_items" : "excl_rowptr", excl_rowptr ? "excl_rowptr" : "excl_items");
+    CBRS_REQUIRE(n_rows >= 0 && n_cols >= 0 && ld >= n_cols && col_base >= 0, CBRS_E_INVALID,
+                 "exclude_cols: n_rows=%lld n_cols=%d ld=%lld col_base=%d", (long long)n_rows, n_cols, (long long)ld, col_base);
+    if (!excl_rowptr || n_rows == 0 || n_cols == 0) return CBRS_OK;
+    exclude_cols_kernel<<<(unsigned)cdiv(n_rows, kExclThreads / 32), kExclThreads, 0, (cudaStream_t)stream>>>(
+        scores, ld, n_rows, n_cols, col_base, excl_rowptr, excl_items);
+    CBRS_CHECK_LAUNCH("exclude_cols");
+    return CBRS_OK;
+}
 
 extern "C" int cbrs_topk_rows(const float *scores, int64_t ld, int64_t n_users, int32_t n_items, int32_t k,
                               int32_t *ids_out, float *vals_out, void *stream) {

@@ -9,6 +9,9 @@ and loader lookup by name (:107-118), loader / optimiser keyword filtering by si
 dispatch on the model family (:136-153), compile -> one call to create the weights -> summary (:155-170), fit with the
 log callback (:172-188), evaluate -> predict -> per-user top-5 / top-10 written as
 predictions/top_<k>/predictions_1.tsv -> P/R/F1@k (:190-222), one failed experiment does not stop the others (:299-302).
+What is added, off unless a config sets the top-level key `catalog_metrics: true`: P/R/F1@k of full-catalog top-k lists
+(every item ranked for every user, the user's training items excluded) against the test ratings, reported as
+catalog_{precision,recall,f1}_at_{k}.
 What is replaced: MLflow run management by a directory per run holding config.yaml, log.txt, metrics.json;
 ruamel.yaml by PyYAML with the YAML-1.2 float forms the files use (`1e-4`); the Java evaluator by
 utilities.metrics.top_k_metrics.
@@ -24,6 +27,7 @@ import time
 import traceback
 
 import numpy as np
+import pandas as pd
 import yaml
 
 from . import models  # noqa: F401  (model modules are looked up by name below)
@@ -33,7 +37,8 @@ from .models.basic import BasicGNN, BasicKnowledgeGCN, BasicRS, BasicTSGNN, Basi
 from .models.hybrid import HybridBertGNN, HybridCBRS
 from .training import Adam
 from .utilities.keras import LogCallback, get_total_parameters
-from .utilities.metrics import top_k_metrics, top_k_predictions
+from .scoring import ItemLists
+from .utilities.metrics import catalog_predictions, precision_recall_f1_at_k, top_k_metrics, top_k_predictions
 from .utilities.utils import get_experiment_logger, make_grid, nested_dict_update
 
 PARAMS_PATH = 'config.yaml'
@@ -93,6 +98,12 @@ class Experimenter:
         self.config = Config(config)
         set_seed(self.config.seed)
         name = self.config.model.name
+        module_name, class_name = name.split('.')
+        self.model_class = getattr(importlib.import_module(models.__name__ + '.' + module_name), class_name)
+        self.catalog_metrics = bool(self.config.get('catalog_metrics'))
+        if self.catalog_metrics and not hasattr(self.model_class, 'recommend_top_k'):
+            raise ValueError("catalog_metrics: {} scores pre-computed embedding rows and has no full-catalog top-k "
+                             "(recommend_top_k); use a graph model".format(name))
         self.exp_name = time.strftime("%m_%d-%H_%M") + '-' + name
         if BasicRS.__name__ in name:
             pass
@@ -113,8 +124,6 @@ class Experimenter:
             yaml.safe_dump(config, fp)
         self.logger = get_experiment_logger(self.dest)
         self.logger.info('CONFIG\n' + yaml.safe_dump(config))
-        module_name, class_name = name.split('.')
-        self.model_class = getattr(importlib.import_module(models.__name__ + '.' + module_name), class_name)
         self.load_function = getattr(loaders, self.config.dataset.load_function_name)
         if self.config.parameters.optimizer.name != 'Adam':
             raise NotImplementedError("optimizer '{}' (the reference's configs use Adam)".format(self.config.parameters.optimizer.name))
@@ -168,10 +177,29 @@ class Experimenter:
             res = top_k_metrics(self.config.dataset.test_ratings_filepath, top_k_dest)[k]
             self.metrics.update({"precision_at_{}".format(k): res["precision"], "recall_at_{}".format(k): res["recall"],
                                  "f1_at_{}".format(k): res["f1"]})
-        table = "\n".join("{}@{}: {:.6f}".format(m, k, self.metrics["{}_at_{}".format(m, k)])
-                          for m in ("precision", "recall", "f1") for k in METRICS_TOP_KS)
+        prefixes = ("",)
+        if self.catalog_metrics:
+            self.evaluate_catalog()
+            prefixes = ("", "catalog_")
+        table = "\n".join("{}{}@{}: {:.6f}".format(p, m, k, self.metrics["{}{}_at_{}".format(p, m, k)])
+                          for p in prefixes for m in ("precision", "recall", "f1") for k in METRICS_TOP_KS)
         self.logger.info('\n' + table)
         print('\n' + table)
+
+    def evaluate_catalog(self):
+        """P/R/F1@k of each user's top-k over the WHOLE catalog, its training items excluded, against the test ratings
+        (the same RiVal restatement as the test-pair metrics)."""
+        users, items = self.trainset.users, self.trainset.items
+        if isinstance(self.model, HybridBertGNN) and self.model.content_table is None:
+            self.model.set_content_table(self.trainset.embeddings.embeddings)
+        seen = ItemLists.from_ratings(self.trainset.ratings, len(users), len(items), device="cuda")
+        ids, vals = self.model.recommend_top_k(len(users), len(items), max(METRICS_TOP_KS), exclude=seen)
+        top = catalog_predictions(ids, vals, users, items)
+        test = pd.read_csv(self.config.dataset.test_ratings_filepath, sep='\t', header=None).to_numpy()
+        for k in METRICS_TOP_KS:
+            res = precision_recall_f1_at_k(test, top.to_numpy(), k)
+            self.metrics.update({"catalog_precision_at_{}".format(k): res["precision"],
+                                 "catalog_recall_at_{}".format(k): res["recall"], "catalog_f1_at_{}".format(k): res["f1"]})
 
     def run(self):
         try:

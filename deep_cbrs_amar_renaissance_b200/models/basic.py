@@ -98,14 +98,17 @@ class BasicGNN(Model, abc.ABC):
         return self.rs.call_sources((embeddings, _ids(u)), (embeddings, _ids(i)))
 
     # -- full-catalog scoring + per-user top-k (new capability, scope row T) ----------------
-    def recommend_top_k(self, n_users, n_items, k=10, users=None, user_block=None, fused=True, precision="fp32"):
+    def recommend_top_k(self, n_users, n_items, k=10, users=None, user_block=None, fused=True, precision="fp32",
+                        exclude=None):
         """Top-k items for every user (or `users`) over the whole catalog.
 
         Returns (item_index int32 [U,k] in [0, n_items), score float32 [U,k]); ties go to
         the lower item index, which equals "score every pair with the reference scorer,
-        stable-sort descending"."""
+        stable-sort descending".  exclude: a scoring.ItemLists (e.g. ItemLists.from_ratings of
+        the training ratings) whose items are kept out of each user's list; slots past the
+        number of eligible items hold -1 / -inf."""
         from ..scoring import catalog_top_k
-        return catalog_top_k(self, self.propagate(), n_users, n_items, k, users, user_block, fused, precision)
+        return catalog_top_k(self, self.propagate(), n_users, n_items, k, users, user_block, fused, precision, exclude)
 
 
 class BasicTSGNN(BasicGNN):

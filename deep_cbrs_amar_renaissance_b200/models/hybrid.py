@@ -158,9 +158,10 @@ class HybridBertGNN(Model, abc.ABC):
         return self.rs.call_sources((embeddings, _ids(ug)), (embeddings, _ids(ig)), (_rows(ub), None),
                                     (_rows(ib), None))
 
-    def recommend_top_k(self, n_users, n_items, k=10, users=None, user_block=None, fused=True, precision="fp32"):
+    def recommend_top_k(self, n_users, n_items, k=10, users=None, user_block=None, fused=True, precision="fp32",
+                        exclude=None):
         from ..scoring import catalog_top_k
-        return catalog_top_k(self, self.propagate(), n_users, n_items, k, users, user_block, fused, precision)
+        return catalog_top_k(self, self.propagate(), n_users, n_items, k, users, user_block, fused, precision, exclude)
 
 
 def BasicGNNFactory(name, Parent, GNN):

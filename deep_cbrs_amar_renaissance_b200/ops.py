@@ -608,6 +608,33 @@ def topk_rows(scores, k):
     return ids, vals
 
 
+def _exclusion(exclude, n_rows):
+    """(rowptr, items) pointers of per-row exclusion lists (include/cbrs_b200.h, above cbrs_score_catalog_topk_ex), or
+    (None, None).  rowptr: CUDA int64 with at least n_rows + 1 entries (row r = the r-th scored row); items: CUDA int32."""
+    if exclude is None:
+        return None, None
+    rowptr, items = exclude
+    if rowptr.dim() != 1 or rowptr.numel() < n_rows + 1 or (rowptr.numel() > 1 and rowptr.stride(0) != 1):
+        raise L.CbrsError("exclusion rowptr must be a contiguous 1-D tensor of at least n_rows + 1 = {} entries".format(n_rows + 1))
+    if items.dim() != 1 or (items.numel() > 1 and items.stride(0) != 1):
+        raise L.CbrsError("exclusion items must be a contiguous 1-D tensor")
+    if items.numel() == 0:   # an empty tensor has no address; every row is empty, so any valid pointer will do
+        items = torch.zeros(1, dtype=torch.int32, device=rowptr.device)
+    return _ptr(rowptr, torch.int64), _ptr(items, torch.int32)
+
+
+def exclude_cols(scores, col_base, exclude):
+    """Overwrite with -inf, in place, the listed items of each row of the score block scores [n_rows, n_cols] whose
+    columns are catalog items col_base .. col_base + n_cols - 1 (cbrs_exclude_cols).  exclude = (rowptr, items)."""
+    lib = L.load()
+    scores, ld = _rowmajor(scores)
+    n_rows, n_cols = scores.shape
+    rp, it = _exclusion(exclude, n_rows)
+    L.check(lib.cbrs_exclude_cols(_ptr(scores), ld, n_rows, n_cols, col_base, rp, it, _stream()), "cbrs_exclude_cols")
+    _count(1)
+    return scores
+
+
 def topk_pairs(users, scores, n_users, k):
     """Rows of the pair list kept by the reference's per-user head(k), in (user asc, score desc) order."""
     lib = L.load()
@@ -620,12 +647,14 @@ def topk_pairs(users, scores, n_users, k):
     return order[rank < k].to(torch.int64)
 
 
-def score_catalog_topk(P, Q, w2, b2, w3, b3, k, precision="fp32"):
+def score_catalog_topk(P, Q, w2, b2, w3, b3, k, precision="fp32", exclude=None):
     """Fused BasicRS catalog scorer: P [U,c1] (bias folded in), Q [I,c1] -> (ids int32 [U,k], scores [U,k]).
     precision 'fp32' = fp32-accurate (1e-5 parity): the 3xTF32 tensor-core kernel for the shapes it takes (c1 in {32, 64},
     c2 <= 64: the reference's grids), the FFMA kernel otherwise; 'fp32-ffma' forces the FFMA kernel (CBRS_SCORE_FP32=ffma
-    does the same for a whole process); 'bf16' = bf16 operands on the tensor cores."""
+    does the same for a whole process); 'bf16' = bf16 operands on the tensor cores.
+    exclude = (rowptr, items): per-row lists of catalog items kept out of row r's top-k (row r = row r of P)."""
     lib = L.load()
+    rp, it = _exclusion(exclude, P.shape[0])
     if precision == "fp32" and os.environ.get("CBRS_SCORE_FP32", "") != "ffma" and \
             lib.cbrs_score_catalog_topk_tf32x3_eligible(P.shape[1], w2.shape[1]):
         P, ldp = _rowmajor(P)
@@ -635,10 +664,10 @@ def score_catalog_topk(P, Q, w2, b2, w3, b3, k, precision="fp32"):
         ids = torch.empty(n_users, k, dtype=torch.int32, device=P.device)
         vals = torch.empty(n_users, k, dtype=torch.float32, device=P.device)
         ws = _ws(lib.cbrs_score_catalog_topk_tf32x3_workspace_bytes(c1, c2), P.device)
-        L.check(lib.cbrs_score_catalog_topk_tf32x3(_ptr(P), ldp, _ptr(Q), ldq, n_users, Q.shape[0], c1,
-                                                   _ptr(w2, torch.float32), _ptr(b2, torch.float32), c2,
-                                                   _ptr(w3, torch.float32), _ptr(b3, torch.float32), k, _ptr(ids),
-                                                   _ptr(vals), _ptr(ws), ws.numel(), _stream()),
+        L.check(lib.cbrs_score_catalog_topk_tf32x3_ex(_ptr(P), ldp, _ptr(Q), ldq, n_users, Q.shape[0], c1,
+                                                      _ptr(w2, torch.float32), _ptr(b2, torch.float32), c2,
+                                                      _ptr(w3, torch.float32), _ptr(b3, torch.float32), k, _ptr(ids),
+                                                      _ptr(vals), rp, it, _ptr(ws), ws.numel(), _stream()),
                 "cbrs_score_catalog_topk_tf32x3")
         _count(2)
         return ids, vals
@@ -652,10 +681,10 @@ def score_catalog_topk(P, Q, w2, b2, w3, b3, k, precision="fp32"):
         ids = torch.empty(n_users, k, dtype=torch.int32, device=P.device)
         vals = torch.empty(n_users, k, dtype=torch.float32, device=P.device)
         ws = _ws(lib.cbrs_score_catalog_topk_bf16_workspace_bytes(Q.shape[0], c1, c2), P.device)
-        L.check(lib.cbrs_score_catalog_topk_bf16(_ptr(P), ldp, _ptr(Q), ldq, n_users, Q.shape[0], c1,
-                                                 _ptr(w2, torch.float32), _ptr(b2, torch.float32), c2,
-                                                 _ptr(w3, torch.float32), _ptr(b3, torch.float32), k, _ptr(ids),
-                                                 _ptr(vals), _ptr(ws), ws.numel(), _stream()),
+        L.check(lib.cbrs_score_catalog_topk_bf16_ex(_ptr(P), ldp, _ptr(Q), ldq, n_users, Q.shape[0], c1,
+                                                    _ptr(w2, torch.float32), _ptr(b2, torch.float32), c2,
+                                                    _ptr(w3, torch.float32), _ptr(b3, torch.float32), k, _ptr(ids),
+                                                    _ptr(vals), rp, it, _ptr(ws), ws.numel(), _stream()),
                 "cbrs_score_catalog_topk_bf16")
         _count(4 if (c1 <= 64 and c2 <= 64) else (3 if c1 <= 64 and c2 <= 128 else 2))
         return ids, vals
@@ -666,29 +695,31 @@ def score_catalog_topk(P, Q, w2, b2, w3, b3, k, precision="fp32"):
     c2 = w2.shape[1]
     ids = torch.empty(n_users, k, dtype=torch.int32, device=P.device)
     vals = torch.empty(n_users, k, dtype=torch.float32, device=P.device)
-    L.check(lib.cbrs_score_catalog_topk(_ptr(P), ldp, _ptr(Q), ldq, n_users, n_items, c1, _ptr(w2, torch.float32),
-                                        _ptr(b2, torch.float32), c2, _ptr(w3, torch.float32), _ptr(b3, torch.float32),
-                                        k, _ptr(ids), _ptr(vals), _stream()), "cbrs_score_catalog_topk")
+    L.check(lib.cbrs_score_catalog_topk_ex(_ptr(P), ldp, _ptr(Q), ldq, n_users, n_items, c1, _ptr(w2, torch.float32),
+                                           _ptr(b2, torch.float32), c2, _ptr(w3, torch.float32), _ptr(b3, torch.float32),
+                                           k, _ptr(ids), _ptr(vals), rp, it, _stream()), "cbrs_score_catalog_topk")
     _count(1)
     return ids, vals
 
 
 # ------------------------------------------------------------------ misc
-def score_hybrid_topk_bf16(P1, Q1, P2, Q2, w3a2, b3a2, w3b2, b3b2, wc1, bc1, wc2, bc2, wc3, bc3, k):
+def score_hybrid_topk_bf16(P1, Q1, P2, Q2, w3a2, b3a2, w3b2, b3b2, wc1, bc1, wc2, bc2, wc3, bc3, k, exclude=None):
     """Feature-based hybrid scorer over the whole catalog + per-user top-k, chained tcgen05 kernel
-    (cbrs_score_hybrid_topk_bf16).  Returns (item index int32 [U, k], score float32 [U, k])."""
+    (cbrs_score_hybrid_topk_bf16).  Returns (item index int32 [U, k], score float32 [U, k]).
+    exclude = (rowptr, items) as in score_catalog_topk."""
     lib = L.load()
     ts = [t.contiguous() for t in (P1, Q1, P2, Q2, w3a2, b3a2, w3b2, b3b2, wc1, bc1, wc2, bc2, wc3, bc3)]
     n_users, c = ts[0].shape
+    rp, it = _exclusion(exclude, n_users)
     n_items = ts[1].shape[0]
     dev = ts[0].device
     ids = torch.empty(n_users, k, dtype=torch.int32, device=dev)
     vals = torch.empty(n_users, k, dtype=torch.float32, device=dev)
     ws = _ws(lib.cbrs_score_hybrid_topk_bf16_workspace_bytes(), dev)
-    L.check(lib.cbrs_score_hybrid_topk_bf16(_ptr(ts[0], torch.float32), _ptr(ts[1], torch.float32), _ptr(ts[2], torch.float32),
-                                            _ptr(ts[3], torch.float32), n_users, n_items, c,
-                                            *[_ptr(t, torch.float32) for t in ts[4:]], k, _ptr(ids), _ptr(vals), _ptr(ws),
-                                            ws.numel(), _stream()), "cbrs_score_hybrid_topk_bf16")
+    L.check(lib.cbrs_score_hybrid_topk_bf16_ex(_ptr(ts[0], torch.float32), _ptr(ts[1], torch.float32),
+                                               _ptr(ts[2], torch.float32), _ptr(ts[3], torch.float32), n_users, n_items, c,
+                                               *[_ptr(t, torch.float32) for t in ts[4:]], k, _ptr(ids), _ptr(vals), rp, it,
+                                               _ptr(ws), ws.numel(), _stream()), "cbrs_score_hybrid_topk_bf16")
     _count(2)
     return ids, vals
 

@@ -7,12 +7,85 @@ src/models/hybrid.py:74-77) is hoisted and computed once per user / item; the pa
 part runs over blocks of users x all items, the tower rows being gathered inside the
 first pairwise Dense kernel, and each block's [UB, I] scores go through cbrs_topk_rows.
 Users are independent => sharded across ranks with no collective (SURVEY 8e).
+
+Every path takes per-user exclusion lists (ItemLists, typically the items a user rated in training): they are kept out
+of that user's top-k, inside the fused kernels or on the generic path's score blocks (cbrs_exclude_cols).
 """
+import numpy as np
 import torch
 
 from . import ops
 
 _PAIR_BUDGET = 1 << 18  # pairs per block: keeps a block's 64-wide activations L2-resident
+
+
+class ItemLists:
+    """Per-user lists of catalog items, CSR over GLOBAL user ids: user u's items are items[rowptr[u]:rowptr[u + 1]],
+    sorted ascending, as catalog indices in [0, n_items) (item node id - n_users).  Passed as `exclude=` to
+    catalog_top_k / recommend_top_k, which keep those items out of the user's top-k."""
+
+    def __init__(self, rowptr, items, n_items):
+        if not (torch.is_tensor(rowptr) and rowptr.dim() == 1 and rowptr.dtype == torch.int64 and rowptr.numel() >= 1):
+            raise ValueError("ItemLists: rowptr must be a 1-D int64 tensor of n_users + 1 offsets")
+        if not (torch.is_tensor(items) and items.dim() == 1 and items.dtype == torch.int32):
+            raise ValueError("ItemLists: items must be a 1-D int32 tensor")
+        if int(rowptr[0]) != 0 or int(rowptr[-1]) != items.numel():
+            raise ValueError("ItemLists: rowptr must run from 0 to len(items) = {}, got {} .. {}".format(
+                items.numel(), int(rowptr[0]), int(rowptr[-1])))
+        self.rowptr, self.items, self.n_items = rowptr.contiguous(), items.contiguous(), int(n_items)
+
+    @property
+    def n_users(self):
+        return self.rowptr.numel() - 1
+
+    @classmethod
+    def from_ratings(cls, ratings, n_users, n_items, device=None):
+        """Seen items per user from the [R, >= 2] ratings format of a training set (`trainset.ratings`): column 0 the
+        user index, column 1 the item index offset by n_users.  Every row counts, whatever its rating: a rated item is
+        a seen item; a pair rated twice is listed twice.  Built on `device` (default: the tensor's own device, or CUDA
+        for a numpy array when one is present)."""
+        r = ratings if torch.is_tensor(ratings) else torch.as_tensor(np.asarray(ratings)[:, :2].astype(np.int64))
+        if device is None:
+            device = r.device if torch.is_tensor(ratings) else ("cuda" if torch.cuda.is_available() else "cpu")
+        if r.dim() != 2 or r.shape[1] < 2:
+            raise ValueError("ItemLists.from_ratings: expected a [R, >= 2] ratings array")
+        r = r[:, :2].to(device=device, dtype=torch.int64)
+        user, item = r[:, 0], r[:, 1] - n_users
+        if r.shape[0] and (bool((user < 0).any()) or bool((user >= n_users).any()) or bool((item < 0).any())
+                           or bool((item >= n_items).any())):
+            raise ValueError("ItemLists.from_ratings: user ids must lie in [0, {}) and item ids in [{}, {})".format(
+                n_users, n_users, n_users + n_items))
+        key = torch.sort(user * n_items + item).values
+        counts = torch.bincount(key // n_items, minlength=n_users)
+        rowptr = torch.zeros(n_users + 1, dtype=torch.int64, device=device)
+        torch.cumsum(counts, 0, out=rowptr[1:])
+        return cls(rowptr, (key % n_items).to(torch.int32), n_items)
+
+
+def _exclusion_rows(exclude, n_users, n_items, users, all_users):
+    """(rowptr, items) whose row r is the list of the r-th scored user, or None.  The whole user range uses the lists
+    as they are, a contiguous range a view of rowptr (offsets are absolute), any other subset gathers its sub-lists."""
+    if exclude is None:
+        return None
+    if not isinstance(exclude, ItemLists):
+        raise TypeError("exclude must be an ItemLists")
+    if exclude.n_users != n_users or exclude.n_items != n_items:
+        raise ValueError("exclude holds lists for {} users x {} items, the catalog is {} x {}".format(
+            exclude.n_users, exclude.n_items, n_users, n_items))
+    rowptr, items = exclude.rowptr.to(users.device), exclude.items.to(users.device)
+    n = users.numel()
+    if all_users or n == 0:
+        return rowptr, items
+    if bool((users < 0).any()) or bool((users >= n_users).any()):
+        raise ValueError("users must lie in [0, {})".format(n_users))
+    u0 = int(users[0])
+    if bool(torch.equal(users, torch.arange(u0, u0 + n, device=users.device))):
+        return rowptr[u0:u0 + n + 1], items
+    begin, counts = rowptr[users], rowptr[users + 1] - rowptr[users]
+    sub = torch.zeros(n + 1, dtype=torch.int64, device=users.device)
+    torch.cumsum(counts, 0, out=sub[1:])
+    pos = torch.arange(int(sub[-1]), device=users.device) - torch.repeat_interleave(sub[:-1] - begin, counts)
+    return sub, items[pos]
 
 
 def _blocks(n_users, n_items, user_block=None, budget=_PAIR_BUDGET):
@@ -99,7 +172,7 @@ def _hoisted_sources(model, emb, users, items):
     return (x1, None), (x2, None), rs.clf
 
 
-def _fused_basic(model, emb, users, items, k, precision="fp32"):
+def _fused_basic(model, emb, users, items, k, precision="fp32", exclude=None):
     """Scorers of the form clf([f(user) || g(item)]) with two hidden classifier layers -> the fused kernel
     (cbrs_score_catalog_topk: hoisted first layer, second layer, output, sigmoid and running top-k in one pass)."""
     clf = model.rs.clf
@@ -120,10 +193,10 @@ def _fused_basic(model, emb, users, items, k, precision="fp32"):
     l3.build_for(l2.units)
     P = ops.dense(u_src[0], l1.kernel[:du], l1.bias, None, idx1=u_src[1])   # bias folded into the user half
     Q = ops.dense(i_src[0], l1.kernel[du:], None, None, idx1=i_src[1])
-    return ops.score_catalog_topk(P, Q, l2.kernel, l2.bias, l3.kernel.reshape(-1), l3.bias, k, precision)
+    return ops.score_catalog_topk(P, Q, l2.kernel, l2.bias, l3.kernel.reshape(-1), l3.bias, k, precision, exclude)
 
 
-def _fused_hybrid_feature(model, emb, users, items, k):
+def _fused_hybrid_feature(model, emb, users, items, k, exclude=None):
     """Feature-based HybridCBRS with the shapes of every hybrid grid of the reference (dense3a / dense3b = two 64-wide
     layers, classifier 64 -> 64 -> 1, relu, plain concatenation) -> the chained tensor-core kernel
     (cbrs_score_hybrid_topk_bf16).  None when the scorer has another shape."""
@@ -152,17 +225,22 @@ def _fused_hybrid_feature(model, emb, users, items, k):
     Q2 = ops.dense(ib, d3b[0].kernel[c:], None, None)
     return ops.score_hybrid_topk_bf16(P1, Q1, P2, Q2, d3a[1].kernel, d3a[1].bias, d3b[1].kernel, d3b[1].bias,
                                       clf[0].kernel, clf[0].bias, clf[1].kernel, clf[1].bias, clf[2].kernel.reshape(-1),
-                                      clf[2].bias, k)
+                                      clf[2].bias, k, exclude)
 
 
-def catalog_top_k(model, emb, n_users, n_items, k=10, users=None, user_block=None, fused=True, precision="fp32"):
+def catalog_top_k(model, emb, n_users, n_items, k=10, users=None, user_block=None, fused=True, precision="fp32",
+                  exclude=None):
+    """exclude: an ItemLists over all n_users; each user's listed items are kept out of its top-k (slots past the number
+    of eligible items hold -1 / -inf)."""
     dev = emb.device
+    all_users = users is None
     users = torch.arange(n_users, device=dev, dtype=torch.int64) if users is None else users.to(dev, torch.int64)
     items = torch.arange(n_users, n_users + n_items, device=dev, dtype=torch.int64)
+    excl = _exclusion_rows(exclude, n_users, n_items, users, all_users)
     if fused:
-        out = _fused_basic(model, emb, users, items, k, precision)
+        out = _fused_basic(model, emb, users, items, k, precision, excl)
         if out is None and precision == "bf16":
-            out = _fused_hybrid_feature(model, emb, users, items, k)
+            out = _fused_hybrid_feature(model, emb, users, items, k, excl)
         if out is not None:
             return out
     score = _pair_scorer(model, emb, users, items)
@@ -177,6 +255,8 @@ def catalog_top_k(model, emb, n_users, n_items, k=10, users=None, user_block=Non
             ni = min(ib, n_items - i0)
             pu, pi = _block_indices(cache, nb, ni, dev)
             s = score(pu + u0, pi + i0).reshape(nb, ni)
+            if excl is not None:   # scores are sigmoid outputs: -inf marks an excluded item and nothing else
+                ops.exclude_cols(s, i0, (excl[0][u0:], excl[1]))
             bi, bv = ops.topk_rows(s, min(k, ni))
             bi = bi + i0
             if best_i is None:
@@ -189,5 +269,7 @@ def catalog_top_k(model, emb, n_users, n_items, k=10, users=None, user_block=Non
             cand_i = torch.cat([best_i, bi], dim=1)
             sel, best_v = ops.topk_rows(cand_v, min(k, cand_v.shape[1]))
             best_i = torch.gather(cand_i, 1, sel.long())
+        if excl is not None:
+            best_i = torch.where(torch.isneginf(best_v), torch.full_like(best_i, -1), best_i)
         ids[u0:u0 + nb, :best_i.shape[1]], vals[u0:u0 + nb, :best_v.shape[1]] = best_i, best_v
     return ids, vals

@@ -35,6 +35,20 @@ def top_k_predictions(predictions, users, items, k=5):
     return df
 
 
+def catalog_predictions(ids, vals, users, items):
+    """Full-catalog top-k (recommend_top_k's ids / scores [U, k]) as the DataFrame(users, items, scores) frame
+    top_k_predictions returns: ORIGINAL ids (row r is users[r], catalog index i is items[i]), rows in input order,
+    each row's items by score descending.  Slots holding -1 (fewer eligible items than k) are dropped."""
+    ids = ids.cpu().numpy() if torch.is_tensor(ids) else np.asarray(ids)
+    vals = vals.cpu().numpy() if torch.is_tensor(vals) else np.asarray(vals)
+    rows, cols = np.nonzero(ids >= 0)
+    df = pd.DataFrame()
+    df['users'] = np.asarray(users)[rows]
+    df['items'] = np.asarray(items)[ids[rows, cols].astype(np.int64)]
+    df['scores'] = vals[rows, cols]
+    return df
+
+
 def precision_recall_f1_at_k(test_ratings, predictions, k, relevance_threshold=1):
     """Precision@k, Recall@k and F1@k in the sense of RiVal 0.2 (the library inside mimir.jar):
 

@@ -219,6 +219,13 @@ int cbrs_score_hybrid_topk_bf16(const float *P1, const float *Q1, const float *P
                                 const float *b3b2, const float *wc1, const float *bc1, const float *wc2,
                                 const float *bc2, const float *wc3, const float *bc3, int32_t k, int32_t *ids_out,
                                 float *scores_out, void *workspace, size_t workspace_bytes, void *stream);
+/* With per-user exclusion lists (contract above cbrs_score_catalog_topk_ex).  Null lists: cbrs_score_hybrid_topk_bf16. */
+int cbrs_score_hybrid_topk_bf16_ex(const float *P1, const float *Q1, const float *P2, const float *Q2, int64_t n_users,
+                                   int32_t n_items, int32_t c, const float *w3a2, const float *b3a2, const float *w3b2,
+                                   const float *b3b2, const float *wc1, const float *bc1, const float *wc2,
+                                   const float *bc2, const float *wc3, const float *bc3, int32_t k, int32_t *ids_out,
+                                   float *scores_out, const int64_t *excl_rowptr, const int32_t *excl_items,
+                                   void *workspace, size_t workspace_bytes, void *stream);
 
 /* Grouped transform of the relational layer (row R: "R-GCN per-relation transform plus scatter as a grouped kernel"):
  * ONE launch computes X[m, f] . [W_0 | ... | W_{R-1}] (w_cat: contiguous [f, n_groups*h], Keras layout) and stores
@@ -290,6 +297,11 @@ int cbrs_gather_rows(const float *x, int64_t ldx, const int64_t *idx, int64_t m,
  * reference scorer's output).  k <= 128.                                        */
 int cbrs_topk_rows(const float *scores, int64_t ld, int64_t n_users, int32_t n_items, int32_t k,
                    int32_t *ids_out, float *vals_out, void *stream);
+/* Exclusion lists on a materialised score block (the generic catalog path): scores [n_rows, n_cols] (leading
+ * dimension ld) holds catalog columns col_base .. col_base + n_cols - 1; every listed item of row r (contract above
+ * cbrs_score_catalog_topk_ex) that falls in that range is overwritten with -inf.  Both lists null: nothing to do. */
+int cbrs_exclude_cols(float *scores, int64_t ld, int64_t n_rows, int32_t n_cols, int32_t col_base,
+                      const int64_t *excl_rowptr, const int32_t *excl_items, void *stream);
 /* Pair-list form (src/utilities/metrics.py:21-34): stable sort by (user asc,
  * score desc), first k rows per user.  order_out [n_pairs] = input row of each
  * sorted position; rank_out [n_pairs] = position inside its user's run (keep rows
@@ -312,6 +324,23 @@ int cbrs_score_catalog_topk(const float *P, int64_t ldp, const float *Q, int64_t
                             const float *w3, const float *b3, int32_t k, int32_t *ids_out,
                             float *scores_out, void *stream);
 
+/* ---- exclusion lists of the catalog scorers (the *_ex entry points and cbrs_exclude_cols) ----
+ * Per scored user, catalog items that must not appear in its top-k (typically the items it rated in training).
+ *   excl_rowptr int64 [n_users + 1]: absolute offsets into excl_items; row r's list is
+ *   excl_items[excl_rowptr[r] .. excl_rowptr[r + 1]) (int32).  Row r is the r-th SCORED user (row r of P / of the
+ *   score block), not a global user id: for the contiguous users u0.. pass excl_rowptr + u0, no copy needed.
+ *   Items are catalog indices in [0, n_items) (item node id - n_users), the space ids_out uses; other values never match.
+ *   Each list is sorted ascending; duplicates and empty rows are allowed.  An UNSORTED row may exclude any subset of its
+ *   own items, and never causes a read outside [excl_rowptr[r], excl_rowptr[r + 1]).
+ * Output form is unchanged (score desc, ties to the lower item index); slots past the number of eligible items hold
+ * -1 / -inf.  Both pointers null: no lists, the same kernel bit for bit as the entry point without _ex; empty lists give
+ * the same bits as no lists.  Exactly one of the two null: CBRS_E_INVALID.  Workspace sizes do not change.  The fused
+ * kernels search a user's list only for a candidate that beats its current k-th score.                              */
+int cbrs_score_catalog_topk_ex(const float *P, int64_t ldp, const float *Q, int64_t ldq, int64_t n_users,
+                               int32_t n_items, int32_t c1, const float *w2, const float *b2, int32_t c2,
+                               const float *w3, const float *b3, int32_t k, int32_t *ids_out, float *scores_out,
+                               const int64_t *excl_rowptr, const int32_t *excl_items, void *stream);
+
 /* The same scorer with the 64 x 64 product on the tensor cores at fp32 accuracy (3xTF32: h = relu(P[u]+Q[i]) and W2 are
  * split into a tf32 part and an exact remainder, three kind::tf32 MMAs per K step accumulate in fp32; the A operand is
  * written by its threads straight into tensor memory).  Same contract, outputs and tie rule as cbrs_score_catalog_topk;
@@ -323,6 +352,11 @@ int cbrs_score_catalog_topk_tf32x3(const float *P, int64_t ldp, const float *Q, 
                                    int32_t n_items, int32_t c1, const float *w2, const float *b2, int32_t c2,
                                    const float *w3, const float *b3, int32_t k, int32_t *ids_out,
                                    float *scores_out, void *workspace, size_t workspace_bytes, void *stream);
+int cbrs_score_catalog_topk_tf32x3_ex(const float *P, int64_t ldp, const float *Q, int64_t ldq, int64_t n_users,
+                                      int32_t n_items, int32_t c1, const float *w2, const float *b2, int32_t c2,
+                                      const float *w3, const float *b3, int32_t k, int32_t *ids_out, float *scores_out,
+                                      const int64_t *excl_rowptr, const int32_t *excl_items, void *workspace,
+                                      size_t workspace_bytes, void *stream);
 
 /* bf16 tensor-core variant (tcgen05.mma, TMEM accumulator): same contract and arguments; the
  * per-pair activations relu(P[u]+Q[i]) and W2 are rounded to bf16, accumulation is fp32, so
@@ -338,6 +372,11 @@ int cbrs_score_catalog_topk_bf16(const float *P, int64_t ldp, const float *Q, in
                                  int32_t n_items, int32_t c1, const float *w2, const float *b2, int32_t c2,
                                  const float *w3, const float *b3, int32_t k, int32_t *ids_out,
                                  float *scores_out, void *workspace, size_t workspace_bytes, void *stream);
+int cbrs_score_catalog_topk_bf16_ex(const float *P, int64_t ldp, const float *Q, int64_t ldq, int64_t n_users,
+                                    int32_t n_items, int32_t c1, const float *w2, const float *b2, int32_t c2,
+                                    const float *w3, const float *b3, int32_t k, int32_t *ids_out, float *scores_out,
+                                    const int64_t *excl_rowptr, const int32_t *excl_items, void *workspace,
+                                    size_t workspace_bytes, void *stream);
 
 /* ---- synthetic scaled graph (SURVEY 8d, config 5) --------------------------------
  * Counter-based generator: edge e connects user hash_u(seed,e) % n_users with an
