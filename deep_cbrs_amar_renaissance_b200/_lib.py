@@ -62,6 +62,9 @@ _SIGS = {
                                             c_size_t, P]),
     "cbrs_score_hybrid_topk_bf16_ex": (c_int, [P, P, P, P, c_int64, c_int32, c_int32, P, P, P, P, P, P, P, P, P, P, c_int32, P, P,
                                                P, P, P, c_size_t, P]),
+    "cbrs_score_hybrid_topk_tf32x3_workspace_bytes": (c_size_t, []),
+    "cbrs_score_hybrid_topk_tf32x3": (c_int, [P, P, P, P, c_int64, c_int32, c_int32, P, P, P, P, P, P, P, P, P, P, c_int32, P, P,
+                                              P, P, P, c_size_t, P]),
     "cbrs_dense_grouped": (c_int, [P, c_int64, P, c_int64, c_int32, c_int32, c_int32, P, c_int64, c_int64, c_int,
                                    POINTER(c_void_p), c_int, P]),
     "cbrs_dense_tf32x3_eligible": (c_int, [c_int32, c_int32]),

@@ -95,4 +95,43 @@ __device__ __forceinline__ bool excluded_item(const int64_t *__restrict__ rowptr
     return lo < end && __ldg(items + lo) == item;
 }
 
+// Candidate lists of the tensor-core catalog scorers (score_tf32.cu, score_hybrid_tf32.cu): 64-bit keys
+// (orderable(logit) << 32) | ~item, so that a larger key is a higher score, ties going to the lower item id.
+__device__ __forceinline__ uint32_t orderable_f32(float f) {
+    const uint32_t u = __float_as_uint(f);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float from_orderable_f32(uint32_t o) {
+    return __uint_as_float((o & 0x80000000u) ? (o & 0x7fffffffu) : ~o);
+}
+// one warp: keep the best min(k, n) keys of c[0..n) in c[0..), descending; *thr becomes the k-th key once k are held
+static __device__ void topk_compact(unsigned long long *c, int *cnt, unsigned long long *thr, int k, int lane) {
+    const int n = *cnt;
+    const int keep = n < k ? n : k;
+    for (int r = 0; r < keep; ++r) {
+        unsigned long long best = 0ull;
+        int bi = -1;
+        for (int i = r + lane; i < n; i += 32) {
+            const unsigned long long v = c[i];
+            if (v > best) { best = v; bi = i; }
+        }
+        unsigned long long m = best;
+#pragma unroll
+        for (int o = 16; o; o >>= 1) {
+            const unsigned long long t = __shfl_xor_sync(0xffffffffu, m, o);
+            m = t > m ? t : m;
+        }
+        if (best == m && bi >= 0) {
+            c[bi] = c[r];
+            c[r] = m;
+        }
+        __syncwarp();
+    }
+    if (lane == 0) {
+        *cnt = keep;
+        *thr = (keep == k) ? c[k - 1] : 0ull;
+    }
+    __syncwarp();
+}
+
 }  // namespace cbrs

@@ -44,87 +44,10 @@ struct ScoreT3Params {
 constexpr int kS3TU = 16;   // users per CTA (4 passes of 4 users per item tile)
 constexpr int kS3TI = 32;   // items per tile
 
-__device__ __forceinline__ uint32_t s3_orderable(float f) {
-    const uint32_t u = __float_as_uint(f);
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float s3_from_orderable(uint32_t o) {
-    return __uint_as_float((o & 0x80000000u) ? (o & 0x7fffffffu) : ~o);
-}
-// one warp: keep the best min(k, n) keys of c[0..n) in c[0..), descending
-__device__ void s3_compact(unsigned long long *c, int *cnt, unsigned long long *thr, int k, int lane) {
-    const int n = *cnt;
-    const int keep = n < k ? n : k;
-    for (int r = 0; r < keep; ++r) {
-        unsigned long long best = 0ull;
-        int bi = -1;
-        for (int i = r + lane; i < n; i += 32) {
-            const unsigned long long v = c[i];
-            if (v > best) { best = v; bi = i; }
-        }
-        unsigned long long m = best;
-#pragma unroll
-        for (int o = 16; o; o >>= 1) {
-            const unsigned long long t = __shfl_xor_sync(0xffffffffu, m, o);
-            m = t > m ? t : m;
-        }
-        if (best == m && bi >= 0) {
-            c[bi] = c[r];
-            c[r] = m;
-        }
-        __syncwarp();
-    }
-    if (lane == 0) {
-        *cnt = keep;
-        *thr = (keep == k) ? c[k - 1] : 0ull;
-    }
-    __syncwarp();
-}
-__device__ __forceinline__ float s3_hi(float x) {   // nearest tf32, low 13 mantissa bits zero
-    uint32_t r;
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
-    return __uint_as_float(r);
-}
-// kind::tf32 instruction descriptor: D fp32, A/B tf32, both K-major, dense
-__host__ __device__ constexpr uint32_t s3_idesc(int m, int n) {
-    return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
-}
-// D[tmem] (+)= A[tmem] * B[smem]: A is read from tensor memory (lane = row, one 32-bit column per k)
-__device__ __forceinline__ void s3_mma_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n\t}" ::"r"(tmem_d),
-        "r"(tmem_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// 32 lanes x 32 columns of 32-bit: thread t of the warp writes lane (base_lane + t), columns c..c+31
-__device__ __forceinline__ void s3_tmem_st32(uint32_t taddr, const uint32_t (&v)[32]) {
-    asm volatile(
-        "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
-        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
-        "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};" ::"r"(taddr),
-        "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]), "r"(v[9]), "r"(v[10]),
-        "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15]), "r"(v[16]), "r"(v[17]), "r"(v[18]), "r"(v[19]), "r"(v[20]),
-        "r"(v[21]), "r"(v[22]), "r"(v[23]), "r"(v[24]), "r"(v[25]), "r"(v[26]), "r"(v[27]), "r"(v[28]), "r"(v[29]), "r"(v[30]),
-        "r"(v[31])
-        : "memory");
-}
 constexpr int kS3WsThreads = 416;   // warp-specialised kernel: 8 producer warps, the MMA warp, 4 epilogue warps
 __device__ __forceinline__ void s3_arrive(uint64_t *bar) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(tc::smem_u32(bar)) : "memory");
 }
-__device__ __forceinline__ void s3_tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-
-__device__ __forceinline__ void s3_tmem_st16(uint32_t taddr, const uint32_t (&v)[16]) {
-    asm volatile(
-        "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
-        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};" ::"r"(taddr),
-        "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]), "r"(v[9]), "r"(v[10]),
-        "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15])
-        : "memory");
-}
-
 // ---------------------------------------------------------------------------------------------------------------------
 // Warp-specialised.  The first versions were barrier-synchronous (produce -> __syncthreads -> issue -> mbarrier wait ->
 // epilogue, 128 or 256 threads, two CTAs per SM): 15-18 G pairs/s, and ~2,300 cycles per 128-pair step of serialised
@@ -225,7 +148,7 @@ __global__ void __launch_bounds__(kS3WsThreads, 1) score_tf32x3_ws_kernel(const 
                 const float4 pv = prow[j], qv = qreg[j];
                 const float h0 = fmaxf(pv.x + qv.x, 0.f), h1 = fmaxf(pv.y + qv.y, 0.f);
                 const float h2 = fmaxf(pv.z + qv.z, 0.f), h3 = fmaxf(pv.w + qv.w, 0.f);
-                const float g0 = s3_hi(h0), g1 = s3_hi(h1), g2 = s3_hi(h2), g3 = s3_hi(h3);
+                const float g0 = tc::tf32_hi(h0), g1 = tc::tf32_hi(h1), g2 = tc::tf32_hi(h2), g3 = tc::tf32_hi(h3);
                 hi[4 * j] = __float_as_uint(g0); hi[4 * j + 1] = __float_as_uint(g1);
                 hi[4 * j + 2] = __float_as_uint(g2); hi[4 * j + 3] = __float_as_uint(g3);
                 lo[4 * j] = __float_as_uint(h0 - g0); lo[4 * j + 1] = __float_as_uint(h1 - g1);
@@ -238,13 +161,13 @@ __global__ void __launch_bounds__(kS3WsThreads, 1) score_tf32x3_ws_kernel(const 
             }
             const uint32_t ta = trow + (uint32_t)buf * 2 * C1;
             if constexpr (E == 32) {
-                s3_tmem_st32(ta, hi);
-                s3_tmem_st32(ta + C1, lo);
+                tc::tmem_st32(ta, hi);
+                tc::tmem_st32(ta + C1, lo);
             } else {
-                s3_tmem_st16(ta, hi);
-                s3_tmem_st16(ta + C1, lo);
+                tc::tmem_st16(ta, hi);
+                tc::tmem_st16(ta + C1, lo);
             }
-            s3_tmem_st_wait();
+            tc::tmem_st_wait();
             tc::tc_fence_before_sync();
             __syncwarp();
             if (lane == 0) s3_arrive(a_full + buf);
@@ -259,7 +182,7 @@ __global__ void __launch_bounds__(kS3WsThreads, 1) score_tf32x3_ws_kernel(const 
     } else if (warp == 8) {
         // ---------------- MMA issuer: one elected lane (elect.sync: UTCHMMA issued once, no per-lane loop) ----------------
         if (tc::elect_one()) {
-            const uint32_t idesc = s3_idesc(128, NP);
+            const uint32_t idesc = tc::idesc_tf32_f32(128, NP);
             const int n_steps = n_tiles * kPasses;
             for (int step = 0; step < n_steps; ++step) {
                 const int buf = step & 1;
@@ -273,9 +196,9 @@ __global__ void __launch_bounds__(kS3WsThreads, 1) score_tf32x3_ws_kernel(const 
                     const uint32_t boff = (uint32_t)(ks >> 2) * NP * 128 + (uint32_t)(ks & 3) * 32;
                     const uint64_t dbh = tc::smem_desc_sw128(wh_addr + boff), dbl = tc::smem_desc_sw128(wl_addr + boff);
                     const uint32_t ahi = a + (uint32_t)ks * 8, alo = a + C1 + (uint32_t)ks * 8;
-                    s3_mma_ts(d, alo, dbh, idesc, ks > 0 ? 1u : 0u);
-                    s3_mma_ts(d, ahi, dbl, idesc, 1u);
-                    s3_mma_ts(d, ahi, dbh, idesc, 1u);
+                    tc::mma_tf32_ts(d, alo, dbh, idesc, ks > 0 ? 1u : 0u);
+                    tc::mma_tf32_ts(d, ahi, dbl, idesc, 1u);
+                    tc::mma_tf32_ts(d, ahi, dbh, idesc, 1u);
                 }
                 tc::mma_commit(a_empty + buf);   // the operand buffer may be rewritten once these MMAs have read it
                 tc::mma_commit(d_full + buf);    // ... and the accumulator is complete
@@ -293,7 +216,7 @@ __global__ void __launch_bounds__(kS3WsThreads, 1) score_tf32x3_ws_kernel(const 
         for (int tile = 0; tile < n_tiles; ++tile) {
             // a user's list must have room for the 32 candidates one item tile can add
             for (int ul = quad; ul < kS3TU; ul += 4)   // user ul is only ever touched by warp 9 + ul % 4
-                if (cnt[ul] > cap - kS3TI) s3_compact(cand + ul * cap, cnt + ul, thr + ul, p.k, lane);
+                if (cnt[ul] > cap - kS3TI) topk_compact(cand + ul * cap, cnt + ul, thr + ul, p.k, lane);
 #pragma unroll 1
             for (int pass = 0; pass < kPasses; ++pass, ++step) {
                 const int buf = step & 1;
@@ -320,7 +243,7 @@ __global__ void __launch_bounds__(kS3WsThreads, 1) score_tf32x3_ws_kernel(const 
                 const int64_t user = u0 + ul;
                 if (item < p.n_items && user < p.n_users) {
                     // candidates are ranked by the logit (sigmoid is monotonic); the sigmoid is applied to the k winners
-                    const unsigned long long key = ((unsigned long long)s3_orderable(logit + b3) << 32) |
+                    const unsigned long long key = ((unsigned long long)orderable_f32(logit + b3) << 32) |
                                                    (unsigned long long)(0xffffffffu - (uint32_t)item);
                     if (key > thr[ul] && !(kExcl && excluded_item(p.excl_rowptr, p.excl_items, user, item))) {
                         const int pos = atomicAdd(cnt + ul, 1);
@@ -337,7 +260,7 @@ __global__ void __launch_bounds__(kS3WsThreads, 1) score_tf32x3_ws_kernel(const 
         tc::tmem_dealloc(tmem_base, kCols);
     }
     for (int ul = warp; ul < kS3TU; ul += kThreads / 32) {
-        s3_compact(cand + ul * cap, cnt + ul, thr + ul, p.k, lane);
+        topk_compact(cand + ul * cap, cnt + ul, thr + ul, p.k, lane);
         const int64_t user = u0 + ul;
         if (user >= p.n_users) continue;
         const int n = cnt[ul];
@@ -346,7 +269,7 @@ __global__ void __launch_bounds__(kS3WsThreads, 1) score_tf32x3_ws_kernel(const 
             if (r < n) {
                 const unsigned long long key = cand[ul * cap + r];
                 p.ids_out[o] = (int32_t)(0xffffffffu - (uint32_t)(key & 0xffffffffull));
-                p.scores_out[o] = 1.f / (1.f + expf(-s3_from_orderable((uint32_t)(key >> 32))));
+                p.scores_out[o] = 1.f / (1.f + expf(-from_orderable_f32((uint32_t)(key >> 32))));
             } else {
                 p.ids_out[o] = -1;
                 p.scores_out[o] = -INFINITY;

@@ -111,6 +111,48 @@ __device__ __forceinline__ void mma_commit(uint64_t *bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 
+// ---- 3xTF32 with the A operand in tensor memory (score_tf32.cu, score_hybrid_tf32.cu) ------------------------------
+// nearest tf32 of x (low 13 mantissa bits zero); x - tf32_hi(x) is exact and is the "lo" part of the split
+__device__ __forceinline__ float tf32_hi(float x) {
+    uint32_t r;
+    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
+    return __uint_as_float(r);
+}
+// kind::tf32 instruction descriptor: D fp32, A/B tf32, both K-major, dense
+__host__ __device__ constexpr uint32_t idesc_tf32_f32(int m, int n) {
+    return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
+}
+// D[tmem] (+)= A[tmem] * B[smem]: A is read from tensor memory (lane = row, one 32-bit column per k)
+__device__ __forceinline__ void mma_tf32_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n\t}" ::"r"(tmem_d),
+        "r"(tmem_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+        : "memory");
+}
+// 32 lanes x 32 / 16 columns of 32-bit: thread t of the warp writes lane (base_lane + t), columns c..c+31 / c..c+15
+__device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t (&v)[32]) {
+    asm volatile(
+        "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
+        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
+        "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};" ::"r"(taddr),
+        "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]), "r"(v[9]), "r"(v[10]),
+        "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15]), "r"(v[16]), "r"(v[17]), "r"(v[18]), "r"(v[19]), "r"(v[20]),
+        "r"(v[21]), "r"(v[22]), "r"(v[23]), "r"(v[24]), "r"(v[25]), "r"(v[26]), "r"(v[27]), "r"(v[28]), "r"(v[29]), "r"(v[30]),
+        "r"(v[31])
+        : "memory");
+}
+__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&v)[16]) {
+    asm volatile(
+        "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
+        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};" ::"r"(taddr),
+        "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]), "r"(v[9]), "r"(v[10]),
+        "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15])
+        : "memory");
+}
+__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+
 // byte offset of 16-byte chunk c (0..7) of row r inside a SWIZZLE_128B K-major tile
 __device__ __forceinline__ uint32_t sw128_offset(int r, int c) { return (uint32_t)(r * 128 + ((c ^ (r & 7)) << 4)); }
 

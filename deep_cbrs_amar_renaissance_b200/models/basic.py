@@ -106,7 +106,12 @@ class BasicGNN(Model, abc.ABC):
         the lower item index, which equals "score every pair with the reference scorer,
         stable-sort descending".  exclude: a scoring.ItemLists (e.g. ItemLists.from_ratings of
         the training ratings) whose items are kept out of each user's list; slots past the
-        number of eligible items hold -1 / -inf."""
+        number of eligible items hold -1 / -inf.
+
+        precision (fused=True): 'fp32' (fp32 accuracy, 1e-5) runs the 3xTF32 tensor-core kernel
+        (cbrs_score_catalog_topk_tf32x3) for classifier widths c1 in {32, 64}, c2 <= 64, and the
+        FFMA kernel otherwise; 'fp32-ffma' always the FFMA kernel; 'bf16' the bf16 tensor-core
+        kernel.  fused=False runs the generic blocked pair pipeline."""
         from ..scoring import catalog_top_k
         return catalog_top_k(self, self.propagate(), n_users, n_items, k, users, user_block, fused, precision, exclude)
 

@@ -160,6 +160,15 @@ class HybridBertGNN(Model, abc.ABC):
 
     def recommend_top_k(self, n_users, n_items, k=10, users=None, user_block=None, fused=True, precision="fp32",
                         exclude=None):
+        """Top-k items for every user (or `users`) over the whole catalog; returns, ties and `exclude` as
+        BasicGNN.recommend_top_k.  Which kernel runs:
+          * feature-based scorer with the reference grids' shapes (dense3a / dense3b two 64-wide relu layers,
+            classifier 64 -> 64 -> 1, plain concatenation, no residual, content table set, k <= 128):
+            precision 'fp32' the chained 3xTF32 tensor-core kernel (cbrs_score_hybrid_topk_tf32x3, fp32 accuracy,
+            1e-5; also needs k <= n_items), 'bf16' the chained bf16 kernel (cbrs_score_hybrid_topk_bf16);
+            'fp32-ffma' the generic pair pipeline;
+          * entity-based scorer with plain concatenation: the fused BasicRS kernels, as BasicGNN.recommend_top_k;
+          * any other shape, and fused=False: the generic blocked pair pipeline (HybridCBRS.tail over item blocks)."""
         from ..scoring import catalog_top_k
         return catalog_top_k(self, self.propagate(), n_users, n_items, k, users, user_block, fused, precision, exclude)
 

@@ -724,6 +724,26 @@ def score_hybrid_topk_bf16(P1, Q1, P2, Q2, w3a2, b3a2, w3b2, b3b2, wc1, bc1, wc2
     return ids, vals
 
 
+def score_hybrid_topk_tf32x3(P1, Q1, P2, Q2, w3a2, b3a2, w3b2, b3b2, wc1, bc1, wc2, bc2, wc3, bc3, k, exclude=None):
+    """The scorer of score_hybrid_topk_bf16 at fp32 accuracy (1e-5): the five 64 x 64 products as 3xTF32 on the tensor
+    cores (cbrs_score_hybrid_topk_tf32x3).  Same arguments and return value as score_hybrid_topk_bf16."""
+    lib = L.load()
+    ts = [t.contiguous() for t in (P1, Q1, P2, Q2, w3a2, b3a2, w3b2, b3b2, wc1, bc1, wc2, bc2, wc3, bc3)]
+    n_users, c = ts[0].shape
+    rp, it = _exclusion(exclude, n_users)
+    n_items = ts[1].shape[0]
+    dev = ts[0].device
+    ids = torch.empty(n_users, k, dtype=torch.int32, device=dev)
+    vals = torch.empty(n_users, k, dtype=torch.float32, device=dev)
+    ws = _ws(lib.cbrs_score_hybrid_topk_tf32x3_workspace_bytes(), dev)
+    L.check(lib.cbrs_score_hybrid_topk_tf32x3(_ptr(ts[0], torch.float32), _ptr(ts[1], torch.float32),
+                                              _ptr(ts[2], torch.float32), _ptr(ts[3], torch.float32), n_users, n_items, c,
+                                              *[_ptr(t, torch.float32) for t in ts[4:]], k, _ptr(ids), _ptr(vals), rp, it,
+                                              _ptr(ws), ws.numel(), _stream()), "cbrs_score_hybrid_topk_tf32x3")
+    _count(6)
+    return ids, vals
+
+
 def synth_bipartite(n_users, n_items, n_edges, seed, device, scatter_items=True):
     lib = L.load()
     row = torch.empty(2 * n_edges, dtype=torch.int32, device=device)

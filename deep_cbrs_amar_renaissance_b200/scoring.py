@@ -196,12 +196,15 @@ def _fused_basic(model, emb, users, items, k, precision="fp32", exclude=None):
     return ops.score_catalog_topk(P, Q, l2.kernel, l2.bias, l3.kernel.reshape(-1), l3.bias, k, precision, exclude)
 
 
-def _fused_hybrid_feature(model, emb, users, items, k, exclude=None):
+def _fused_hybrid_feature(model, emb, users, items, k, exclude=None, precision="bf16"):
     """Feature-based HybridCBRS with the shapes of every hybrid grid of the reference (dense3a / dense3b = two 64-wide
-    layers, classifier 64 -> 64 -> 1, relu, plain concatenation) -> the chained tensor-core kernel
-    (cbrs_score_hybrid_topk_bf16).  None when the scorer has another shape."""
+    layers, classifier 64 -> 64 -> 1, relu, plain concatenation) -> a chained tensor-core kernel: precision 'bf16'
+    cbrs_score_hybrid_topk_bf16 (bf16 operands), 'fp32' cbrs_score_hybrid_topk_tf32x3 (3xTF32, fp32 accuracy; k must
+    not exceed the catalog).  None when the scorer has another shape or the precision has no such kernel."""
     rs = model.rs
     if hasattr(rs, "unet") or not rs.feature_based or rs.residual is not None or model.content_table is None or k > 128:
+        return None
+    if precision not in ("bf16", "fp32") or (precision == "fp32" and k > items.numel()):
         return None
     if any(f.method != 'concatenate' for f in (rs.fuse1a, rs.fuse1b, rs.fuse2)):
         return None
@@ -223,9 +226,9 @@ def _fused_hybrid_feature(model, emb, users, items, k, exclude=None):
     Q1 = ops.dense(ig, d3a[0].kernel[g:], None, None)
     P2 = ops.dense(ub, d3b[0].kernel[:c], d3b[0].bias, None)
     Q2 = ops.dense(ib, d3b[0].kernel[c:], None, None)
-    return ops.score_hybrid_topk_bf16(P1, Q1, P2, Q2, d3a[1].kernel, d3a[1].bias, d3b[1].kernel, d3b[1].bias,
-                                      clf[0].kernel, clf[0].bias, clf[1].kernel, clf[1].bias, clf[2].kernel.reshape(-1),
-                                      clf[2].bias, k, exclude)
+    kernel = ops.score_hybrid_topk_bf16 if precision == "bf16" else ops.score_hybrid_topk_tf32x3
+    return kernel(P1, Q1, P2, Q2, d3a[1].kernel, d3a[1].bias, d3b[1].kernel, d3b[1].bias, clf[0].kernel, clf[0].bias,
+                  clf[1].kernel, clf[1].bias, clf[2].kernel.reshape(-1), clf[2].bias, k, exclude)
 
 
 def catalog_top_k(model, emb, n_users, n_items, k=10, users=None, user_block=None, fused=True, precision="fp32",
@@ -239,8 +242,8 @@ def catalog_top_k(model, emb, n_users, n_items, k=10, users=None, user_block=Non
     excl = _exclusion_rows(exclude, n_users, n_items, users, all_users)
     if fused:
         out = _fused_basic(model, emb, users, items, k, precision, excl)
-        if out is None and precision == "bf16":
-            out = _fused_hybrid_feature(model, emb, users, items, k, excl)
+        if out is None and precision in ("bf16", "fp32"):   # 'fp32-ffma' keeps the generic path for hybrids
+            out = _fused_hybrid_feature(model, emb, users, items, k, excl, precision)
         if out is not None:
             return out
     score = _pair_scorer(model, emb, users, items)

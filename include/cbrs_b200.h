@@ -226,6 +226,20 @@ int cbrs_score_hybrid_topk_bf16_ex(const float *P1, const float *Q1, const float
                                    const float *bc2, const float *wc3, const float *bc3, int32_t k, int32_t *ids_out,
                                    float *scores_out, const int64_t *excl_rowptr, const int32_t *excl_items,
                                    void *workspace, size_t workspace_bytes, void *stream);
+/* The same scorer at fp32 accuracy (1e-5 on the scores): each of the five 64 x 64 products runs as 3xTF32 on the tensor
+ * cores (as cbrs_score_catalog_topk_tf32x3), every activation that feeds one split into a tf32 part and its remainder;
+ * bias, relu, the output dot and the sigmoid in fp32.  Arguments and outputs as cbrs_score_hybrid_topk_bf16_ex, with
+ * k in [1, min(128, n_items)]; slots past a user's eligible items hold -1 / -inf.  Exclusion lists as above
+ * cbrs_score_catalog_topk_ex (both null: none; exactly one null: CBRS_E_INVALID).  c != 64: CBRS_E_UNSUPPORTED;
+ * workspace: at least cbrs_score_hybrid_topk_tf32x3_workspace_bytes(), 16-byte aligned, else CBRS_E_WORKSPACE;
+ * n_users == 0 writes nothing.                                                                                    */
+size_t cbrs_score_hybrid_topk_tf32x3_workspace_bytes(void);
+int cbrs_score_hybrid_topk_tf32x3(const float *P1, const float *Q1, const float *P2, const float *Q2, int64_t n_users,
+                                  int32_t n_items, int32_t c, const float *w3a2, const float *b3a2, const float *w3b2,
+                                  const float *b3b2, const float *wc1, const float *bc1, const float *wc2,
+                                  const float *bc2, const float *wc3, const float *bc3, int32_t k, int32_t *ids_out,
+                                  float *scores_out, const int64_t *excl_rowptr, const int32_t *excl_items,
+                                  void *workspace, size_t workspace_bytes, void *stream);
 
 /* Grouped transform of the relational layer (row R: "R-GCN per-relation transform plus scatter as a grouped kernel"):
  * ONE launch computes X[m, f] . [W_0 | ... | W_{R-1}] (w_cat: contiguous [f, n_groups*h], Keras layout) and stores
