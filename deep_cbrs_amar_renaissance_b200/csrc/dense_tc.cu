@@ -21,7 +21,6 @@
 #include "dense_tc.cuh"
 
 #include <algorithm>
-#include <stdlib.h>
 
 namespace cbrs {
 
@@ -252,9 +251,8 @@ extern "C" int cbrs_dense_tc(const float *x1, int64_t ld1, const int64_t *idx1, 
     p.w_image = (const uint8_t *)w_image; p.b = b; p.m = m; p.n = n; p.act = act; p.out = out; p.ldo = ldo;
     // two kernels, chosen by depth (profiles/r02_dense_tc_bench_{shipped,variant4}.jsonl, 2^20 rows): the 256-thread
     // kernel with loop-invariant row pointers (dense_tc_x.cu) wins on deep layers (768 -> 256: 1.54 vs 1.65 ms), the
-    // 128-thread one on shallow layers (256 -> 64: 0.34 vs 0.40 ms).  CBRS_DENSE_TC_VARIANT=3|4 forces one (tests).
-    static const int variant = getenv("CBRS_DENSE_TC_VARIANT") ? atoi(getenv("CBRS_DENSE_TC_VARIANT")) : 0;
-    if (variant == 4 || (variant == 0 && f1 + f2 >= 512)) return dense_tc_launch_x(p, (cudaStream_t)stream);
+    // 128-thread one on shallow layers (256 -> 64: 0.34 vs 0.40 ms).
+    if (f1 + f2 >= 512) return dense_tc_launch_x(p, (cudaStream_t)stream);
     dense_tc_kernel<<<(unsigned)cdiv(m, kDtRows), kDtThreads, smem, (cudaStream_t)stream>>>(p);
     CBRS_CHECK_LAUNCH("cbrs_dense_tc");
     return CBRS_OK;

@@ -1,4 +1,4 @@
-// Shared between the tensor-core Dense kernels (dense_tc.cu: the shipped kernel; dense_tc_x.cu: the experimental variant).
+// Shared between the tensor-core Dense kernels (dense_tc.cu: shallow layers; dense_tc_x.cu: deep layers, f1 + f2 >= 512).
 #pragma once
 #include "common.cuh"
 #include "tc05.cuh"
@@ -43,7 +43,7 @@ __device__ __forceinline__ float4 dt_ld_stream4(const float *p) {   // read-once
     return v;
 }
 
-// experimental variant (dense_tc_x.cu), selected by CBRS_DENSE_TC_VARIANT=4; not part of the validated path
+// deep-layer kernel (dense_tc_x.cu): cbrs_dense_tc runs it when f1 + f2 >= 512
 int dense_tc_launch_x(const DenseTcParams &p, cudaStream_t stream);
 
 }  // namespace cbrs

@@ -29,7 +29,6 @@
 #include "tc05.cuh"
 
 #include <cuda.h>  // CUtensorMap; the encoder is looked up through the runtime (no -lcuda)
-#include <stdlib.h>
 
 namespace cbrs {
 
@@ -359,13 +358,8 @@ static tm_encode_fn tm_encoder() {
 }
 // L2 promotion of the loads: a row is read in 128-byte slices, one K block at a time; promoting each miss to 256 B brings the
 // next K block's slice of the same row along (measured, 768 -> 256 at 2^20 rows: 0.543 vs 0.558 ms consecutive, 0.609 vs
-// 0.623 ms gathered, profiles/r02_dense_tc_tma_bench_l2p{128,256}.jsonl).  CBRS_TMA_L2_PROMOTION=64|128|256 overrides.
-static CUtensorMapL2promotion tm_l2_promotion(bool gather) {
-    static const int forced = getenv("CBRS_TMA_L2_PROMOTION") ? atoi(getenv("CBRS_TMA_L2_PROMOTION")) : 0;
-    (void)gather;
-    const int v = forced ? forced : 256;
-    return v == 256 ? CU_TENSOR_MAP_L2_PROMOTION_L2_256B : (v == 64 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B : CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
-}
+// 0.623 ms gathered, profiles/r02_dense_tc_tma_bench_l2p{128,256}.jsonl).
+constexpr CUtensorMapL2promotion kTmL2Promotion = CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
 // rows of `f` bf16 out of a [rows, ld] table; box = 64 columns x (1 row for tile::gather4 | 64 rows tiled)
 static int tm_make_map(CUtensorMap *map, const void *x, int64_t ld, int64_t rows, int32_t f, bool gather) {
     tm_encode_fn encode = tm_encoder();
@@ -375,8 +369,7 @@ static int tm_make_map(CUtensorMap *map, const void *x, int64_t ld, int64_t rows
     const cuuint32_t box[2] = {(cuuint32_t)kTmKB, gather ? 1u : 64u};
     const cuuint32_t estr[2] = {1, 1};
     CUresult r = encode(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void *>(x), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                        tm_l2_promotion(gather),
+                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, kTmL2Promotion,
                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     CBRS_REQUIRE(r == CUDA_SUCCESS, CBRS_E_CUDA, "cbrs_dense_tc_bf16: cuTensorMapEncodeTiled failed (%d)", (int)r);
     return CBRS_OK;

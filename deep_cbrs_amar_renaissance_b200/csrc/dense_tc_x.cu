@@ -1,7 +1,7 @@
 // Second tensor-core Dense kernel (see dense_tc.cu): cbrs_dense_tc uses it for deep layers (f1 + f2 >= 512, e.g. the
 // hybrid scorer's 768 -> 256 BERT tower: 1.54 ms per 2^20 rows against 1.65 ms with dense_tc_kernel,
-// profiles/r02_dense_tc_bench_variant4.jsonl); CBRS_DENSE_TC_VARIANT=3|4 forces one kernel on every shape, which is
-// how tests/test_zz_gpu_dense_tc.py::test_each_kernel_variant_on_every_shape covers both.
+// profiles/r02_dense_tc_bench_variant4.jsonl).  tests/test_zz_gpu_dense_tc.py runs its parity cases at both depths and
+// checks which kernel each depth gets.
 // Written from the ncu evidence on dense_tc_kernel (profiles/r01_ncu_dense_tc_v3_stalls.txt: 8 warps per SM, ~535
 // instructions per warp and K block, 26 % of the stall samples on the row-pointer LDS -> address arithmetic chain).
 //

@@ -19,7 +19,6 @@
 #include "common.cuh"
 #include "tc05.cuh"
 
-#include <stdlib.h>
 #include <string.h>
 
 namespace cbrs {
@@ -290,7 +289,8 @@ __global__ void __launch_bounds__(kTcThreads, QREG ? 4 : 3) score_tc_kernel(cons
 //    h1 = bf16(bf16(P) + bf16(Q)), relu - the bf16 oracle in the tests does the same roundings;
 //  * A tiles and TMEM accumulators are double buffered: the A tile of step s+1 is produced and its MMA issued
 //    BEFORE the epilogue of step s, so the tensor core's issue->commit latency hides behind CUDA-core work;
-//  * the epilogue uses the packed fp32 pipe (add.rn.f32x2 / fma.rn.f32x2) for bias and the output layer.
+//  * the epilogue reads bias and output-layer weights from shared memory and sums the output layer in eight
+//    independent fp32 chains.
 struct ScoreTc2Params {
     const float *P; int64_t ldp;
     const uint4 *Qb;            // [n_items_pad][8] : 64 bf16 per item, zero padded
@@ -302,13 +302,6 @@ struct ScoreTc2Params {
     int32_t *ids_out; float *scores_out;
     const int64_t *excl_rowptr; const int32_t *excl_items;   // exclusion lists (both null: none)
 };
-
-// bias and output-layer weights in constant memory: the fully unrolled epilogue (NP > 0) reads them as
-// instruction operands (c[bank][offset]) - no shared-memory load per column.  Filled stream-ordered by
-// cudaMemcpyToSymbolAsync (device to device, no host synchronisation); concurrent scorer calls on DIFFERENT
-// streams with different weights would race on it (stated in the header).
-__constant__ float g_score_b2[128];
-__constant__ float g_score_w3[128];
 
 __global__ void score_tc_qprep_kernel(const float *__restrict__ Q, int64_t ldq, int32_t n_items, int32_t n_items_pad,
                                       int32_t c1, uint4 *__restrict__ Qb) {
@@ -331,25 +324,12 @@ __device__ __forceinline__ uint32_t bf16x2_add_relu(uint32_t a, uint32_t b) {
     const __nv_bfloat162 r = __hmax2(__hadd2(x, y), __float2bfloat162_rn(0.f));
     return *reinterpret_cast<const uint32_t *>(&r);
 }
-__device__ __forceinline__ unsigned long long f32x2_pack(float lo, float hi) {
-    return ((unsigned long long)__float_as_uint(hi) << 32) | (unsigned long long)__float_as_uint(lo);
-}
-__device__ __forceinline__ unsigned long long f32x2_add(unsigned long long a, unsigned long long b) {
-    unsigned long long d;
-    asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
-    return d;
-}
-__device__ __forceinline__ unsigned long long f32x2_fma(unsigned long long a, unsigned long long b, unsigned long long c) {
-    unsigned long long d;
-    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c));
-    return d;
-}
 
-template <bool kPackedEpilogue, int NP, bool kExcl>   // kExcl: exclusion lists given
+template <bool kExcl>   // exclusion lists given
 __global__ void __launch_bounds__(kTcThreads, 4) score_tc2_kernel(const __grid_constant__ ScoreTc2Params p) {
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     const int c1 = p.c1;
-    const int n_pad = NP > 0 ? NP : (p.c2 + 15) / 16 * 16;
+    const int n_pad = (p.c2 + 15) / 16 * 16;
     const int cap = 2 * p.k + kTcTI;
     unsigned char *As = smem_raw;                                    // [2][128][128 B]
     unsigned char *Bs = As + 2 * 16384;                              // [n_pad][128 B]
@@ -474,25 +454,7 @@ __global__ void __launch_bounds__(kTcThreads, 4) score_tc2_kernel(const __grid_c
         tc::tc_fence_after_sync();
         // ---- epilogue of `step`: accumulator row `tid` ------------------------------------------------------
         const uint32_t trow = tmem_row + (uint32_t)(step & 1) * buf_cols;
-        unsigned long long logit2 = 0ull;
         float lacc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};  // independent chains: 4 warps per scheduler hide little latency
-        if constexpr (NP > 0) {
-#pragma unroll
-            for (int cb = 0; cb < NP; cb += 32) {
-                uint32_t v0[16], v1[16];
-                tc::tmem_ld16(trow + (uint32_t)cb, v0);
-                if (cb + 16 < NP) tc::tmem_ld16(trow + (uint32_t)cb + 16, v1);
-                tc::tmem_ld_wait();
-#pragma unroll
-                for (int j = 0; j < 16; ++j)
-                    lacc[j & 7] = fmaf(fmaxf(__uint_as_float(v0[j]) + g_score_b2[cb + j], 0.f), g_score_w3[cb + j], lacc[j & 7]);
-                if (cb + 16 < NP) {
-#pragma unroll
-                    for (int j = 0; j < 16; ++j)
-                        lacc[j & 7] = fmaf(fmaxf(__uint_as_float(v1[j]) + g_score_b2[cb + 16 + j], 0.f), g_score_w3[cb + 16 + j], lacc[j & 7]);
-                }
-            }
-        } else
         for (int cb = 0; cb < n_pad; cb += 32) {
             uint32_t v0[16], v1[16];
             tc::tmem_ld16(trow + (uint32_t)cb, v0);
@@ -501,31 +463,19 @@ __global__ void __launch_bounds__(kTcThreads, 4) score_tc2_kernel(const __grid_c
 #pragma unroll
             for (int j = 0; j < 16; j += 2) {
                 const float4 t = bw[(cb + j) >> 1];
-                if (kPackedEpilogue) {
-                    const unsigned long long x = f32x2_add(((unsigned long long)v0[j + 1] << 32) | v0[j], f32x2_pack(t.x, t.y));
-                    const float lo = fmaxf(__uint_as_float((uint32_t)x), 0.f), hi = fmaxf(__uint_as_float((uint32_t)(x >> 32)), 0.f);
-                    logit2 = f32x2_fma(f32x2_pack(lo, hi), f32x2_pack(t.z, t.w), logit2);
-                } else {
-                    lacc[j & 7] = fmaf(fmaxf(__uint_as_float(v0[j]) + t.x, 0.f), t.z, lacc[j & 7]);
-                    lacc[(j + 1) & 7] = fmaf(fmaxf(__uint_as_float(v0[j + 1]) + t.y, 0.f), t.w, lacc[(j + 1) & 7]);
-                }
+                lacc[j & 7] = fmaf(fmaxf(__uint_as_float(v0[j]) + t.x, 0.f), t.z, lacc[j & 7]);
+                lacc[(j + 1) & 7] = fmaf(fmaxf(__uint_as_float(v0[j + 1]) + t.y, 0.f), t.w, lacc[(j + 1) & 7]);
             }
             if (cb + 16 < n_pad) {
 #pragma unroll
                 for (int j = 0; j < 16; j += 2) {
                     const float4 t = bw[(cb + 16 + j) >> 1];
-                    if (kPackedEpilogue) {
-                        const unsigned long long x = f32x2_add(((unsigned long long)v1[j + 1] << 32) | v1[j], f32x2_pack(t.x, t.y));
-                        const float lo = fmaxf(__uint_as_float((uint32_t)x), 0.f), hi = fmaxf(__uint_as_float((uint32_t)(x >> 32)), 0.f);
-                        logit2 = f32x2_fma(f32x2_pack(lo, hi), f32x2_pack(t.z, t.w), logit2);
-                    } else {
-                        lacc[j & 7] = fmaf(fmaxf(__uint_as_float(v1[j]) + t.x, 0.f), t.z, lacc[j & 7]);
-                        lacc[(j + 1) & 7] = fmaf(fmaxf(__uint_as_float(v1[j + 1]) + t.y, 0.f), t.w, lacc[(j + 1) & 7]);
-                    }
+                    lacc[j & 7] = fmaf(fmaxf(__uint_as_float(v1[j]) + t.x, 0.f), t.z, lacc[j & 7]);
+                    lacc[(j + 1) & 7] = fmaf(fmaxf(__uint_as_float(v1[j + 1]) + t.y, 0.f), t.w, lacc[(j + 1) & 7]);
                 }
             }
         }
-        const float logit = (kPackedEpilogue && NP == 0) ? __uint_as_float((uint32_t)logit2) + __uint_as_float((uint32_t)(logit2 >> 32)) : ((lacc[0] + lacc[1]) + (lacc[2] + lacc[3])) + ((lacc[4] + lacc[5]) + (lacc[6] + lacc[7]));
+        const float logit = ((lacc[0] + lacc[1]) + (lacc[2] + lacc[3])) + ((lacc[4] + lacc[5]) + (lacc[6] + lacc[7]));
         const int ul = pass * 4 + warp;
         const int item = tile * kTcTI + lane;
         const int64_t user = u0 + ul;
@@ -911,10 +861,7 @@ static size_t score_tc_smem(int c1, int c2, int k) {
 using namespace cbrs;
 
 static bool score_tc_use_v2(int c1, int c2) { return c1 <= 64 && c2 <= 128; }
-static bool score_tc_use_v3(int c1, int c2) {   // CBRS_SCORE_BF16_KERNEL=2 keeps v2 (measurements)
-    static const int forced = getenv("CBRS_SCORE_BF16_KERNEL") ? atoi(getenv("CBRS_SCORE_BF16_KERNEL")) : 0;
-    return forced != 2 && c1 <= 64 && c2 <= 64;
-}
+static bool score_tc_use_v3(int c1, int c2) { return c1 <= 64 && c2 <= 64; }
 constexpr size_t kTc3ImageBytes = 2 * 8192 + 2048;
 
 extern "C" size_t cbrs_score_catalog_topk_bf16_workspace_bytes(int32_t n_items, int32_t c1, int32_t c2) {
@@ -977,32 +924,12 @@ extern "C" int cbrs_score_catalog_topk_bf16_ex(const float *P, int64_t ldp, cons
         }
         const size_t smem2 = score_tc2_smem(c2, k);
         CBRS_REQUIRE(smem2 <= 220 * 1024, CBRS_E_UNSUPPORTED, "score_catalog_bf16: needs %zu bytes of shared memory", smem2);
-        static const int mode = getenv("CBRS_SCORE_EPILOGUE") ? atoi(getenv("CBRS_SCORE_EPILOGUE")) : 0;  // tuning knob
         ScoreTc2Params p2{P, ldp, Qb, n_users, n_items, c1, c2, (const uint8_t *)workspace, b2, w3, b3, k, ids_out, scores_out,
                           excl_rowptr, excl_items};
-        const unsigned grid = (unsigned)cdiv(n_users, kTcTU);
-        // mode 0: n_pad == 64 -> constant-bank epilogue (b2/w3 copied to constant memory);
-        // mode 1: shared-memory scalar epilogue; mode 2: shared-memory packed fp32x2 epilogue
-        if (mode == 0 && c2 == 64) {
-            CBRS_REQUIRE(c2 == 64, CBRS_E_INVALID, "score_catalog_bf16: internal: constant epilogue needs c2 == 64");
-            cudaError_t ec = cudaMemcpyToSymbolAsync(g_score_b2, b2, sizeof(float) * c2, 0, cudaMemcpyDeviceToDevice, s);
-            if (ec == cudaSuccess) ec = cudaMemcpyToSymbolAsync(g_score_w3, w3, sizeof(float) * c2, 0, cudaMemcpyDeviceToDevice, s);
-            CBRS_REQUIRE(ec == cudaSuccess, CBRS_E_CUDA, "score_catalog_bf16: staging b2/w3: %s", cudaGetErrorString(ec));
-            auto k2 = excl_rowptr ? score_tc2_kernel<false, 64, true> : score_tc2_kernel<false, 64, false>;
-            cudaError_t e2 = cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
-            CBRS_REQUIRE(e2 == cudaSuccess, CBRS_E_CUDA, "score_catalog_bf16: cudaFuncSetAttribute: %s", cudaGetErrorString(e2));
-            k2<<<grid, kTcThreads, smem2, s>>>(p2);
-        } else if (mode == 2) {
-            auto k2 = excl_rowptr ? score_tc2_kernel<true, 0, true> : score_tc2_kernel<true, 0, false>;
-            cudaError_t e2 = cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
-            CBRS_REQUIRE(e2 == cudaSuccess, CBRS_E_CUDA, "score_catalog_bf16: cudaFuncSetAttribute: %s", cudaGetErrorString(e2));
-            k2<<<grid, kTcThreads, smem2, s>>>(p2);
-        } else {
-            auto k2 = excl_rowptr ? score_tc2_kernel<false, 0, true> : score_tc2_kernel<false, 0, false>;
-            cudaError_t e2 = cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
-            CBRS_REQUIRE(e2 == cudaSuccess, CBRS_E_CUDA, "score_catalog_bf16: cudaFuncSetAttribute: %s", cudaGetErrorString(e2));
-            k2<<<grid, kTcThreads, smem2, s>>>(p2);
-        }
+        auto k2 = excl_rowptr ? score_tc2_kernel<true> : score_tc2_kernel<false>;
+        cudaError_t e2 = cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
+        CBRS_REQUIRE(e2 == cudaSuccess, CBRS_E_CUDA, "score_catalog_bf16: cudaFuncSetAttribute: %s", cudaGetErrorString(e2));
+        k2<<<(unsigned)cdiv(n_users, kTcTU), kTcThreads, smem2, s>>>(p2);
         CBRS_CHECK_LAUNCH("score_tc2");
         return CBRS_OK;
     }

@@ -16,7 +16,6 @@
 #include "common.cuh"
 
 #include <cuda_bf16.h>
-#include <stdlib.h>
 
 #include <type_traits>
 
@@ -99,12 +98,6 @@ template <>
 struct Vec<8> {
     float4 a, b;
     __device__ __forceinline__ void zero() { a = make_float4(0.f, 0.f, 0.f, 0.f); b = a; }
-    // one 256-bit load (LDG.E.256, sm_100): a 128-wide fp32 row is 16 lanes, two chunks share a warp
-    __device__ __forceinline__ void load(const float *p) {
-        asm volatile("ld.global.nc.v8.f32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-                     : "=f"(a.x), "=f"(a.y), "=f"(a.z), "=f"(a.w), "=f"(b.x), "=f"(b.y), "=f"(b.z), "=f"(b.w)
-                     : "l"(p));
-    }
     __device__ __forceinline__ void load_plain(const float *p) {
         a = *reinterpret_cast<const float4 *>(p); b = *reinterpret_cast<const float4 *>(p + 4);
     }
@@ -452,54 +445,15 @@ __global__ void __launch_bounds__(256) spmm_gcn_fused_heavy_kernel(const FusedPa
     fused_store_z(fp, row, lane, row_times_w(acc.v, fp.w_next, lane));
 }
 
-// tuning knob (bench/tuning only): CBRS_SPMM_VARIANT selects loads-in-flight x occupancy for the
-// 128-wide fp32 kernel; the default is the measured best
-static int spmm_variant() {
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("CBRS_SPMM_VARIANT");
-        v = e ? atoi(e) : 0;
-    }
-    return v;
-}
-
 template <int G, int VEC, typename XT = float>
 static int launch(const SpmmParams &p, cudaStream_t s) {
     const int64_t threads = p.n_chunks * G;
     if (threads > 0) {
-        const unsigned grid = (unsigned)cdiv(threads, kSpmmThreads);
-        if (!std::is_same<XT, float>::value) {
-            switch (spmm_variant()) {  // CBRS_SPMM_VARIANT: loads in flight for the bf16 kernel (tuning knob)
-                case 1: spmm_chunk_kernel<G, VEC, 4, 4, XT><<<grid, kSpmmThreads, 0, s>>>(p); break;
-                case 2: spmm_chunk_kernel<G, VEC, 16, 3, XT><<<grid, kSpmmThreads, 0, s>>>(p); break;
-                case 3: spmm_chunk_kernel<G, VEC, 8, 3, XT><<<grid, kSpmmThreads, 0, s>>>(p); break;
-                case 4: spmm_chunk_kernel<G, VEC, 6, 4, XT><<<grid, kSpmmThreads, 0, s>>>(p); break;
-                default:
-                    if (VEC == 8) spmm_chunk_kernel<G, VEC, 4, 4, XT><<<grid, kSpmmThreads, 0, s>>>(p);
-                    else spmm_chunk_kernel<G, VEC, 8, 4, XT><<<grid, kSpmmThreads, 0, s>>>(p);
-                    break;
-            }
-        } else if (G == 32 && VEC == 4) {
-            // measured on config 5 (profiles/r01_tune_spmm.log): 4 loads in flight x 32 warps/SM beats
-            // 8 x 16 by 1.45x - occupancy, not per-warp MLP, is what saturates HBM here
-            switch (spmm_variant()) {
-                case 1: spmm_chunk_kernel<32, 4, 8, 2><<<grid, kSpmmThreads, 0, s>>>(p); break;
-                case 2: spmm_chunk_kernel<32, 4, 8, 4><<<grid, kSpmmThreads, 0, s>>>(p); break;
-                case 3: spmm_chunk_kernel<32, 4, 2, 8><<<grid, kSpmmThreads, 0, s>>>(p); break;
-                case 4: spmm_chunk_kernel<32, 4, 4, 5><<<grid, kSpmmThreads, 0, s>>>(p); break;
-                case 5: spmm_chunk_kernel<32, 4, 2, 6><<<grid, kSpmmThreads, 0, s>>>(p); break;
-                default: spmm_chunk_kernel<32, 4, 4, 4><<<grid, kSpmmThreads, 0, s>>>(p); break;
-            }
-        } else if (G == 16 && VEC == 8) {
-            switch (spmm_variant()) {   // fp32, 256-bit loads: loads in flight x occupancy
-                case 7: spmm_chunk_kernel<16, 8, 4, 3><<<grid, kSpmmThreads, 0, s>>>(p); break;
-                case 8: spmm_chunk_kernel<16, 8, 2, 4><<<grid, kSpmmThreads, 0, s>>>(p); break;
-                case 9: spmm_chunk_kernel<16, 8, 8, 2><<<grid, kSpmmThreads, 0, s>>>(p); break;
-                default: spmm_chunk_kernel<16, 8, 4, 4><<<grid, kSpmmThreads, 0, s>>>(p); break;
-            }
-        } else {
-            spmm_chunk_kernel<G, VEC><<<grid, kSpmmThreads, 0, s>>>(p);
-        }
+        // row loads in flight per group: 4, or 8 for the half-width bf16 loads of VEC 1 and 4 (the same bytes in
+        // flight per lane as the fp32 kernel).  Measured on config 5 (profiles/r01_tune_spmm.log): 4 loads in
+        // flight x 32 warps/SM beats 8 x 16 by 1.45x - occupancy, not per-warp MLP, is what saturates HBM here
+        constexpr int kLoads = (!std::is_same<XT, float>::value && VEC != 8) ? 8 : 4;
+        spmm_chunk_kernel<G, VEC, kLoads, 4, XT><<<(unsigned)cdiv(threads, kSpmmThreads), kSpmmThreads, 0, s>>>(p);
         CBRS_CHECK_LAUNCH("spmm_chunk");
     }
     if (p.n_heavy > 0) {
@@ -570,13 +524,10 @@ static int spmm_impl(const cbrs_csr_t *g, const void *x, int64_t ldx, void *y, i
         // a 4-wide bf16 group is an 8-byte load: same lane layout as fp32, half the bytes per edge
         const bool v4 = (d % 4 == 0) && (ldx % 4 == 0) && (ldy % 4 == 0) && ((uintptr_t)x % 8 == 0) && ((uintptr_t)y % 16 == 0) &&
                         ((uintptr_t)workspace % 16 == 0) && (!bias || (uintptr_t)bias % 16 == 0) && vec4_peers;
-        const bool v8 = v4 && (d % 8 == 0) && (ldx % 8 == 0) && ((uintptr_t)x % 16 == 0) && spmm_variant() != 9;
+        const bool v8 = v4 && (d % 8 == 0) && (ldx % 8 == 0) && ((uintptr_t)x % 16 == 0);
         if (v8) return dispatch_g<8, __nv_bfloat16>(d / 8, p, s);  // 16-byte loads, half the lanes per row
         return v4 ? dispatch_g<4, __nv_bfloat16>(d / 4, p, s) : dispatch_g<1, __nv_bfloat16>(d, p, s);
     }
-    // CBRS_SPMM_VARIANT=6: 256-bit row loads (fp32 rows 32-byte aligned, d % 8 == 0) - tuning knob
-    const bool vec8 = vec4 && (d % 8 == 0) && (ldx % 8 == 0) && ((uintptr_t)x % 32 == 0) && spmm_variant() >= 6;
-    if (vec8) return dispatch_g<8>(d / 8, p, s);
     return vec4 ? dispatch_g<4>(d / 4, p, s) : dispatch_g<1>(d, p, s);
 }
 

@@ -4,7 +4,6 @@ Every function takes CUDA torch tensors, launches on torch's current stream and
 returns torch tensors.  No CPU path exists: a non-CUDA tensor raises.
 """
 import ctypes
-import os
 
 import torch
 
@@ -276,8 +275,9 @@ def dense(x1, w, b=None, act=None, x2=None, idx1=None, idx2=None, rowop=L.ROWOP_
 # ---- the GCN transform Z = X W: fp32 FFMA kernel or the fp32-accurate tensor-core kernel (3xTF32) ----------------
 # "auto": tensor cores from TF32X3_MIN_ROWS graph nodes up (below that the layer is launch-latency bound and the FFMA
 # kernel keeps the round-1 bits of every MovieLens-sized parity case).  The choice is made on the GLOBAL node count, so
-# all ranks of a row partition and the single-GPU run take the same kernel.  CBRS_GCN_TRANSFORM=ffma|tf32x3 forces one.
-GCN_TRANSFORM = os.environ.get("CBRS_GCN_TRANSFORM", "auto")
+# all ranks of a row partition and the single-GPU run take the same kernel.  Setting GCN_TRANSFORM to "ffma" or "tf32x3"
+# forces one.
+GCN_TRANSFORM = "auto"
 TF32X3_MIN_ROWS = 1 << 16
 
 
@@ -650,13 +650,12 @@ def topk_pairs(users, scores, n_users, k):
 def score_catalog_topk(P, Q, w2, b2, w3, b3, k, precision="fp32", exclude=None):
     """Fused BasicRS catalog scorer: P [U,c1] (bias folded in), Q [I,c1] -> (ids int32 [U,k], scores [U,k]).
     precision 'fp32' = fp32-accurate (1e-5 parity): the 3xTF32 tensor-core kernel for the shapes it takes (c1 in {32, 64},
-    c2 <= 64: the reference's grids), the FFMA kernel otherwise; 'fp32-ffma' forces the FFMA kernel (CBRS_SCORE_FP32=ffma
-    does the same for a whole process); 'bf16' = bf16 operands on the tensor cores.
+    c2 <= 64: the reference's grids), the FFMA kernel otherwise; 'fp32-ffma' forces the FFMA kernel;
+    'bf16' = bf16 operands on the tensor cores.
     exclude = (rowptr, items): per-row lists of catalog items kept out of row r's top-k (row r = row r of P)."""
     lib = L.load()
     rp, it = _exclusion(exclude, P.shape[0])
-    if precision == "fp32" and os.environ.get("CBRS_SCORE_FP32", "") != "ffma" and \
-            lib.cbrs_score_catalog_topk_tf32x3_eligible(P.shape[1], w2.shape[1]):
+    if precision == "fp32" and lib.cbrs_score_catalog_topk_tf32x3_eligible(P.shape[1], w2.shape[1]):
         P, ldp = _rowmajor(P)
         Q, ldq = _rowmajor(Q)
         n_users, c1 = P.shape

@@ -377,10 +377,7 @@ int cbrs_score_catalog_topk_tf32x3_ex(const float *P, int64_t ldp, const float *
  * scores differ from the fp32 kernel by O(1e-3) (tolerance stated in tests).  c1 % 8 == 0,
  * c1 <= 256, c2 <= 256.  For c1 <= 64 (the reference's grids) P and Q themselves are rounded to bf16 and
  * added with add.rn.bf16x2: h1 = bf16(bf16(P) + bf16(Q)); for wider c1 the sum is formed in fp32 and
- * rounded once.  Workspace: the pre-swizzled bf16 image of W2^T (+ Q as bf16 when c1 <= 64).
- * With c2 == 64 the bias and output weights are staged in __constant__ memory (stream-ordered device-to-device
- * copy, no host synchronisation) so the epilogue reads them as instruction operands: calls with DIFFERENT
- * weights must not run concurrently on different streams.                                                  */
+ * rounded once.  Workspace: the pre-swizzled bf16 image of W2^T (+ Q as bf16 when c1 <= 64).              */
 size_t cbrs_score_catalog_topk_bf16_workspace_bytes(int32_t n_items, int32_t c1, int32_t c2);
 int cbrs_score_catalog_topk_bf16(const float *P, int64_t ldp, const float *Q, int64_t ldq, int64_t n_users,
                                  int32_t n_items, int32_t c1, const float *w2, const float *b2, int32_t c2,

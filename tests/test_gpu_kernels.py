@@ -383,7 +383,8 @@ def _bf16_round(x):
 
 @pytest.mark.parametrize("n_users,n_items,c1,c2,k", [(37, 3706, 64, 64, 10), (50, 1000, 48, 48, 5), (5, 7, 64, 64, 10),
                                                       (40, 333, 128, 128, 20), (130, 2049, 64, 32, 10),
-                                                      (33, 500, 8, 16, 3), (20, 700, 72, 80, 10)])
+                                                      (33, 500, 8, 16, 3), (20, 700, 72, 80, 10),
+                                                      (41, 1500, 64, 128, 10), (9, 300, 32, 96, 7)])
 def test_tensor_core_catalog_scorer_matches_bf16_oracle(dev, n_users, n_items, c1, c2, k):
     """tcgen05 path: operands rounded to bf16, fp32 accumulate.  Oracle = the same rounding in numpy;
     tolerance 2e-5 on scores (fp32 summation order inside the MMA is unspecified; 1e-4 for the v3 kernel, where an

@@ -3,10 +3,6 @@ rounds the same operands to bf16 and sums in float64.  Tolerance 1e-4 of the out
 accumulation order inside the tensor core is not specified; a layout or descriptor bug gives O(1) errors).
 Model level: a hybrid model with set_scorer_precision('bf16') against the same rounding oracle, and against its own
 fp32 scores within 2e-2."""
-import os
-import subprocess
-import sys
-
 import numpy as np
 import pytest
 import torch
@@ -40,8 +36,11 @@ def close(got, want, what, rtol=1e-4):
     assert err <= rtol * scale, "{}: max abs err {:.3e} (scale {:.3e})".format(what, err, scale)
 
 
+# k < 512 runs dense_tc_kernel, k >= 512 dense_tc_x_kernel: each kernel at the same widths, activations and bias settings
 @pytest.mark.parametrize("m,k,n,act,bias", [(300, 768, 256, "relu", True), (128, 64, 64, None, True), (77, 24, 16, "tanh", False),
-                                            (1000, 200, 40, None, True), (5, 256, 8, "sigmoid", True), (4097, 128, 128, "relu", True)])
+                                            (1000, 200, 40, None, True), (5, 256, 8, "sigmoid", True), (4097, 128, 128, "relu", True),
+                                            (128, 576, 64, None, True), (77, 512, 16, "tanh", False), (1000, 520, 40, None, True),
+                                            (5, 768, 8, "sigmoid", True), (4097, 1024, 128, "relu", True)])
 def test_dense_tc_single_source(m, k, n, act, bias):
     from deep_cbrs_amar_renaissance_b200 import ops
     rng = np.random.RandomState(m + k + n)
@@ -53,27 +52,58 @@ def test_dense_tc_single_source(m, k, n, act, bias):
     close(got, oracle_dense_bf16(a, w, b, act), "dense_tc %dx%dx%d %s" % (m, k, n, act))
 
 
-def test_dense_tc_gather_concat_strided():
+def _gather_concat_strided(f1, f2, n, seed):
     """two gathered sources (the scorer's lookup + concat), a column-slice source and a strided output"""
     from deep_cbrs_amar_renaissance_b200 import ops
-    rng = np.random.RandomState(1)
-    t1 = rng.standard_normal((500, 96 + 8)).astype(np.float32)
-    t2 = rng.standard_normal((400, 48)).astype(np.float32)
+    rng = np.random.RandomState(seed)
+    t1 = rng.standard_normal((500, f1 + 8)).astype(np.float32)
+    t2 = rng.standard_normal((400, f2)).astype(np.float32)
     i1 = rng.randint(0, 500, size=1000)
     i1[:64] = i1[0]
     i2 = rng.randint(0, 400, size=1000)
-    w = (rng.standard_normal((144, 64)) / 12).astype(np.float32)
-    b = (rng.standard_normal(64) * 0.1).astype(np.float32)
-    src1 = cuda(t1)[:, 4:100]          # ld 104, offset 16 bytes
-    buf = torch.zeros(1000, 72, device="cuda")
-    out = ops.dense_tc(src1, cuda(w), cuda(b), "sigmoid", x2=cuda(t2), idx1=cuda(i1), idx2=cuda(i2), out=buf[:, 4:68])
-    a = np.concatenate([t1[i1][:, 4:100], t2[i2]], axis=1)
-    close(out.cpu().numpy(), oracle_dense_bf16(a, w, b, "sigmoid"), "gather + concat")
-    assert float(buf[:, :4].abs().max()) == 0.0 and float(buf[:, 68:].abs().max()) == 0.0   # nothing written outside the view
+    w = (rng.standard_normal((f1 + f2, n)) / np.sqrt(f1 + f2)).astype(np.float32)
+    b = (rng.standard_normal(n) * 0.1).astype(np.float32)
+    src1 = cuda(t1)[:, 4:4 + f1]        # ld f1 + 8, offset 16 bytes
+    buf = torch.zeros(1000, n + 8, device="cuda")
+    out = ops.dense_tc(src1, cuda(w), cuda(b), "sigmoid", x2=cuda(t2), idx1=cuda(i1), idx2=cuda(i2), out=buf[:, 4:4 + n])
+    a = np.concatenate([t1[i1][:, 4:4 + f1], t2[i2]], axis=1)
+    close(out.cpu().numpy(), oracle_dense_bf16(a, w, b, "sigmoid"), "gather + concat %d + %d -> %d" % (f1, f2, n))
+    assert float(buf[:, :4].abs().max()) == 0.0 and float(buf[:, 4 + n:].abs().max()) == 0.0   # nothing written outside the view
     # a prepared image can be reused across calls
     image = ops.dense_tc_image(cuda(w))
     again = ops.dense_tc(src1, cuda(w), cuda(b), "sigmoid", x2=cuda(t2), idx1=cuda(i1), idx2=cuda(i2), image=image)
     assert torch.equal(again, out.contiguous())
+
+
+def test_dense_tc_gather_concat_strided():
+    _gather_concat_strided(96, 48, 64, seed=1)
+
+
+def test_dense_tc_gather_concat_strided_deep():
+    """the same at the depth of the hybrid scorer's concatenated towers (f1 + f2 >= 512: dense_tc_x_kernel)"""
+    _gather_concat_strided(512, 256, 64, seed=2)
+
+
+@pytest.mark.parametrize("f1,f2,kernel", [(504, 0, "dense_tc_kernel"), (512, 0, "dense_tc_x_kernel"),
+                                          (256, 248, "dense_tc_kernel"), (256, 256, "dense_tc_x_kernel")])
+def test_dense_tc_kernel_chosen_by_depth(f1, f2, kernel):
+    """cbrs_dense_tc runs dense_tc_x_kernel from f1 + f2 = 512 up and dense_tc_kernel below, whatever the split"""
+    from deep_cbrs_amar_renaissance_b200 import ops
+    rng = np.random.RandomState(f1 + f2)
+    m, n = 300, 64
+    a = rng.standard_normal((m, f1 + f2)).astype(np.float32)
+    w = (rng.standard_normal((f1 + f2, n)) / np.sqrt(f1 + f2)).astype(np.float32)
+    b = (rng.standard_normal(n) * 0.1).astype(np.float32)
+    x1, x2 = cuda(a[:, :f1]), (cuda(a[:, f1:]) if f2 else None)
+    wd, bd = cuda(w), cuda(b)
+    torch.cuda.synchronize()
+    with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
+        got = ops.dense_tc(x1, wd, bd, "relu", x2=x2)
+        torch.cuda.synchronize()
+    names = {e.name for e in prof.events()}
+    ran = {k for k in ("dense_tc_kernel", "dense_tc_x_kernel") if any(k in name for name in names)}
+    assert ran == {kernel}, sorted(name for name in names if "dense_tc" in name)
+    close(got.cpu().numpy(), oracle_dense_bf16(a, w, b, "relu"), "dense_tc %d + %d -> %d" % (f1, f2, n))
 
 
 def test_dense_tc_refuses_what_it_cannot_take():
@@ -130,13 +160,3 @@ def test_hybrid_scorer_on_tensor_cores():
     x2 = stack(np.concatenate([ub, ib], 1), w["dense3b"])
     want = stack(np.concatenate([x1, x2], 1), w["clf"], last="sigmoid")
     close(got, want, "bf16 hybrid scores", rtol=2e-3)   # bf16 re-rounding of near-tie activations between layers
-
-
-@pytest.mark.parametrize("variant", ["3", "4"])
-def test_each_kernel_variant_on_every_shape(variant):
-    """cbrs_dense_tc picks one of two kernels by depth (dense_tc.cu / dense_tc_x.cu); the same parity cases with each
-    kernel forced on every shape (CBRS_DENSE_TC_VARIANT is read once per process, hence the child process)"""
-    env = dict(os.environ, CBRS_DENSE_TC_VARIANT=variant)
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-q", "-x", "-k",
-                        "single_source or gather_concat or hybrid_scorer"], env=env, capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
