@@ -80,6 +80,9 @@ _SIGS = {
     "cbrs_gather_rows": (c_int, [P, c_int64, P, c_int64, c_int32, P, c_int64, P]),
     "cbrs_topk_rows": (c_int, [P, c_int64, c_int64, c_int32, c_int32, P, P, P]),
     "cbrs_exclude_cols": (c_int, [P, c_int64, c_int64, c_int32, c_int32, P, P, P]),
+    "cbrs_rank_metrics_workspace_bytes": (c_size_t, [c_int64, c_int32]),
+    "cbrs_rank_metrics": (c_int, [P, c_int64, c_int64, c_int32, c_int32, P, c_int64, P, P, POINTER(c_int32), c_int32, P, P,
+                                  P, c_size_t, P]),
     "cbrs_topk_pairs_workspace_bytes": (c_size_t, [c_int64]),
     "cbrs_topk_pairs": (c_int, [P, P, c_int64, c_int64, P, P, P, c_size_t, P]),
     "cbrs_score_catalog_topk": (c_int, [P, c_int64, P, c_int64, c_int64, c_int32, c_int32, P, P, c_int32, P, P, c_int32,

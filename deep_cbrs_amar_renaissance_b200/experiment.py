@@ -11,7 +11,8 @@ log callback (:172-188), evaluate -> predict -> per-user top-5 / top-10 written 
 predictions/top_<k>/predictions_1.tsv -> P/R/F1@k (:190-222), one failed experiment does not stop the others (:299-302).
 What is added, off unless a config sets the top-level key `catalog_metrics: true`: P/R/F1@k of full-catalog top-k lists
 (every item ranked for every user, the user's training items excluded) against the test ratings, reported as
-catalog_{precision,recall,f1}_at_{k}.
+catalog_{precision,recall,f1}_at_{k}; `catalog_metrics: all` adds catalog_{ndcg,map,hit_rate,mrr}_at_{k}.  The metrics
+are computed on the device from the lists and the test ratings (utilities.metrics.catalog_ranking_metrics).
 What is replaced: MLflow run management by a directory per run holding config.yaml, log.txt, metrics.json;
 ruamel.yaml by PyYAML with the YAML-1.2 float forms the files use (`1e-4`); the Java evaluator by
 utilities.metrics.top_k_metrics.
@@ -27,7 +28,6 @@ import time
 import traceback
 
 import numpy as np
-import pandas as pd
 import yaml
 
 from . import models  # noqa: F401  (model modules are looked up by name below)
@@ -38,7 +38,7 @@ from .models.hybrid import HybridBertGNN, HybridCBRS
 from .training import Adam
 from .utilities.keras import LogCallback, get_total_parameters
 from .scoring import ItemLists
-from .utilities.metrics import catalog_predictions, precision_recall_f1_at_k, top_k_metrics, top_k_predictions
+from .utilities.metrics import RANKING_METRICS, catalog_ranking_metrics, top_k_metrics, top_k_predictions
 from .utilities.utils import get_experiment_logger, make_grid, nested_dict_update
 
 PARAMS_PATH = 'config.yaml'
@@ -46,6 +46,7 @@ EXPERIMENTS_PATH = 'experiments.yaml'
 RUNS_PATH = './runs'
 LOG_FREQUENCY = 100
 METRICS_TOP_KS = [5, 10]
+CATALOG_METRICS = ("precision", "recall", "f1")   # catalog_metrics: true; `all` reports every RANKING_METRICS entry
 
 
 class _Loader(yaml.SafeLoader):
@@ -100,7 +101,9 @@ class Experimenter:
         name = self.config.model.name
         module_name, class_name = name.split('.')
         self.model_class = getattr(importlib.import_module(models.__name__ + '.' + module_name), class_name)
-        self.catalog_metrics = bool(self.config.get('catalog_metrics'))
+        catalog = self.config.get('catalog_metrics')
+        self.catalog_metrics = bool(catalog)
+        self.catalog_metric_names = RANKING_METRICS if catalog == 'all' else CATALOG_METRICS
         if self.catalog_metrics and not hasattr(self.model_class, 'recommend_top_k'):
             raise ValueError("catalog_metrics: {} scores pre-computed embedding rows and has no full-catalog top-k "
                              "(recommend_top_k); use a graph model".format(name))
@@ -177,29 +180,30 @@ class Experimenter:
             res = top_k_metrics(self.config.dataset.test_ratings_filepath, top_k_dest)[k]
             self.metrics.update({"precision_at_{}".format(k): res["precision"], "recall_at_{}".format(k): res["recall"],
                                  "f1_at_{}".format(k): res["f1"]})
-        prefixes = ("",)
+        rows = [("", m) for m in CATALOG_METRICS]
         if self.catalog_metrics:
             self.evaluate_catalog()
-            prefixes = ("", "catalog_")
+            rows += [("catalog_", m) for m in self.catalog_metric_names]
         table = "\n".join("{}{}@{}: {:.6f}".format(p, m, k, self.metrics["{}{}_at_{}".format(p, m, k)])
-                          for p in prefixes for m in ("precision", "recall", "f1") for k in METRICS_TOP_KS)
+                          for p, m in rows for k in METRICS_TOP_KS)
         self.logger.info('\n' + table)
         print('\n' + table)
 
     def evaluate_catalog(self):
-        """P/R/F1@k of each user's top-k over the WHOLE catalog, its training items excluded, against the test ratings
-        (the same RiVal restatement as the test-pair metrics)."""
+        """P/R/F1@k (with `catalog_metrics: all` also NDCG, MAP, hit rate and MRR @k) of each user's top-k over the WHOLE
+        catalog, its training items excluded, against the test ratings: the items a user rated >= 1 in the test set are
+        its relevant items, as in the RiVal restatement of the test-pair metrics.  Lists and relevance stay on the
+        device; one kernel computes every metric at both cutoffs."""
         users, items = self.trainset.users, self.trainset.items
         if isinstance(self.model, HybridBertGNN) and self.model.content_table is None:
             self.model.set_content_table(self.trainset.embeddings.embeddings)
         seen = ItemLists.from_ratings(self.trainset.ratings, len(users), len(items), device="cuda")
-        ids, vals = self.model.recommend_top_k(len(users), len(items), max(METRICS_TOP_KS), exclude=seen)
-        top = catalog_predictions(ids, vals, users, items)
-        test = pd.read_csv(self.config.dataset.test_ratings_filepath, sep='\t', header=None).to_numpy()
-        for k in METRICS_TOP_KS:
-            res = precision_recall_f1_at_k(test, top.to_numpy(), k)
-            self.metrics.update({"catalog_precision_at_{}".format(k): res["precision"],
-                                 "catalog_recall_at_{}".format(k): res["recall"], "catalog_f1_at_{}".format(k): res["f1"]})
+        ids, _ = self.model.recommend_top_k(len(users), len(items), max(METRICS_TOP_KS), exclude=seen)
+        # the loader maps every test id into the training vocabulary, so the test ratings index the same catalog
+        relevant = ItemLists.from_ratings(self.testset.ratings, len(users), len(items), device="cuda", min_rating=1,
+                                          distinct=True)
+        res = catalog_ranking_metrics(ids, relevant, cutoffs=METRICS_TOP_KS, metrics=self.catalog_metric_names)
+        self.metrics.update({"catalog_" + key: value for key, value in res.items() if key != "users"})
 
     def run(self):
         try:

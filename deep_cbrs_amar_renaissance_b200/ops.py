@@ -635,6 +635,52 @@ def exclude_cols(scores, col_base, exclude):
     return scores
 
 
+RANK_METRICS = ("precision", "recall", "hit_rate", "mrr", "ndcg", "map")   # the per-user columns of cbrs_rank_metrics
+
+
+def rank_metrics_cutoffs(ids, cutoffs):
+    """The cutoffs as a list of ints, or CbrsError (before any device work) unless ids is a 2-D int32 tensor with unit
+    column stride and cutoffs are 1..8 strictly ascending values in [1, k]."""
+    if not torch.is_tensor(ids) or ids.dim() != 2 or ids.dtype != torch.int32 or (ids.shape[1] > 1 and ids.stride(1) != 1):
+        raise L.CbrsError("rank_metrics: ids must be a 2-D int32 tensor with unit column stride")
+    k = ids.shape[1]
+    cutoffs = [int(c) for c in cutoffs]
+    if not cutoffs or len(cutoffs) > 8 or k > 128 or any(c < 1 or c > k for c in cutoffs) \
+            or any(b <= a for a, b in zip(cutoffs, cutoffs[1:])):
+        raise L.CbrsError("rank_metrics: cutoffs {} must be 1..8 strictly ascending values in [1, k = {}], k <= 128".format(
+            cutoffs, k))
+    return cutoffs
+
+
+def rank_metrics(ids, rel, users, cutoffs, per_user=False, n_items=None):
+    """Ranking metrics of top-k lists against per-user relevance lists (cbrs_rank_metrics), on the device.
+    ids [n_rows, k] int32 (row r = the list of users[r], or of user r when users is None; -1 = empty slot);
+    rel = (rowptr, items): CSR over global user ids, sorted distinct catalog indices per row; n_items: ids at or past it
+    never hit (default: no bound beyond the lists).  cutoffs: strictly ascending, each in [1, k], at most 8.
+    Returns (sums fp64 [n_cutoffs, 7] on the device: columns RANK_METRICS summed over the scored users with at least one
+    relevant item, then their count; per_user fp64 [n_rows, n_cutoffs, 6] (NaN for rows without one) or None)."""
+    cutoffs = rank_metrics_cutoffs(ids, cutoffs)
+    lib = L.load()
+    n_rows, k = ids.shape
+    ld = ids.stride(0) if n_rows > 1 else k
+    rowptr, items = rel
+    n_users = rowptr.numel() - 1
+    rp, it = _exclusion(rel, n_users)
+    if users is not None:
+        users = users.to(ids.device, torch.int64).contiguous()
+        if users.numel() != n_rows:
+            raise L.CbrsError("rank_metrics: {} users for {} lists".format(users.numel(), n_rows))
+    nc = len(cutoffs)
+    sums = torch.empty(nc, 7, dtype=torch.float64, device=ids.device)
+    pu = torch.empty(n_rows, nc, 6, dtype=torch.float64, device=ids.device) if per_user else None
+    ws = _ws(lib.cbrs_rank_metrics_workspace_bytes(n_rows, nc), ids.device)
+    L.check(lib.cbrs_rank_metrics(_ptr(ids), ld, n_rows, k, (1 << 31) - 1 if n_items is None else int(n_items),
+                                  _ptr(users, torch.int64), n_users, rp, it, (ctypes.c_int32 * nc)(*cutoffs), nc,
+                                  _ptr(sums), _ptr(pu), _ptr(ws), ws.numel(), _stream()), "cbrs_rank_metrics")
+    _count(2)
+    return sums, pu
+
+
 def topk_pairs(users, scores, n_users, k):
     """Rows of the pair list kept by the reference's per-user head(k), in (user asc, score desc) order."""
     lib = L.load()

@@ -39,23 +39,33 @@ class ItemLists:
         return self.rowptr.numel() - 1
 
     @classmethod
-    def from_ratings(cls, ratings, n_users, n_items, device=None):
-        """Seen items per user from the [R, >= 2] ratings format of a training set (`trainset.ratings`): column 0 the
-        user index, column 1 the item index offset by n_users.  Every row counts, whatever its rating: a rated item is
-        a seen item; a pair rated twice is listed twice.  Built on `device` (default: the tensor's own device, or CUDA
-        for a numpy array when one is present)."""
-        r = ratings if torch.is_tensor(ratings) else torch.as_tensor(np.asarray(ratings)[:, :2].astype(np.int64))
+    def from_ratings(cls, ratings, n_users, n_items, device=None, min_rating=None, distinct=False):
+        """Items per user from the [R, >= 2] ratings format of a dataset (`trainset.ratings`, `testset.ratings`): column
+        0 the user index, column 1 the item index offset by n_users, column 2 the rating.  Built on `device` (default:
+        the tensor's own device, or CUDA for a numpy array when one is present).
+        Defaults (the seen items of a training set): every row counts, whatever its rating: a rated item is a seen
+        item; a pair rated twice is listed twice.
+        min_rating: keep only the rows whose rating is >= min_rating (needs column 2).  distinct: one entry per
+        (user, item).  `min_rating=1, distinct=True` on test ratings gives the relevance sets of
+        utilities.metrics.precision_recall_f1_at_k, the input of catalog_ranking_metrics."""
+        arr = None if torch.is_tensor(ratings) else np.asarray(ratings)
+        r = ratings if arr is None else torch.as_tensor(arr[:, :2].astype(np.int64))
         if device is None:
-            device = r.device if torch.is_tensor(ratings) else ("cuda" if torch.cuda.is_available() else "cpu")
+            device = r.device if arr is None else ("cuda" if torch.cuda.is_available() else "cpu")
         if r.dim() != 2 or r.shape[1] < 2:
             raise ValueError("ItemLists.from_ratings: expected a [R, >= 2] ratings array")
+        if min_rating is not None:
+            if (ratings if arr is None else arr).shape[1] < 3:
+                raise ValueError("ItemLists.from_ratings: min_rating needs a rating column (column 2)")
+            rating = ratings[:, 2] if arr is None else torch.as_tensor(arr[:, 2].astype(np.float64))
+            r = r[rating >= min_rating]
         r = r[:, :2].to(device=device, dtype=torch.int64)
         user, item = r[:, 0], r[:, 1] - n_users
         if r.shape[0] and (bool((user < 0).any()) or bool((user >= n_users).any()) or bool((item < 0).any())
                            or bool((item >= n_items).any())):
             raise ValueError("ItemLists.from_ratings: user ids must lie in [0, {}) and item ids in [{}, {})".format(
                 n_users, n_users, n_users + n_items))
-        key = torch.sort(user * n_items + item).values
+        key = torch.unique(user * n_items + item) if distinct else torch.sort(user * n_items + item).values
         counts = torch.bincount(key // n_items, minlength=n_users)
         rowptr = torch.zeros(n_users + 1, dtype=torch.int64, device=device)
         torch.cumsum(counts, 0, out=rowptr[1:])

@@ -83,6 +83,47 @@ def precision_recall_f1_at_k(test_ratings, predictions, k, relevance_threshold=1
     return dict(precision=prec, recall=rec, f1=f1, users=len(ps))
 
 
+RANKING_METRICS = ("precision", "recall", "f1", "ndcg", "map", "hit_rate", "mrr")
+
+
+def catalog_ranking_metrics(ids, relevant, users=None, cutoffs=(5, 10), metrics=RANKING_METRICS, per_user=False):
+    """Full-ranking metrics of top-k lists at each cutoff, computed on the device (cbrs_rank_metrics): only the sums
+    come back to the host.
+
+    ids: CUDA int32 [n_rows, k], the lists of recommend_top_k (catalog indices, best first, -1 = empty slot); row r is
+    user users[r] (users: int64 [n_rows], distinct), or user r when users is None.
+    relevant: scoring.ItemLists over all users, e.g. ItemLists.from_ratings(testset.ratings, ..., min_rating=1,
+    distinct=True).  Binary relevance; the definitions are those above cbrs_rank_metrics in include/cbrs_b200.h.
+
+    As in precision_recall_f1_at_k (RiVal 0.2): every mean is over ALL users with at least one relevant item, those
+    that were not scored counting 0; F1 = 2PR / (P + R) of the means.
+    Returns {"<metric>_at_<c>": float} for each metric of `metrics` (names in RANKING_METRICS) and cutoff, "users": the
+    number of users with a relevant item, and with per_user=True "per_user": fp64 [n_rows, n_cutoffs, 6] of the columns
+    ops.RANK_METRICS per scored row (NaN for a row without relevant items) for paired comparisons."""
+    from ..scoring import ItemLists
+    metrics = tuple(metrics)
+    unknown = [m for m in metrics if m not in RANKING_METRICS]
+    if unknown:
+        raise ValueError("unknown ranking metrics {}; known: {}".format(unknown, RANKING_METRICS))
+    if not isinstance(relevant, ItemLists):
+        raise TypeError("relevant must be an ItemLists")
+    cutoffs = ops.rank_metrics_cutoffs(ids, cutoffs)
+    rowptr, items = relevant.rowptr.to(ids.device), relevant.items.to(ids.device)
+    sums, pu = ops.rank_metrics(ids, (rowptr, items), users, cutoffs, per_user=per_user, n_items=relevant.n_items)
+    n_rel = int((rowptr[1:] > rowptr[:-1]).sum())
+    sums = sums.cpu().numpy()
+    out = {}
+    for ci, c in enumerate(cutoffs):
+        mean = {m: float(sums[ci, j]) / n_rel if n_rel else 0.0 for j, m in enumerate(ops.RANK_METRICS)}
+        p, r = mean["precision"], mean["recall"]
+        mean["f1"] = 2 * p * r / (p + r) if p + r > 0 else 0.0
+        out.update({"{}_at_{}".format(m, c): mean[m] for m in metrics})
+    out["users"] = n_rel
+    if per_user:
+        out["per_user"] = pu
+    return out
+
+
 def top_k_metrics(test_filepath, predictions_path, relevance_threshold=1, sep='\t'):
     """Same directory walk as the reference (metrics.py:37-80): every `top_<k>` directory holding
     predictions*.tsv gets a results.tsv with Precision / Recall / F1 at that cutoff (averaged over the

@@ -355,6 +355,32 @@ int cbrs_score_catalog_topk_ex(const float *P, int64_t ldp, const float *Q, int6
                                const float *w3, const float *b3, int32_t k, int32_t *ids_out, float *scores_out,
                                const int64_t *excl_rowptr, const int32_t *excl_items, void *stream);
 
+/* ---- full-catalog ranking metrics of top-k lists (binary relevance) -------------------------------------------------
+ * ids [n_rows, k] int32, leading dimension ld >= k: row r is the top-k list of user users[r] (users null: user r), best
+ * first, as the catalog scorers write it.  -1 marks an empty slot; no value outside [0, n_items) is ever a hit.
+ * Relevance lists: rel_rowptr int64 [n_users + 1] / rel_items int32, the CSR form of the exclusion lists above, but rows
+ * are GLOBAL user ids (row u = user u, whichever rows are scored).  Each row is sorted ascending, distinct, catalog
+ * indices.  An unsorted or duplicated row may lose hits (a duplicate also counts in R_u); it never causes a read
+ * outside [rel_rowptr[u], rel_rowptr[u + 1]).  A user outside [0, n_users), or both pointers null, has no relevant
+ * items.  Exactly one of the two pointers null: CBRS_E_INVALID.
+ * cutoffs_host: n_cutoffs (1..8) strictly ascending cutoffs c in [1, k], host memory; k <= 128.
+ * Per scored user with R_u = |rel_u| >= 1, hit_r = (slot r is in rel_u), at each cutoff c:
+ *   P = sum_{r<c} hit_r / c            R = sum_{r<c} hit_r / R_u            HR = 1 if any hit_r with r < c
+ *   MRR = 1 / (r + 1) of the first hit at r < c, else 0
+ *   NDCG = DCG / IDCG, DCG = sum_{r<c} hit_r / log2(r + 2), IDCG = sum_{r<min(c, R_u)} 1 / log2(r + 2)
+ *   AP = sum_{r<c} hit_r * (sum_{s<=r} hit_s) / (r + 1) / min(c, R_u)
+ * sums_out fp64 [n_cutoffs, 7] (device): columns P, R, HR, MRR, NDCG, AP summed over the scored users with R_u >= 1,
+ * and column 6 the number of those users.  Rows without relevant items add nothing.  The sums are bit-identical from
+ * run to run and do not depend on ld: the rows are added in a fixed tree over fixed blocks of rows.
+ * per_user_out fp64 [n_rows, n_cutoffs, 6] (may be null): the six values of row r; NaN for a row with R_u = 0.
+ * Workspace: cbrs_rank_metrics_workspace_bytes(n_rows, n_cutoffs) bytes, 8-byte aligned, else CBRS_E_WORKSPACE.
+ * Every argument is checked before any launch.                                                                      */
+size_t cbrs_rank_metrics_workspace_bytes(int64_t n_rows, int32_t n_cutoffs);
+int cbrs_rank_metrics(const int32_t *ids, int64_t ld, int64_t n_rows, int32_t k, int32_t n_items, const int64_t *users,
+                      int64_t n_users, const int64_t *rel_rowptr, const int32_t *rel_items, const int32_t *cutoffs_host,
+                      int32_t n_cutoffs, double *sums_out, double *per_user_out, void *workspace,
+                      size_t workspace_bytes, void *stream);
+
 /* The same scorer with the 64 x 64 product on the tensor cores at fp32 accuracy (3xTF32: h = relu(P[u]+Q[i]) and W2 are
  * split into a tf32 part and an exact remainder, three kind::tf32 MMAs per K step accumulate in fp32; the A operand is
  * written by its threads straight into tensor memory).  Same contract, outputs and tie rule as cbrs_score_catalog_topk;
