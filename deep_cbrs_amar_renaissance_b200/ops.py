@@ -563,7 +563,10 @@ def gather_rows(x, idx, out=None):
 
 def push_rows(view, buf):
     """Store the finished row block `view` (a view into the local copy of the SymmetricBuffer `buf`) into every rank's copy:
-    one coalesced pass to the NVSwitch multicast mapping when the buffer has one, else one per peer (cbrs_push_rows)."""
+    one coalesced pass to the NVSwitch multicast mapping when the buffer has one, else one per peer (cbrs_push_rows).
+    An empty block stores nothing (torch gives it no address inside the buffer)."""
+    if view.numel() == 0:
+        return
     lib = L.load()
     v = view if view.dim() == 2 else view.reshape(-1, 1)
     v, ld = _rowmajor(v)
@@ -582,9 +585,12 @@ def push_rows(view, buf):
 
 
 def peer_copy(dst_addr, src):
-    """copy-engine transfer of a contiguous tensor into a peer-mapped address (cbrs_peer_copy)"""
+    """copy-engine transfer of a contiguous tensor into a peer-mapped address (cbrs_peer_copy); an empty tensor (which
+    torch gives a null address) moves nothing"""
     if not src.is_contiguous():
         raise L.CbrsError("peer_copy: source must be contiguous")
+    if src.numel() == 0:
+        return
     if PROFILE_ON:
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
