@@ -148,6 +148,11 @@ _SIGS = {
     "cbrs_gat_backward_workspace_bytes": (c_size_t, [c_int64]),
     "cbrs_gat_backward": (c_int, [POINTER(CsrDesc), P, c_int64, P, P, P, c_int64, P, P, c_int64, c_int32, P, P, P, c_int64,
                                   P, P, P, c_size_t, P]),
+    "cbrs_gat_backward_stats_rows": (c_int, [POINTER(CsrDesc), c_int64, P, P, P, c_int64, P, P, c_int64, c_int32, P,
+                                             POINTER(c_void_p), c_int, P]),
+    "cbrs_gat_backward_grad_rows": (c_int, [POINTER(CsrDesc), c_int64, P, c_int64, P, P, P, c_int64, c_int32, P, P, P,
+                                            P, c_int64, P, P, POINTER(c_void_p), POINTER(c_void_p), POINTER(c_void_p),
+                                            c_int, P]),
     "cbrs_adam_step_multi": (c_int, [c_int32, POINTER(c_void_p), POINTER(c_void_p), POINTER(c_void_p), POINTER(c_void_p),
                                      POINTER(c_int64), POINTER(c_float), c_float, P, c_float, c_float, c_float, P]),
     "cbrs_synth_bipartite": (c_int, [c_int64, c_int64, c_int64, c_uint64, P, P, P]),

@@ -167,9 +167,203 @@ __global__ void gat_bwd_combine_kernel(float *__restrict__ dz, int64_t lddz, con
     dz[r * lddz + c] = fmaf(dq[r], a_neigh[c], fmaf(dp[r], a_self[c], dz[r * lddz + c]));
 }
 
+// ---- row-slice form for the row partition (cbrs_gat_backward_stats_rows / cbrs_gat_backward_grad_rows) ----------
+// The same per-row arithmetic as the two kernels above, on rows [row_offset, row_offset + n_rows) of a graph whose
+// column ids are global, so every output row has the bits of the whole-graph call.  Inputs are whole-graph arrays read
+// at global rows; outputs are views of the slice's rows (as in cbrs_gat_csr).  The stats live in a caller-owned [N, 3]
+// array (m, S, t) instead of the workspace: the rows phase reads the stats of neighbour rows, which another rank
+// computed and stored into this rank's copy.  The combine (dz += dp a_self + dq a_neigh) is folded into the rows
+// kernel's epilogue with the operand order of gat_bwd_combine_kernel, so no kernel reads back an output (an output may
+// be a multicast address).
+struct GatBwdSliceParams {
+    const int64_t *rowptr;
+    const int32_t *colidx;
+    int64_t n_rows, row_offset;
+    const float *z; int64_t ldz;
+    const float *p; const float *q;
+    const float *y; int64_t ldy;
+    const float *bias;
+    const float *d_o; int64_t ldo;
+    int32_t h;
+    const float *stats_in;            // [N, 3], read by the rows phase
+    float *stats;                     // [n_rows, 3], written by the stats phase
+    const float *a_self; const float *a_neigh;
+    float *dp; float *dq;             // [n_rows]
+    float *dz; int64_t lddz;          // [n_rows, h]
+    float *stats_peer[CBRS_MAX_PEERS - 1];
+    float *dp_peer[CBRS_MAX_PEERS - 1];
+    float *dq_peer[CBRS_MAX_PEERS - 1];
+    float *dz_peer[CBRS_MAX_PEERS - 1];
+    int n_peer;
+};
+
+__global__ void __launch_bounds__(256) gat_bwd_stats_slice_kernel(const GatBwdSliceParams p) {
+    const int64_t row = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (row >= p.n_rows) return;
+    const int64_t g = row + p.row_offset;
+    const int64_t b = p.rowptr[row], e = p.rowptr[row + 1];
+    const float pi = p.p[g];
+    float m = lrelu02(pi + p.q[g]);
+    for (int64_t k = b + lane; k < e; k += 32) {
+        const int c = p.colidx[k];
+        if (c != g) m = fmaxf(m, lrelu02(pi + p.q[c]));
+    }
+    m = warp_max(m);
+    float s = 0.f;
+    for (int64_t k = b + lane; k < e; k += 32) {
+        const int c = p.colidx[k];
+        if (c != g) s += expf(lrelu02(pi + p.q[c]) - m);
+    }
+    s = warp_sum(s) + expf(lrelu02(pi + p.q[g]) - m);
+    float t = 0.f;
+    for (int c = lane; c < p.h; c += 32) {
+        const float gr = p.d_o[g * p.ldo + c];
+        if (gr != 0.f) t = fmaf(gr, p.y[g * p.ldy + c] - (p.bias ? p.bias[c] : 0.f), t);
+    }
+    t = warp_sum(t);
+    if (lane < 3) {
+        const float v = lane == 0 ? m : (lane == 1 ? s + 1e-9f : t);
+        p.stats[row * 3 + lane] = v;
+        for (int r = 0; r < p.n_peer; ++r) p.stats_peer[r][row * 3 + lane] = v;
+    }
+}
+
+__global__ void __launch_bounds__(256) gat_bwd_rows_slice_kernel(const GatBwdSliceParams p, int vec4) {
+    const int64_t row = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (row >= p.n_rows) return;
+    const int64_t g = row + p.row_offset;
+    const int64_t b = p.rowptr[row], e = p.rowptr[row + 1];
+    const int64_t n_edges = e - b + 1;
+    const float p_r = p.p[g], q_r = p.q[g];
+    const float m_r = p.stats_in[g * 3], s_r = p.stats_in[g * 3 + 1], t_r = p.stats_in[g * 3 + 2];
+    const float *do_r = p.d_o + g * p.ldo;
+    const float *z_r = p.z + g * p.ldz;
+    float dp_lane = 0.f, dq_lane = 0.f;
+    float acc[kGatBwdMaxAcc];
+#pragma unroll
+    for (int k = 0; k < kGatBwdMaxAcc; ++k) acc[k] = 0.f;
+    for (int64_t base = 0; base < n_edges; base += 32) {
+        const int64_t k = base + lane;
+        int c = -1;
+        float coef = 0.f;
+        if (k < n_edges) {
+            c = k < n_edges - 1 ? p.colidx[b + k] : (int)g;
+            if (k < n_edges - 1 && c == g) c = -1;
+        }
+        if (c >= 0) {
+            const float s_a = p_r + p.q[c];
+            const float alpha_a = expf(lrelu02(s_a) - m_r) / s_r;
+            const float dal_a = row_dot(do_r, p.z + (int64_t)c * p.ldz, p.h, vec4);
+            dp_lane += alpha_a * (dal_a - t_r) * (s_a > 0.f ? 1.f : 0.2f);
+            const float s_b = p.p[c] + q_r;
+            coef = expf(lrelu02(s_b) - p.stats_in[(int64_t)c * 3]) / p.stats_in[(int64_t)c * 3 + 1];
+            const float dal_b = row_dot(p.d_o + (int64_t)c * p.ldo, z_r, p.h, vec4);
+            dq_lane += coef * (dal_b - p.stats_in[(int64_t)c * 3 + 2]) * (s_b > 0.f ? 1.f : 0.2f);
+        }
+        const int cnt = n_edges - base < 32 ? (int)(n_edges - base) : 32;
+        for (int u = 0; u < cnt; ++u) {
+            const int cu = __shfl_sync(0xffffffffu, c, u);
+            const float au = __shfl_sync(0xffffffffu, coef, u);
+            if (cu < 0) continue;
+            const float *src = p.d_o + (int64_t)cu * p.ldo;
+#pragma unroll
+            for (int k2 = 0; k2 < kGatBwdMaxAcc; ++k2) {
+                const int col = lane + 32 * k2;
+                if (col < p.h) acc[k2] = fmaf(au, src[col], acc[k2]);
+            }
+        }
+    }
+    // the xor butterfly leaves the same sum in every lane, so each lane can apply the combine itself
+    dp_lane = warp_sum(dp_lane);
+    dq_lane = warp_sum(dq_lane);
+    if (lane == 0) {
+        p.dp[row] = dp_lane;
+        p.dq[row] = dq_lane;
+        for (int r = 0; r < p.n_peer; ++r) {
+            p.dp_peer[r][row] = dp_lane;
+            p.dq_peer[r][row] = dq_lane;
+        }
+    }
+#pragma unroll
+    for (int k2 = 0; k2 < kGatBwdMaxAcc; ++k2) {
+        const int col = lane + 32 * k2;
+        if (col < p.h) {
+            const float v = fmaf(dq_lane, p.a_neigh[col], fmaf(dp_lane, p.a_self[col], acc[k2]));
+            p.dz[row * p.lddz + col] = v;
+            for (int r = 0; r < p.n_peer; ++r) p.dz_peer[r][row * p.lddz + col] = v;
+        }
+    }
+}
+
 }  // namespace cbrs
 
 using namespace cbrs;
+
+// copies a host list of n peer addresses into dst[CBRS_MAX_PEERS - 1]; false when the list or an entry is null
+static bool take_peers(float **dst, void *const *host, int n) {
+    for (int r = 0; r < CBRS_MAX_PEERS - 1; ++r) dst[r] = nullptr;
+    if (n > 0 && !host) return false;
+    for (int r = 0; r < n; ++r) {
+        dst[r] = (float *)host[r];
+        if (!dst[r]) return false;
+    }
+    return true;
+}
+
+extern "C" int cbrs_gat_backward_stats_rows(const cbrs_csr_t *g, int64_t row_offset, const float *pvec,
+                                            const float *qvec, const float *y, int64_t ldy, const float *bias,
+                                            const float *d_o, int64_t ldo, int32_t h, float *stats,
+                                            void *const *stats_peers_host, int n_peers, void *stream) {
+    CBRS_REQUIRE(g && pvec && qvec && y && d_o && stats, CBRS_E_INVALID, "gat_backward_stats_rows: null argument");
+    CBRS_REQUIRE(h > 0 && ldy >= h && ldo >= h && row_offset >= 0, CBRS_E_INVALID,
+                 "gat_backward_stats_rows: h=%d ldy=%lld ldo=%lld row_offset=%lld", h, (long long)ldy, (long long)ldo,
+                 (long long)row_offset);
+    CBRS_REQUIRE(n_peers >= 0 && n_peers < CBRS_MAX_PEERS, CBRS_E_INVALID,
+                 "gat_backward_stats_rows: n_peers=%d (at most %d peer copies)", n_peers, CBRS_MAX_PEERS - 1);
+    CBRS_REQUIRE(g->n_rows >= 0 && (g->n_rows == 0 || g->rowptr) && (g->nnz == 0 || g->colidx), CBRS_E_INVALID,
+                 "gat_backward_stats_rows: bad graph descriptor");
+    GatBwdSliceParams p = {};
+    CBRS_REQUIRE(take_peers(p.stats_peer, stats_peers_host, n_peers), CBRS_E_INVALID,
+                 "gat_backward_stats_rows: null peer copy");
+    if (g->n_rows == 0) return CBRS_OK;
+    p.rowptr = g->rowptr; p.colidx = g->colidx; p.n_rows = g->n_rows; p.row_offset = row_offset;
+    p.p = pvec; p.q = qvec; p.y = y; p.ldy = ldy; p.bias = bias; p.d_o = d_o; p.ldo = ldo; p.h = h;
+    p.stats = stats; p.n_peer = n_peers;
+    gat_bwd_stats_slice_kernel<<<(unsigned)cdiv(g->n_rows * 32, 256), 256, 0, (cudaStream_t)stream>>>(p);
+    CBRS_CHECK_LAUNCH("gat_bwd_stats_slice");
+    return CBRS_OK;
+}
+
+extern "C" int cbrs_gat_backward_grad_rows(const cbrs_csr_t *g, int64_t row_offset, const float *z, int64_t ldz,
+                                           const float *pvec, const float *qvec, const float *d_o, int64_t ldo,
+                                           int32_t h, const float *stats, const float *a_self, const float *a_neigh,
+                                           float *dz, int64_t lddz, float *dp, float *dq, void *const *dz_peers_host,
+                                           void *const *dp_peers_host, void *const *dq_peers_host, int n_peers,
+                                           void *stream) {
+    CBRS_REQUIRE(g && z && pvec && qvec && d_o && stats && a_self && a_neigh && dz && dp && dq, CBRS_E_INVALID,
+                 "gat_backward_grad_rows: null argument");
+    CBRS_REQUIRE(h > 0 && h <= 32 * kGatBwdMaxAcc && ldz >= h && ldo >= h && lddz >= h && row_offset >= 0,
+                 CBRS_E_INVALID, "gat_backward_grad_rows: h=%d (max %d), a leading dimension or row_offset is bad", h,
+                 32 * kGatBwdMaxAcc);
+    CBRS_REQUIRE(n_peers >= 0 && n_peers < CBRS_MAX_PEERS, CBRS_E_INVALID,
+                 "gat_backward_grad_rows: n_peers=%d (at most %d peer copies)", n_peers, CBRS_MAX_PEERS - 1);
+    CBRS_REQUIRE(g->n_rows >= 0 && (g->n_rows == 0 || g->rowptr) && (g->nnz == 0 || g->colidx), CBRS_E_INVALID,
+                 "gat_backward_grad_rows: bad graph descriptor");
+    GatBwdSliceParams p = {};
+    CBRS_REQUIRE(take_peers(p.dz_peer, dz_peers_host, n_peers) && take_peers(p.dp_peer, dp_peers_host, n_peers) &&
+                     take_peers(p.dq_peer, dq_peers_host, n_peers),
+                 CBRS_E_INVALID, "gat_backward_grad_rows: null peer copy");
+    if (g->n_rows == 0) return CBRS_OK;
+    p.rowptr = g->rowptr; p.colidx = g->colidx; p.n_rows = g->n_rows; p.row_offset = row_offset;
+    p.z = z; p.ldz = ldz; p.p = pvec; p.q = qvec; p.d_o = d_o; p.ldo = ldo; p.h = h; p.stats_in = stats;
+    p.a_self = a_self; p.a_neigh = a_neigh; p.dz = dz; p.lddz = lddz; p.dp = dp; p.dq = dq; p.n_peer = n_peers;
+    const int vec4 = (h % 4 == 0) && (ldz % 4 == 0) && (ldo % 4 == 0) && ((uintptr_t)z % 16 == 0) && ((uintptr_t)d_o % 16 == 0);
+    gat_bwd_rows_slice_kernel<<<(unsigned)cdiv(g->n_rows * 32, 256), 256, 0, (cudaStream_t)stream>>>(p, vec4);
+    CBRS_CHECK_LAUNCH("gat_bwd_rows_slice");
+    return CBRS_OK;
+}
 
 extern "C" size_t cbrs_gat_backward_workspace_bytes(int64_t n_rows) {
     return 3 * align_up((size_t)n_rows * sizeof(float)) + 256;

@@ -429,6 +429,69 @@ class RowPartition:
             self._sym[key] = (sb, sb.matrix(n, w, dtype))
         return self._sym[key]
 
+    @staticmethod
+    def _targets(sb, view):
+        """keyword arguments for the sparse kernels that make their stores of `view` reach every rank's copy of the
+        SymmetricBuffer `sb`: one store to the multicast mapping when the buffer has one, else a store per peer copy"""
+        mc = sb.mc_addr(view)
+        return {"mc": mc} if mc else {"peers": sb.peer_addrs(view)}
+
+    # ------------------------------------------------------------------ training (row-split sparse products)
+    def buffer(self, key, rows, w):
+        """[rows, w] float32 output buffer for sparse_rows, kept across steps: symmetric under the peer exchange"""
+        if self.heap is not None:
+            return self._symbuf(("train",) + tuple(key), rows, w)[1]
+        return self._buf(("train",) + tuple(key), rows, w, torch.device("cuda", torch.cuda.current_device()))
+
+    def _owner(self, view):
+        for sb, _ in self._sym.values():
+            if sb.local <= view.data_ptr() < sb.local + sb.nbytes:
+                return sb
+        raise ValueError("sparse_rows: output is not a view of a RowPartition.buffer")
+
+    def sparse_rows(self, csr, outs, launch):
+        """Run a sparse product on this rank's rows of the operator `csr` and leave every output complete on every rank.
+
+        csr: a whole operator (a graph view or its transpose) of G*N rows, N = the partitioned node count; the stacked
+        transpose of the relational operator has one group of N rows per relation, and this rank owns its row blocks of
+        every group.  outs: [G*N, w] views of RowPartition.buffer tensors, one per kernel output.
+        launch(sl, views, targets) launches the kernel on the row slice `sl` (global column ids, sl.row_offset = its
+        first row) with views[k] = outs[k][its rows] and targets[k] = the keyword arguments (peers= / mc=) that make
+        output k's stores reach the other ranks.  Under the peer exchange those stores are the exchange: a flag barrier
+        before (no rank still reads a copy from an earlier use of the buffers) and one after (every row has landed).
+        Under "nccl" the kernel writes own rows and exchange_rows moves them.  Row results do not depend on the
+        slicing, so every output equals the single-GPU product bit for bit."""
+        n = sum(self.n_rows_by_type)
+        if csr.n_rows % n or any(o.shape[0] != csr.n_rows for o in outs):
+            raise ValueError("sparse_rows: operator of {} rows, outputs of {} rows, {} nodes".format(
+                csr.n_rows, [o.shape[0] for o in outs], n))
+        key = ("rows", id(csr))
+        if key not in self._slices:
+            self._slices[key] = (csr, [csr.row_slice(g * n + a, g * n + b)
+                                       for g in range(csr.n_rows // n) for a, b in self.mine])
+        slices = self._slices[key][1]
+        peer = self.heap is not None
+        owners = [self._owner(o) for o in outs] if peer else None
+        if peer:
+            self.heap.barrier()
+        for sl in slices:
+            a, b = sl.row_offset, sl.row_offset + sl.n_rows
+            views = [o[a:b] for o in outs]
+            launch(sl, views, [self._targets(sb, v) for sb, v in zip(owners, views)] if peer else [{}] * len(outs))
+        if peer:
+            self.heap.barrier()
+            return outs
+        for o in outs:
+            for g in range(csr.n_rows // n):
+                blk = o[g * n:(g + 1) * n]
+                if blk.is_contiguous():
+                    self._exchange(blk)
+                else:   # a column slice (the 'concatenation' buffer): the collectives move contiguous rows
+                    tmp = blk.contiguous()
+                    self._exchange(tmp)
+                    blk.copy_(tmp)
+        return outs
+
     def _type_of(self, a):
         base = 0
         for t, cnt in enumerate(self.n_rows_by_type):
@@ -496,12 +559,7 @@ class RowPartition:
                 return osb.peer_addrs(view) if (everywhere or is_final(a)) else None
 
             def out_targets(view, a):
-                """keyword arguments for the sparse kernels: one store to the multicast mapping when the buffer has
-                one, else a store per peer copy"""
-                if not (everywhere or is_final(a)):
-                    return {}
-                mc = osb.mc_addr(view)
-                return {"mc": mc} if mc else {"peers": osb.peer_addrs(view)}
+                return self._targets(osb, view) if (everywhere or is_final(a)) else {}
 
             if isinstance(layer, GCNConv) and self.pipeline == "replicate":
                 # Every rank computes the WHOLE transform Z = X W itself (2.5 ms for 1.1e7 x 128 x 128 on the tensor

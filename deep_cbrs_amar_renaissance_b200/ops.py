@@ -192,14 +192,19 @@ def spmm_gcn_fused(csr, z, out, bias, relu, w_next, z_next, y_peers=None, z_peer
     return out
 
 
-def gat(csr, z, p, q, out, bias=None, relu=True, row_offset=0, workspace=None, peers=None):
+def gat(csr, z, p, q, out, bias=None, relu=True, row_offset=0, workspace=None, peers=None, mc=None):
+    """mc: as for spmm, the multicast address of `out` (the kernel only stores to its output)"""
     lib = L.load()
     z, ldz = _rowmajor(z)
     out, ldy = _rowmajor(out)
     h = z.shape[1]
     need = lib.cbrs_gat_workspace_bytes(ctypes.byref(csr.desc), h)
     ws = workspace if workspace is not None and workspace.numel() >= need else _ws(need, z.device)
-    if peers:
+    if mc:
+        L.check(lib.cbrs_gat_csr(ctypes.byref(csr.desc), row_offset, _ptr(z), ldz, _ptr(p, torch.float32),
+                                 _ptr(q, torch.float32), ctypes.c_void_p(int(mc)), ldy, h, _ptr(bias, torch.float32),
+                                 1 if relu else 0, _ptr(ws), ws.numel(), _stream()), "cbrs_gat_csr")
+    elif peers:
         L.check(lib.cbrs_gat_csr_bcast(ctypes.byref(csr.desc), row_offset, _ptr(z), ldz, _ptr(p, torch.float32),
                                        _ptr(q, torch.float32), _ptr(out), ldy, h, _ptr(bias, torch.float32),
                                        1 if relu else 0, _ptr_array(peers), len(peers), _ptr(ws), ws.numel(),
@@ -995,6 +1000,61 @@ def gat_backward(csr, z, p, q, y, bias, d_o, a_self, a_neigh):
                                   _ptr(a_self, torch.float32), _ptr(a_neigh, torch.float32), _ptr(dz), h, _ptr(dp),
                                   _ptr(dq), _ptr(ws), ws.numel(), _stream()), "cbrs_gat_backward")
     _count(3)
+    return dz, dp, dq
+
+
+def _out_targets(out, targets, what):
+    """(address the kernel stores `out` to, host array of peer addresses, peer count) for one output of a row-slice
+    kernel: targets = None / {} (local only), {"peers": [addresses]} or {"mc": multicast address}"""
+    targets = targets or {}
+    if targets.get("mc"):
+        return ctypes.c_void_p(int(targets["mc"])), None, 0
+    peers = targets.get("peers") or []
+    if len(peers) >= L.MAX_PEERS:
+        raise L.CbrsError("{}: {} peer copies (at most {})".format(what, len(peers), L.MAX_PEERS - 1))
+    return _ptr(out), (_ptr_array(peers) if peers else None), len(peers)
+
+
+def gat_backward_stats_rows(csr, p, q, y, bias, d_o, stats, peers=None, mc=None):
+    """Phase 1 of gat_backward on the row slice `csr` (rows csr.row_offset + [0, n_rows)): (m, S, t) of its rows into
+    `stats` ([n_rows, 3] view) and into the peers' copies (or once, to the multicast address `mc`) - cbrs_gat_backward_stats_rows.
+    p, q [N], y, d_o [N, h] are whole-graph tensors."""
+    lib = L.load()
+    y, ldy = _rowmajor(y)
+    d_o, ldo = _rowmajor(d_o)
+    stats, _ = _rowmajor(stats)
+    if tuple(stats.shape) != (csr.n_rows, 3) or not stats.is_contiguous():
+        raise L.CbrsError("gat_backward_stats_rows: stats must be a contiguous [{}, 3] view".format(csr.n_rows))
+    dst, arr, n_peers = _out_targets(stats, {"peers": peers, "mc": mc}, "gat_backward_stats_rows")
+    L.check(lib.cbrs_gat_backward_stats_rows(ctypes.byref(csr.desc), csr.row_offset, _ptr(p, torch.float32),
+                                             _ptr(q, torch.float32), _ptr(y), ldy, _ptr(bias, torch.float32), _ptr(d_o),
+                                             ldo, y.shape[1], dst, arr, n_peers, _stream()),
+            "cbrs_gat_backward_stats_rows")
+    _count(1)
+    return stats
+
+
+def gat_backward_grad_rows(csr, z, p, q, d_o, stats, a_self, a_neigh, dz, dp, dq, targets=None):
+    """Phase 2 of gat_backward on the row slice `csr`: dz ([n_rows, h] view, the dp/dq terms included), dp, dq
+    ([n_rows, 1] views) of its rows - cbrs_gat_backward_grad_rows.  `stats` is the whole [N, 3] array of phase 1.
+    targets: None, or one dict per output (dz, dp, dq) as for _out_targets; every output takes the same kind."""
+    lib = L.load()
+    z, ldz = _rowmajor(z)
+    d_o, ldo = _rowmajor(d_o)
+    dz, lddz = _rowmajor(dz)
+    h = z.shape[1]
+    if dz.shape[1] != h or not all(t.shape[0] == csr.n_rows and t.numel() == csr.n_rows for t in (dp, dq)):
+        raise L.CbrsError("gat_backward_grad_rows: outputs do not match the slice's {} rows".format(csr.n_rows))
+    targets = list(targets) if targets else [None] * 3
+    outs = [_out_targets(t, tg, "gat_backward_grad_rows") for t, tg in zip((dz, dp, dq), targets)]
+    if len({o[2] for o in outs}) != 1:
+        raise L.CbrsError("gat_backward_grad_rows: dz, dp and dq need the same number of peer copies")
+    L.check(lib.cbrs_gat_backward_grad_rows(ctypes.byref(csr.desc), csr.row_offset, _ptr(z), ldz, _ptr(p, torch.float32),
+                                            _ptr(q, torch.float32), _ptr(d_o), ldo, h, _ptr(stats, torch.float32),
+                                            _ptr(a_self, torch.float32), _ptr(a_neigh, torch.float32), outs[0][0], lddz,
+                                            outs[1][0], outs[2][0], outs[0][1], outs[1][1], outs[2][1], outs[0][2],
+                                            _stream()), "cbrs_gat_backward_grad_rows")
+    _count(1)
     return dz, dp, dq
 
 

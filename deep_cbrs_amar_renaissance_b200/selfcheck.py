@@ -196,3 +196,105 @@ def partition_parity(group=None, log=None, families=("BasicGCN", "BasicGraphSage
     dist.all_gather_object(gathered, failures, group=group)
     all_failures = sorted({f for fl in gathered for f in fl})
     return {"bit_identical": bool(int(flag.item()) == 1), "cases": cases, "failures": all_failures}
+
+
+def _train_model(name, adj, sizes, relational):
+    """a small model of family `name` with fixed weights (non-zero biases) and a compiled Adam"""
+    import zlib
+    from .models import hybrid
+    set_seed(31)
+    kw = dict(embedding_dim=16, final_node="concatenation")
+    if name == "HybridBertGCN":
+        m = hybrid.HybridBertGCN(adj, n_hiddens=[16, 16], dense_units=[[48, 48], [32, 32], [32, 32]], clf_units=[16, 16],
+                                 **kw)
+        m.build_weights(24)
+    else:
+        if name == "BasicLightGCN":
+            m = basic.BasicLightGCN(adj, n_layers=2, dense_units=[32, 16], clf_units=[16, 16], **kw)
+        else:
+            m = getattr(basic, name)(relational if name == "BasicRGCN" else adj, n_hiddens=[16, 16],
+                                     dense_units=[32, 16], clf_units=[16, 16], **kw)
+        m.build_weights()
+    with torch.no_grad():
+        for nm, w in m.named_weights():
+            if nm.endswith("bias"):
+                g = torch.Generator(w.device).manual_seed(zlib.crc32(nm.encode()) % 1000)
+                w.copy_(torch.randn(w.shape, device=w.device, generator=g) * 0.05)
+    m.compile(loss="binary_crossentropy", optimizer={"learning_rate": 1e-2})
+    return m
+
+
+def _train_steps(model, name, sizes, steps=3):
+    """`steps` train_on_batch calls on the same seeded batches on every rank -> host copies of (losses, weights,
+    Adam m, Adam v)"""
+    rng = np.random.RandomState(11)
+    losses = []
+    for k in range(steps):
+        u = rng.randint(0, sizes[0], size=256)
+        i = rng.randint(0, sizes[1], size=256) + sizes[0]
+        y = (rng.rand(256) < 0.5).astype(np.float32)
+        x = (u, i)
+        if name == "HybridBertGCN":
+            g = torch.Generator("cuda").manual_seed(100 + k)
+            x = (u, i, torch.randn(256, 24, device="cuda", generator=g), torch.randn(256, 24, device="cuda", generator=g))
+        loss, _ = model.train_on_batch(x, y)
+        losses.append(loss.clone())
+    torch.cuda.synchronize()
+    st = model._adam._state
+    ws = list(model.weights)
+    return ([t.cpu() for t in losses], [w.detach().cpu().clone() for w in ws],
+            [st[id(w)][0].cpu() for w in ws if id(w) in st], [st[id(w)][1].cpu() for w in ws if id(w) in st])
+
+
+def training_parity(group=None, log=None, families=("BasicGCN", "BasicRGCN", "BasicLightGCN", "BasicGraphSage",
+                                                    "BasicGAT", "HybridBertGCN")):
+    """Collective.  The row-partitioned training step must equal the single-GPU step BIT FOR BIT: for each family,
+    three optimiser steps unpartitioned and then partitioned - peer stores and the NCCL all-gather, even and
+    edge-balanced cuts, the row-major and the column-blocked schedule - compared with torch.equal on the losses, every
+    weight (the embedding table included) and the Adam moments.  Returns {"bit_identical", "cases", "failures"} (the
+    same on every rank)."""
+    from .graph import DeviceGraph
+    rank, world = dist.get_rank(group), dist.get_world_size(group)
+    failures, cases = [], 0
+
+    def say(msg):
+        if log is not None and rank == 0:
+            log(msg)
+
+    n_users, n_items, n_props = 3001, 1999, 500
+    adj = small_graph(n_users, n_items, 60000, seed=23, n_props=n_props, n_links=4000, dup_links=300)
+    dev = torch.device("cuda", torch.cuda.current_device())
+    rel = ((adj.row >= n_users + n_items) | (adj.col >= n_users + n_items)).astype(np.int32)
+    t = lambda v, dt: torch.from_numpy(np.ascontiguousarray(v, dt)).to(dev)  # noqa: E731
+    sizes = [n_users, n_items, n_props]
+    for blocking in (None, (257, 40)):
+        G.FORCED_BLOCKING = blocking
+        try:
+            for name in families:
+                relational = DeviceGraph(t(adj.row, np.int32), t(adj.col, np.int32), t(adj.data, np.float32),
+                                         adj.shape[0], rel=t(rel, np.int32), n_rel=2)
+                want = _train_steps(_train_model(name, adj, sizes, relational), name, sizes)
+                for exchange in ("peer", "nccl"):
+                    for balanced in (False, True):
+                        model = _train_model(name, adj, sizes, relational)
+                        seq = model.gnn.gnn_layers
+                        part = RowPartition(sizes, group=group, exchange=exchange,
+                                            balance_rowptr=seq.adj_matrix.norm.rowptr if balanced else None).attach(seq)
+                        got = _train_steps(model, name, sizes)
+                        part.close()
+                        seq.partition = None
+                        cases += 1
+                        ok = all(len(a) == len(b) and all(torch.equal(x, y) for x, y in zip(a, b))
+                                 for a, b in zip(got, want))
+                        if not ok:
+                            failures.append("%s %s %s%s" % (name, exchange, "edge-balanced" if balanced else "even",
+                                                            " blocked" if blocking else ""))
+                say("training parity: %s%s done" % (name, " blocked" if blocking else ""))
+        finally:
+            G.FORCED_BLOCKING = None
+    flag = torch.tensor([0 if failures else 1], dtype=torch.int32, device=dev)
+    dist.all_reduce(flag, op=dist.ReduceOp.MIN, group=group)
+    gathered = [None] * world
+    dist.all_gather_object(gathered, failures, group=group)
+    return {"bit_identical": bool(int(flag.item()) == 1), "cases": cases,
+            "failures": sorted({f for fl in gathered for f in fl})}

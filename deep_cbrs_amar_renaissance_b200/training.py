@@ -181,20 +181,26 @@ def _bwd_csr(graph, view):
     return csr if graph.symmetric else csr.transposed()
 
 
-def _gcn_train(tape, layer, x_node, graph, out):
+def _gcn_train(tape, layer, x_node, graph, out, part=None):
     """GCNConv / RGCNConv: y = act(A_hat (x W) + b).  Backward: dPre = dY*act'(y); db = colsum dPre;
     dZ = A_hat^T dPre (= A_hat dPre on a symmetric graph); dW = x^T dZ; dx = dZ W^T.
     Relational operator (stacked layout [N, R*N]: column r*N + j carries relation r): ONE product with the transposed
     stacked operator gives every relation's dZ_r at once (rows r*N .. (r+1)*N of the result), whatever the symmetry of
-    the individual relation blocks."""
+    the individual relation blocks.
+    part: a RowPartition; the sparse products then run on this rank's rows (RowPartition.sparse_rows), everything else
+    as on one GPU."""
     x = x_node.x
     csr = graph.norm
     n = x.shape[0]
     relational = isinstance(layer, RGCNConv)
     kernels = layer.kernels if relational else [layer.kernel]
+    relu = layer.activation == "relu"
     z = torch.empty(len(kernels) * n, layer.channels, dtype=torch.float32, device=x.device)
     ops.dense_grouped(x, kernels, z, n)
-    y = ops.spmm(csr, z, out, bias=layer.bias, relu=layer.activation == "relu")
+    if part is None:
+        y = ops.spmm(csr, z, out, bias=layer.bias, relu=relu)
+    else:
+        y, = part.sparse_rows(csr, [out], lambda sl, v, t: ops.spmm(sl, z, v[0], bias=layer.bias, relu=relu, **t[0]))
     node = Node(y)
 
     def bwd():
@@ -204,14 +210,23 @@ def _gcn_train(tape, layer, x_node, graph, out):
         if layer.bias is not None:
             tape.wgrad(layer.bias, ops.colsum(dpre))
         if not relational:
-            dz = torch.empty(n, layer.channels, dtype=torch.float32, device=x.device)
-            ops.spmm(_bwd_csr(graph, "norm"), dpre, dz)
+            if part is None:
+                dz = torch.empty(n, layer.channels, dtype=torch.float32, device=x.device)
+                ops.spmm(_bwd_csr(graph, "norm"), dpre, dz)
+            else:
+                dz, = part.sparse_rows(_bwd_csr(graph, "norm"), [part.buffer(("gcn_dz", id(layer)), n, layer.channels)],
+                                       lambda sl, v, t: ops.spmm(sl, dpre, v[0], **t[0]))
             dw, _ = ops.dense_grad_w(x, dz, want_bias=False)
             tape.wgrad(layer.kernel, dw)
             x_node.add_grad(ops.dense(dz, ops.transpose(layer.kernel)))
             return
-        dz_all = torch.empty(len(kernels) * n, layer.channels, dtype=torch.float32, device=x.device)
-        ops.spmm(csr.transposed(), dpre, dz_all)
+        if part is None:
+            dz_all = torch.empty(len(kernels) * n, layer.channels, dtype=torch.float32, device=x.device)
+            ops.spmm(csr.transposed(), dpre, dz_all)
+        else:
+            dz_all, = part.sparse_rows(csr.transposed(),
+                                       [part.buffer(("rgcn_dz", id(layer)), len(kernels) * n, layer.channels)],
+                                       lambda sl, v, t: ops.spmm(sl, dpre, v[0], **t[0]))
         dx = None
         for r, w in enumerate(kernels):
             dz = dz_all[r * n:(r + 1) * n]
@@ -225,17 +240,25 @@ def _gcn_train(tape, layer, x_node, graph, out):
     return node
 
 
-def _lightgcn_train(tape, layer, x_node, graph, out):
+def _lightgcn_train(tape, layer, x_node, graph, out, part=None):
     csr = graph.norm
-    y = ops.spmm(csr, x_node.x, out)
+    x = x_node.x
+    if part is None:
+        y = ops.spmm(csr, x, out)
+    else:
+        y, = part.sparse_rows(csr, [out], lambda sl, v, t: ops.spmm(sl, x, v[0], **t[0]))
     node = Node(y)
 
     def bwd():
         if node.grad is None:
             return
-        dx = torch.empty_like(y) if y.is_contiguous() else torch.empty(y.shape, dtype=torch.float32, device=y.device)
         g = node.grad if node.grad.stride(1) == 1 else node.grad.contiguous()
-        ops.spmm(_bwd_csr(graph, "norm"), g, dx)
+        if part is None:
+            dx = torch.empty_like(y) if y.is_contiguous() else torch.empty(y.shape, dtype=torch.float32, device=y.device)
+            ops.spmm(_bwd_csr(graph, "norm"), g, dx)
+        else:
+            dx, = part.sparse_rows(_bwd_csr(graph, "norm"), [part.buffer(("lightgcn_dx", id(layer)), *y.shape)],
+                                   lambda sl, v, t: ops.spmm(sl, g, v[0], **t[0]))
         x_node.add_grad(dx)
 
     tape.ops.append(bwd)
@@ -264,15 +287,19 @@ def _dgcf_train(tape, layer, x_node, graph, out):
     return node
 
 
-def _sage_train(tape, layer, x_node, graph, out):
+def _sage_train(tape, layer, x_node, graph, out, part=None):
     """GraphSageConv: agg = mean/sum over the raw edge list; v = [x || agg] W + b; out = relu(v / |v|).
     Training keeps v (the fused inference epilogue does not), so the epilogue is its own kernel."""
     x = x_node.x
     csr = graph.raw
     f = x.shape[1]
     mean = layer.aggregate == "mean"
-    agg = torch.empty(csr.n_rows, f, dtype=torch.float32, device=x.device)
-    ops.spmm(csr, x, agg, agg=L.AGG_MEAN if mean else L.AGG_SUM)
+    if part is None:
+        agg = torch.empty(csr.n_rows, f, dtype=torch.float32, device=x.device)
+        ops.spmm(csr, x, agg, agg=L.AGG_MEAN if mean else L.AGG_SUM)
+    else:
+        agg, = part.sparse_rows(csr, [part.buffer(("sage_agg", id(layer)), csr.n_rows, f)],
+                                lambda sl, v, t: ops.spmm(sl, x, v[0], agg=L.AGG_MEAN if mean else L.AGG_SUM, **t[0]))
     v = ops.dense(x, layer.kernel, layer.bias, None, x2=agg)
     relu = layer.activation == "relu"
     y = ops.l2norm_act(v, relu=relu, out=out)
@@ -288,16 +315,20 @@ def _sage_train(tape, layer, x_node, graph, out):
         da = ops.dense(dv, ops.transpose(layer.kernel))
         dagg = da[:, f:]
         t = ops.scale_rows_inv_degree(dagg, csr.rowptr) if mean else dagg.contiguous()
-        dxa = torch.empty(csr.n_rows, f, dtype=torch.float32, device=x.device)
         # A^T = A on a symmetric graph (the raw edge list holds both directions of every edge); else the transpose
-        ops.spmm(_bwd_csr(graph, "raw"), t, dxa, agg=L.AGG_SUM)
+        if part is None:
+            dxa = torch.empty(csr.n_rows, f, dtype=torch.float32, device=x.device)
+            ops.spmm(_bwd_csr(graph, "raw"), t, dxa, agg=L.AGG_SUM)
+        else:
+            dxa, = part.sparse_rows(_bwd_csr(graph, "raw"), [part.buffer(("sage_dxa", id(layer)), csr.n_rows, f)],
+                                    lambda sl, v, tg: ops.spmm(sl, t, v[0], agg=L.AGG_SUM, **tg[0]))
         x_node.add_grad(ops.axpby(da[:, :f], 1.0, dxa, 1.0))
 
     tape.ops.append(bwd)
     return node
 
 
-def _gat_train(tape, layer, x_node, graph, out):
+def _gat_train(tape, layer, x_node, graph, out, part=None):
     """GATConv: z = x W, p = z.a_self, q = z.a_neigh, fused edge softmax + aggregate (csrc/gat.cu);
     backward = csrc/gat_bwd.cu, then the dense pieces."""
     x = x_node.x
@@ -310,7 +341,12 @@ def _gat_train(tape, layer, x_node, graph, out):
     w2 = layer.kernel.reshape(f, layer.channels)
     a_s, a_n = layer.attn_kernel_self.reshape(-1), layer.attn_kernel_neighs.reshape(-1)
     z, p, q = ops.dense(x, w2, rowop=L.ROWOP_ATTN, a_self=a_s, a_neigh=a_n)
-    y = ops.gat(csr, z, p, q, out, bias=layer.bias, relu=layer.activation == "relu")
+    relu = layer.activation == "relu"
+    if part is None:
+        y = ops.gat(csr, z, p, q, out, bias=layer.bias, relu=relu)
+    else:
+        y, = part.sparse_rows(csr, [out], lambda sl, v, t: ops.gat(sl, z, p, q, v[0], bias=layer.bias, relu=relu,
+                                                                   row_offset=sl.row_offset, **t[0]))
     node = Node(y)
 
     def bwd():
@@ -319,7 +355,18 @@ def _gat_train(tape, layer, x_node, graph, out):
         d_o = ops.act_grad(node.grad, y, layer.activation)
         if layer.bias is not None:
             tape.wgrad(layer.bias, ops.colsum(d_o))
-        dz, dp, dq = ops.gat_backward(csr, z, p, q, y, layer.bias, d_o, a_s, a_n)
+        if part is None:
+            dz, dp, dq = ops.gat_backward(csr, z, p, q, y, layer.bias, d_o, a_s, a_n)
+        else:
+            # two row-split phases: every rank needs the softmax stats of its rows' neighbours before the gradients
+            n, h = z.shape
+            stats, = part.sparse_rows(csr, [part.buffer(("gat_stats", id(layer)), n, 3)],
+                                      lambda sl, v, t: ops.gat_backward_stats_rows(sl, p, q, y, layer.bias, d_o, v[0],
+                                                                                   **t[0]))
+            dz, dp, dq = part.sparse_rows(
+                csr, [part.buffer(("gat_dz", id(layer)), n, h), part.buffer(("gat_dp", id(layer)), n, 1),
+                      part.buffer(("gat_dq", id(layer)), n, 1)],
+                lambda sl, v, t: ops.gat_backward_grad_rows(sl, z, p, q, d_o, stats, a_s, a_n, *v, targets=t))
         da_s, _ = ops.dense_grad_w(z, dp.reshape(-1, 1), want_bias=False)
         da_n, _ = ops.dense_grad_w(z, dq.reshape(-1, 1), want_bias=False)
         tape.wgrad(layer.attn_kernel_self, da_s)
@@ -378,6 +425,17 @@ def concat_rows_train(tape, nodes):
     return out
 
 
+PARTITIONED_LAYERS = (GCNConv, RGCNConv, LightGCNConv, GraphSageConv, GATConv)
+
+
+def check_partitioned_training(seq):
+    """Raises NotImplementedError, before any device work, for a partitioned stack the row-split tape does not cover."""
+    for layer in seq.seq_layers:
+        if not isinstance(layer, PARTITIONED_LAYERS):
+            raise NotImplementedError("training {} layers under a RowPartition (no partitioned form; train them on one "
+                                      "GPU)".format(type(layer).__name__))
+
+
 def gnn_train(tape, seq, x_node=None):
     """SequentialGNN.call (/root/reference/src/models/gnn.py:74-84) on the tape -> Node of [N, D_out].
     x_node: the initial node features when they are not the GNN's own embeddings alone
@@ -388,12 +446,16 @@ def gnn_train(tape, seq, x_node=None):
     n = emb.shape[0]
     widths = seq._widths()
     graph = seq.adj_matrix
-    if seq.partition is not None:
-        raise NotImplementedError("training runs on one GPU (the row partition covers the forward path)")
+    part = seq.partition
+    if part is not None:
+        check_partitioned_training(seq)
     concat = seq.final_node == 'concatenation'
     if seq.final_node not in ('concatenation', 'mean', 'sum', 'last'):
         raise NotImplementedError("training with final_node='%s'" % seq.final_node)
-    buf = torch.empty(n, sum(widths), dtype=torch.float32, device=emb.device) if concat else None
+    if part is None:
+        buf = torch.empty(n, sum(widths), dtype=torch.float32, device=emb.device) if concat else None
+    else:
+        buf = part.buffer(("concat",), n, sum(widths)) if concat else None
     nodes = [x_node]
     off = widths[0]
     if concat:
@@ -402,16 +464,21 @@ def gnn_train(tape, seq, x_node=None):
         if not layer.built:
             layer.build([(n, x_node.x.shape[1]), None])
             layer.built = True
-        out = buf[:, off:off + w] if concat else torch.empty(n, w, dtype=torch.float32, device=emb.device)
+        if concat:
+            out = buf[:, off:off + w]
+        elif part is None:
+            out = torch.empty(n, w, dtype=torch.float32, device=emb.device)
+        else:
+            out = part.buffer(("h", id(layer)), n, w)
         off += w
         if isinstance(layer, (GCNConv, RGCNConv)):
-            x_node = _gcn_train(tape, layer, x_node, graph, out)
+            x_node = _gcn_train(tape, layer, x_node, graph, out, part)
         elif isinstance(layer, LightGCNConv):
-            x_node = _lightgcn_train(tape, layer, x_node, graph, out)
+            x_node = _lightgcn_train(tape, layer, x_node, graph, out, part)
         elif isinstance(layer, GraphSageConv):
-            x_node = _sage_train(tape, layer, x_node, graph, out)
+            x_node = _sage_train(tape, layer, x_node, graph, out, part)
         elif isinstance(layer, GATConv):
-            x_node = _gat_train(tape, layer, x_node, graph, out)
+            x_node = _gat_train(tape, layer, x_node, graph, out, part)
         elif isinstance(layer, DGCFConv):
             x_node = _dgcf_train(tape, layer, x_node, graph, out)
         else:
@@ -453,6 +520,12 @@ def model_gnn_train(tape, gnn):
     TwoWayGNN (twgnn.py:93-100)."""
     from .models.tsgnn import TwoStepGNN
     from .models.twgnn import TwoWayGNN
+    if isinstance(gnn, (TwoStepGNN, TwoWayGNN)):
+        stacks = [getattr(gnn, k) for k in ("step_one_gnn_layers", "way_one_gnn_layers", "way_two_gnn_layers",
+                                            "step_two_gnn_layers") if hasattr(gnn, k)]
+        if any(getattr(s, "partition", None) is not None for s in stacks):
+            raise NotImplementedError("training a {} under a RowPartition (no partitioned form; train it on one GPU)"
+                                      .format(type(gnn).__name__))
     if isinstance(gnn, TwoStepGNN):
         items = head_rows_train(tape, gnn_train(tape, gnn.step_one_gnn_layers), gnn.n_embeddings)
         two = gnn.step_two_gnn_layers
@@ -615,6 +688,13 @@ class GraphedTrainStep:
 
     def __init__(self, model, optimizer, batch_size, content_dim=None):
         import numpy as np
+        from .models.gnn import SequentialGNN
+        gnn = getattr(model, "gnn", None)
+        stacks = [s for s in vars(gnn).values() if isinstance(s, SequentialGNN)] if gnn is not None else []
+        if any(s.partition is not None for s in stacks):
+            # the flag barrier of the peer exchange takes a new epoch per call, which a replayed graph cannot
+            raise NotImplementedError("a CUDA-graphed training step under a RowPartition (train eagerly: "
+                                      "train_on_batch / fit(cuda_graph=False))")
         self.model, self.optimizer, self.batch_size = model, optimizer, int(batch_size)
         dev = torch.device("cuda", torch.cuda.current_device())
         self.u = torch.zeros(self.batch_size, dtype=torch.int64, device=dev)

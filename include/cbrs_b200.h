@@ -587,6 +587,25 @@ int cbrs_gat_backward(const cbrs_csr_t *g, const float *z, int64_t ldz, const fl
                       const float *y, int64_t ldy, const float *bias, const float *d_o, int64_t ldo, int32_t h,
                       const float *a_self, const float *a_neigh, float *dz, int64_t lddz, float *dp, float *dq,
                       void *workspace, size_t workspace_bytes, void *stream);
+/* cbrs_gat_backward on rows [row_offset, row_offset + g->n_rows) of the graph (a row slice with global column ids,
+ * as cbrs_gat_csr takes), in two phases so that an exchange can sit between them under a row partition:
+ *   stats_rows: (m_i, S_i, t_i) of the slice's rows into `stats` (the slice's rows of an [N, 3] contiguous array) and
+ *               into stats_peers_host[0..n_peers) (each a peer's address of the same view);
+ *   grad_rows:  dz, dp, dq of the slice's rows, the combine included, into dz/dp/dq and the peers' copies.  `stats` is
+ *               the whole [N, 3] array: the phase reads the stats of every neighbour row, so all rows' stats must be
+ *               there first.
+ * Inputs p, q, y, d_o and z are whole-graph arrays ([N] / [N, ld]) read at global rows; outputs are views of the
+ * slice's rows, as cbrs_gat_csr's y.  Each output row has the bits the whole-graph call gives it.  For an NVSwitch multicast target pass the multicast address of the output as the output and n_peers = 0: no
+ * kernel reads its outputs back.  Null arguments, a null peer copy, n_peers > CBRS_MAX_PEERS - 1, h > 256 and a bad
+ * leading dimension or row_offset return CBRS_E_INVALID before any launch.  No workspace.                       */
+int cbrs_gat_backward_stats_rows(const cbrs_csr_t *g, int64_t row_offset, const float *p, const float *q,
+                                 const float *y, int64_t ldy, const float *bias, const float *d_o, int64_t ldo,
+                                 int32_t h, float *stats, void *const *stats_peers_host, int n_peers, void *stream);
+int cbrs_gat_backward_grad_rows(const cbrs_csr_t *g, int64_t row_offset, const float *z, int64_t ldz, const float *p,
+                                const float *q, const float *d_o, int64_t ldo, int32_t h, const float *stats,
+                                const float *a_self, const float *a_neigh, float *dz, int64_t lddz, float *dp,
+                                float *dq, void *const *dz_peers_host, void *const *dp_peers_host,
+                                void *const *dq_peers_host, int n_peers, void *stream);
 /* the same update for all n_tensors weight tensors of a model in one launch (host arrays of device pointers) */
 int cbrs_adam_step_multi(int32_t n_tensors, void *const *w_host, const void *const *g_host, void *const *m_host,
                          void *const *v_host, const int64_t *n_host, const float *l2_host, float lr_t,
