@@ -106,11 +106,8 @@ _SIGS = {
     "cbrs_peer_open": (c_int, [P, POINTER(c_void_p)]),
     "cbrs_peer_close": (c_int, [P]),
     "cbrs_push_rows": (c_int, [P, c_int64, P, c_int64, c_int64, c_int32, P]),
-    "cbrs_peer_copy": (c_int, [P, P, c_size_t, P]),
     "cbrs_peer_barrier": (c_int, [POINTER(c_void_p), c_int, c_int, c_uint64, P, c_double, P]),
     "cbrs_spmm_csr_bcast": (c_int, [POINTER(CsrDesc), P, c_int64, P, c_int64, c_int32, c_int, P, c_int, c_int,
-                                    POINTER(c_void_p), c_int, P, c_size_t, P]),
-    "cbrs_spmm_gcn_fused": (c_int, [POINTER(CsrDesc), P, c_int64, P, c_int64, P, c_int, P, P, c_int64, POINTER(c_void_p), c_int,
                                     POINTER(c_void_p), c_int, P, c_size_t, P]),
     "cbrs_gat_csr_bcast": (c_int, [POINTER(CsrDesc), c_int64, P, c_int64, P, P, P, c_int64, c_int32, P, c_int,
                                    POINTER(c_void_p), c_int, P, c_size_t, P]),

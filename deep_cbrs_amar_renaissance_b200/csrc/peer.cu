@@ -130,17 +130,6 @@ extern "C" int cbrs_peer_close(void *ptr) {
     return CBRS_OK;
 }
 
-extern "C" int cbrs_peer_copy(void *dst, const void *src, size_t bytes, void *stream) {
-    CBRS_REQUIRE(dst && src, CBRS_E_INVALID, "peer_copy: null argument");
-    if (bytes == 0) return CBRS_OK;
-    cudaError_t e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDefault, (cudaStream_t)stream);
-    if (e != cudaSuccess) {
-        set_error("peer_copy: %s", cudaGetErrorString(e));
-        return CBRS_E_CUDA;
-    }
-    return CBRS_OK;
-}
-
 // Row block -> a mapped address (a peer's copy of a symmetric buffer, or its NVSwitch multicast mapping), coalesced:
 // consecutive threads write consecutive 16-byte pieces of a row, so the fabric sees full 128-byte lines.
 __global__ void push_rows_kernel(const float *__restrict__ src, int64_t lds, float *__restrict__ dst, int64_t ldd, int64_t m, int w4) {

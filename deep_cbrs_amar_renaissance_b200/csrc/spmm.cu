@@ -266,185 +266,6 @@ __global__ void __launch_bounds__(kSpmmThreads) spmm_heavy_kernel(const SpmmPara
     }
 }
 
-// ---------------------------------------------------------------------------------------------------------
-// GCN layer l fused with layer l+1's transform and its all-gather (multi-GPU, SURVEY 8e):
-//   y_i  = relu(sum_j A_ij z_j + b)          (this layer's output row, written to the local [N, D_out] buffer and,
-//                                              for item rows, to every rank's copy)
-//   z'_i = y_i . W_next                       (the NEXT layer's gather operand, row i) -> stored into EVERY rank's
-//                                              copy of Z^(l+1) over NVLink straight from the sparse kernel's epilogue
-// so the exchange of Z^(l+1) is spread over the whole duration of the sparse kernel instead of following it as a
-// transform-with-stores kernel that runs at NVLink speed.  D = 128 in, 128 out (one warp per row, lane l holds
-// elements 4l..4l+3).  W_next (64 KB fp32) is brought into shared memory once per CTA with cp.async.bulk on an
-// mbarrier that each warp waits on only when it reaches its epilogue - the copy hides behind the edge loop and no
-// CTA-wide barrier follows it.  The row x matrix product walks k ascending with one fmaf chain per output element,
-// exactly like dense_fast_kernel, so Z^(l+1) has the same bits as the unfused path.
-// Measured on one GPU at config 5 (profiles/r01_layer_rooflines_c5.jsonl): 152 ms against 133.6 (sparse) + 10.6
-// (transform) separately - the row x W product is a 128-step dependent fmaf chain per output that the warp runs after
-// its gather, and it costs more in the sparse kernel than in the tiled dense kernel.  Two cheaper-looking forms were
-// tried and were SLOWER: 4 rows per pass over W (170 ms: a warp's critical path gets 4x longer) and the packed
-// fma.rn.f32x2 pipe with y duplicated in shared memory (171 ms).  The fusion pays off once the transform-with-stores
-// kernel it replaces is NVLink-bound, i.e. from 4 GPUs up (profiles/r01_scaling_exchange_modes.json).
-struct FusedParams {
-    SpmmParams sp;
-    const float *w_next;   // [128, 128] row-major (Keras kernel [in, out])
-    float *z_next;         // [N_local_rows, 128] view of the local Z^(l+1) at this slice's rows
-    int64_t ldz;
-    float *z_peer[CBRS_MAX_PEERS - 1];
-    int n_zpeer;
-};
-
-constexpr int kFusedThreads = 512, kFusedD = 128;
-
-__device__ __forceinline__ void fused_mbar_init(uint64_t *bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"((uint32_t)__cvta_generic_to_shared(bar)), "r"(count));
-}
-__device__ __forceinline__ void fused_mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"((uint32_t)__cvta_generic_to_shared(bar)), "r"(bytes)
-                 : "memory");
-}
-__device__ __forceinline__ void fused_bulk_g2s(void *dst, const void *src, uint32_t bytes, uint64_t *bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                     (uint32_t)__cvta_generic_to_shared(dst)),
-                 "l"(src), "r"(bytes), "r"((uint32_t)__cvta_generic_to_shared(bar))
-                 : "memory");
-}
-__device__ __forceinline__ void fused_mbar_wait(uint64_t *bar, uint32_t parity) {
-    uint32_t ok = 0;
-    for (uint32_t spins = 0; !ok; ++spins) {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(ok)
-            : "r"((uint32_t)__cvta_generic_to_shared(bar)), "r"(parity)
-            : "memory");
-        if (spins > (1u << 26)) __trap();  // a protocol bug traps instead of hanging the GPU
-    }
-}
-
-// z'[4*lane .. 4*lane+3] = sum_k y_k W[k][4*lane ..], k ascending; y is spread 4 elements per lane
-__device__ __forceinline__ float4 row_times_w(const float4 y, const float *__restrict__ w, int lane) {
-    float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-    const float4 *wl = reinterpret_cast<const float4 *>(w) + lane;  // row k starts at float4 index k*32
-#pragma unroll 4
-    for (int kl = 0; kl < 32; ++kl) {
-        const float y0 = __shfl_sync(0xffffffffu, y.x, kl), y1 = __shfl_sync(0xffffffffu, y.y, kl);
-        const float y2 = __shfl_sync(0xffffffffu, y.z, kl), y3 = __shfl_sync(0xffffffffu, y.w, kl);
-        const float4 w0 = wl[(4 * kl + 0) * 32], w1 = wl[(4 * kl + 1) * 32], w2 = wl[(4 * kl + 2) * 32], w3 = wl[(4 * kl + 3) * 32];
-        z.x = fmaf(y0, w0.x, z.x); z.y = fmaf(y0, w0.y, z.y); z.z = fmaf(y0, w0.z, z.z); z.w = fmaf(y0, w0.w, z.w);
-        z.x = fmaf(y1, w1.x, z.x); z.y = fmaf(y1, w1.y, z.y); z.z = fmaf(y1, w1.z, z.z); z.w = fmaf(y1, w1.w, z.w);
-        z.x = fmaf(y2, w2.x, z.x); z.y = fmaf(y2, w2.y, z.y); z.z = fmaf(y2, w2.z, z.z); z.w = fmaf(y2, w2.w, z.w);
-        z.x = fmaf(y3, w3.x, z.x); z.y = fmaf(y3, w3.y, z.y); z.z = fmaf(y3, w3.z, z.z); z.w = fmaf(y3, w3.w, z.w);
-    }
-    return z;
-}
-
-__device__ __forceinline__ void fused_store_z(const FusedParams &p, int32_t row, int lane, const float4 z) {
-    const int64_t off = (int64_t)row * p.ldz + 4 * lane;
-    *reinterpret_cast<float4 *>(p.z_next + off) = z;
-    for (int q = 0; q < p.n_zpeer; ++q) *reinterpret_cast<float4 *>(p.z_peer[q] + off) = z;
-}
-
-__global__ void __launch_bounds__(kFusedThreads, 2) spmm_gcn_fused_kernel(const FusedParams fp) {
-    extern __shared__ __align__(128) unsigned char fused_smem[];
-    float *Ws = reinterpret_cast<float *>(fused_smem);                       // [128][128]
-    uint64_t *bar = reinterpret_cast<uint64_t *>(Ws + kFusedD * kFusedD);
-    const SpmmParams &p = fp.sp;
-    if (threadIdx.x == 0) {
-        fused_mbar_init(bar, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        fused_mbar_expect_tx(bar, kFusedD * kFusedD * 4);
-#pragma unroll
-        for (int c = 0; c < 4; ++c)
-            fused_bulk_g2s(Ws + c * (kFusedD * kFusedD / 4), fp.w_next + c * (kFusedD * kFusedD / 4), kFusedD * kFusedD, bar);
-    }
-    constexpr int U = 4;
-    const int lane = threadIdx.x & 31;
-    const int64_t gid = (int64_t)blockIdx.x * (kFusedThreads / 32) + (threadIdx.x >> 5);
-    // every exit path waits for the bulk copy: a CTA must not retire with a copy into its shared memory in flight
-    if (gid >= p.n_chunks) { fused_mbar_wait(bar, 0); return; }
-    const int32_t row = p.chunk_row[gid];
-    const int64_t row_e = p.rowptr[row + 1];
-    const int64_t b = p.chunk_begin[gid];
-    const int64_t e = p.chunk_len ? b + p.chunk_len[gid] : ((b + p.chunk_edges < row_e) ? b + p.chunk_edges : row_e);
-    const int32_t slot = p.chunk_slot[gid];
-    const bool weighted = p.vals != nullptr;
-    const float *xcol = reinterpret_cast<const float *>(p.x) + lane * 4;
-    Vec<4> acc;
-    acc.zero();
-    int c_next = 0;
-    float v_next = 0.f;
-    if (b + lane < e) {
-        c_next = ld_stream_i32(p.colidx + b + lane);
-        v_next = weighted ? ld_stream_f32(p.vals + b + lane) : 1.f;
-    }
-    for (int64_t base = b; base < e; base += 32) {
-        const int c = c_next;
-        const float v = v_next;
-        const int64_t nidx = base + 32 + lane;
-        c_next = 0;
-        v_next = 0.f;
-        if (nidx < e) {
-            c_next = ld_stream_i32(p.colidx + nidx);
-            v_next = weighted ? ld_stream_f32(p.vals + nidx) : 1.f;
-        }
-        const int cnt = (e - base < 32) ? (int)(e - base) : 32;
-#pragma unroll
-        for (int k0 = 0; k0 < 32; k0 += U) {
-            if (k0 >= cnt) break;
-            int cc[U];
-            float vv[U];
-            Vec<4> xr[U];
-#pragma unroll
-            for (int u = 0; u < U; ++u) {
-                cc[u] = __shfl_sync(0xffffffffu, c, k0 + u);
-                vv[u] = __shfl_sync(0xffffffffu, v, k0 + u);
-            }
-#pragma unroll
-            for (int u = 0; u < U; ++u)
-                if (k0 + u < cnt) xr[u].load(xcol + (int64_t)cc[u] * p.ldx);
-#pragma unroll
-            for (int u = 0; u < U; ++u)
-                if (k0 + u < cnt) acc.fma(vv[u], xr[u]);
-        }
-    }
-    const int col = lane * 4;
-    if (slot >= 0) {  // heavy row: park the partial; spmm_gcn_fused_heavy_kernel finishes the row and its transform
-        acc.store(p.partial + (int64_t)slot * kFusedD + col);
-        fused_mbar_wait(bar, 0);
-        return;
-    }
-    acc.epilogue(p.bias ? p.bias + col : nullptr, p.relu);
-    acc.store(p.y + (int64_t)row * p.ldy + col);
-    for (int q = 0; q < p.n_peer; ++q) acc.store(p.y_peer[q] + (int64_t)row * p.ldy + col);
-    fused_mbar_wait(bar, 0);
-    fused_store_z(fp, row, lane, row_times_w(acc.v, Ws, lane));
-}
-
-// heavy rows: ascending-chunk merge (as spmm_heavy_kernel), then the same transform with W read through L1/L2
-__global__ void __launch_bounds__(256) spmm_gcn_fused_heavy_kernel(const FusedParams fp) {
-    const SpmmParams &p = fp.sp;
-    const int64_t gid = ((int64_t)blockIdx.x * 256 + threadIdx.x) >> 5;
-    if (gid >= p.n_heavy) return;
-    const int lane = threadIdx.x & 31;
-    const int32_t row = p.heavy_row[gid];
-    const int col = lane * 4;
-    Vec<4> acc;
-    acc.zero();
-    for (int64_t s = p.heavy_slot_ptr[gid]; s < p.heavy_slot_ptr[gid + 1]; ++s) {
-        Vec<4> t;
-        t.load_plain(p.partial + s * kFusedD + col);
-        acc.add(t);
-    }
-    acc.epilogue(p.bias ? p.bias + col : nullptr, p.relu);
-    acc.store(p.y + (int64_t)row * p.ldy + col);
-    for (int q = 0; q < p.n_peer; ++q) acc.store(p.y_peer[q] + (int64_t)row * p.ldy + col);
-    fused_store_z(fp, row, lane, row_times_w(acc.v, fp.w_next, lane));
-}
-
 template <int G, int VEC, typename XT = float>
 static int launch(const SpmmParams &p, cudaStream_t s) {
     const int64_t threads = p.n_chunks * G;
@@ -529,59 +350,6 @@ static int spmm_impl(const cbrs_csr_t *g, const void *x, int64_t ldx, void *y, i
         return v4 ? dispatch_g<4, __nv_bfloat16>(d / 4, p, s) : dispatch_g<1, __nv_bfloat16>(d, p, s);
     }
     return vec4 ? dispatch_g<4>(d / 4, p, s) : dispatch_g<1>(d, p, s);
-}
-
-extern "C" int cbrs_spmm_gcn_fused(const cbrs_csr_t *g, const float *z, int64_t ldz_in, float *y, int64_t ldy, const float *bias,
-                                   int relu, const float *w_next, float *z_next, int64_t ldz_next, void *const *y_peers_host,
-                                   int n_ypeers, void *const *z_peers_host, int n_zpeers, void *workspace,
-                                   size_t workspace_bytes, void *stream) {
-    CBRS_REQUIRE(g && z && y && w_next && z_next, CBRS_E_INVALID, "spmm_gcn_fused: null argument");
-    CBRS_REQUIRE(ldz_in >= kFusedD && ldy >= kFusedD && ldz_next >= kFusedD && ldz_in % 4 == 0 && ldy % 4 == 0 && ldz_next % 4 == 0,
-                 CBRS_E_INVALID, "spmm_gcn_fused: built for 128-wide layers with 16-byte aligned rows");
-    CBRS_REQUIRE(n_ypeers >= 0 && n_ypeers < CBRS_MAX_PEERS && n_zpeers >= 0 && n_zpeers < CBRS_MAX_PEERS &&
-                     (n_ypeers == 0 || y_peers_host) && (n_zpeers == 0 || z_peers_host),
-                 CBRS_E_INVALID, "spmm_gcn_fused: peer lists");
-    CBRS_REQUIRE(g->n_rows >= 0 && g->n_chunks >= 0 && g->chunk_edges > 0, CBRS_E_INVALID, "spmm_gcn_fused: bad graph descriptor");
-    if (g->n_rows == 0) return CBRS_OK;
-    const size_t need = (size_t)g->n_slots * kFusedD * sizeof(float);
-    CBRS_REQUIRE(g->n_slots == 0 || (workspace && workspace_bytes >= need), CBRS_E_WORKSPACE, "spmm_gcn_fused: workspace too small");
-    auto al16 = [](const void *q) { return ((uintptr_t)q % 16) == 0; };
-    CBRS_REQUIRE(al16(z) && al16(y) && al16(w_next) && al16(z_next) && al16(workspace) && (!bias || al16(bias)), CBRS_E_INVALID,
-                 "spmm_gcn_fused: pointers must be 16-byte aligned");
-    FusedParams fp;
-    SpmmParams &p = fp.sp;
-    p.rowptr = g->rowptr; p.colidx = g->colidx; p.vals = g->vals;
-    p.chunk_row = g->chunk_row; p.chunk_begin = g->chunk_begin; p.chunk_slot = g->chunk_slot; p.chunk_len = g->chunk_len;
-    p.n_chunks = g->n_chunks; p.chunk_edges = g->chunk_edges;
-    p.x = z; p.ldx = ldz_in; p.y = y; p.ldy = ldy; p.d = kFusedD; p.agg = CBRS_AGG_WEIGHTED;
-    p.bias = bias; p.relu = relu; p.partial = (float *)workspace;
-    p.heavy_row = g->heavy_row; p.heavy_slot_ptr = g->heavy_slot_ptr; p.n_heavy = g->n_heavy;
-    p.n_peer = n_ypeers;
-    fp.n_zpeer = n_zpeers;
-    for (int q = 0; q < CBRS_MAX_PEERS - 1; ++q) {
-        p.y_peer[q] = q < n_ypeers ? (float *)y_peers_host[q] : nullptr;
-        fp.z_peer[q] = q < n_zpeers ? (float *)z_peers_host[q] : nullptr;
-        CBRS_REQUIRE((q >= n_ypeers || (p.y_peer[q] && al16(p.y_peer[q]))) && (q >= n_zpeers || (fp.z_peer[q] && al16(fp.z_peer[q]))),
-                     CBRS_E_INVALID, "spmm_gcn_fused: peer copy %d is null or misaligned", q);
-    }
-    fp.w_next = w_next; fp.z_next = z_next; fp.ldz = ldz_next;
-    cudaStream_t s = (cudaStream_t)stream;
-    constexpr int smem = kFusedD * kFusedD * 4 + 16;
-    static bool configured = false;
-    if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(spmm_gcn_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        CBRS_REQUIRE(e == cudaSuccess, CBRS_E_CUDA, "spmm_gcn_fused: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-        configured = true;
-    }
-    if (p.n_chunks > 0) {
-        spmm_gcn_fused_kernel<<<(unsigned)cdiv(p.n_chunks, kFusedThreads / 32), kFusedThreads, smem, s>>>(fp);
-        CBRS_CHECK_LAUNCH("spmm_gcn_fused");
-    }
-    if (p.n_heavy > 0) {
-        spmm_gcn_fused_heavy_kernel<<<(unsigned)cdiv(p.n_heavy * 32, 256), 256, 0, s>>>(fp);
-        CBRS_CHECK_LAUNCH("spmm_gcn_fused_heavy");
-    }
-    return CBRS_OK;
 }
 
 extern "C" int cbrs_spmm_csr(const cbrs_csr_t *g, const void *x, int64_t ldx, void *y, int64_t ldy, int32_t d, int agg,

@@ -296,17 +296,23 @@ class PeerHeap:
 class RowPartition:
     """Attach to a SequentialGNN to run its layer loop on this rank's row blocks.
 
-    What travels per layer is the [N, H] operand the sparse kernel gathers from:
-      GCN / RGCN : Z = X W is computed for OWN rows only, all-gathered, then A_hat Z on own rows
-                   (the dense transform is never replicated; X itself is never exchanged);
+    What travels per layer:
+      GCN        : under the peer exchange, the layer OUTPUT: every rank computes the whole transform
+                   Z = X W from a layer input that is complete on every rank; under "nccl", Z for OWN
+                   rows only, all-gathered, then A_hat Z on own rows;
+      RGCN       : the stacked Z = [X W_r] for OWN rows only, all-gathered, then A_hat Z on own rows;
       GAT        : z = X W, q = z.a_neigh for own rows, all-gathered; p stays local;
       GraphSage / LightGCN : the layer INPUT X^(l) is all-gathered (layer 0 reads the
                    replicated embedding table).
     After the last layer only the node types in `final_types` (default: everything but users)
     are exchanged, because scoring is sharded by user."""
 
-    def __init__(self, n_rows_by_type, group=None, final_types=None, exchange=None, pipeline=None,
-                 row_blocks=None, balance_rowptr=None, balance_min_len=0):
+    # the peer exchange's one GCN schedule: every rank transforms all rows, only layer outputs travel (DESIGN.md section 5).
+    # Nothing in the package reads it; bench.py and tools/scale_families.py report it in their output.
+    pipeline = "replicate"
+
+    def __init__(self, n_rows_by_type, group=None, final_types=None, exchange=None, balance_rowptr=None,
+                 balance_min_len=0):
         self.group = group
         exchange = exchange or os.environ.get("CBRS_EXCHANGE") or ("peer" if torch.cuda.is_available() else "nccl")
         if exchange not in ("peer", "nccl"):
@@ -331,23 +337,6 @@ class RowPartition:
                 warnings.warn("peer-memory exchange unavailable ({}); using the NCCL all-gather".format(
                     why if not ok else "another rank could not map its peers"))
                 self.exchange = "nccl"
-        # peer exchange of a GCN stack: "off" = transform+stores, barrier, sparse kernel, in order;
-        # "kernel" = the next layer's fused transform+stores of row block b runs on a high-priority side
-        # stream while the sparse kernel works on block b+1; "ce" = same, but the rows travel by copy engine
-        # "fused" (default) = where both layers are 128-wide fp32 GCN layers, layer l's sparse kernel also computes the next
-        # layer's transform row by row and stores it into every rank's copy from its epilogue (cbrs_spmm_gcn_fused): the
-        # exchange is spread over the whole sparse kernel; other shapes fall back to "off"
-        # measured on config 5: the fused sparse kernel is ~10 % slower than the plain one, which pays off once the
-        # transform-with-stores kernel it replaces is NVLink-bound: 8 GPUs 84.0 -> 94.2 G edges/s, 2 GPUs 27.1 -> 26.2
-        # "replicate" (default, round 2): GCN layers compute the whole transform on every rank and exchange the layer
-        # OUTPUT from the sparse kernel's epilogue instead (see _propagate_peer); with the tensor-core transform this
-        # beats every exchange of Z: nothing NVLink-bound is exposed and no software pipeline is needed
-        self.pipeline = pipeline or os.environ.get("CBRS_PIPELINE", "replicate")
-        if self.pipeline not in ("off", "kernel", "ce", "fused", "replicate"):
-            raise ValueError("pipeline must be 'replicate', 'off', 'fused', 'kernel' or 'ce'")
-        self.row_blocks = int(row_blocks or os.environ.get("CBRS_ROW_BLOCKS", "1" if self.pipeline in ("off", "fused", "replicate") else "2"))
-        self.replicate_l0 = os.environ.get("CBRS_REPLICATE_L0", "1") != "0"
-        self._side = None
         self._sym = {}
         self.n_rows_by_type = list(n_rows_by_type)
         self.world = dist.get_world_size(group)
@@ -375,23 +364,10 @@ class RowPartition:
             self.heap = None
 
     def csr_slices(self, view_name, graph):
-        """This rank's rows of a CSR view: one slice per owned node-type block, each cut further into
-        `row_blocks` pieces of about equal edge count (the pipelined GCN overlaps the exchange of
-        piece b's transform with the sparse kernel of piece b+1)."""
+        """This rank's rows of a CSR view: one slice per owned node-type block."""
         if view_name not in self._slices:
             full = getattr(graph, view_name)
-            out = []
-            for a, b in self.mine:
-                cuts = [a, b]
-                if self.row_blocks > 1 and b - a >= self.row_blocks:
-                    rp = full.rowptr[a:b + 1]
-                    lo, hi = int(rp[0].item()), int(rp[-1].item())
-                    targets = torch.tensor([lo + (hi - lo) * k // self.row_blocks for k in range(1, self.row_blocks)],
-                                           dtype=rp.dtype, device=rp.device)
-                    mids = (torch.searchsorted(rp, targets) + a).tolist()
-                    cuts = sorted(set([a] + [min(max(m, a), b) for m in mids] + [b]))
-                out.extend(full.row_slice(c0, c1) for c0, c1 in zip(cuts[:-1], cuts[1:]) if c1 > c0)
-            self._slices[view_name] = out
+            self._slices[view_name] = [full.row_slice(a, b) for a, b in self.mine]
         return self._slices[view_name]
 
     def release_full_views(self, graph):
@@ -538,12 +514,10 @@ class RowPartition:
                     emb[type_lo[t]:type_lo[t] + self.n_rows_by_type[t]])
         x_full, hs = emb, [h0]
         off = widths[0]
-        z_ahead = False  # this layer's transform was already produced and exchanged by the previous layer
         for l, layer in enumerate(layers):
             if not layer.built:
                 layer.build([(n, widths[l]), None])
                 layer.built = True
-            h = layer.channels if hasattr(layer, "channels") else widths[l]
             if concat:
                 osb, out = csb, cbuf[:, off:off + widths[l + 1]]
                 off += widths[l + 1]
@@ -552,8 +526,7 @@ class RowPartition:
             relu = getattr(layer, "activation", None) == "relu"
             nxt = layers[l + 1] if l + 1 < len(layers) else None
             # the next layer's sparse kernel gathers from this output directly -> every row travels
-            everywhere = isinstance(nxt, (GraphSageConv, LightGCNConv)) or (self.pipeline == "replicate" and
-                                                                             isinstance(nxt, GCNConv))
+            everywhere = isinstance(nxt, (GCNConv, GraphSageConv, LightGCNConv))
 
             def out_peers(view, a):
                 return osb.peer_addrs(view) if (everywhere or is_final(a)) else None
@@ -561,7 +534,7 @@ class RowPartition:
             def out_targets(view, a):
                 return self._targets(osb, view) if (everywhere or is_final(a)) else {}
 
-            if isinstance(layer, GCNConv) and self.pipeline == "replicate":
+            if isinstance(layer, GCNConv):
                 # Every rank computes the WHOLE transform Z = X W itself (2.5 ms for 1.1e7 x 128 x 128 on the tensor
                 # cores) from a layer input that is complete on every rank: layer 0 reads the replicated embedding
                 # table, later layers read the previous output, whose rows the sparse kernel's epilogue stored into
@@ -570,84 +543,23 @@ class RowPartition:
                 if l > 0:
                     heap.barrier()   # the previous output's remote rows have landed
                 zdt = torch.bfloat16 if getattr(layer, "feature_dtype", "fp32") == "bf16" else torch.float32
-                z = self._buf(("zrep",), n, layer.channels, emb.device, zdt)
+                z = self._buf(("zrep", layer.channels), n, layer.channels, emb.device, zdt)
                 ops.gcn_transform(x_full, layer.kernel, n, out=z)
                 for sl in self.csr_slices("norm", graph):
                     a, b = sl.row_offset, sl.row_offset + sl.n_rows
                     ov = out[a:b]
                     ops.spmm(sl, z, ov, bias=layer.bias, relu=relu, **out_targets(ov, a))
-                z_ahead = False
-            elif isinstance(layer, (GCNConv, RGCNConv)):
-                kernels = layer.kernels if isinstance(layer, RGCNConv) else [layer.kernel]
-                zdt = torch.bfloat16 if getattr(layer, "feature_dtype", "fp32") == "bf16" else torch.float32
-                zsb, z = self._symbuf(("z", l), len(kernels) * n, layer.channels, zdt)
-                if not z_ahead and l == 0 and len(kernels) == 1 and self.replicate_l0 and x_full is emb and zdt == torch.float32:
-                    # layer 0 reads the REPLICATED embedding table: every rank transforms all rows itself (2.5 ms on the
-                    # tensor cores at config 5) instead of its own rows + an exposed, NVLink-bound exchange (6.5 ms)
-                    ops.gcn_transform(emb, kernels[0], n, out=z[0:n])
-                elif not z_ahead:
-                    for a, b in self.mine:
-                        if len(kernels) > 1:   # relational: every relation's transform of the block in one launch
-                            zv = z[a:(len(kernels) - 1) * n + b]
-                            ops.dense_grouped(x_full[a:b], kernels, zv, n, peers=zsb.peer_addrs(zv))
-                        else:
-                            zv = z[a:b]
-                            ops.gcn_transform(x_full[a:b], kernels[0], n, out=zv, peers=zsb.peer_addrs(zv))
-                    heap.barrier()
-                # software pipeline: while the sparse kernel works on row block b+1, the NEXT layer's transform
-                # of block b is computed and stored into every rank's copy on a side stream
-                # (its epilogue is the FFMA chain of dense.cu: only taken when the standalone transform is the FFMA kernel
-                # too, otherwise the partitioned result would differ in the last bits from the single-GPU one)
-                fuse_next = (self.pipeline == "fused" and isinstance(layer, GCNConv) and isinstance(nxt, GCNConv)
-                             and layer.channels == 128 and nxt.channels == 128 and zdt == torch.float32
-                             and getattr(nxt, "feature_dtype", "fp32") == "fp32"
-                             and not ops.tf32x3_chosen(n, 128, 128))
-                if fuse_next:
-                    if not nxt.built:
-                        nxt.build([(n, widths[l + 1]), None])
-                        nxt.built = True
-                    nsb, nz = self._symbuf(("z", l + 1), n, nxt.channels)
-                    for sl in self.csr_slices("norm", graph):
-                        a, b = sl.row_offset, sl.row_offset + sl.n_rows
-                        ov, zv = out[a:b], nz[a:b]
-                        ops.spmm_gcn_fused(sl, z, ov, layer.bias, relu, nxt.kernel, zv, y_peers=out_peers(ov, a),
-                                           z_peers=nsb.peer_addrs(zv))
-                    heap.barrier()
-                    z_ahead = True
-                    x_full = out
-                    hs.append(out)
-                    continue
-                z_ahead = self.pipeline in ("kernel", "ce") and isinstance(nxt, GCNConv)
-                if z_ahead:
-                    if not nxt.built:
-                        nxt.build([(n, widths[l + 1]), None])
-                        nxt.built = True
-                    ndt = torch.bfloat16 if getattr(nxt, "feature_dtype", "fp32") == "bf16" else torch.float32
-                    nsb, nz = self._symbuf(("z", l + 1), n, nxt.channels, ndt)
-                    if self._side is None:
-                        self._side = torch.cuda.Stream(device=emb.device, priority=-1)
-                    main = torch.cuda.current_stream(emb.device)
+            elif isinstance(layer, RGCNConv):
+                # own rows of every relation's transform, stored into every rank's copy of the stacked operand
+                n_rel = len(layer.kernels)
+                zsb, z = self._symbuf(("z", l), n_rel * n, layer.channels)
+                for a, b in self.mine:
+                    zv = z[a:(n_rel - 1) * n + b]
+                    ops.dense_grouped(x_full[a:b], layer.kernels, zv, n, peers=zsb.peer_addrs(zv))
+                heap.barrier()
                 for sl in self.csr_slices("norm", graph):
-                    a, b = sl.row_offset, sl.row_offset + sl.n_rows
-                    ov = out[a:b]
-                    ops.spmm(sl, z, ov, bias=layer.bias, relu=relu, **out_targets(ov, a))
-                    if z_ahead:
-                        done = torch.cuda.Event()
-                        done.record(main)
-                        with torch.cuda.stream(self._side):
-                            self._side.wait_event(done)
-                            zv = nz[a:b]
-                            if self.pipeline == "ce":
-                                ops.gcn_transform(ov, nxt.kernel, n, out=zv)
-                                for addr in nsb.peer_addrs(zv):
-                                    ops.peer_copy(addr, zv)
-                            else:
-                                ops.gcn_transform(ov, nxt.kernel, n, out=zv, peers=nsb.peer_addrs(zv))
-                if z_ahead:
-                    pushed = torch.cuda.Event()
-                    pushed.record(self._side)
-                    main.wait_event(pushed)
-                    heap.barrier()
+                    ov = out[sl.row_offset:sl.row_offset + sl.n_rows]
+                    ops.spmm(sl, z, ov, bias=layer.bias, relu=relu, **out_targets(ov, sl.row_offset))
             elif isinstance(layer, GATConv):
                 zsb, z = self._symbuf(("z", l), n, layer.channels)
                 qsb, q = self._symbuf(("q", l), n, 1)
@@ -730,8 +642,8 @@ class RowPartition:
                 kernels = layer.kernels if isinstance(layer, RGCNConv) else [layer.kernel]
                 zdt = torch.bfloat16 if getattr(layer, "feature_dtype", "fp32") == "bf16" else torch.float32
                 z = self._buf(("z", l), len(kernels) * n, layer.channels, dev, zdt)
-                for a, b in self.mine:
-                    if len(kernels) > 1:
+                for a, b in self.mine:   # the transform each layer type runs on one GPU (GCNConv.call, RGCNConv.call)
+                    if isinstance(layer, RGCNConv):
                         ops.dense_grouped(x_full[a:b], kernels, z[a:(len(kernels) - 1) * n + b], n)
                     else:
                         ops.gcn_transform(x_full[a:b], kernels[0], n, out=z[a:b])

@@ -165,33 +165,6 @@ def spmm(csr, x, out, agg=L.AGG_WEIGHTED, bias=None, relu=False, workspace=None,
     return out
 
 
-def spmm_gcn_fused(csr, z, out, bias, relu, w_next, z_next, y_peers=None, z_peers=None, workspace=None):
-    """GCN sparse step fused with the next layer's transform (cbrs_spmm_gcn_fused), 128-wide layers:
-    out = act(A z + bias) for this slice's rows, z_next[rows] = out @ w_next; both also stored into the peers' copies."""
-    lib = L.load()
-    z, ldz = _rowmajor(z)
-    out, ldy = _rowmajor(out)
-    z_next, ldn = _rowmajor(z_next)
-    if z.shape[1] != 128 or tuple(w_next.shape) != (128, 128) or z_next.shape[1] != 128 or not w_next.is_contiguous():
-        raise L.CbrsError("spmm_gcn_fused is built for 128-wide layers")
-    need = lib.cbrs_spmm_workspace_bytes(ctypes.byref(csr.desc), 128)
-    ws = workspace if workspace is not None and workspace.numel() >= need else _ws(need, z.device)
-    if PROFILE_ON:
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-    L.check(lib.cbrs_spmm_gcn_fused(ctypes.byref(csr.desc), _ptr(z), ldz, _ptr(out), ldy, _ptr(bias, torch.float32),
-                                    1 if relu else 0, _ptr(w_next, torch.float32), _ptr(z_next), ldn,
-                                    _ptr_array(y_peers) if y_peers else None, len(y_peers) if y_peers else 0,
-                                    _ptr_array(z_peers) if z_peers else None, len(z_peers) if z_peers else 0,
-                                    _ptr(ws), ws.numel(), _stream()), "cbrs_spmm_gcn_fused")
-    if PROFILE_ON:
-        e1.record()
-        PROFILE.append(("spmm", e0, e1, {"nnz": csr.nnz, "rows": csr.n_rows, "d": 128, "fused_transform": True,
-                                         "bytes": csr.nnz * (8 + 4 * 128) + csr.n_rows * (4 * 128 + 8)}))
-    _count(1 + (1 if csr.chunks["n_heavy"] else 0))
-    return out
-
-
 def gat(csr, z, p, q, out, bias=None, relu=True, row_offset=0, workspace=None, peers=None, mc=None):
     """mc: as for spmm, the multicast address of `out` (the kernel only stores to its output)"""
     lib = L.load()
@@ -587,23 +560,6 @@ def push_rows(view, buf):
     if PROFILE_ON:
         e1.record()
         PROFILE.append(("push", e0, e1, m * w * 4))
-
-
-def peer_copy(dst_addr, src):
-    """copy-engine transfer of a contiguous tensor into a peer-mapped address (cbrs_peer_copy); an empty tensor (which
-    torch gives a null address) moves nothing"""
-    if not src.is_contiguous():
-        raise L.CbrsError("peer_copy: source must be contiguous")
-    if src.numel() == 0:
-        return
-    if PROFILE_ON:
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-    L.check(L.load().cbrs_peer_copy(ctypes.c_void_p(dst_addr), _ptr(src), src.numel() * src.element_size(), _stream()),
-            "cbrs_peer_copy")
-    if PROFILE_ON:
-        e1.record()
-        PROFILE.append(("peer_copy", e0, e1, src.numel() * src.element_size()))
 
 
 # ------------------------------------------------------------------ top-k

@@ -3,8 +3,8 @@
 
 Called by bench.py before timing whenever WORLD_SIZE > 1 (the JSON line carries the outcome as "partition_parity")
 and by tests/multi_gpu_check.py.  Every rank builds the same small graph and weights, runs each layer family once
-unpartitioned and then partitioned - ragged and even blocks, peer stores and the NCCL all-gather, the software
-pipelines, the fused sparse + transform kernel, the column-blocked schedule - and compares with torch.equal.
+unpartitioned and then partitioned - ragged and even blocks, peer stores and the NCCL all-gather, both GCN transform
+kernels, the column-blocked schedule - and compares with torch.equal.
 Nothing here is timed; the graphs are MovieLens-sized so the whole check takes a few seconds."""
 import numpy as np
 import torch
@@ -68,8 +68,7 @@ def partition_parity(group=None, log=None, families=("BasicGCN", "BasicGraphSage
     adj = small_graph(n_users, n_items, 150000, seed=21, n_props=n_props, n_links=4000, dup_links=300)
     u = np.arange(512) % n_users
     i = np.arange(512) % n_items + n_users
-    modes = ([("peer", "replicate"), ("peer", "off"), ("peer", "kernel"), ("peer", "ce"), ("nccl", "off")] if gpu
-             else [("nccl", "off")])
+    exchanges = ("peer", "nccl") if gpu else ("nccl",)
     for blocking in (None, (257, 40)):          # row-major schedule, then the column-blocked one on the same graph
         G.FORCED_BLOCKING = blocking
         try:
@@ -87,13 +86,9 @@ def partition_parity(group=None, log=None, families=("BasicGCN", "BasicGraphSage
                     seq = model.gnn.gnn_layers
                     model((u, i))
                     full = model.gnn(None).clone()
-                    for exchange, pipeline in modes:
-                        if pipeline != "off" and (name != "BasicGCN" or (blocking is not None and pipeline != "replicate")):
-                            continue  # the pipelines exist for GCN stacks
-                        tag = "%s %s %s/%s%s" % (name, "even" if even else "ragged", exchange, pipeline,
-                                                 " blocked" if blocking else "")
-                        part = RowPartition(sizes, group=group, final_types=[0, 1, 2], exchange=exchange, pipeline=pipeline,
-                                            row_blocks=3 if pipeline in ("kernel", "ce") else 1).attach(seq)
+                    for exchange in exchanges:
+                        tag = "%s %s %s%s" % (name, "even" if even else "ragged", exchange, " blocked" if blocking else "")
+                        part = RowPartition(sizes, group=group, final_types=[0, 1, 2], exchange=exchange).attach(seq)
                         for rep in range(3):  # repeated calls reuse the symmetric buffers
                             got = model.gnn(None)
                             if gpu:
@@ -115,14 +110,13 @@ def partition_parity(group=None, log=None, families=("BasicGCN", "BasicGraphSage
                         seq.partition = None
                     say("partition parity: %s %s%s done" % (name, "even" if even else "ragged", " blocked" if blocking else ""))
             if gpu:
-                # 128-wide GCN stack, once with each transform kernel.  "ffma": the sparse kernel of layer l may also
-                # produce layer l+1's transform and store it into every rank's copy (cbrs_spmm_gcn_fused); "tf32x3": the
-                # tensor-core transform (forced here: the graph is below its automatic threshold), whole-table on every
-                # rank ("replicate") or own rows + peer stores ("off").  All must equal the single-GPU result bit for bit.
+                # 128-wide GCN stack under the peer exchange, once with each transform kernel: the FFMA kernel and the
+                # tensor-core one (forced here: the graph is below its automatic threshold).  Both must equal the
+                # single-GPU result bit for bit.
                 from . import ops
                 saved = ops.GCN_TRANSFORM
                 try:
-                    for transform, pipelines in (("ffma", ("fused", "replicate", "off")), ("tf32x3", ("replicate", "off"))):
+                    for transform in ("ffma", "tf32x3"):
                         ops.GCN_TRANSFORM = transform
                         set_seed(11)
                         model = basic.BasicGCN(adj, n_hiddens=[128, 128, 128], embedding_dim=128, dense_units=[48, 48],
@@ -130,16 +124,15 @@ def partition_parity(group=None, log=None, families=("BasicGCN", "BasicGraphSage
                         seq = model.gnn.gnn_layers
                         model((u, i))
                         full = model.gnn(None).clone()
-                        for pipeline in pipelines:
-                            part = RowPartition([n_users, n_items, n_props], group=group, final_types=[0, 1, 2],
-                                                exchange="peer", pipeline=pipeline).attach(seq)
-                            for rep in range(2):
-                                got = model.gnn(None)
-                                torch.cuda.synchronize()
-                                check(torch.equal(got, full), "128-wide GCN %s pipeline=%s%s rep %d" % (
-                                    transform, pipeline, " blocked" if blocking else "", rep))
-                            part.close()
-                            seq.partition = None
+                        part = RowPartition([n_users, n_items, n_props], group=group, final_types=[0, 1, 2],
+                                            exchange="peer").attach(seq)
+                        for rep in range(2):
+                            got = model.gnn(None)
+                            torch.cuda.synchronize()
+                            check(torch.equal(got, full), "128-wide GCN %s%s rep %d" % (
+                                transform, " blocked" if blocking else "", rep))
+                        part.close()
+                        seq.partition = None
                         if transform == "tf32x3":   # the GAT transform (z, p, q) on the tensor-core kernel, partitioned
                             set_seed(13)
                             model = basic.BasicGAT(adj, n_hiddens=[64, 64], embedding_dim=64, dense_units=[48, 48],
@@ -170,7 +163,7 @@ def partition_parity(group=None, log=None, families=("BasicGCN", "BasicGraphSage
                             seq.partition = None
                 finally:
                     ops.GCN_TRANSFORM = saved
-                say("partition parity: 128-wide GCN (fused / replicated / tensor-core transform)%s done" % (" blocked" if blocking else ""))
+                say("partition parity: 128-wide GCN (FFMA / tensor-core transform)%s done" % (" blocked" if blocking else ""))
         finally:
             G.FORCED_BLOCKING = None
     if gpu:

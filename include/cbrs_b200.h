@@ -426,7 +426,7 @@ int cbrs_synth_bipartite(int64_t n_users, int64_t n_items, int64_t n_edges, uint
 int cbrs_synth_bipartite_ex(int64_t n_users, int64_t n_items, int64_t n_edges, uint64_t seed, int scatter_items,
                             int32_t *coo_row, int32_t *coo_col, void *stream);
 
-/* ---- peer memory + fused producer -> all-gather kernels (SURVEY 8e; multi-GPU extension) -----
+/* ---- peer memory + producer kernels that store into every rank's copy (SURVEY 8e; multi-GPU) ---
  * One process per GPU.  Every rank allocates the same ("symmetric") buffers with
  * cbrs_peer_alloc, exports an IPC handle (CBRS_IPC_HANDLE_BYTES opaque bytes, exchanged by
  * the host, e.g. torch.distributed.all_gather_object) and maps its peers' copies with
@@ -448,9 +448,6 @@ int cbrs_peer_free(void *ptr);
 int cbrs_peer_export(void *ptr, unsigned char *handle_host);
 int cbrs_peer_open(const unsigned char *handle_host, void **ptr_out);
 int cbrs_peer_close(void *ptr);
-/* copy-engine transfer into a peer-mapped buffer (no SMs): the alternative to the fused stores when the
- * producer's rows should travel while ANOTHER kernel owns the SMs */
-int cbrs_peer_copy(void *dst, const void *src, size_t bytes, void *stream);
 
 /* Coalesced copy of a row block (m rows of w floats, leading dimensions in elements) into a MAPPED address: the same view
  * in a peer's copy of a symmetric buffer, or in the buffer's NVSwitch multicast mapping (one store reaches every copy).
@@ -464,14 +461,6 @@ int cbrs_peer_barrier(void *const *flags_peers_host, int n_ranks, int my_rank, u
 int cbrs_spmm_csr_bcast(const cbrs_csr_t *g, const void *x, int64_t ldx, void *y, int64_t ldy, int32_t d,
                         int agg, const float *bias, int relu, int dtype, void *const *y_peers_host,
                         int n_peers, void *workspace, size_t workspace_bytes, void *stream);
-/* GCN layer l fused with layer l+1's transform and its all-gather, 128-wide layers:
- *   y = relu(A_hat z + bias) -> y (+ y_peers), and z_next[row] = y[row] @ w_next[128,128] -> z_next (+ z_peers),
- * both from the sparse kernel's epilogue, so the exchange of the next operand is spread over the whole sparse kernel.
- * z_next has the bits cbrs_dense would produce from y (same k-ascending fmaf chain).  Workspace as cbrs_spmm_csr. */
-int cbrs_spmm_gcn_fused(const cbrs_csr_t *g, const float *z, int64_t ldz_in, float *y, int64_t ldy, const float *bias,
-                        int relu, const float *w_next, float *z_next, int64_t ldz_next, void *const *y_peers_host,
-                        int n_ypeers, void *const *z_peers_host, int n_zpeers, void *workspace,
-                        size_t workspace_bytes, void *stream);
 int cbrs_gat_csr_bcast(const cbrs_csr_t *g, int64_t row_offset, const float *z, int64_t ldz, const float *p,
                        const float *q, float *y, int64_t ldy, int32_t h, const float *bias, int relu,
                        void *const *y_peers_host, int n_peers, void *workspace, size_t workspace_bytes,

@@ -2,7 +2,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 tests/multi_gpu_check.py
 Every rank builds the same graph and weights, runs the propagation once unpartitioned and once
 row-partitioned, and requires the two to be BIT-identical for all four layer families, ragged and even blocks,
-peer stores / NCCL / the software pipelines / the fused kernel, row-major and column-blocked schedules; then checks
+peer stores / NCCL, both GCN transform kernels, row-major and column-blocked schedules; then checks
 user-sharded catalog top-k.  The body lives in deep_cbrs_amar_renaissance_b200/selfcheck.py because bench.py runs
 the same check before timing whenever WORLD_SIZE > 1 (its JSON line carries "partition_parity")."""
 import json

@@ -185,24 +185,6 @@ def test_gat_blocked_matches_oracle_and_partition(dev):
     assert torch.equal(part, out)
 
 
-def test_fused_gcn_kernel_on_blocked_schedule_equals_unfused(dev):
-    from deep_cbrs_amar_renaissance_b200 import ops
-    adj = random_bipartite(300, 60, 9000, seed=2)
-    g, reblock = _graphs(adj, dev, (40, 25), chunk_edges=64)
-    norm = reblock(g.norm)
-    n = adj.shape[0]
-    gen = torch.Generator(dev).manual_seed(7)
-    z = torch.randn(n, 128, device=dev, generator=gen)
-    w = torch.randn(128, 128, device=dev, generator=gen) * 0.1
-    b = torch.randn(128, device=dev, generator=gen)
-    y_ref, z_ref = torch.empty(n, 128, device=dev), torch.empty(n, 128, device=dev)
-    ops.spmm(norm, z, y_ref, bias=b, relu=True)
-    ops.dense(y_ref, w, out=z_ref)
-    y, zn = torch.empty_like(y_ref), torch.empty_like(z_ref)
-    ops.spmm_gcn_fused(norm, z, y, b, True, w, zn)
-    assert torch.equal(y, y_ref) and torch.equal(zn, z_ref)
-
-
 def test_default_policy_leaves_small_graphs_row_major(dev):
     from deep_cbrs_amar_renaissance_b200.graph import DeviceGraph, blocking_policy
     assert blocking_policy(9746) == (0, 0) and blocking_policy(11_000_000)[0] > 0

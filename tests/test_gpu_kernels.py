@@ -497,36 +497,6 @@ def test_loader_device_ids_give_the_same_arrays(tmp_path):
     assert (host[2] != dev[2]).nnz == 0 and np.array_equal(host[2].row, dev[2].row)
 
 
-# ------------------------------------------------------------------ fused sparse step + next transform
-@pytest.mark.parametrize("chunk_edges,relu,with_bias", [(128, True, True), (1024, False, False), (32, True, False)])
-def test_spmm_gcn_fused_equals_spmm_then_dense_bit_for_bit(dev, chunk_edges, relu, with_bias):
-    """cbrs_spmm_gcn_fused (no peers): y == cbrs_spmm_csr's output and z_next == cbrs_dense(y, W) exactly, for rows
-    finished by the chunk kernel and for heavy rows finished by the merge kernel; strided y (a column slice)."""
-    from deep_cbrs_amar_renaissance_b200 import ops
-    from deep_cbrs_amar_renaissance_b200.graph import DeviceGraph
-    n_items = 200 if chunk_edges < 1024 else 40   # item rows must exceed a chunk so the heavy-row merge runs
-    adj = random_bipartite(3000, n_items, 70000, seed=chunk_edges)
-    g = DeviceGraph.from_scipy(adj, chunk_edges=chunk_edges)
-    csr = g.norm
-    assert csr.chunks["n_heavy"] > 0
-    n = 3000 + n_items
-    rng = np.random.RandomState(1)
-    x = _t(rng.standard_normal((n, 128)).astype(np.float32), dev)
-    w = _t((rng.standard_normal((128, 128)) * 0.1).astype(np.float32), dev)
-    b = _t((rng.standard_normal(128) * 0.1).astype(np.float32), dev) if with_bias else None
-    buf1 = torch.zeros(n, 384, device=dev)
-    buf2 = torch.zeros(n, 384, device=dev)
-    y1, y2 = buf1[:, 128:256], buf2[:, 128:256]
-    ops.spmm(csr, x, y1, bias=b, relu=relu)
-    z1 = ops.dense(y1, w)
-    z2 = torch.empty(n, 128, device=dev)
-    ops.spmm_gcn_fused(csr, x, y2, b, relu, w, z2)
-    assert torch.equal(buf1, buf2)
-    assert torch.equal(z1, z2)
-    with pytest.raises(RuntimeError):
-        ops.spmm_gcn_fused(csr, x[:, :64].contiguous(), y2, b, relu, w, z2)
-
-
 @pytest.mark.parametrize("m,f,h,r", [(300, 16, 16, 2), (1000, 64, 64, 3), (77, 10, 6, 2), (513, 128, 128, 2), (200, 32, 8, 5)])
 def test_dense_grouped_writes_every_relation_block_in_one_launch(dev, m, f, h, r):
     """cbrs_dense_grouped (row R): X . [W_0 | ... | W_{R-1}] stored straight into the stacked [R*N, H] operand; same

@@ -1,7 +1,7 @@
 """The multi-GPU exchange, tested on one GPU.
 
 Under the row partition (distributed.py) the producing kernels store every finished row into the local buffer AND into
-each peer's copy of it (the *_bcast / *_peers forms), push_rows / peer_copy move finished blocks, and cbrs_peer_barrier
+each peer's copy of it (the *_bcast / *_peers forms), push_rows moves finished blocks, and cbrs_peer_barrier
 orders producers before consumers.  Every peer store is a plain store to an address the caller supplies, so a separate
 allocation on the same device stands in for another rank's copy and nothing in the kernel changes but the address.
 
@@ -11,14 +11,16 @@ A. Kernel by kernel: the same call without peers, then with 1 and with 7 (CBRS_M
    layout (same leading dimension and alignment, as every rank's copy of a symmetric buffer has); the layouts used are
    packed rows, column slices of wider rows and rows that start off a 16-byte boundary.  The entry points must also
    refuse peer lists they cannot serve, before any launch.
-B. SymmetricBuffer addresses, push_rows (vector and scalar paths, the multicast target) and peer_copy.
+B. SymmetricBuffer addresses and push_rows (vector and scalar paths, the multicast target).
 C. The flag barrier, only in configurations where every flag it waits for is already set: the kernel traps when a
    peer does not arrive, so no configuration that could make it wait is run.
-D. A loopback of the partitioned layer loop: 2 and 3 ranks emulated in one process on one stream, each rank running
-   its row slice and storing into its own copy and, through SymmetricBuffer.peer_addrs, into the others', composed as
-   RowPartition._propagate_peer composes them.  Every copy of every layer output must equal the single-GPU layer
-   output bit for bit - the claim selfcheck.partition_parity makes on several GPUs."""
+D. A loopback of the partitioned layer loop: RowPartition.propagate itself on 2 and 3 ranks emulated by threads of one
+   process, all launching on one stream, over an emulated heap of symmetric buffers and a host-side barrier.  Every
+   rank's result, with every layer's output concatenated, must equal the single-GPU SequentialGNN result bit for bit,
+   on the first call and on a second that reuses the buffers - the claim selfcheck.partition_parity makes on several
+   GPUs."""
 import ctypes
+import threading
 import types
 
 import numpy as np
@@ -207,27 +209,6 @@ def test_spmm_misaligned_peer_drops_to_scalar_stores(dev, graph, blocking):
 
 
 @pytest.mark.parametrize("blocking", [(0, 0), (23, 9)])
-@pytest.mark.parametrize("chunk_edges", [32, 1024])
-def test_fused_gcn_peer_stores(dev, graph, chunk_edges, blocking):
-    """y and z_next both go to the peers; z_next in every copy is ops.dense(y, w_next) bit for bit"""
-    from deep_cbrs_amar_renaissance_b200 import ops
-    adj, g = graph
-    n = adj.shape[0]
-    csr = _sched(g, "norm", blocking, chunk_edges)
-    z, w, b = _randn((n, 128), dev, 1), _randn((128, 128), dev, 2, 0.1), _randn((128,), dev, 3)
-
-    def run(v, peers):
-        ops.spmm_gcn_fused(csr, z, v[0], b, True, w, v[1], y_peers=peers[0] if peers else None,
-                           z_peers=peers[1] if peers else None)
-    ref, _ = check_peer_stores(dev, [(n, 128, 136, F32, 4), (n, 128, 128, F32, 0)], run,
-                               "spmm_gcn_fused chunk_edges=%d blocking=%s" % (chunk_edges, blocking))
-    assert same_bits(ref[1], ops.dense(ref[0], w))
-    y = torch.empty(n, 128, device=dev)
-    ops.spmm(csr, z, y, bias=b, relu=True)
-    assert same_bits(ref[0], y)
-
-
-@pytest.mark.parametrize("blocking", [(0, 0), (23, 9)])
 @pytest.mark.parametrize("h", [8, 20, 128])
 def test_gat_peer_stores(dev, graph, h, blocking):
     from deep_cbrs_amar_renaissance_b200 import ops
@@ -406,14 +387,6 @@ def test_peer_lists_the_kernels_cannot_serve_are_refused_before_any_launch(dev, 
         ("spmm, a null peer", E_INVALID, lambda: ops.spmm(csr, x, out, peers=[copies[0], 0])),
         ("gat, 8 peers", E_INVALID, lambda: ops.gat(g.raw, x, p, q, out, peers=copies)),
         ("gat, a null peer", E_INVALID, lambda: ops.gat(g.raw, x, p, q, out, peers=[0])),
-        ("spmm_gcn_fused, 8 peers", E_INVALID, lambda: ops.spmm_gcn_fused(csr, x, out, b, True, w, out160[:, :128],
-                                                                            y_peers=copies)),
-        ("spmm_gcn_fused, misaligned y peer", E_INVALID,
-         lambda: ops.spmm_gcn_fused(csr, x, out, b, True, w, out160[:, :128], y_peers=[copies[0] + 4])),
-        ("spmm_gcn_fused, misaligned z peer", E_INVALID,
-         lambda: ops.spmm_gcn_fused(csr, x, out, b, True, w, out160[:, :128], z_peers=[copies[0], copies[1] + 8])),
-        ("spmm_gcn_fused, null z peer", E_INVALID,
-         lambda: ops.spmm_gcn_fused(csr, x, out, b, True, w, out160[:, :128], z_peers=[0])),
         ("dense, 8 peers", E_INVALID, lambda: ops.dense(x, w, b, out=out, peers=copies)),
         ("dense, a null peer", E_INVALID, lambda: ops.dense(x, w, b, out=out, peers=[copies[0], 0])),
         ("dense, peer aligned differently mod 16", E_INVALID, lambda: ops.dense(x, w, b, out=out, peers=[copies[0] + 4])),
@@ -443,7 +416,7 @@ def test_peer_lists_the_kernels_cannot_serve_are_refused_before_any_launch(dev, 
         assert bool((a.buf == SENT).all()), what + ": refused, but something was written"
 
 
-# ------------------------------------------------------------------------------- B. addresses, pushes and copies
+# ------------------------------------------------------------------------------------- B. addresses and pushes
 def _stub(rank):
     return types.SimpleNamespace(rank=rank)
 
@@ -512,27 +485,6 @@ def test_push_rows(dev, name, multicast):
     a.check("push_rows %s%s" % (name, " (multicast)" if multicast else ""))
 
 
-def test_peer_copy(dev):
-    from deep_cbrs_amar_renaissance_b200 import _lib as L
-    from deep_cbrs_amar_renaissance_b200 import ops
-    a = Arena(dev, 2 * GUARD + 2 * (37 * 13 + 8 + GUARD))
-    dst = a.take(37, 13)
-    src = _randn((37, 13), dev, 4)
-    ops.peer_copy(dst.data_ptr(), src)
-    torch.cuda.synchronize()
-    assert same_bits(dst, src)
-    a.check("peer_copy")
-    other = a.take(37, 13, mark=False)
-    ops.peer_copy(other.data_ptr(), src[5:5])          # an empty block: nothing moves
-    stream = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
-    L.check(L.load().cbrs_peer_copy(ctypes.c_void_p(other.data_ptr()), ctypes.c_void_p(src.data_ptr()), 0, stream),
-            "cbrs_peer_copy")
-    torch.cuda.synchronize()
-    a.check("0-byte peer_copy")
-    with pytest.raises(L.CbrsError):
-        ops.peer_copy(other.data_ptr(), src.t())          # not contiguous
-
-
 # ----------------------------------------------------------------------------------------------- C. the flag barrier
 @pytest.mark.parametrize("n_ranks,me", [(1, 0), (2, 0), (2, 1), (8, 0), (8, 5)])
 def test_flag_barrier_publishes_its_epoch(dev, n_ranks, me):
@@ -568,132 +520,108 @@ def test_flag_barrier_publishes_its_epoch(dev, n_ranks, me):
 
 
 # ------------------------------------------------------------------------- D. loopback of the partitioned layer loop
-class _Sym:
-    """A symmetric [n, w] buffer of `world` emulated ranks: one allocation per rank and each rank's SymmetricBuffer."""
+class _Heap:
+    """What the peer layer loop uses of a PeerHeap, for one of `world` ranks emulated by threads of this process.
+    alloc() is collective, as PeerHeap.alloc is: the k-th call of every rank returns a SymmetricBuffer over the same
+    `world` sentinel-filled allocations.  barrier() is a host-side rendezvous of the threads.  Every thread launches on
+    one stream, so when the rendezvous opens, every rank's earlier launches are queued ahead of every rank's later
+    ones: the ordering the flag barrier gives across GPUs."""
 
-    def __init__(self, world, n, w, dtype, dev):
+    def __init__(self, shared, rank):
+        self.shared, self.rank, self.n_allocs = shared, rank, 0
+
+    def alloc(self, nbytes):
         from deep_cbrs_amar_renaissance_b200.distributed import SymmetricBuffer
-        self.copies = [torch.full((n, w), -3.0e38, dtype=dtype, device=dev) for _ in range(world)]
-        nbytes = n * w * self.copies[0].element_size()
-        self.sb = [SymmetricBuffer(_stub(r), nbytes, [c.data_ptr() for c in self.copies]) for r in range(world)]
+        nbytes = (int(nbytes) + 255) // 256 * 256
+        sh = self.shared
+        with sh.lock:
+            if self.n_allocs == len(sh.allocs):
+                sh.allocs.append((nbytes, [torch.full((nbytes // 4,), SENT, device=sh.dev) for _ in range(sh.world)]))
+            size, copies = sh.allocs[self.n_allocs]
+        self.n_allocs += 1
+        assert size == nbytes, "rank %d asked for %d bytes, another rank for %d" % (self.rank, nbytes, size)
+        return SymmetricBuffer(self, nbytes, [c.data_ptr() for c in copies])
+
+    def barrier(self):
+        self.shared.rendezvous.wait()
 
 
-LOOPBACK = [("gcn", p, t, dt) for p in ("replicate", "off", "kernel", "ce") for t in ("ffma", "tf32x3") for dt in ("fp32", "bf16")]
-LOOPBACK += [("gcn", "fused", "ffma", "fp32"), ("rgcn", "off", "ffma", "fp32")]
+def _ranks(sizes, cuts, dev):
+    """One RowPartition per emulated rank, rank r owning rows cuts[r]:cuts[r+1], with the attributes
+    RowPartition.__init__ sets that the peer layer loop reads.  Every node type is final, so every rank ends up with
+    every row."""
+    from deep_cbrs_amar_renaissance_b200.distributed import RowPartition
+    world = len(cuts) - 1
+    shared = types.SimpleNamespace(world=world, dev=dev, lock=threading.Lock(), allocs=[],
+                                   rendezvous=threading.Barrier(world, timeout=120))
+    parts = []
+    for r in range(world):
+        p = RowPartition.__new__(RowPartition)
+        p.group, p.exchange, p.heap = None, "peer", _Heap(shared, r)
+        p.n_rows_by_type, p.world, p.rank = list(sizes), world, r
+        p.mine = [(cuts[r], cuts[r + 1])]
+        p.final_types = list(range(len(sizes)))
+        p._sym, p._slices, p._bufs = {}, {}, {}
+        parts.append(p)
+    return shared, parts
+
+
+def _propagate_on_every_rank(shared, parts, seq, calls=2):
+    """RowPartition.propagate `calls` times on every emulated rank, each rank in its own thread, all on the caller's
+    stream -> [[copy of the result of each call] per rank].  A rank that raises breaks the rendezvous, so the others
+    stop waiting for it, and its error is raised here."""
+    stream = torch.cuda.current_stream()
+    results = [[] for _ in parts]
+    errors = [None] * len(parts)
+
+    def run(r):
+        try:
+            with torch.cuda.stream(stream):
+                for _ in range(calls):
+                    results[r].append(parts[r].propagate(seq).clone())
+        except BaseException as e:  # noqa: BLE001
+            errors[r] = e
+            shared.rendezvous.abort()
+    threads = [threading.Thread(target=run, args=(r,)) for r in range(len(parts))]
+    for t in threads:
+        t.start()
+    for t in threads:
+        t.join()
+    raised = [e for e in errors if e is not None]
+    if raised:
+        raise next((e for e in raised if not isinstance(e, threading.BrokenBarrierError)), raised[0])
+    torch.cuda.synchronize()
+    return results
+
+
+# (family, variant, transform, dtype).  Variants: "64-32-48" = GCN layers of those widths, "2rel" / "1rel" = RGCN with
+# that many relations (one relation: the tensor-core transform, which GCNConv would take at this width, is forced)
+LOOPBACK = [("gcn", "replicate", t, dt) for t in ("ffma", "tf32x3") for dt in ("fp32", "bf16")]
+LOOPBACK += [("gcn", "64-32-48", "ffma", "fp32"), ("rgcn", "2rel", "-", "fp32"), ("rgcn", "1rel", "tf32x3", "fp32")]
 LOOPBACK += [(f, "-", t, "fp32") for f in ("gat", "sage") for t in ("ffma", "tf32x3")] + [("lightgcn", "-", "-", "fp32")]
 
 
-def _layers(family, width, dev, n, dtype):
+def _stack(family, variant, dtype, g, emb):
+    """a three-layer SequentialGNN of `family` over g with the embedding table emb, concatenating every layer's output"""
     from deep_cbrs_amar_renaissance_b200.keras_like import set_seed
     from deep_cbrs_amar_renaissance_b200.layers import GATConv, GCNConv, GraphSageConv, LightGCNConv, RGCNConv
+    from deep_cbrs_amar_renaissance_b200.models.gnn import SequentialGNN
     set_seed(23)
-    make = {"gcn": lambda: GCNConv(width, activation="relu"), "rgcn": lambda: RGCNConv(width, 2, activation="relu"),
-            "gat": lambda: GATConv(width, activation="relu", dropout_rate=0.0),
-            "sage": lambda: GraphSageConv(width, activation="relu"), "lightgcn": lambda: LightGCNConv()}[family]
-    layers = [make() for _ in range(3)]
-    for l, ly in enumerate(layers):
-        ly.build([(n, width), None])
-        ly.built = True
-        if getattr(ly, "bias", None) is not None:
-            with torch.no_grad():
-                ly.bias.copy_(_randn(ly.bias.shape, dev, 30 + l, 0.1))
-        if dtype == "bf16":
-            ly.feature_dtype = "bf16"
-    return layers
-
-
-def _loopback(family, pipeline, g, emb, layers, cuts, zdt):
-    """The layer loop of RowPartition._propagate_peer with every rank run in turn; returns [[copy per rank] per layer]."""
-    from deep_cbrs_amar_renaissance_b200 import _lib as L
-    from deep_cbrs_amar_renaissance_b200 import ops
-    n, dev, world = emb.shape[0], emb.device, len(cuts) - 1
-    ranks = range(world)
-    own = [(cuts[r], cuts[r + 1]) for r in ranks]
-    full = g.raw if family in ("gat", "sage") else g.norm
-    slices = [full.row_slice(a, b) for a, b in own]
-    x = [emb] * world             # every rank's layer input: the replicated table, then its copy of the last output
-    outs, keep, z_ahead = [], [], None
-    for l, ly in enumerate(layers):
-        nxt = layers[l + 1] if l + 1 < len(layers) else None
-        o = _Sym(world, n, getattr(ly, "channels", emb.shape[1]), F32, dev)
-        if family == "gcn" and pipeline == "replicate":
-            for r in ranks:       # the whole transform on every rank, own rows of the output to everybody
-                z = torch.empty(n, ly.channels, dtype=zdt, device=dev)
-                ops.gcn_transform(x[r], ly.kernel, n, out=z)
-                ov = o.copies[r][own[r][0]:own[r][1]]
-                ops.spmm(slices[r], z, ov, bias=ly.bias, relu=True, peers=o.sb[r].peer_addrs(ov))
-        elif family in ("gcn", "rgcn"):
-            kernels = ly.kernels if family == "rgcn" else [ly.kernel]
-            zs, z_ahead = z_ahead, None
-            if zs is None:        # own rows of the transform, stored into every rank's copy ("off")
-                zs = _Sym(world, len(kernels) * n, ly.channels, zdt, dev)
-                for r in ranks:
-                    a, b = own[r]
-                    if len(kernels) > 1:
-                        zv = zs.copies[r][a:(len(kernels) - 1) * n + b]
-                        ops.dense_grouped(x[r][a:b], kernels, zv, n, peers=zs.sb[r].peer_addrs(zv))
-                    else:
-                        zv = zs.copies[r][a:b]
-                        ops.gcn_transform(x[r][a:b], kernels[0], n, out=zv, peers=zs.sb[r].peer_addrs(zv))
-            keep.append(zs)
-            if pipeline == "fused" and nxt is not None:   # the sparse kernel also produces the next transform
-                z_ahead = _Sym(world, n, nxt.channels, F32, dev)
-                for r in ranks:
-                    a, b = own[r]
-                    ov, zv = o.copies[r][a:b], z_ahead.copies[r][a:b]
-                    ops.spmm_gcn_fused(slices[r], zs.copies[r], ov, ly.bias, True, nxt.kernel, zv,
-                                       y_peers=o.sb[r].peer_addrs(ov), z_peers=z_ahead.sb[r].peer_addrs(zv))
-            else:
-                ahead = pipeline in ("kernel", "ce") and nxt is not None
-                if ahead:
-                    z_ahead = _Sym(world, n, nxt.channels, zdt, dev)
-                for r in ranks:
-                    a, b = own[r]
-                    ov = o.copies[r][a:b]
-                    ops.spmm(slices[r], zs.copies[r], ov, bias=ly.bias, relu=True, peers=o.sb[r].peer_addrs(ov))
-                    if ahead:     # the next layer's transform of these rows, to every rank's copy
-                        zv = z_ahead.copies[r][a:b]
-                        if pipeline == "ce":
-                            ops.gcn_transform(ov, nxt.kernel, n, out=zv)
-                            for addr in z_ahead.sb[r].peer_addrs(zv):
-                                ops.peer_copy(addr, zv)
-                        else:
-                            ops.gcn_transform(ov, nxt.kernel, n, out=zv, peers=z_ahead.sb[r].peer_addrs(zv))
-        elif family == "gat":
-            zs, qs = _Sym(world, n, ly.channels, F32, dev), _Sym(world, n, 1, F32, dev)
-            ps = [torch.empty(n, 1, device=dev) for _ in ranks]
-            keep += [zs, qs]
-            for r in ranks:       # transform locally, then push the finished block of z and q
-                a, b = own[r]
-                zv = zs.copies[r][a:b]
-                _, pp, _ = ops.gat_transform(x[r][a:b], ly.kernel.reshape(x[r].shape[1], ly.channels),
-                                             ly.attn_kernel_self.reshape(-1), ly.attn_kernel_neighs.reshape(-1), n,
-                                             out=zv, q_out=qs.copies[r][a:b, 0])
-                ops.push_rows(zv, zs.sb[r])
-                ops.push_rows(qs.copies[r][a:b], qs.sb[r])
-                ps[r][a:b, 0].copy_(pp)
-            for r in ranks:
-                a, b = own[r]
-                ov = o.copies[r][a:b]
-                ops.gat(slices[r], zs.copies[r], ps[r].reshape(-1), qs.copies[r].reshape(-1), ov, bias=ly.bias, relu=True,
-                        row_offset=a, peers=o.sb[r].peer_addrs(ov))
-        elif family == "sage":
-            for r in ranks:
-                a, b = own[r]
-                agg = torch.empty(b - a, x[r].shape[1], device=dev)
-                ops.spmm(slices[r], x[r], agg, agg=L.AGG_MEAN)
-                ov = o.copies[r][a:b]
-                ops.sage_dense(x[r][a:b], agg, ly.kernel, ly.bias, ly.activation, n, out=ov)
-                ops.push_rows(ov, o.sb[r])
-        else:
-            for r in ranks:
-                ov = o.copies[r][own[r][0]:own[r][1]]
-                ops.spmm(slices[r], x[r], ov, peers=o.sb[r].peer_addrs(ov))
-        outs.append(o.copies)
-        keep.append(o)
-        x = o.copies
-    torch.cuda.synchronize()
-    return outs
+    make = {"gcn": lambda w: GCNConv(w, activation="relu"),
+            "rgcn": lambda w: RGCNConv(w, 2 if variant == "2rel" else 1, activation="relu"),
+            "gat": lambda w: GATConv(w, activation="relu", dropout_rate=0.0),
+            "sage": lambda w: GraphSageConv(w, activation="relu"), "lightgcn": lambda w: LightGCNConv()}[family]
+    widths = [64, 32, 48] if variant == "64-32-48" else [emb.shape[1]] * 3
+    seq = SequentialGNN(g, [make(w) for w in widths], embedding_dim=emb.shape[1], final_node="concatenation")
+    seq.build_layers()
+    with torch.no_grad():
+        seq.embeddings.copy_(emb)
+        for l, ly in enumerate(seq.seq_layers):
+            if getattr(ly, "bias", None) is not None:
+                ly.bias.copy_(_randn(ly.bias.shape, emb.device, 30 + l, 0.1))
+    if dtype == "bf16":
+        seq.set_feature_dtype("bf16")
+    return seq
 
 
 @pytest.fixture(scope="module")
@@ -703,17 +631,18 @@ def loopback_adj():
 
 
 @pytest.mark.parametrize("blocked", [False, True], ids=["row-major", "blocked"])
-@pytest.mark.parametrize("family,pipeline,transform,dtype", LOOPBACK, ids=["-".join(c) for c in LOOPBACK])
-def test_partitioned_layer_loop_loopback(dev, loopback_adj, monkeypatch, family, pipeline, transform, dtype, blocked):
+@pytest.mark.parametrize("family,variant,transform,dtype", LOOPBACK, ids=["-".join(c) for c in LOOPBACK])
+def test_partitioned_layer_loop_loopback(dev, loopback_adj, monkeypatch, family, variant, transform, dtype, blocked):
+    from deep_cbrs_amar_renaissance_b200 import _lib as L
     from deep_cbrs_amar_renaissance_b200 import graph as G
     from deep_cbrs_amar_renaissance_b200 import ops
-    adj, (nu, ni, _) = loopback_adj
+    adj, sizes = loopback_adj
     n = adj.shape[0]
     monkeypatch.setattr(G, "FORCED_BLOCKING", (97, 25) if blocked else None)
     if transform != "-":
         monkeypatch.setattr(ops, "GCN_TRANSFORM", transform)
-    if family == "rgcn":          # item <-> property links are relation 1 (tests/helpers.relation_blocks)
-        rel = ((adj.row >= nu + ni) | (adj.col >= nu + ni)).astype(np.int32)
+    if variant == "2rel":         # item <-> property links are relation 1 (tests/helpers.relation_blocks)
+        rel = ((adj.row >= sizes[0] + sizes[1]) | (adj.col >= sizes[0] + sizes[1])).astype(np.int32)
 
         def t(v, dt):
             return torch.from_numpy(np.ascontiguousarray(v, dt)).to(dev)
@@ -721,21 +650,18 @@ def test_partitioned_layer_loop_loopback(dev, loopback_adj, monkeypatch, family,
                           n_rel=2)
     else:
         g = G.DeviceGraph.from_scipy(adj, dev, chunk_edges=16)
-    width = 128 if family == "gcn" else 64
-    emb = _randn((n, width), dev, 11)
-    layers = _layers(family, width, dev, n, dtype)
-    full = g.raw if family in ("gat", "sage") else g.norm
+    emb = _randn((n, 128 if family == "gcn" else 64), dev, 11)
+    if variant == "1rel":
+        assert ops.tf32x3_chosen(n, 64, 64, emb)
+    seq = _stack(family, variant, dtype, g, emb)
+    full = g.raw if family in ("gat", "sage") else g.norm    # built before the threads start, which only read it
     assert full.blocking == ((97, 25) if blocked else (0, 0)) and full.chunks["n_heavy"] > 0
-    ref, h = [], emb
-    for ly in layers:             # the single-GPU layer loop
-        h = ly([h, g])
-        ref.append(h)
-    torch.cuda.synchronize()
+    ref = seq.call(None).clone()  # the single-GPU layer loop
+    L.load()
     hv = _heavy_row(full)
     for cuts in ([0, hv, n], [0, 37, hv + 1, n]):     # uneven cuts; a rank starts, or ends, at a heavy row
-        zdt = BF16 if dtype == "bf16" else F32
-        outs = _loopback(family, pipeline, g, emb, layers, cuts, zdt)
-        for l, copies in enumerate(outs):
-            for r, c in enumerate(copies):
-                assert same_bits(c, ref[l]), "%s %s %s %s: layer %d, copy of rank %d of %d (cuts %s)" % (
-                    family, pipeline, transform, dtype, l, r, len(cuts) - 1, cuts)
+        shared, parts = _ranks(sizes, cuts, dev)
+        for r, got in enumerate(_propagate_on_every_rank(shared, parts, seq)):
+            for k, out in enumerate(got):
+                assert same_bits(out, ref), "%s %s %s %s: call %d, rank %d of %d (cuts %s)" % (
+                    family, variant, transform, dtype, k, r, len(cuts) - 1, cuts)

@@ -99,10 +99,6 @@ def main():
     z, p, q = ops.dense(x, w, rowop=L.ROWOP_ATTN, a_self=a_s, a_neigh=a_n)
     ms = timeit(lambda: ops.gat(raw, z, p, q, out, bias=bias, relu=True))
     report("GAT fused score+softmax+aggregate (raw A + self loops)", ms, raw.nnz + n, raw.nnz * (8 + d * s) + n * (d * s + 16))
-    # GCN sparse step fused with the next layer's transform (no peers here: isolates the cost of the row x W product)
-    zn = torch.empty(n, d, device=dev)
-    ms = timeit(lambda: ops.spmm_gcn_fused(norm, x, out, bias, True, w, zn))
-    report("GCN SpMM + next transform fused (cbrs_spmm_gcn_fused)", ms, norm.nnz, norm.nnz * (8 + d * s) + n * (2 * d * s + 8))
     # bf16 operand storage
     z16 = x.to(torch.bfloat16)
     ms = timeit(lambda: ops.spmm(norm, z16, out, bias=bias, relu=True))
