@@ -42,6 +42,9 @@ _SIGS = {
     "cbrs_chunks_blocked_count": (c_int, [P, P, c_int64, c_int64, c_int64, c_int32, c_int32, c_int64, P, P, c_size_t, P]),
     "cbrs_chunks_blocked_fill": (c_int, [P, P, c_int64, c_int64, c_int64, c_int32, c_int32, c_int64, P, P, P, P, P, P, P,
                                          c_size_t, P]),
+    "cbrs_csr_subset_workspace_bytes": (c_size_t, [POINTER(CsrDesc)]),
+    "cbrs_csr_subset_count": (c_int, [POINTER(CsrDesc), P, c_int64, P, P, c_size_t, P]),
+    "cbrs_csr_subset_fill": (c_int, [POINTER(CsrDesc), P, P, P, P, P, P, P, c_size_t, P]),
     "cbrs_spmm_workspace_bytes": (c_size_t, [POINTER(CsrDesc), c_int32]),
     "cbrs_spmm_csr": (c_int, [POINTER(CsrDesc), P, c_int64, P, c_int64, c_int32, c_int, P, c_int, c_int, P, c_size_t, P]),
     "cbrs_gat_workspace_bytes": (c_size_t, [POINTER(CsrDesc), c_int32]),

@@ -42,6 +42,26 @@ def blocking_policy(n_cols):
     return cols, min_len
 
 
+# Per-batch model call: a GCN / LightGCN stack whose layers are concatenated is read by the scorer only at the batch's
+# rows, so its LAST layer's sparse product may run on those rows alone (graph.CsrSubset).  Layers before it stay full:
+# their outputs feed the last layer at every neighbour.  The subset costs a few passes over the chunk list and one
+# small device-to-host copy per call; on graphs of at least this many rows that is far below the rows it skips
+# (config 5, 1.1e7 rows: ~3.5 % of the last layer's edges are needed by a 65,536-pair batch).  The MovieLens-1M-sized
+# graphs (~1e4 rows, a batch needs ~40 % of them) stay on the full product, and their launch count.
+SUBSET_MIN_ROWS = 1 << 20
+FORCED_SUBSET = None        # True / False: tests decide the size condition with it
+
+
+def last_layer_subset_policy(n_rows, partitioned, concatenated, last_layer_gcn):
+    """True when the per-batch call computes the last layer's sparse product only at the rows its batch scores.
+    Never under a row partition, for other reductions or layer families, or while a CUDA graph is being captured (a
+    replay must stay valid for any ids)."""
+    if partitioned or not concatenated or not last_layer_gcn:
+        return False
+    large = bool(FORCED_SUBSET) if FORCED_SUBSET is not None else n_rows >= SUBSET_MIN_ROWS
+    return large and not torch.cuda.is_current_stream_capturing()
+
+
 class CsrSlice:
     """Rows [row_offset, row_offset + n_rows) of a CSR matrix plus its work decomposition."""
 
@@ -54,19 +74,7 @@ class CsrSlice:
         self.chunk_edges = chunk_edges
         self.blocking = blocking_policy(n_cols) if blocking is None else tuple(blocking)
         self.chunks = ops.build_chunks(rowptr, chunk_edges, colidx, n_cols, *self.blocking)
-        c = self.chunks
-        d = L.CsrDesc()
-        d.n_rows, d.nnz = self.n_rows, self.nnz
-        d.rowptr, d.colidx = rowptr.data_ptr(), colidx.data_ptr()
-        d.vals = vals.data_ptr() if vals is not None else None
-        d.chunk_edges, d.n_chunks = chunk_edges, c["n_chunks"]
-        d.chunk_row, d.chunk_begin, d.chunk_slot = (c["chunk_row"].data_ptr(), c["chunk_begin"].data_ptr(),
-                                                    c["chunk_slot"].data_ptr())
-        d.n_heavy, d.n_slots = c["n_heavy"], c["n_slots"]
-        d.heavy_row = c["heavy_row"].data_ptr() if c["n_heavy"] else None
-        d.heavy_slot_ptr = c["heavy_slot_ptr"].data_ptr()
-        d.chunk_len = c["chunk_len"].data_ptr() if c["chunk_len"] is not None else None
-        self.desc = d
+        self.desc = _desc(self, self.chunks)
 
     def row_slice(self, r0, r1, chunk_edges=None):
         """Rows [r0, r1) with global column ids (1-D row partition, SURVEY 8e)."""
@@ -75,6 +83,10 @@ class CsrSlice:
         vals = self.vals[b:e].contiguous() if self.vals is not None else None
         return CsrSlice(rowptr, self.colidx[b:e].contiguous(), vals, self.n_cols,
                         chunk_edges or self.chunk_edges, self.row_offset + r0, blocking=self.blocking)
+
+    def row_subset(self, ids):
+        """The rows `ids` of this slice as a CsrSubset (int64 device ids, local row numbers)."""
+        return CsrSubset(self, ids)
 
     def coo_rows(self):
         """row id of every stored entry (int32 [nnz])"""
@@ -98,6 +110,38 @@ class CsrSlice:
         vals = (self.vals if self.vals is not None else torch.ones_like(self.colidx, dtype=torch.float32)).cpu().numpy()
         return sparse.csr_matrix((vals, self.colidx.cpu().numpy(), self.rowptr.cpu().numpy()),
                                  shape=(self.n_rows, self.n_cols))
+
+
+def _desc(csr, c):
+    """cbrs_csr_t of the matrix held by `csr` under the chunk decomposition `c` (ops.build_chunks / ops.csr_subset)"""
+    d = L.CsrDesc()
+    d.n_rows, d.nnz = csr.n_rows, csr.colidx.numel()
+    d.rowptr, d.colidx = csr.rowptr.data_ptr(), csr.colidx.data_ptr()
+    d.vals = csr.vals.data_ptr() if csr.vals is not None else None
+    d.chunk_edges, d.n_chunks = csr.chunk_edges, c["n_chunks"]
+    d.chunk_row, d.chunk_begin, d.chunk_slot = (c["chunk_row"].data_ptr(), c["chunk_begin"].data_ptr(),
+                                                c["chunk_slot"].data_ptr())
+    d.n_heavy, d.n_slots = c["n_heavy"], c["n_slots"]
+    d.heavy_row = c["heavy_row"].data_ptr() if c["n_heavy"] else None
+    d.heavy_slot_ptr = c["heavy_slot_ptr"].data_ptr()
+    d.chunk_len = c["chunk_len"].data_ptr() if c["chunk_len"] is not None else None
+    return d
+
+
+class CsrSubset:
+    """Some rows of a CsrSlice: the same matrix, with only those rows' chunks, in their original order, and their
+    partial slots renumbered in order (cbrs_csr_subset_*).  A propagation launch on it writes exactly those rows of its
+    [n_rows, D] output, each with the bits the full launch gives it, and leaves every other row as it was."""
+
+    def __init__(self, full, ids):
+        self.full = full    # keeps the shared rowptr / colidx / vals alive
+        self.rowptr, self.colidx, self.vals = full.rowptr, full.colidx, full.vals
+        self.n_rows, self.n_cols, self.row_offset = full.n_rows, full.n_cols, full.row_offset
+        self.chunk_edges, self.blocking = full.chunk_edges, full.blocking
+        self.chunks = ops.csr_subset(full, ids)
+        self.n_needed = self.chunks["rows"]     # distinct rows a launch computes
+        self.nnz = self.chunks["edges"]         # the edges it gathers
+        self.desc = _desc(self, self.chunks)
 
 
 class DeviceGraph:

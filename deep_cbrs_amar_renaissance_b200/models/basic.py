@@ -11,7 +11,7 @@ import torch
 
 from ..keras_like import Model, default_device
 from .dense import build_dense_classifier, build_dense_network
-from .gnn import GAT, GCN, DGCF, RGCN, GraphSage, LightGCN
+from .gnn import GAT, GCN, DGCF, GNN, RGCN, GraphSage, LightGCN
 from .tsgnn import TwoStepDGCF, TwoStepGAT, TwoStepGCN, TwoStepGraphSage, TwoStepLightGCN
 from .twgnn import TwoWayDGCF, TwoWayGAT, TwoWayGCN, TwoWayGraphSage, TwoWayLightGCN
 
@@ -90,6 +90,15 @@ class BasicGNN(Model, abc.ABC):
         return self
 
     def call(self, inputs, **kwargs):
+        seq = getattr(self.gnn, "gnn_layers", None)
+        if not self.cache_propagation and isinstance(self.gnn, GNN) and seq.last_layer_subset():
+            # the scorer reads the table at the batch's rows only: the last layer is computed there alone.  The
+            # partly filled table never leaves this call (nor stays cached)
+            u, i = inputs
+            u, i = _ids(u), _ids(i)
+            self._cached = None
+            emb = seq._run(seq.embeddings, rows=torch.cat([u, i]))
+            return self.rs.call_sources((emb, u), (emb, i))
         updated_embeddings = self.propagate()
         return self.embed_recommend(updated_embeddings, inputs)
 

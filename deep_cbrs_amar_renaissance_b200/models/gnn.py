@@ -10,6 +10,7 @@ import abc
 
 import torch
 
+from .. import graph
 from ..graph import DeviceGraph
 from ..keras_like import L2, Model, default_device
 from ..layers import DGCFConv, GATConv, GCNConv, GraphSageConv, LightGCNConv, ReductionLayer, RGCNConv
@@ -80,10 +81,22 @@ class SequentialGNN(Model):
             return self.partition.propagate(self)
         return self._run(self.embeddings)
 
-    def _run(self, x):
-        """the layer loop + reduction of gnn.py:74-84 on the initial node features x"""
+    def last_layer_subset(self):
+        """True when a call that only reads the output at some rows may run the last layer's sparse product on those
+        rows alone (graph.last_layer_subset_policy)."""
+        last = self.seq_layers[-1] if self.seq_layers else None
+        return graph.last_layer_subset_policy(self.n_nodes, self.partition is not None,
+                                              self.final_node == 'concatenation',
+                                              isinstance(last, (GCNConv, LightGCNConv)))
+
+    def _run(self, x, rows=None):
+        """the layer loop + reduction of gnn.py:74-84 on the initial node features x.
+        rows (int64 device ids; only when last_layer_subset() holds): the last layer's output is computed at these
+        rows only - every other row of its slice is left unfilled, so the result must not leave the caller."""
         n = x.shape[0]
         if self.final_node == 'concatenation':
+            # the subset is built before layer 1 is enqueued: its one device-to-host copy exposes only a launch gap
+            last_csr = self.adj_matrix.norm.row_subset(rows) if rows is not None else None
             widths = self._widths()
             if self._buf is None or self._buf.shape != (n, sum(widths)):
                 self._buf = torch.empty(n, sum(widths), dtype=torch.float32, device=x.device)
@@ -91,9 +104,12 @@ class SequentialGNN(Model):
             buf[:, :widths[0]].copy_(x)
             hs = [buf[:, :widths[0]]]
             off = widths[0]
-            for layer, w in zip(self.seq_layers, widths[1:]):
+            for k, (layer, w) in enumerate(zip(self.seq_layers, widths[1:])):
                 out = buf[:, off:off + w]
-                x = layer([x, self.adj_matrix], out=out)
+                if last_csr is not None and k == len(self.seq_layers) - 1:
+                    x = layer([x, self.adj_matrix], out=out, csr=last_csr)
+                else:
+                    x = layer([x, self.adj_matrix], out=out)
                 hs.append(out)
                 off += w
             for h in hs:

@@ -118,6 +118,33 @@ def build_chunks(rowptr, chunk_edges, colidx=None, n_cols=0, block_cols=0, block
                 heavy_slot_ptr=heavy_slot_ptr, chunk_len=chunk_len)
 
 
+def csr_subset(csr, ids):
+    """Chunk decomposition of the rows `ids` (int64, any order, duplicates allowed, out-of-range ids ignored) of a
+    graph.CsrSlice, as build_chunks returns it plus rows / edges (the distinct needed rows and their edge count).
+    One device-to-host copy of the counts (cbrs_csr_subset_*)."""
+    lib = L.load()
+    dev = csr.rowptr.device
+    desc = ctypes.byref(csr.desc)
+    ws = _ws(lib.cbrs_csr_subset_workspace_bytes(desc), dev)
+    counts = torch.empty(5, dtype=torch.int64, device=dev)
+    L.check(lib.cbrs_csr_subset_count(desc, _ptr(ids, torch.int64), ids.numel(), _ptr(counts), _ptr(ws), ws.numel(),
+                                      _stream()), "cbrs_csr_subset_count")
+    n_chunks, n_heavy, n_slots, rows, edges = (int(v) for v in counts.tolist())
+    chunk_row = torch.empty(max(n_chunks, 1), dtype=torch.int32, device=dev)
+    chunk_begin = torch.empty(max(n_chunks, 1), dtype=torch.int64, device=dev)
+    chunk_slot = torch.empty(max(n_chunks, 1), dtype=torch.int32, device=dev)
+    chunk_len = torch.empty(max(n_chunks, 1), dtype=torch.int32, device=dev) if csr.desc.chunk_len else None
+    heavy_row = torch.empty(max(n_heavy, 1), dtype=torch.int32, device=dev)
+    heavy_slot_ptr = torch.zeros(n_heavy + 1, dtype=torch.int64, device=dev)
+    L.check(lib.cbrs_csr_subset_fill(desc, _ptr(chunk_row), _ptr(chunk_begin), _ptr(chunk_len), _ptr(chunk_slot),
+                                     _ptr(heavy_row), _ptr(heavy_slot_ptr), _ptr(ws), ws.numel(), _stream()),
+            "cbrs_csr_subset_fill")
+    return dict(n_chunks=n_chunks, n_heavy=n_heavy, n_slots=n_slots, chunk_row=chunk_row[:n_chunks],
+                chunk_begin=chunk_begin[:n_chunks], chunk_slot=chunk_slot[:n_chunks], heavy_row=heavy_row[:n_heavy],
+                heavy_slot_ptr=heavy_slot_ptr, chunk_len=chunk_len[:n_chunks] if chunk_len is not None else None,
+                rows=rows, edges=edges)
+
+
 # ------------------------------------------------------------------ propagation
 def _ptr_array(addresses):
     """host array of device addresses for the *_bcast entry points"""
@@ -158,9 +185,11 @@ def spmm(csr, x, out, agg=L.AGG_WEIGHTED, bias=None, relu=False, workspace=None,
     if PROFILE_ON:
         e1.record()
         # algorithmic bytes of this launch (SURVEY 8d): nnz*(4 col + 4 val + d*4 row) + rows*(d*4 out + 8 rowptr)
+        # (a graph.CsrSubset counts the rows and edges it computes)
         xb = x.element_size()
-        PROFILE.append(("spmm", e0, e1, {"nnz": csr.nnz, "rows": csr.n_rows, "d": d,
-                                         "bytes": csr.nnz * (8 + xb * d) + csr.n_rows * (4 * d + 8)}))
+        rows = getattr(csr, "n_needed", csr.n_rows)
+        PROFILE.append(("spmm", e0, e1, {"nnz": csr.nnz, "rows": rows, "d": d,
+                                         "bytes": csr.nnz * (8 + xb * d) + rows * (4 * d + 8)}))
     _count(1 + (1 if csr.chunks["n_heavy"] else 0))
     return out
 

@@ -129,6 +129,20 @@ int cbrs_chunks_blocked_fill(const int64_t *rowptr, const int32_t *colidx, int64
                              int32_t *heavy_row, int64_t *heavy_slot_ptr, void *workspace,
                              size_t workspace_bytes, void *stream);
 
+/* Row subset of a decomposition: the chunks of the rows listed in ids[0, n_ids) (duplicates allowed; ids outside
+ * [0, n_rows) select nothing), in their original list order, with the needed heavy rows and their slots renumbered
+ * compactly in the same order.  The result shares rowptr/colidx/vals/chunk_edges with g; a propagation kernel run on
+ * it writes exactly the needed rows of Y, with the bits the full launch gives them.
+ * Pass 1: counts_out (device int64[5]) = {n_chunks, n_heavy, n_slots, needed rows, their edges}.
+ * Pass 2: fill (same workspace, untouched since pass 1); chunk_len is written when g has one, heavy_slot_ptr
+ * [n_heavy + 1] must come zeroed.  The subset's spmm workspace is at most cbrs_spmm_workspace_bytes(g, d).        */
+size_t cbrs_csr_subset_workspace_bytes(const cbrs_csr_t *g);
+int cbrs_csr_subset_count(const cbrs_csr_t *g, const int64_t *ids, int64_t n_ids, int64_t *counts_out,
+                          void *workspace, size_t workspace_bytes, void *stream);
+int cbrs_csr_subset_fill(const cbrs_csr_t *g, int32_t *chunk_row, int64_t *chunk_begin, int32_t *chunk_len,
+                         int32_t *chunk_slot, int32_t *heavy_row, int64_t *heavy_slot_ptr, void *workspace,
+                         size_t workspace_bytes, void *stream);
+
 /* ---- propagation kernels (rows P1, P2 aggregate, P4) ---------------------
  * Y[i, 0:D] = epilogue( reduce_j A_ij * X[col_j, 0:D] ), j over row i ascending.
  * Replaces tf.sparse.sparse_dense_matmul as invoked by spektral GCNConv /
