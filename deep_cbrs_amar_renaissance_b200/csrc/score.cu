@@ -218,7 +218,8 @@ static size_t score_smem_bytes(int c1, int k) {
 template <int CT>
 static int launch_score(const ScoreParams &p, cudaStream_t s) {
     const size_t smem = score_smem_bytes<CT>(p.c1, p.k);
-    CBRS_REQUIRE(smem <= 200 * 1024, CBRS_E_UNSUPPORTED, "score_catalog: needs %zu bytes of shared memory", smem);
+    // up to the 227 KB a CTA may have: the widest classifier (c1 = 256, c2 = 128) at k = 128 needs 217 KB
+    CBRS_REQUIRE(smem <= 227 * 1024, CBRS_E_UNSUPPORTED, "score_catalog: needs %zu bytes of shared memory", smem);
     auto kernel = p.excl_rowptr ? score_catalog_kernel<CT, true> : score_catalog_kernel<CT, false>;
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     CBRS_REQUIRE(e == cudaSuccess, CBRS_E_CUDA, "score_catalog: cudaFuncSetAttribute: %s", cudaGetErrorString(e));

@@ -165,8 +165,8 @@ class HybridBertGNN(Model, abc.ABC):
           * feature-based scorer with the reference grids' shapes (dense3a / dense3b two 64-wide relu layers,
             classifier 64 -> 64 -> 1, plain concatenation, no residual, content table set, k <= 128):
             precision 'fp32' the chained 3xTF32 tensor-core kernel (cbrs_score_hybrid_topk_tf32x3, fp32 accuracy,
-            1e-5; also needs k <= n_items), 'bf16' the chained bf16 kernel (cbrs_score_hybrid_topk_bf16);
-            'fp32-ffma' the generic pair pipeline;
+            1e-5), 'bf16' the chained bf16 kernel (cbrs_score_hybrid_topk_bf16), both when k <= n_items;
+            'fp32-ffma' and k > n_items the generic pair pipeline;
           * entity-based scorer with plain concatenation: the fused BasicRS kernels, as BasicGNN.recommend_top_k;
           * any other shape, and fused=False: the generic blocked pair pipeline (HybridCBRS.tail over item blocks)."""
         from ..scoring import catalog_top_k

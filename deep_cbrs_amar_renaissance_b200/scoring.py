@@ -209,12 +209,12 @@ def _fused_basic(model, emb, users, items, k, precision="fp32", exclude=None):
 def _fused_hybrid_feature(model, emb, users, items, k, exclude=None, precision="bf16"):
     """Feature-based HybridCBRS with the shapes of every hybrid grid of the reference (dense3a / dense3b = two 64-wide
     layers, classifier 64 -> 64 -> 1, relu, plain concatenation) -> a chained tensor-core kernel: precision 'bf16'
-    cbrs_score_hybrid_topk_bf16 (bf16 operands), 'fp32' cbrs_score_hybrid_topk_tf32x3 (3xTF32, fp32 accuracy; k must
-    not exceed the catalog).  None when the scorer has another shape or the precision has no such kernel."""
+    cbrs_score_hybrid_topk_bf16 (bf16 operands), 'fp32' cbrs_score_hybrid_topk_tf32x3 (3xTF32, fp32 accuracy).  None
+    when the scorer has another shape, the precision has no such kernel or k exceeds the catalog."""
     rs = model.rs
     if hasattr(rs, "unet") or not rs.feature_based or rs.residual is not None or model.content_table is None or k > 128:
         return None
-    if precision not in ("bf16", "fp32") or (precision == "fp32" and k > items.numel()):
+    if precision not in ("bf16", "fp32") or k > items.numel():   # both chained kernels refuse k > n_items
         return None
     if any(f.method != 'concatenate' for f in (rs.fuse1a, rs.fuse1b, rs.fuse2)):
         return None
@@ -259,8 +259,9 @@ def catalog_top_k(model, emb, n_users, n_items, k=10, users=None, user_block=Non
     score = _pair_scorer(model, emb, users, items)
     cache = {}
     ub, ib = _blocks(users.numel(), n_items, user_block)
-    ids = torch.empty(users.numel(), k, dtype=torch.int32, device=dev)
-    vals = torch.empty(users.numel(), k, dtype=torch.float32, device=dev)
+    # slots past the catalog (k > n_items) keep -1 / -inf, as the fused kernels write them
+    ids = torch.full((users.numel(), k), -1, dtype=torch.int32, device=dev)
+    vals = torch.full((users.numel(), k), -float("inf"), dtype=torch.float32, device=dev)
     for u0 in range(0, users.numel(), ub):
         nb = min(ub, users.numel() - u0)
         best_i = best_v = None

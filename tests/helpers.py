@@ -2,6 +2,8 @@
 import numpy as np
 from scipy import sparse
 
+from oracle import layers as ol
+
 RTOL = 1e-5  # north star: embeddings and scores within 1e-5 relative (fp32)
 
 
@@ -58,6 +60,127 @@ def assert_topk_equivalent(ids, vals, oracle_scores, k, tol=2e-6):
     clear = (gaps > tol) & (prev_gap > tol)
     assert (ids[clear] == order[clear]).all(), "top-k ids differ where the ranking is unambiguous"
     return float(clear.mean()) if clear.size else 1.0
+
+
+# ------------------------------------------------------------------ catalog scorer oracles
+def bf16_round(x):
+    """round-to-nearest-even fp32 -> bf16 -> fp32 (numpy)"""
+    u = np.asarray(x, np.float32).view(np.uint32).astype(np.uint64)
+    u = (u + 0x7FFF + ((u >> 16) & 1)) & 0xFFFF0000
+    return u.astype(np.uint32).view(np.float32)
+
+
+def tf32_round(x):
+    """round to the nearest tf32 (10 explicit mantissa bits), ties away from zero as cvt.rna"""
+    b = np.asarray(x, np.float32).view(np.uint32).astype(np.uint64)
+    return ((b + 0x1000) & 0xFFFFE000).astype(np.uint32).view(np.float32)
+
+
+def _user_blocks(n_users, n_items, pairs=1 << 17):
+    step = max(1, pairs // max(n_items, 1))
+    return [(u0, min(u0 + step, n_users)) for u0 in range(0, n_users, step)]
+
+
+def basic_chain(P, Q, w2, b2, w3, b3):
+    """The fused BasicRS scorer (cbrs_score_catalog_topk*) in float64: sigmoid(relu(relu(P[u] + Q[i]) W2 + b2) w3 + b3)
+    for every (user, item) -> [U, I]"""
+    f8 = np.float64
+    out = np.empty((len(P), len(Q)))
+    for u0, u1 in _user_blocks(len(P), len(Q)):
+        h1 = np.maximum(P[u0:u1, None, :].astype(f8) + Q[None, :, :], 0)
+        h2 = np.maximum(h1 @ w2.astype(f8) + b2, 0)
+        out[u0:u1] = 1.0 / (1.0 + np.exp(-(h2 @ w3.astype(f8) + f8(b3[0]))))
+    return out
+
+
+def bf16_basic_chain(P, Q, w2, b2, w3, b3):
+    """The bf16 catalog scorer (cbrs_score_catalog_topk_bf16) with its operands rounded where each kernel variant rounds
+    them, sums in float64 -> [U, I].  Tolerances of the kernels against it: 1e-4 for v3 (c1 <= 64, c2 <= 64: an
+    activation within an fp32 ulp of a bf16 rounding boundary may round the other way before the output product),
+    2e-5 for v2 / v1 (fp32 summation order inside the MMA is unspecified)."""
+    c1, c2 = w2.shape
+    f8 = np.float64
+    out = np.empty((len(P), len(Q)), np.float32)
+    for u0, u1 in _user_blocks(len(P), len(Q)):
+        nu = u1 - u0
+        if c1 <= 64 and c2 <= 128:  # v2 / v3: P and Q rounded first, bf16 add (exact sum rounded once), relu
+            h1 = bf16_round(bf16_round(P[u0:u1])[:, None, :] + bf16_round(Q)[None, :, :])
+            h1 = np.maximum(h1, 0).reshape(-1, c1)
+        else:                       # v1
+            h1 = bf16_round(np.maximum(P[u0:u1, None, :] + Q[None, :, :], 0).reshape(-1, c1))
+        if c1 <= 64 and c2 <= 64:
+            # v3 (every product on the tensor core): the bias is a row of the bf16 image of W2, relu(h1 W2 + b2) is
+            # rounded to bf16 and the output layer is a second product against bf16(w3)
+            acc = h1.astype(f8) @ bf16_round(w2).astype(f8) + bf16_round(b2).astype(f8)
+            h2 = bf16_round(np.maximum(acc, 0).astype(np.float32))
+            s = ol.sigmoid((h2.astype(f8) @ bf16_round(w3).astype(f8)).astype(np.float32) + b3)
+        else:
+            h2 = np.maximum(h1.astype(f8) @ bf16_round(w2).astype(f8) + b2, 0).astype(np.float32)
+            s = ol.sigmoid((h2.astype(f8) @ w3.astype(f8)).astype(np.float32) + b3)
+        out[u0:u1] = s.reshape(nu, len(Q))
+    return out
+
+
+HYBRID_WEIGHTS = ("w3a2", "b3a2", "w3b2", "b3b2", "wc1", "bc1", "wc2", "bc2", "wc3", "bc3")   # argument order
+
+
+def hybrid_tables(n_users, n_items, seed):
+    """Seeded operands of the chained hybrid scorers: tables (P1, Q1, P2, Q2) [*, 64] and the weights by name"""
+    rng = np.random.RandomState(seed)
+    c = 64
+    P1, P2 = (rng.standard_normal((n_users, c)).astype(np.float32) for _ in range(2))
+    Q1, Q2 = (rng.standard_normal((n_items, c)).astype(np.float32) for _ in range(2))
+    w = dict(w3a2=glorot(rng, (c, c)), w3b2=glorot(rng, (c, c)), wc1=glorot(rng, (2 * c, c)), wc2=glorot(rng, (c, c)),
+             wc3=glorot(rng, (c, 1)).reshape(-1), bc3=np.array([0.05], np.float32))
+    for b in ("b3a2", "b3b2", "bc1", "bc2"):
+        w[b] = (rng.standard_normal(c) * 0.1).astype(np.float32)
+    return (P1, Q1, P2, Q2), w
+
+
+def hybrid_chain(P1, Q1, P2, Q2, w, uu, ii, rounded=False):
+    """The chained hybrid scorer in float64: sigmoid scores of the pairs (uu[j], ii[j]); rounded: every product operand
+    rounded to tf32 (a single-TF32 evaluation)"""
+    f8 = np.float64
+    r = (lambda x: tf32_round(x).astype(f8)) if rounded else (lambda x: np.asarray(x, f8))
+    relu = lambda x: np.maximum(x, 0)
+    h1 = relu(P1[uu].astype(f8) + Q1[ii])
+    h2 = relu(P2[uu].astype(f8) + Q2[ii])
+    x1 = relu(r(h1) @ r(w["w3a2"]) + w["b3a2"])
+    x2 = relu(r(h2) @ r(w["w3b2"]) + w["b3b2"])
+    g = relu(r(x1) @ r(w["wc1"][:64]) + r(x2) @ r(w["wc1"][64:]) + w["bc1"])
+    h = relu(r(g) @ r(w["wc2"]) + w["bc2"])
+    return 1.0 / (1.0 + np.exp(-(h @ w["wc3"].astype(f8) + f8(w["bc3"][0]))))
+
+
+def hybrid_chain_scores(tabs, w):
+    """hybrid_chain over every (user, item) -> [U, I] float64"""
+    n_users, n_items = len(tabs[0]), len(tabs[1])
+    out = np.empty((n_users, n_items))
+    for u0, u1 in _user_blocks(n_users, n_items):
+        uu, ii = np.repeat(np.arange(u0, u1), n_items), np.tile(np.arange(n_items), u1 - u0)
+        out[u0:u1] = hybrid_chain(*tabs, w, uu, ii).reshape(u1 - u0, n_items)
+    return out
+
+
+def hybrid_bf16_scores(P1, Q1, P2, Q2, w, rounded=True):
+    """The chained bf16 hybrid scorer (cbrs_score_hybrid_topk_bf16): every MMA operand rounded to bf16 where the kernel
+    rounds it (h1, h2, x1, x2, g and all weight matrices), float64 sums -> [U, I].  rounded=False: the exact fp32 chain."""
+    r = bf16_round if rounded else (lambda x: np.asarray(x, np.float32))
+    f8 = np.float64
+    out = np.empty((len(P1), len(Q1)), np.float32)
+
+    def layer(x, k, b):
+        return np.maximum(r(x).astype(f8) @ r(k).astype(f8) + b, 0).astype(np.float32)
+
+    for u0, u1 in _user_blocks(len(P1), len(Q1)):
+        pairs = lambda P, Q: np.maximum(P[u0:u1, None, :] + Q[None, :, :], 0).reshape(-1, P.shape[1]).astype(np.float32)
+        x1 = layer(pairs(P1, Q1), w["w3a2"], w["b3a2"])
+        x2 = layer(pairs(P2, Q2), w["w3b2"], w["b3b2"])
+        g = layer(np.concatenate([x1, x2], 1), w["wc1"], w["bc1"])
+        h = layer(g, w["wc2"], w["bc2"])
+        logit = (h.astype(f8) @ w["wc3"].astype(f8) + w["bc3"]).astype(np.float32)
+        out[u0:u1] = ol.sigmoid(logit).reshape(u1 - u0, len(Q1))
+    return out
 
 
 def weights_struct(w, proj_first=None):

@@ -12,7 +12,7 @@ import torch
 
 from oracle import graph as og
 from oracle import layers as ol
-from tests.helpers import assert_topk_equivalent, export_weights, glorot, random_bipartite
+from tests.helpers import assert_topk_equivalent, export_weights, hybrid_bf16_scores, hybrid_tables, random_bipartite
 
 pytestmark = pytest.mark.gpu
 
@@ -28,34 +28,11 @@ def _t(a, dev):
     return torch.from_numpy(np.ascontiguousarray(a)).to(dev)
 
 
-def _oracle(P1, Q1, P2, Q2, w, rounded=True):
-    r = ol.bf16_round if rounded else (lambda x: np.asarray(x, np.float32))
-    f8 = np.float64
-
-    def pairs(P, Q):
-        return np.maximum(P[:, None, :] + Q[None, :, :], 0).reshape(-1, P.shape[1]).astype(np.float32)
-
-    def layer(x, k, b):
-        return np.maximum(r(x).astype(f8) @ r(k).astype(f8) + b, 0).astype(np.float32)
-    x1 = layer(pairs(P1, Q1), w["w3a2"], w["b3a2"])
-    x2 = layer(pairs(P2, Q2), w["w3b2"], w["b3b2"])
-    g = layer(np.concatenate([x1, x2], 1), w["wc1"], w["bc1"])
-    h = layer(g, w["wc2"], w["bc2"])
-    return ol.sigmoid((h @ w["wc3"] + w["bc3"]).astype(np.float32)).reshape(len(P1), len(Q1))
-
-
 @pytest.mark.parametrize("n_users,n_items,k", [(37, 1000, 10), (5, 7, 5), (130, 333, 20), (16, 32, 3), (1, 2049, 10),
                                                (4800, 40, 5)])   # 4800 users: 24 users per CTA (one wave of 2 CTAs per SM)
 def test_chained_hybrid_scorer_matches_bf16_oracle(dev, n_users, n_items, k):
     from deep_cbrs_amar_renaissance_b200 import ops
-    rng = np.random.RandomState(n_users + n_items)
-    c = 64
-    P1, P2 = (rng.standard_normal((n_users, c)).astype(np.float32) for _ in range(2))
-    Q1, Q2 = (rng.standard_normal((n_items, c)).astype(np.float32) for _ in range(2))
-    w = dict(w3a2=glorot(rng, (c, c)), w3b2=glorot(rng, (c, c)), wc1=glorot(rng, (2 * c, c)), wc2=glorot(rng, (c, c)),
-             wc3=glorot(rng, (c, 1)).reshape(-1), bc3=np.array([0.05], np.float32))
-    for b in ("b3a2", "b3b2", "bc1", "bc2"):
-        w[b] = (rng.standard_normal(c) * 0.1).astype(np.float32)
+    (P1, Q1, P2, Q2), w = hybrid_tables(n_users, n_items, n_users + n_items)
     ids, vals = ops.score_hybrid_topk_bf16(_t(P1, dev), _t(Q1, dev), _t(P2, dev), _t(Q2, dev), _t(w["w3a2"], dev),
                                            _t(w["b3a2"], dev), _t(w["w3b2"], dev), _t(w["b3b2"], dev), _t(w["wc1"], dev),
                                            _t(w["bc1"], dev), _t(w["wc2"], dev), _t(w["bc2"], dev), _t(w["wc3"], dev),
@@ -65,8 +42,8 @@ def test_chained_hybrid_scorer_matches_bf16_oracle(dev, n_users, n_items, k):
     assert (ids_np >= 0).all() and (ids_np < n_items).all()
     assert all(len(set(row)) == kk for row in ids_np[:, :kk])          # no item twice
     assert (np.diff(vals_np[:, :kk], axis=1) <= 0).all()                 # descending
-    assert_topk_equivalent(ids_np[:, :kk], vals_np[:, :kk], _oracle(P1, Q1, P2, Q2, w), kk, tol=2e-3)
-    exact = _oracle(P1, Q1, P2, Q2, w, rounded=False)
+    assert_topk_equivalent(ids_np[:, :kk], vals_np[:, :kk], hybrid_bf16_scores(P1, Q1, P2, Q2, w), kk, tol=2e-3)
+    exact = hybrid_bf16_scores(P1, Q1, P2, Q2, w, rounded=False)
     got_exact = np.take_along_axis(exact, ids_np[:, :kk].astype(np.int64), axis=1)
     assert np.abs(got_exact - vals_np[:, :kk]).max() < 3e-2
 

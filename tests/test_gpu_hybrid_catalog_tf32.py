@@ -10,7 +10,8 @@ import numpy as np
 import pytest
 import torch
 
-from tests.helpers import assert_topk_equivalent, glorot, random_bipartite
+from tests.helpers import (HYBRID_WEIGHTS, assert_topk_equivalent, hybrid_chain, hybrid_chain_scores, hybrid_tables,
+                           random_bipartite)
 from tests.test_gpu_catalog_exclusion import (GUARD, _Arena, _check_exact, _csr, _guarded_lists, _hybrid_tables,
                                               _item_lists, _random_lists, _rival)
 
@@ -30,72 +31,27 @@ def _t(a, dev):
     return torch.from_numpy(np.ascontiguousarray(a)).to(dev)
 
 
-def _tables(n_users, n_items, seed):
-    rng = np.random.RandomState(seed)
-    c = 64
-    P1, P2 = (rng.standard_normal((n_users, c)).astype(np.float32) for _ in range(2))
-    Q1, Q2 = (rng.standard_normal((n_items, c)).astype(np.float32) for _ in range(2))
-    w = dict(w3a2=glorot(rng, (c, c)), w3b2=glorot(rng, (c, c)), wc1=glorot(rng, (2 * c, c)), wc2=glorot(rng, (c, c)),
-             wc3=glorot(rng, (c, 1)).reshape(-1), bc3=np.array([0.05], np.float32))
-    for b in ("b3a2", "b3b2", "bc1", "bc2"):
-        w[b] = (rng.standard_normal(c) * 0.1).astype(np.float32)
-    return (P1, Q1, P2, Q2), w
-
-
-WORDER = ("w3a2", "b3a2", "w3b2", "b3b2", "wc1", "bc1", "wc2", "bc2", "wc3", "bc3")
-
-
 def _run(tabs, w, k, dev, exclude=None):
     from deep_cbrs_amar_renaissance_b200 import ops
-    return ops.score_hybrid_topk_tf32x3(*[_t(x, dev) for x in tabs], *[_t(w[n], dev) for n in WORDER], k, exclude=exclude)
-
-
-def _tf32(x):
-    """round to the nearest tf32 (10 explicit mantissa bits), ties away from zero as cvt.rna"""
-    b = np.asarray(x, np.float32).view(np.uint32).astype(np.uint64)
-    return ((b + 0x1000) & 0xFFFFE000).astype(np.uint32).view(np.float32)
-
-
-def _chain(P1, Q1, P2, Q2, w, uu, ii, rounded=False):
-    """sigmoid scores of the pairs (uu[j], ii[j]) in float64; rounded: every product operand rounded to tf32"""
-    f8 = np.float64
-    r = (lambda x: _tf32(x).astype(f8)) if rounded else (lambda x: np.asarray(x, f8))
-    relu = lambda x: np.maximum(x, 0)
-    h1 = relu(P1[uu].astype(f8) + Q1[ii])
-    h2 = relu(P2[uu].astype(f8) + Q2[ii])
-    x1 = relu(r(h1) @ r(w["w3a2"]) + w["b3a2"])
-    x2 = relu(r(h2) @ r(w["w3b2"]) + w["b3b2"])
-    g = relu(r(x1) @ r(w["wc1"][:64]) + r(x2) @ r(w["wc1"][64:]) + w["bc1"])
-    h = relu(r(g) @ r(w["wc2"]) + w["bc2"])
-    return 1.0 / (1.0 + np.exp(-(h @ w["wc3"].astype(f8) + f8(w["bc3"][0]))))
-
-
-def _oracle(tabs, w):
-    n_users, n_items = len(tabs[0]), len(tabs[1])
-    out = np.empty((n_users, n_items))
-    step = max(1, 200000 // n_items)
-    for u0 in range(0, n_users, step):
-        nu = min(step, n_users - u0)
-        uu, ii = np.repeat(np.arange(u0, u0 + nu), n_items), np.tile(np.arange(n_items), nu)
-        out[u0:u0 + nu] = _chain(*tabs, w, uu, ii).reshape(nu, n_items)
-    return out
+    return ops.score_hybrid_topk_tf32x3(*[_t(x, dev) for x in tabs], *[_t(w[n], dev) for n in HYBRID_WEIGHTS], k,
+                                        exclude=exclude)
 
 
 @pytest.mark.parametrize("n_users,n_items,k", [(37, 1000, 10), (5, 7, 5), (130, 333, 20), (16, 32, 3), (1, 2049, 10),
                                                (4800, 40, 5), (300, 5000, 64), (64, 300, 128)])
 def test_against_float64_chain(dev, n_users, n_items, k):
-    tabs, w = _tables(n_users, n_items, n_users + n_items)
+    tabs, w = hybrid_tables(n_users, n_items, n_users + n_items)
     ids, vals = (x.cpu().numpy() for x in _run(tabs, w, k, dev))
     assert (ids >= 0).all() and (ids < n_items).all()
     assert all(len(set(row)) == k for row in ids)                       # no item twice
     assert (np.diff(vals, axis=1) <= 0).all()                           # descending
-    oracle = _oracle(tabs, w)
+    oracle = hybrid_chain_scores(tabs, w)
     assert_topk_equivalent(ids, vals, oracle, k, tol=TOL)
     uu = np.repeat(np.arange(n_users), k)
     got = np.take_along_axis(oracle, ids.astype(np.int64), 1)
     assert np.abs(got - vals).max() <= TOL
     # a single-TF32 evaluation of the same pairs misses the tolerance: the kernel's accuracy comes from the split
-    single = _chain(*tabs, w, uu, ids.reshape(-1).astype(np.int64), rounded=True).reshape(n_users, k)
+    single = hybrid_chain(*tabs, w, uu, ids.reshape(-1).astype(np.int64), rounded=True).reshape(n_users, k)
     assert np.abs(single - got).max() > TOL
 
 

@@ -346,7 +346,7 @@ def test_fused_catalog_scorer_matches_oracle(dev, n_users, n_items, c1, c2, k, p
         launches = ops.LAUNCHES
         tensor = bool(_lib.load().cbrs_score_catalog_topk_tf32x3_eligible(c1, c2))
         assert tensor == (c1 in (32, 64) and c2 <= 64)
-    from tests.helpers import assert_topk_equivalent
+    from tests.helpers import assert_topk_equivalent, basic_chain
     rng = np.random.RandomState(n_items + c2)
     P = rng.standard_normal((n_users, c1)).astype(np.float32)
     Q = rng.standard_normal((n_items, c1)).astype(np.float32)
@@ -358,9 +358,7 @@ def test_fused_catalog_scorer_matches_oracle(dev, n_users, n_items, c1, c2, k, p
                                        precision=precision)
     if precision == "fp32":
         assert ops.LAUNCHES - launches == (2 if tensor else 1)   # operand-image prep + scorer | the FFMA scorer
-    h1 = np.maximum(P[:, None, :] + Q[None, :, :], 0).reshape(-1, c1)
-    h2 = np.maximum(h1 @ w2 + b2, 0)
-    scores = ol.sigmoid(h2 @ w3 + b3).reshape(n_users, n_items)
+    scores = basic_chain(P, Q, w2, b2, w3, b3)
     kk = min(k, n_items)
     ids_np, vals_np = ids.cpu().numpy(), vals.cpu().numpy()
     assert (ids_np[:, kk:] == -1).all()
@@ -374,13 +372,6 @@ def test_fused_catalog_scorer_matches_oracle(dev, n_users, n_items, c1, c2, k, p
                 assert not (a + 10 in pos and a not in pos)
 
 
-def _bf16_round(x):
-    """round-to-nearest-even fp32 -> bf16 -> fp32 (numpy)"""
-    u = np.asarray(x, np.float32).view(np.uint32).astype(np.uint64)
-    u = (u + 0x7FFF + ((u >> 16) & 1)) & 0xFFFF0000
-    return u.astype(np.uint32).view(np.float32)
-
-
 @pytest.mark.parametrize("n_users,n_items,c1,c2,k", [(37, 3706, 64, 64, 10), (50, 1000, 48, 48, 5), (5, 7, 64, 64, 10),
                                                       (40, 333, 128, 128, 20), (130, 2049, 64, 32, 10),
                                                       (33, 500, 8, 16, 3), (20, 700, 72, 80, 10),
@@ -390,7 +381,7 @@ def test_tensor_core_catalog_scorer_matches_bf16_oracle(dev, n_users, n_items, c
     tolerance 2e-5 on scores (fp32 summation order inside the MMA is unspecified; 1e-4 for the v3 kernel, where an
     activation within an fp32 ulp of a bf16 rounding boundary may round the other way before the output product)."""
     from deep_cbrs_amar_renaissance_b200 import ops
-    from tests.helpers import assert_topk_equivalent
+    from tests.helpers import assert_topk_equivalent, bf16_basic_chain
     rng = np.random.RandomState(n_items + c2)
     P = rng.standard_normal((n_users, c1)).astype(np.float32)
     Q = rng.standard_normal((n_items, c1)).astype(np.float32)
@@ -398,20 +389,7 @@ def test_tensor_core_catalog_scorer_matches_bf16_oracle(dev, n_users, n_items, c
     w3, b3 = glorot(rng, (c2, 1)).reshape(-1), np.array([0.05], np.float32)
     ids, vals = ops.score_catalog_topk(_t(P, dev), _t(Q, dev), _t(w2, dev), _t(b2, dev), _t(w3, dev), _t(b3, dev), k,
                                        precision="bf16")
-    if c1 <= 64 and c2 <= 128:  # v2 kernel: P and Q rounded first, bf16 add (exact sum rounded once), relu
-        h1 = np.maximum(_bf16_round(_bf16_round(P)[:, None, :] + _bf16_round(Q)[None, :, :]), 0).reshape(-1, c1)
-    else:
-        h1 = _bf16_round(np.maximum(P[:, None, :] + Q[None, :, :], 0).reshape(-1, c1))
-    if c1 <= 64 and c2 <= 64:
-        # v3 kernel (every product on the tensor core): the bias is a row of the bf16 image of W2, relu(h1 W2 + b2) is
-        # rounded to bf16 and the output layer is a second product against bf16(w3)
-        acc = h1.astype(np.float64) @ _bf16_round(w2).astype(np.float64) + _bf16_round(b2).astype(np.float64)
-        h2 = _bf16_round(np.maximum(acc, 0).astype(np.float32))
-        scores = ol.sigmoid((h2.astype(np.float64) @ _bf16_round(w3).astype(np.float64)).astype(np.float32) + b3)
-        scores = scores.reshape(n_users, n_items)
-    else:
-        h2 = np.maximum(h1.astype(np.float64) @ _bf16_round(w2).astype(np.float64) + b2, 0).astype(np.float32)
-        scores = ol.sigmoid(h2 @ w3 + b3).reshape(n_users, n_items)
+    scores = bf16_basic_chain(P, Q, w2, b2, w3, b3)
     kk = min(k, n_items)
     ids_np, vals_np = ids.cpu().numpy(), vals.cpu().numpy()
     assert (ids_np[:, kk:] == -1).all()
