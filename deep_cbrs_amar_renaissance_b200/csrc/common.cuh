@@ -95,8 +95,15 @@ __device__ __forceinline__ bool excluded_item(const int64_t *__restrict__ rowptr
     return lo < end && __ldg(items + lo) == item;
 }
 
-// Candidate lists of the tensor-core catalog scorers (score_tf32.cu, score_hybrid_tf32.cu): 64-bit keys
-// (orderable(logit) << 32) | ~item, so that a larger key is a higher score, ties going to the lower item id.
+// ---- per-user candidate lists of the fused catalog scorers (score*.cu) --------------------------------------------
+// A CTA keeps, for each of its users, a list of 64-bit keys (orderable(value) << 32) | ~item in shared memory: a larger
+// key is a higher value, ties going to the lower item id, so the result does not depend on insertion order.  Key 0 is
+// below every real key (the low word of one is ~item >= 2^31).  A candidate is appended (topk_offer) when it beats the
+// user's current k-th key; before every item tile a list that could overflow is cut back to its best k
+// (topk_make_room), and at the end topk_write compacts once more and writes the k slots.  The loop over users, and
+// which warp owns user ul, stay with each kernel: a list is only ever touched by one warp at a time.
+
+// order-preserving map float -> uint32 (ascending)
 __device__ __forceinline__ uint32_t orderable_f32(float f) {
     const uint32_t u = __float_as_uint(f);
     return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
@@ -104,6 +111,36 @@ __device__ __forceinline__ uint32_t orderable_f32(float f) {
 __device__ __forceinline__ float from_orderable_f32(uint32_t o) {
     return __uint_as_float((o & 0x80000000u) ? (o & 0x7fffffffu) : ~o);
 }
+__device__ __forceinline__ unsigned long long topk_key(float value, uint32_t item) {
+    return ((unsigned long long)orderable_f32(value) << 32) | (unsigned long long)(0xffffffffu - item);
+}
+__device__ __forceinline__ int32_t topk_key_item(unsigned long long key) {
+    return (int32_t)(0xffffffffu - (uint32_t)(key & 0xffffffffull));
+}
+__device__ __forceinline__ float topk_key_value(unsigned long long key) { return from_orderable_f32((uint32_t)(key >> 32)); }
+
+// one output slot: the item and value of `key` (kSigmoid: the value is a logit, written as its sigmoid), or (-1, -inf)
+// for key 0, a slot the list has no item for
+template <bool kSigmoid>
+__device__ __forceinline__ void topk_store(unsigned long long key, int32_t *id, float *score) {
+    if (key != 0ull) {
+        *id = topk_key_item(key);
+        const float v = topk_key_value(key);
+        *score = kSigmoid ? 1.f / (1.f + expf(-v)) : v;
+    } else {
+        *id = -1;
+        *score = -INFINITY;
+    }
+}
+
+constexpr int kTopkTile = 32;   // most candidates one item tile adds to a user's list
+// a compaction keeps k keys, so a list of 2k + 32 takes one more tile whenever it holds at most 2k
+__host__ __device__ constexpr int topk_list_cap(int k) { return 2 * k + kTopkTile; }
+// shared memory of tu lists: keys [tu][cap], k-th keys [tu] (0 until k are held), counts [tu]
+static inline size_t topk_lists_smem_bytes(int tu, int k) {
+    return (size_t)tu * topk_list_cap(k) * 8 + (size_t)tu * 8 + (size_t)tu * 4;
+}
+
 // one warp: keep the best min(k, n) keys of c[0..n) in c[0..), descending; *thr becomes the k-th key once k are held
 static __device__ void topk_compact(unsigned long long *c, int *cnt, unsigned long long *thr, int k, int lane) {
     const int n = *cnt;
@@ -132,6 +169,70 @@ static __device__ void topk_compact(unsigned long long *c, int *cnt, unsigned lo
         *thr = (keep == k) ? c[k - 1] : 0ull;
     }
     __syncwarp();
+}
+
+// The three operations below address the lists of a CTA's users as in shared memory: keys cand [tu][cap] with
+// cap = topk_list_cap(k), k-th keys thr [tu], counts cnt [tu]; ul is the user's slot in the CTA.
+
+// one warp, before an item tile: compact user ul's list if it might not have room for the tile's candidates
+__device__ __forceinline__ void topk_make_room(unsigned long long *cand, int *cnt, unsigned long long *thr, int cap, int ul,
+                                               int k, int lane) {
+    if (cnt[ul] > cap - kTopkTile) topk_compact(cand + ul * cap, cnt + ul, thr + ul, k, lane);
+}
+
+// one thread: append (value, item) to user ul's list if it beats the list's k-th key and is not on the exclusion list of
+// `user`, the user's global row (kExcl)
+template <bool kExcl>
+__device__ __forceinline__ void topk_offer(unsigned long long *cand, int *cnt, const unsigned long long *thr, int cap, int ul,
+                                           float value, int32_t item, int64_t user, const int64_t *__restrict__ excl_rowptr,
+                                           const int32_t *__restrict__ excl_items) {
+    const unsigned long long key = topk_key(value, (uint32_t)item);
+    if (key > thr[ul] && !(kExcl && excluded_item(excl_rowptr, excl_items, user, item))) {
+        const int pos = atomicAdd(cnt + ul, 1);
+        cand[ul * cap + pos] = key;   // pos < cap: topk_make_room ran before this tile
+    }
+}
+
+// one warp, after the last tile: user ul's k slots to rows user * k .. user * k + k - 1 of ids_out / scores_out (nothing
+// for a user at or past n_users, the CTA's padding); kSigmoid as in topk_store
+template <bool kSigmoid>
+__device__ __forceinline__ void topk_write(unsigned long long *cand, int *cnt, unsigned long long *thr, int cap, int ul,
+                                           int k, int lane, int64_t user, int64_t n_users, int32_t *ids_out,
+                                           float *scores_out) {
+    unsigned long long *c = cand + ul * cap;
+    topk_compact(c, cnt + ul, thr + ul, k, lane);
+    if (user >= n_users) return;
+    const int n = cnt[ul];
+    for (int r = lane; r < k; r += 32) {
+        const int64_t o = user * k + r;
+        topk_store<kSigmoid>(r < n ? c[r] : 0ull, ids_out + o, scores_out + o);
+    }
+}
+
+// ---- host side of the fused catalog scorers -------------------------------------------------------------------------
+// the argument rules they all share; `who` prefixes the messages
+static inline int check_catalog_args(const char *who, const int64_t *excl_rowptr, const int32_t *excl_items,
+                                     int64_t n_users, int32_t n_items, int32_t k) {
+    CBRS_REQUIRE(!excl_rowptr == !excl_items, CBRS_E_INVALID, "%s: %s is null but %s is not", who,
+                 excl_rowptr ? "excl_items" : "excl_rowptr", excl_rowptr ? "excl_rowptr" : "excl_items");
+    CBRS_REQUIRE(n_users >= 0 && n_items > 0 && k > 0 && k <= 128, CBRS_E_INVALID, "%s: n_users=%lld n_items=%d k=%d", who,
+                 (long long)n_users, n_items, k);
+    return CBRS_OK;
+}
+
+// Launches `excl` when the parameters carry exclusion lists, `plain` otherwise, with `smem` bytes of dynamic shared
+// memory (at most smem_limit).  The attribute is set on every call: it belongs to the current device's context.
+template <typename Params>
+static int launch_catalog_scorer(void (*plain)(Params), void (*excl)(Params), const Params &p, unsigned grid,
+                                 unsigned block, size_t smem, size_t smem_limit, cudaStream_t s, const char *who,
+                                 const char *what) {
+    CBRS_REQUIRE(smem <= smem_limit, CBRS_E_UNSUPPORTED, "%s: needs %zu bytes of shared memory", who, smem);
+    auto kernel = p.excl_rowptr ? excl : plain;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    CBRS_REQUIRE(e == cudaSuccess, CBRS_E_CUDA, "%s: cudaFuncSetAttribute: %s", who, cudaGetErrorString(e));
+    kernel<<<grid, block, smem, s>>>(p);
+    CBRS_CHECK_LAUNCH(what);
+    return CBRS_OK;
 }
 
 }  // namespace cbrs

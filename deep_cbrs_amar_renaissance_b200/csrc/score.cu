@@ -13,10 +13,8 @@
 //
 // CTA = 16 users; the item catalog streams through shared memory in tiles of 32 items
 // (transposed, 128-bit reads).  Each thread owns 1 user x 8 items x 8 classifier columns:
-// 64 FFMA per 3 LDS.128 + 16 add/max.  Candidates above the user's current k-th score are
-// appended to a per-user list and compacted (k rounds of warp arg-max) when it fills; keys
-// are (score bits, ~item) so ties go to the lower item index and the result does not depend
-// on insertion order.
+// 64 FFMA per 3 LDS.128 + 16 add/max.  Candidates above the user's current k-th score go to
+// the per-user candidate lists of common.cuh, keyed on the sigmoid score.
 #include "common.cuh"
 
 namespace cbrs {
@@ -37,44 +35,6 @@ constexpr int kScTU = 16;       // users per CTA
 constexpr int kScTI = 32;       // items per tile
 constexpr int kScQS = kScTI + 4;  // padded row of the transposed item tile
 
-__device__ __forceinline__ uint32_t sc_orderable(float f) {
-    const uint32_t u = __float_as_uint(f);
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float sc_from_orderable(uint32_t o) {
-    return __uint_as_float((o & 0x80000000u) ? (o & 0x7fffffffu) : ~o);
-}
-
-// one warp: keep the best min(k, n) keys of c[0..n) in c[0..), descending
-__device__ void sc_compact(unsigned long long *c, int *cnt, unsigned long long *thr, int k, int lane) {
-    const int n = *cnt;
-    const int keep = n < k ? n : k;
-    for (int r = 0; r < keep; ++r) {
-        unsigned long long best = 0ull;
-        int bi = -1;
-        for (int i = r + lane; i < n; i += 32) {
-            const unsigned long long v = c[i];
-            if (v > best) { best = v; bi = i; }
-        }
-        unsigned long long m = best;
-#pragma unroll
-        for (int o = 16; o; o >>= 1) {
-            const unsigned long long t = __shfl_xor_sync(0xffffffffu, m, o);
-            m = t > m ? t : m;
-        }
-        if (best == m && bi >= 0) {  // keys are unique: exactly one lane owns the maximum
-            c[bi] = c[r];
-            c[r] = m;
-        }
-        __syncwarp();
-    }
-    if (lane == 0) {
-        *cnt = keep;
-        *thr = (keep == k) ? c[k - 1] : 0ull;
-    }
-    __syncwarp();
-}
-
 // CT: threads across the classifier's second-layer columns: 8 (c2 <= 64) or 16 (c2 <= 128); kExcl: exclusion lists given
 template <int CT, bool kExcl>
 __global__ void __launch_bounds__(kScThreads, 2) score_catalog_kernel(const ScoreParams p) {
@@ -83,7 +43,7 @@ __global__ void __launch_bounds__(kScThreads, 2) score_catalog_kernel(const Scor
     constexpr int C2P = CT * 8;          // padded second-layer width
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int c1 = p.c1;
-    const int cap = 2 * p.k + kScTI;
+    const int cap = topk_list_cap(p.k);
     float *Ws = reinterpret_cast<float *>(smem_raw);       // [c1][C2P]
     float *Ps = Ws + c1 * C2P;                              // [kScTU][c1]
     float *Qs = Ps + kScTU * c1;                            // [c1][kScQS] (transposed tile)
@@ -119,7 +79,7 @@ __global__ void __launch_bounds__(kScThreads, 2) score_catalog_kernel(const Scor
     for (int t0 = 0; t0 < p.n_items; t0 += kScTI) {
         __syncthreads();  // previous tile fully consumed; candidate lists settled
         for (int ul = warp; ul < kScTU; ul += kScThreads / 32)
-            if (cnt[ul] > cap - kScTI) sc_compact(cand + ul * cap, cnt + ul, thr + ul, p.k, lane);
+            topk_make_room(cand, cnt, thr, cap, ul, p.k, lane);
         for (int e = tid; e < kScTI * (c1 / 4); e += kScThreads) {
             const int it = e / (c1 / 4), k4 = e % (c1 / 4);
             float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -174,58 +134,31 @@ __global__ void __launch_bounds__(kScThreads, 2) score_catalog_kernel(const Scor
             if (ct < 8) {
                 const int item = t0 + item_oct * 8 + ct;
                 const int64_t user = u0 + ul;
-                if (item < p.n_items && user < p.n_users) {
-                    const float score = 1.f / (1.f + expf(-(mine + b3)));
-                    const unsigned long long key =
-                        ((unsigned long long)sc_orderable(score) << 32) | (unsigned long long)(0xffffffffu - (uint32_t)item);
-                    if (key > thr[ul] && !(kExcl && excluded_item(p.excl_rowptr, p.excl_items, user, item))) {
-                        const int pos = atomicAdd(cnt + ul, 1);
-                        cand[ul * cap + pos] = key;  // pos < cap: lists above cap-32 were compacted before this tile
-                    }
-                }
+                if (item < p.n_items && user < p.n_users)
+                    topk_offer<kExcl>(cand, cnt, thr, cap, ul, 1.f / (1.f + expf(-(mine + b3))), item, user,
+                                      p.excl_rowptr, p.excl_items);
             }
         }
     }
     __syncthreads();
-    for (int ul = warp; ul < kScTU; ul += kScThreads / 32) {
-        sc_compact(cand + ul * cap, cnt + ul, thr + ul, p.k, lane);
-        const int64_t user = u0 + ul;
-        if (user >= p.n_users) continue;
-        const int n = cnt[ul];
-        for (int r = lane; r < p.k; r += 32) {
-            const int64_t o = user * p.k + r;
-            if (r < n) {
-                const unsigned long long key = cand[ul * cap + r];
-                p.ids_out[o] = (int32_t)(0xffffffffu - (uint32_t)(key & 0xffffffffull));
-                p.scores_out[o] = sc_from_orderable((uint32_t)(key >> 32));
-            } else {
-                p.ids_out[o] = -1;
-                p.scores_out[o] = -INFINITY;
-            }
-        }
-    }
+    for (int ul = warp; ul < kScTU; ul += kScThreads / 32)
+        topk_write<false>(cand, cnt, thr, cap, ul, p.k, lane, u0 + ul, p.n_users, p.ids_out, p.scores_out);
 }
 
 template <int CT>
 static size_t score_smem_bytes(int c1, int k) {
     const int C2P = CT * 8;
-    const int cap = 2 * k + kScTI;
     size_t f = (size_t)c1 * C2P + (size_t)kScTU * c1 + (size_t)c1 * kScQS + 2 * C2P;
     f = (f + 1) / 2 * 2;  // keep the 64-bit candidate lists 8-byte aligned
-    return f * sizeof(float) + (size_t)kScTU * cap * 8 + kScTU * 8 + kScTU * 4 + 16;
+    return f * sizeof(float) + topk_lists_smem_bytes(kScTU, k) + 16;
 }
 
 template <int CT>
 static int launch_score(const ScoreParams &p, cudaStream_t s) {
-    const size_t smem = score_smem_bytes<CT>(p.c1, p.k);
     // up to the 227 KB a CTA may have: the widest classifier (c1 = 256, c2 = 128) at k = 128 needs 217 KB
-    CBRS_REQUIRE(smem <= 227 * 1024, CBRS_E_UNSUPPORTED, "score_catalog: needs %zu bytes of shared memory", smem);
-    auto kernel = p.excl_rowptr ? score_catalog_kernel<CT, true> : score_catalog_kernel<CT, false>;
-    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    CBRS_REQUIRE(e == cudaSuccess, CBRS_E_CUDA, "score_catalog: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    kernel<<<(unsigned)cdiv(p.n_users, kScTU), kScThreads, smem, s>>>(p);
-    CBRS_CHECK_LAUNCH("score_catalog");
-    return CBRS_OK;
+    return launch_catalog_scorer(score_catalog_kernel<CT, false>, score_catalog_kernel<CT, true>, p,
+                                 (unsigned)cdiv(p.n_users, kScTU), kScThreads, score_smem_bytes<CT>(p.c1, p.k), 227 * 1024,
+                                 s, "score_catalog", "score_catalog");
 }
 
 }  // namespace cbrs
@@ -245,10 +178,8 @@ extern "C" int cbrs_score_catalog_topk_ex(const float *P, int64_t ldp, const flo
                                           const float *w3, const float *b3, int32_t k, int32_t *ids_out, float *scores_out,
                                           const int64_t *excl_rowptr, const int32_t *excl_items, void *stream) {
     CBRS_REQUIRE(P && Q && w2 && b2 && w3 && b3 && ids_out && scores_out, CBRS_E_INVALID, "score_catalog: null argument");
-    CBRS_REQUIRE(!excl_rowptr == !excl_items, CBRS_E_INVALID, "score_catalog: %s is null but %s is not",
-                 excl_rowptr ? "excl_items" : "excl_rowptr", excl_rowptr ? "excl_rowptr" : "excl_items");
-    CBRS_REQUIRE(n_users >= 0 && n_items > 0 && k > 0 && k <= 128, CBRS_E_INVALID, "score_catalog: n_users=%lld n_items=%d k=%d",
-                 (long long)n_users, n_items, k);
+    const int rc = check_catalog_args("score_catalog", excl_rowptr, excl_items, n_users, n_items, k);
+    if (rc != CBRS_OK) return rc;
     CBRS_REQUIRE(c1 > 0 && c1 % 4 == 0 && c1 <= 256 && c2 > 0 && c2 <= 128, CBRS_E_UNSUPPORTED,
                  "score_catalog: classifier widths c1=%d (multiple of 4, <= 256), c2=%d (<= 128)", c1, c2);
     CBRS_REQUIRE(ldp >= c1 && ldq >= c1 && ldq % 4 == 0 && ((uintptr_t)Q % 16) == 0, CBRS_E_INVALID,

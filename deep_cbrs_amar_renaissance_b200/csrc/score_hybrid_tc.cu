@@ -18,7 +18,7 @@
 // one CTA's MMAs overlap the other's CUDA-core phases (same organisation as score_tc_kernel, score_tc.cu).
 // Precision: every operand of an MMA is rounded to bf16 (nearest even), sums are fp32; the parity test compares against
 // an oracle that rounds at the same points (tests/test_gpu_hybrid_catalog.py, tolerance stated there).  Top-k: exact on
-// the kernel's own scores, ties to the lower item id (64-bit (score, ~item) keys as in the other catalog kernels).
+// the kernel's own scores, ties to the lower item id (the candidate lists of common.cuh).
 #include "common.cuh"
 #include "tc05.cuh"
 
@@ -44,44 +44,6 @@ struct HybridTcParams {
     const int64_t *excl_rowptr;          // exclusion lists (both null: none)
     const int32_t *excl_items;
 };
-
-__device__ __forceinline__ uint32_t hy_orderable(float f) {
-    const uint32_t u = __float_as_uint(f);
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float hy_from_orderable(uint32_t o) {
-    return __uint_as_float((o & 0x80000000u) ? (o & 0x7fffffffu) : ~o);
-}
-
-// keep the k largest keys of a candidate list, sorted descending (one warp)
-__device__ void hy_compact(unsigned long long *c, int *cnt, unsigned long long *thr, int k, int lane) {
-    const int n = *cnt;
-    const int keep = n < k ? n : k;
-    for (int r = 0; r < keep; ++r) {
-        unsigned long long best = 0ull;
-        int bi = -1;
-        for (int i = r + lane; i < n; i += 32) {
-            const unsigned long long v = c[i];
-            if (v > best) { best = v; bi = i; }
-        }
-        unsigned long long m = best;
-#pragma unroll
-        for (int o = 16; o; o >>= 1) {
-            const unsigned long long t = __shfl_xor_sync(0xffffffffu, m, o);
-            m = t > m ? t : m;
-        }
-        if (best == m && bi >= 0) {
-            c[bi] = c[r];
-            c[r] = m;
-        }
-        __syncwarp();
-    }
-    if (lane == 0) {
-        *cnt = keep;
-        *thr = (keep == k) ? c[k - 1] : 0ull;
-    }
-    __syncwarp();
-}
 
 // W [64 (in), 64 (out)] fp32, Keras layout, row stride ldw -> B operand image: element (n, kk) = bf16(W[kk][n])
 __global__ void hy_prep_kernel(const float *w3a2, const float *w3b2, const float *wc1, const float *wc2, uint8_t *image) {
@@ -117,7 +79,7 @@ constexpr int kHyQLd = kHyC + 4;   // padded row of the staged Q tile: 8 consecu
 template <int TU, bool kExcl>   // kExcl: exclusion lists given
 __global__ void __launch_bounds__(kHyThreads, 2) score_hybrid_tc_kernel(const HybridTcParams p) {
     extern __shared__ __align__(1024) unsigned char hy_smem[];
-    const int cap = 2 * p.k + kHyTI;
+    const int cap = topk_list_cap(p.k);
     unsigned char *A1 = hy_smem;                               // [128][128 B]
     unsigned char *A2 = A1 + kHyTile;
     unsigned char *Ws = A2 + kHyTile;                          // 5 weight images
@@ -233,7 +195,7 @@ __global__ void __launch_bounds__(kHyThreads, 2) score_hybrid_tc_kernel(const Hy
 
     for (int t0 = 0; t0 < p.n_items; t0 += kHyTI) {
         for (int ul = warp; ul < TU; ul += kHyThreads / 32)   // user ul is always handled by warp ul % 4
-            if (cnt[ul] > cap - kHyTI) hy_compact(cand + ul * cap, cnt + ul, thr + ul, p.k, lane);
+            topk_make_room(cand, cnt, thr, cap, ul, p.k, lane);
         const int item = t0 + lane;
         const bool item_ok = item < p.n_items;
         stage_q();                 // every warp is past the previous tile's producer phases (it passed later barriers)
@@ -297,15 +259,9 @@ __global__ void __launch_bounds__(kHyThreads, 2) score_hybrid_tc_kernel(const Hy
                 }
             }
             const int64_t user = u0 + ul;
-            if (item_ok && user < p.n_users) {
-                // ranked by the logit (sigmoid is monotonic); the sigmoid is applied to the k winners
-                const unsigned long long key =
-                    ((unsigned long long)hy_orderable(logit + bc3) << 32) | (unsigned long long)(0xffffffffu - (uint32_t)item);
-                if (key > thr[ul] && !(kExcl && excluded_item(p.excl_rowptr, p.excl_items, user, item))) {
-                    const int pos = atomicAdd(cnt + ul, 1);
-                    cand[ul * cap + pos] = key;
-                }
-            }
+            // ranked by the logit (sigmoid is monotonic); the sigmoid is applied to the k winners
+            if (item_ok && user < p.n_users)
+                topk_offer<kExcl>(cand, cnt, thr, cap, ul, logit + bc3, item, user, p.excl_rowptr, p.excl_items);
         }
     }
     tc::tc_fence_before_sync();
@@ -314,46 +270,20 @@ __global__ void __launch_bounds__(kHyThreads, 2) score_hybrid_tc_kernel(const Hy
         tc::tc_fence_after_sync();
         tc::tmem_dealloc(tmem_base, kCols);
     }
-    for (int ul = warp; ul < TU; ul += kHyThreads / 32) {
-        hy_compact(cand + ul * cap, cnt + ul, thr + ul, p.k, lane);
-        const int64_t user = u0 + ul;
-        if (user >= p.n_users) continue;
-        const int n = cnt[ul];
-        for (int r = lane; r < p.k; r += 32) {
-            const int64_t o = user * p.k + r;
-            if (r < n) {
-                const unsigned long long key = cand[ul * cap + r];
-                p.ids_out[o] = (int32_t)(0xffffffffu - (uint32_t)(key & 0xffffffffull));
-                p.scores_out[o] = 1.f / (1.f + expf(-hy_from_orderable((uint32_t)(key >> 32))));
-            } else {
-                p.ids_out[o] = -1;
-                p.scores_out[o] = -INFINITY;
-            }
-        }
-    }
+    for (int ul = warp; ul < TU; ul += kHyThreads / 32)
+        topk_write<true>(cand, cnt, thr, cap, ul, p.k, lane, u0 + ul, p.n_users, p.ids_out, p.scores_out);
 }
 
 static size_t hy_smem_bytes(int k, int tu) {
-    const int cap = 2 * k + kHyTI;
     return 2 * (size_t)kHyTile + 5 * (size_t)kHyW + 2 * tu * kHyC * 4 + 5 * kHyC * 4 + 2 * (size_t)kHyTI * kHyQLd * 4 +
-           (size_t)tu * cap * 8 + tu * 8 + 8 + tu * 4 + 16;
+           topk_lists_smem_bytes(tu, k) + 8 + 16;
 }
 
 template <int TU>
 static int hy_launch(const HybridTcParams &p, cudaStream_t s) {
-    const size_t smem = hy_smem_bytes(p.k, TU);
-    CBRS_REQUIRE(smem <= 227 * 1024, CBRS_E_UNSUPPORTED, "score_hybrid_topk_bf16: needs %zu bytes of shared memory", smem);
-    static size_t configured[2] = {0, 0};
-    const int x = p.excl_rowptr ? 1 : 0;
-    auto kernel = x ? score_hybrid_tc_kernel<TU, true> : score_hybrid_tc_kernel<TU, false>;
-    if (smem > configured[x]) {
-        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        CBRS_REQUIRE(e == cudaSuccess, CBRS_E_CUDA, "score_hybrid_topk_bf16: %s", cudaGetErrorString(e));
-        configured[x] = smem;
-    }
-    kernel<<<(unsigned)cdiv(p.n_users, TU), kHyThreads, smem, s>>>(p);
-    CBRS_CHECK_LAUNCH("score_hybrid_topk_bf16");
-    return CBRS_OK;
+    return launch_catalog_scorer(score_hybrid_tc_kernel<TU, false>, score_hybrid_tc_kernel<TU, true>, p,
+                                 (unsigned)cdiv(p.n_users, TU), kHyThreads, hy_smem_bytes(p.k, TU), 227 * 1024, s,
+                                 "score_hybrid_topk_bf16", "score_hybrid_topk_bf16");
 }
 
 }  // namespace cbrs
@@ -381,12 +311,12 @@ extern "C" int cbrs_score_hybrid_topk_bf16_ex(const float *P1, const float *Q1, 
     CBRS_REQUIRE(P1 && Q1 && P2 && Q2 && w3a2 && b3a2 && w3b2 && b3b2 && wc1 && bc1 && wc2 && bc2 && wc3 && bc3 && ids_out &&
                      scores_out && workspace,
                  CBRS_E_INVALID, "score_hybrid_topk_bf16: null argument");
-    CBRS_REQUIRE(!excl_rowptr == !excl_items, CBRS_E_INVALID, "score_hybrid_topk_bf16: %s is null but %s is not",
-                 excl_rowptr ? "excl_items" : "excl_rowptr", excl_rowptr ? "excl_rowptr" : "excl_items");
+    const int rc = check_catalog_args("score_hybrid_topk_bf16", excl_rowptr, excl_items, n_users, n_items, k);
+    if (rc != CBRS_OK) return rc;
     CBRS_REQUIRE(c == kHyC, CBRS_E_UNSUPPORTED, "score_hybrid_topk_bf16: built for %d-wide hidden layers (every hybrid grid of the "
                  "reference), got %d", kHyC, c);
-    CBRS_REQUIRE(n_users >= 0 && n_items > 0 && k > 0 && k <= 128 && k <= n_items, CBRS_E_INVALID,
-                 "score_hybrid_topk_bf16: n_users=%lld n_items=%d k=%d", (long long)n_users, n_items, k);
+    CBRS_REQUIRE(k <= n_items, CBRS_E_INVALID, "score_hybrid_topk_bf16: n_users=%lld n_items=%d k=%d", (long long)n_users,
+                 n_items, k);
     CBRS_REQUIRE(workspace_bytes >= cbrs_score_hybrid_topk_bf16_workspace_bytes() && ((uintptr_t)workspace % 16) == 0,
                  CBRS_E_WORKSPACE, "score_hybrid_topk_bf16: workspace too small or misaligned");
     if (n_users == 0) return CBRS_OK;

@@ -66,7 +66,7 @@ template <int TU, bool kExcl>   // TU: users per CTA (TU / 2 per warp group); kE
 __global__ void __launch_bounds__(kHfThreads, 1) score_hybrid_tf32_kernel(const __grid_constant__ HybridTf32Params p) {
     constexpr int TW = TU / 2;   // users per warp group
     extern __shared__ __align__(1024) unsigned char hf_smem[];
-    const int cap = 2 * p.k + kHfTI;
+    const int cap = topk_list_cap(p.k);
     unsigned char *Ws = hf_smem;                                          // 5 weight images
     float *P1s = reinterpret_cast<float *>(Ws + 5 * kHfImage);            // [TU][64]
     float *P2s = P1s + TU * kHfC;
@@ -211,7 +211,7 @@ __global__ void __launch_bounds__(kHfThreads, 1) score_hybrid_tf32_kernel(const 
 
     for (int t0 = 0; t0 < p.n_items; t0 += kHfTI) {
         for (int ul = ub + quad; ul < ub + TW; ul += 4)   // user ul is only ever touched by warp quad of its group
-            if (cnt[ul] > cap - kHfTI) topk_compact(cand + ul * cap, cnt + ul, thr + ul, p.k, lane);
+            topk_make_room(cand, cnt, thr, cap, ul, p.k, lane);
         const int item = t0 + lane;
         stage_q();          // the group's previous readers of the stage have passed later barriers
         hf_group_sync(group);
@@ -267,15 +267,9 @@ __global__ void __launch_bounds__(kHfThreads, 1) score_hybrid_tf32_kernel(const 
                 logit = ((lacc[0] + lacc[1]) + (lacc[2] + lacc[3])) + ((lacc[4] + lacc[5]) + (lacc[6] + lacc[7]));
             }
             const int64_t user = cta_u0 + ul;
-            if (item < p.n_items && user < p.n_users) {
-                // ranked by the logit (sigmoid is monotonic); the sigmoid is applied to the k winners
-                const unsigned long long key =
-                    ((unsigned long long)orderable_f32(logit + bc3) << 32) | (unsigned long long)(0xffffffffu - (uint32_t)item);
-                if (key > thr[ul] && !(kExcl && excluded_item(p.excl_rowptr, p.excl_items, user, item))) {
-                    const int pos = atomicAdd(cnt + ul, 1);
-                    cand[ul * cap + pos] = key;
-                }
-            }
+            // ranked by the logit (sigmoid is monotonic); the sigmoid is applied to the k winners
+            if (item < p.n_items && user < p.n_users)
+                topk_offer<kExcl>(cand, cnt, thr, cap, ul, logit + bc3, item, user, p.excl_rowptr, p.excl_items);
         }
     }
     tc::tc_fence_before_sync();
@@ -284,41 +278,20 @@ __global__ void __launch_bounds__(kHfThreads, 1) score_hybrid_tf32_kernel(const 
         tc::tc_fence_after_sync();
         tc::tmem_dealloc(tmem_base, kCols);
     }
-    for (int ul = warp; ul < TU; ul += kHfThreads / 32) {
-        topk_compact(cand + ul * cap, cnt + ul, thr + ul, p.k, lane);
-        const int64_t user = cta_u0 + ul;
-        if (user >= p.n_users) continue;
-        const int n = cnt[ul];
-        for (int r = lane; r < p.k; r += 32) {
-            const int64_t o = user * p.k + r;
-            if (r < n) {
-                const unsigned long long key = cand[ul * cap + r];
-                p.ids_out[o] = (int32_t)(0xffffffffu - (uint32_t)(key & 0xffffffffull));
-                p.scores_out[o] = 1.f / (1.f + expf(-from_orderable_f32((uint32_t)(key >> 32))));
-            } else {
-                p.ids_out[o] = -1;
-                p.scores_out[o] = -INFINITY;
-            }
-        }
-    }
+    for (int ul = warp; ul < TU; ul += kHfThreads / 32)
+        topk_write<true>(cand, cnt, thr, cap, ul, p.k, lane, cta_u0 + ul, p.n_users, p.ids_out, p.scores_out);
 }
 
 static size_t hf_smem_bytes(int k, int tu) {
-    const int cap = 2 * k + kHfTI;
     return 5 * (size_t)kHfImage + 2 * (size_t)tu * kHfC * 4 + 5 * kHfC * 4 + 4 * (size_t)kHfTI * kHfQLd * 4 +
-           (size_t)tu * cap * 8 + tu * 8 + 2 * 8 + tu * 4 + 16;
+           topk_lists_smem_bytes(tu, k) + 2 * 8 + 16;
 }
 
 template <int TU>
 static int hf_launch(const HybridTf32Params &p, cudaStream_t s) {
-    const size_t smem = hf_smem_bytes(p.k, TU);
-    CBRS_REQUIRE(smem <= 227 * 1024, CBRS_E_UNSUPPORTED, "score_hybrid_topk_tf32x3: needs %zu bytes of shared memory", smem);
-    auto kernel = p.excl_rowptr ? score_hybrid_tf32_kernel<TU, true> : score_hybrid_tf32_kernel<TU, false>;
-    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    CBRS_REQUIRE(e == cudaSuccess, CBRS_E_CUDA, "score_hybrid_topk_tf32x3: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    kernel<<<(unsigned)cdiv(p.n_users, TU), kHfThreads, smem, s>>>(p);
-    CBRS_CHECK_LAUNCH("score_hybrid_topk_tf32x3");
-    return CBRS_OK;
+    return launch_catalog_scorer(score_hybrid_tf32_kernel<TU, false>, score_hybrid_tf32_kernel<TU, true>, p,
+                                 (unsigned)cdiv(p.n_users, TU), kHfThreads, hf_smem_bytes(p.k, TU), 227 * 1024, s,
+                                 "score_hybrid_topk_tf32x3", "score_hybrid_topk_tf32x3");
 }
 
 }  // namespace cbrs
@@ -337,20 +310,20 @@ extern "C" int cbrs_score_hybrid_topk_tf32x3(const float *P1, const float *Q1, c
     CBRS_REQUIRE(P1 && Q1 && P2 && Q2 && w3a2 && b3a2 && w3b2 && b3b2 && wc1 && bc1 && wc2 && bc2 && wc3 && bc3 && ids_out &&
                      scores_out && workspace,
                  CBRS_E_INVALID, "score_hybrid_topk_tf32x3: null argument");
-    CBRS_REQUIRE(!excl_rowptr == !excl_items, CBRS_E_INVALID, "score_hybrid_topk_tf32x3: %s is null but %s is not",
-                 excl_rowptr ? "excl_items" : "excl_rowptr", excl_rowptr ? "excl_rowptr" : "excl_items");
+    const int rc = check_catalog_args("score_hybrid_topk_tf32x3", excl_rowptr, excl_items, n_users, n_items, k);
+    if (rc != CBRS_OK) return rc;
     CBRS_REQUIRE(c == kHfC, CBRS_E_UNSUPPORTED, "score_hybrid_topk_tf32x3: built for %d-wide hidden layers (every hybrid grid "
                  "of the reference), got %d", kHfC, c);
-    CBRS_REQUIRE(n_users >= 0 && n_items > 0 && k > 0 && k <= 128 && k <= n_items, CBRS_E_INVALID,
-                 "score_hybrid_topk_tf32x3: n_users=%lld n_items=%d k=%d", (long long)n_users, n_items, k);
+    CBRS_REQUIRE(k <= n_items, CBRS_E_INVALID, "score_hybrid_topk_tf32x3: n_users=%lld n_items=%d k=%d", (long long)n_users,
+                 n_items, k);
     CBRS_REQUIRE(workspace_bytes >= cbrs_score_hybrid_topk_tf32x3_workspace_bytes() && ((uintptr_t)workspace % 16) == 0,
                  CBRS_E_WORKSPACE, "score_hybrid_topk_tf32x3: workspace too small or misaligned");
     if (n_users == 0) return CBRS_OK;
     uint8_t *image = (uint8_t *)workspace;
     const float *w[5] = {w3a2, w3b2, wc1, wc1 + kHfC * kHfC, wc2};
     for (int m = 0; m < 5; ++m) {
-        const int rc = cbrs_dense_tf32x3_prepare(w[m], kHfC, kHfC, image + (size_t)m * kHfImage, stream);
-        if (rc != CBRS_OK) return rc;
+        const int rc_prep = cbrs_dense_tf32x3_prepare(w[m], kHfC, kHfC, image + (size_t)m * kHfImage, stream);
+        if (rc_prep != CBRS_OK) return rc_prep;
     }
     HybridTf32Params p;
     p.P1 = P1; p.Q1 = Q1; p.P2 = P2; p.Q2 = Q2; p.n_users = n_users; p.n_items = n_items;

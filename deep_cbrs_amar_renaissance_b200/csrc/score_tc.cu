@@ -39,43 +39,6 @@ constexpr int kTcThreads = 128;
 constexpr int kTcTU = 16;  // users per CTA (4 passes of 4 users per item tile)
 constexpr int kTcTI = 32;  // items per tile
 
-__device__ __forceinline__ uint32_t tcs_orderable(float f) {
-    const uint32_t u = __float_as_uint(f);
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float tcs_from_orderable(uint32_t o) {
-    return __uint_as_float((o & 0x80000000u) ? (o & 0x7fffffffu) : ~o);
-}
-
-__device__ void tcs_compact(unsigned long long *c, int *cnt, unsigned long long *thr, int k, int lane) {
-    const int n = *cnt;
-    const int keep = n < k ? n : k;
-    for (int r = 0; r < keep; ++r) {
-        unsigned long long best = 0ull;
-        int bi = -1;
-        for (int i = r + lane; i < n; i += 32) {
-            const unsigned long long v = c[i];
-            if (v > best) { best = v; bi = i; }
-        }
-        unsigned long long m = best;
-#pragma unroll
-        for (int o = 16; o; o >>= 1) {
-            const unsigned long long t = __shfl_xor_sync(0xffffffffu, m, o);
-            m = t > m ? t : m;
-        }
-        if (best == m && bi >= 0) {
-            c[bi] = c[r];
-            c[r] = m;
-        }
-        __syncwarp();
-    }
-    if (lane == 0) {
-        *cnt = keep;
-        *thr = (keep == k) ? c[k - 1] : 0ull;
-    }
-    __syncwarp();
-}
-
 // W2 [c1, c2] fp32 (Keras [in,out]) -> B operand image: element (n, k) = bf16(W2[k][n]), K-major, SWIZZLE_128B
 __global__ void score_tc_prep_kernel(const float *__restrict__ w2, int c1, int c2, int n_pad, int kb_count,
                                      uint8_t *__restrict__ image) {
@@ -100,7 +63,7 @@ __global__ void __launch_bounds__(kTcThreads, QREG ? 4 : 3) score_tc_kernel(cons
     const int kb_count = (c1 + 63) / 64;
     const int c1p = kb_count * 64;
     const int n_pad = (p.c2 + 15) / 16 * 16;
-    const int cap = 2 * p.k + kTcTI;
+    const int cap = topk_list_cap(p.k);
     // carve shared memory (operand tiles first: SWIZZLE_128B needs 1024-byte alignment)
     // (pointers are derived from the __shared__ array without integer round-trips so that the
     //  compiler keeps them in the shared address space: LDS/STS, not generic LD/ST)
@@ -165,7 +128,7 @@ __global__ void __launch_bounds__(kTcThreads, QREG ? 4 : 3) score_tc_kernel(cons
 
     for (int t0 = 0; t0 < p.n_items; t0 += kTcTI) {
         for (int ul = warp; ul < kTcTU; ul += kTcThreads / 32)   // user ul is always handled by warp ul % 4
-            if (cnt[ul] > cap - kTcTI) tcs_compact(cand + ul * cap, cnt + ul, thr + ul, p.k, lane);
+            topk_make_room(cand, cnt, thr, cap, ul, p.k, lane);
         const int item = t0 + lane;
         const bool item_ok = item < p.n_items;
         const float *qrow = p.Q + (int64_t)(item_ok ? item : 0) * p.ldq;
@@ -245,15 +208,9 @@ __global__ void __launch_bounds__(kTcThreads, QREG ? 4 : 3) score_tc_kernel(cons
                 }
             }
             const int64_t user = u0 + ul;
-            if (item_ok && user < p.n_users) {
-                // candidates are ranked by the logit (sigmoid is monotonic); the sigmoid is applied to the k winners
-                const unsigned long long key =
-                    ((unsigned long long)tcs_orderable(logit + b3) << 32) | (unsigned long long)(0xffffffffu - (uint32_t)item);
-                if (key > thr[ul] && !(kExcl && excluded_item(p.excl_rowptr, p.excl_items, user, item))) {
-                    const int pos = atomicAdd(cnt + ul, 1);
-                    cand[ul * cap + pos] = key;
-                }
-            }
+            // candidates are ranked by the logit (sigmoid is monotonic); the sigmoid is applied to the k winners
+            if (item_ok && user < p.n_users)
+                topk_offer<kExcl>(cand, cnt, thr, cap, ul, logit + b3, item, user, p.excl_rowptr, p.excl_items);
         }
     }
     tc::tc_fence_before_sync();
@@ -262,23 +219,8 @@ __global__ void __launch_bounds__(kTcThreads, QREG ? 4 : 3) score_tc_kernel(cons
         tc::tc_fence_after_sync();
         tc::tmem_dealloc(tmem_base, tmem_cols);
     }
-    for (int ul = warp; ul < kTcTU; ul += kTcThreads / 32) {
-        tcs_compact(cand + ul * cap, cnt + ul, thr + ul, p.k, lane);
-        const int64_t user = u0 + ul;
-        if (user >= p.n_users) continue;
-        const int n = cnt[ul];
-        for (int r = lane; r < p.k; r += 32) {
-            const int64_t o = user * p.k + r;
-            if (r < n) {
-                const unsigned long long key = cand[ul * cap + r];
-                p.ids_out[o] = (int32_t)(0xffffffffu - (uint32_t)(key & 0xffffffffull));
-                p.scores_out[o] = 1.f / (1.f + expf(-tcs_from_orderable((uint32_t)(key >> 32))));
-            } else {
-                p.ids_out[o] = -1;
-                p.scores_out[o] = -INFINITY;
-            }
-        }
-    }
+    for (int ul = warp; ul < kTcTU; ul += kTcThreads / 32)
+        topk_write<true>(cand, cnt, thr, cap, ul, p.k, lane, u0 + ul, p.n_users, p.ids_out, p.scores_out);
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -330,7 +272,7 @@ __global__ void __launch_bounds__(kTcThreads, 4) score_tc2_kernel(const __grid_c
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     const int c1 = p.c1;
     const int n_pad = (p.c2 + 15) / 16 * 16;
-    const int cap = 2 * p.k + kTcTI;
+    const int cap = topk_list_cap(p.k);
     unsigned char *As = smem_raw;                                    // [2][128][128 B]
     unsigned char *Bs = As + 2 * 16384;                              // [n_pad][128 B]
     uint4 *Pb = reinterpret_cast<uint4 *>(Bs + n_pad * 128);         // [TU][8] bf16 rows of P
@@ -438,7 +380,7 @@ __global__ void __launch_bounds__(kTcThreads, 4) score_tc2_kernel(const __grid_c
         const int nxt = step + 1;
         if (pass == 0)
             for (int ul = warp; ul < kTcTU; ul += kTcThreads / 32)
-                if (cnt[ul] > cap - kTcTI) tcs_compact(cand + ul * cap, cnt + ul, thr + ul, p.k, lane);
+                topk_make_room(cand, cnt, thr, cap, ul, p.k, lane);
         if (nxt < n_steps) {
             produce(nxt);                                   // qreg holds the tile of step nxt
             if (nxt % kPasses == kPasses - 1 && nxt + 1 < n_steps) load_q(nxt / kPasses + 1);  // refill for the tile after
@@ -479,14 +421,8 @@ __global__ void __launch_bounds__(kTcThreads, 4) score_tc2_kernel(const __grid_c
         const int ul = pass * 4 + warp;
         const int item = tile * kTcTI + lane;
         const int64_t user = u0 + ul;
-        if (item < p.n_items && user < p.n_users) {
-            const unsigned long long key =
-                ((unsigned long long)tcs_orderable(logit + b3) << 32) | (unsigned long long)(0xffffffffu - (uint32_t)item);
-            if (key > thr[ul] && !(kExcl && excluded_item(p.excl_rowptr, p.excl_items, user, item))) {
-                const int pos = atomicAdd(cnt + ul, 1);
-                cand[ul * cap + pos] = key;
-            }
-        }
+        if (item < p.n_items && user < p.n_users)
+            topk_offer<kExcl>(cand, cnt, thr, cap, ul, logit + b3, item, user, p.excl_rowptr, p.excl_items);
     }
     tc::tc_fence_before_sync();
     __syncthreads();
@@ -494,23 +430,8 @@ __global__ void __launch_bounds__(kTcThreads, 4) score_tc2_kernel(const __grid_c
         tc::tc_fence_after_sync();
         tc::tmem_dealloc(tmem_base, tmem_cols);
     }
-    for (int ul = warp; ul < kTcTU; ul += kTcThreads / 32) {
-        tcs_compact(cand + ul * cap, cnt + ul, thr + ul, p.k, lane);
-        const int64_t user = u0 + ul;
-        if (user >= p.n_users) continue;
-        const int n = cnt[ul];
-        for (int r = lane; r < p.k; r += 32) {
-            const int64_t o = user * p.k + r;
-            if (r < n) {
-                const unsigned long long key = cand[ul * cap + r];
-                p.ids_out[o] = (int32_t)(0xffffffffu - (uint32_t)(key & 0xffffffffull));
-                p.scores_out[o] = 1.f / (1.f + expf(-tcs_from_orderable((uint32_t)(key >> 32))));
-            } else {
-                p.ids_out[o] = -1;
-                p.scores_out[o] = -INFINITY;
-            }
-        }
-    }
+    for (int ul = warp; ul < kTcTU; ul += kTcThreads / 32)
+        topk_write<true>(cand, cnt, thr, cap, ul, p.k, lane, u0 + ul, p.n_users, p.ids_out, p.scores_out);
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -615,7 +536,7 @@ __device__ __forceinline__ uint32_t w3_pack_relu(float lo, float hi) {
 template <bool kExcl>   // exclusion lists given
 __global__ void __launch_bounds__(kW3Threads, 1) score_tc3_kernel(const __grid_constant__ ScoreTc3Params p) {
     extern __shared__ __align__(1024) unsigned char smem_raw[];
-    const int cap = 2 * p.k + kTcTI;
+    const int cap = topk_list_cap(p.k);
     unsigned char *W1 = smem_raw;                                    // [2][64][128 B]
     unsigned char *W3 = W1 + 2 * 8192;                               // [16][128 B]
     uint4 *Pb = reinterpret_cast<uint4 *>(W3 + 2048);                // [TU][8] bf16 rows of P
@@ -754,7 +675,7 @@ __global__ void __launch_bounds__(kW3Threads, 1) score_tc3_kernel(const __grid_c
         int step = 0;
         for (int tile = 0; tile < n_tiles; ++tile) {
             for (int ul = quad; ul < kTcTU; ul += 4)   // user ul is only ever touched by the final warp of quadrant ul % 4
-                if (cnt[ul] > cap - kTcTI) tcs_compact(cand + ul * cap, cnt + ul, thr + ul, p.k, lane);
+                topk_make_room(cand, cnt, thr, cap, ul, p.k, lane);
 #pragma unroll 1
             for (int pass = 0; pass < kPasses; ++pass, ++step) {
                 const int buf = step % kW3NB;
@@ -768,14 +689,8 @@ __global__ void __launch_bounds__(kW3Threads, 1) score_tc3_kernel(const __grid_c
                 const int ul = pass * 4 + quad;
                 const int item = tile * kTcTI + lane;
                 const int64_t user = u0 + ul;
-                if (item < p.n_items && user < p.n_users) {
-                    const unsigned long long key =
-                        ((unsigned long long)tcs_orderable(logit + b3) << 32) | (unsigned long long)(0xffffffffu - (uint32_t)item);
-                    if (key > thr[ul] && !(kExcl && excluded_item(p.excl_rowptr, p.excl_items, user, item))) {
-                        const int pos = atomicAdd(cnt + ul, 1);
-                        cand[ul * cap + pos] = key;
-                    }
-                }
+                if (item < p.n_items && user < p.n_users)
+                    topk_offer<kExcl>(cand, cnt, thr, cap, ul, logit + b3, item, user, p.excl_rowptr, p.excl_items);
             }
         }
     } else {
@@ -820,40 +735,24 @@ __global__ void __launch_bounds__(kW3Threads, 1) score_tc3_kernel(const __grid_c
         tc::tc_fence_after_sync();
         tc::tmem_dealloc(tmem_base, 512);
     }
-    for (int ul = warp; ul < kTcTU; ul += kW3Threads / 32) {
-        tcs_compact(cand + ul * cap, cnt + ul, thr + ul, p.k, lane);
-        const int64_t user = u0 + ul;
-        if (user >= p.n_users) continue;
-        const int n = cnt[ul];
-        for (int r = lane; r < p.k; r += 32) {
-            const int64_t o = user * p.k + r;
-            if (r < n) {
-                const unsigned long long key = cand[ul * cap + r];
-                p.ids_out[o] = (int32_t)(0xffffffffu - (uint32_t)(key & 0xffffffffull));
-                p.scores_out[o] = 1.f / (1.f + expf(-tcs_from_orderable((uint32_t)(key >> 32))));
-            } else {
-                p.ids_out[o] = -1;
-                p.scores_out[o] = -INFINITY;
-            }
-        }
-    }
+    for (int ul = warp; ul < kTcTU; ul += kW3Threads / 32)
+        topk_write<true>(cand, cnt, thr, cap, ul, p.k, lane, u0 + ul, p.n_users, p.ids_out, p.scores_out);
 }
 
 static size_t score_tc3_smem(int k) {
-    const int cap = 2 * k + kTcTI;
-    return 2 * 8192 + 2048 + (size_t)kTcTU * 8 * 16 + (size_t)kTcTU * cap * 8 + kTcTU * 8 + 8 * kW3NB * 8 + kTcTU * 4 + 16;
+    return 2 * 8192 + 2048 + (size_t)kTcTU * 8 * 16 + topk_lists_smem_bytes(kTcTU, k) + 8 * kW3NB * 8 + 16;
 }
 
 static size_t score_tc2_smem(int c2, int k) {
-    const int n_pad = (c2 + 15) / 16 * 16, cap = 2 * k + kTcTI;
+    const int n_pad = (c2 + 15) / 16 * 16;
     return 1024 + 2 * 16384 + (size_t)n_pad * 128 + (size_t)kTcTU * 8 * 16 + (size_t)(n_pad / 2) * 16 +
-           (size_t)kTcTU * cap * 8 + kTcTU * 8 + 16 + kTcTU * 4 + 16;
+           topk_lists_smem_bytes(kTcTU, k) + 16 + 16;
 }
 
 static size_t score_tc_smem(int c1, int c2, int k) {
-    const int kb = (c1 + 63) / 64, n_pad = (c2 + 15) / 16 * 16, cap = 2 * k + kTcTI;
+    const int kb = (c1 + 63) / 64, n_pad = (c2 + 15) / 16 * 16;
     return 1024 + (size_t)kb * 16384 + (size_t)kb * n_pad * 128 + (size_t)kTcTU * kb * 64 * 4 + (size_t)n_pad * 8 +
-           (size_t)kTcTU * cap * 8 + kTcTU * 8 + 8 + kTcTU * 4 + 16;
+           topk_lists_smem_bytes(kTcTU, k) + 8 + 16;
 }
 
 }  // namespace cbrs
@@ -886,10 +785,8 @@ extern "C" int cbrs_score_catalog_topk_bf16_ex(const float *P, int64_t ldp, cons
                                                float *scores_out, const int64_t *excl_rowptr, const int32_t *excl_items,
                                                void *workspace, size_t workspace_bytes, void *stream) {
     CBRS_REQUIRE(P && Q && w2 && b2 && w3 && b3 && ids_out && scores_out, CBRS_E_INVALID, "score_catalog_bf16: null argument");
-    CBRS_REQUIRE(!excl_rowptr == !excl_items, CBRS_E_INVALID, "score_catalog_bf16: %s is null but %s is not",
-                 excl_rowptr ? "excl_items" : "excl_rowptr", excl_rowptr ? "excl_rowptr" : "excl_items");
-    CBRS_REQUIRE(n_users >= 0 && n_items > 0 && k > 0 && k <= 128, CBRS_E_INVALID, "score_catalog_bf16: n_users=%lld n_items=%d k=%d",
-                 (long long)n_users, n_items, k);
+    const int rc = check_catalog_args("score_catalog_bf16", excl_rowptr, excl_items, n_users, n_items, k);
+    if (rc != CBRS_OK) return rc;
     CBRS_REQUIRE(c1 >= 8 && c1 % 8 == 0 && c1 <= 256 && c2 > 0 && c2 <= 256, CBRS_E_UNSUPPORTED,
                  "score_catalog_bf16: classifier widths c1=%d (multiple of 8, <= 256), c2=%d (<= 256)", c1, c2);
     CBRS_REQUIRE(ldp >= c1 && ldq >= c1 && ldq % 4 == 0 && ((uintptr_t)Q % 16) == 0, CBRS_E_INVALID,
@@ -911,38 +808,23 @@ extern "C" int cbrs_score_catalog_topk_bf16_ex(const float *P, int64_t ldp, cons
             uint8_t *img = (uint8_t *)workspace + align_up((size_t)kb * n_pad * 128) + align_up((size_t)n_items_pad * 128);
             score_tc3_prep_kernel<<<8, 256, 0, s>>>(w2, b2, w3, c1, c2, img, img + 2 * 8192);
             CBRS_CHECK_LAUNCH("score_tc3_prep");
-            const size_t smem3 = score_tc3_smem(k);
-            CBRS_REQUIRE(smem3 <= 200 * 1024, CBRS_E_UNSUPPORTED, "score_catalog_bf16: needs %zu bytes of shared memory", smem3);
-            auto k3 = excl_rowptr ? score_tc3_kernel<true> : score_tc3_kernel<false>;
-            cudaError_t e3 = cudaFuncSetAttribute(k3, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem3);
-            CBRS_REQUIRE(e3 == cudaSuccess, CBRS_E_CUDA, "score_catalog_bf16: cudaFuncSetAttribute: %s", cudaGetErrorString(e3));
             ScoreTc3Params p3{P, ldp, Qb, n_users, n_items, c1, c2, img, img + 2 * 8192, b3, k, ids_out, scores_out,
                                excl_rowptr, excl_items};
-            k3<<<(unsigned)cdiv(n_users, kTcTU), kW3Threads, smem3, s>>>(p3);
-            CBRS_CHECK_LAUNCH("score_tc3");
-            return CBRS_OK;
+            return launch_catalog_scorer(score_tc3_kernel<false>, score_tc3_kernel<true>, p3, (unsigned)cdiv(n_users, kTcTU),
+                                         kW3Threads, score_tc3_smem(k), 200 * 1024, s, "score_catalog_bf16", "score_tc3");
         }
-        const size_t smem2 = score_tc2_smem(c2, k);
-        CBRS_REQUIRE(smem2 <= 220 * 1024, CBRS_E_UNSUPPORTED, "score_catalog_bf16: needs %zu bytes of shared memory", smem2);
         ScoreTc2Params p2{P, ldp, Qb, n_users, n_items, c1, c2, (const uint8_t *)workspace, b2, w3, b3, k, ids_out, scores_out,
                           excl_rowptr, excl_items};
-        auto k2 = excl_rowptr ? score_tc2_kernel<true> : score_tc2_kernel<false>;
-        cudaError_t e2 = cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
-        CBRS_REQUIRE(e2 == cudaSuccess, CBRS_E_CUDA, "score_catalog_bf16: cudaFuncSetAttribute: %s", cudaGetErrorString(e2));
-        k2<<<(unsigned)cdiv(n_users, kTcTU), kTcThreads, smem2, s>>>(p2);
-        CBRS_CHECK_LAUNCH("score_tc2");
-        return CBRS_OK;
+        return launch_catalog_scorer(score_tc2_kernel<false>, score_tc2_kernel<true>, p2, (unsigned)cdiv(n_users, kTcTU),
+                                     kTcThreads, score_tc2_smem(c2, k), 220 * 1024, s, "score_catalog_bf16", "score_tc2");
     }
-    const size_t smem = score_tc_smem(c1, c2, k);
-    CBRS_REQUIRE(smem <= 220 * 1024, CBRS_E_UNSUPPORTED, "score_catalog_bf16: needs %zu bytes of shared memory", smem);
     ScoreTcParams p{P, ldp, Q, ldq, n_users, n_items, c1, c2, (const uint8_t *)workspace, b2, w3, b3, k, ids_out, scores_out,
                      excl_rowptr, excl_items};
-    const bool qreg = c1 <= 64;
-    auto k1 = qreg ? (excl_rowptr ? score_tc_kernel<true, true> : score_tc_kernel<true, false>)
-                   : (excl_rowptr ? score_tc_kernel<false, true> : score_tc_kernel<false, false>);
-    cudaError_t e = cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    CBRS_REQUIRE(e == cudaSuccess, CBRS_E_CUDA, "score_catalog_bf16: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    k1<<<(unsigned)cdiv(n_users, kTcTU), kTcThreads, smem, s>>>(p);
-    CBRS_CHECK_LAUNCH("score_tc");
-    return CBRS_OK;
+    const unsigned grid = (unsigned)cdiv(n_users, kTcTU);
+    const size_t smem = score_tc_smem(c1, c2, k);
+    if (c1 <= 64)
+        return launch_catalog_scorer(score_tc_kernel<true, false>, score_tc_kernel<true, true>, p, grid, kTcThreads, smem,
+                                     220 * 1024, s, "score_catalog_bf16", "score_tc");
+    return launch_catalog_scorer(score_tc_kernel<false, false>, score_tc_kernel<false, true>, p, grid, kTcThreads, smem,
+                                 220 * 1024, s, "score_catalog_bf16", "score_tc");
 }

@@ -17,9 +17,8 @@
 // and cap the pipe at 2/3 of its rate).  Wh / Wl sit in shared memory as the K-major SWIZZLE_128B images
 // cbrs_dense_tf32x3_prepare writes.  One thread issues the 3 x c1/8 MMAs (M = 128, N = c2, K = 8) and commits to
 // mbarriers; an epilogue thread reads its accumulator row back (tcgen05.ld), adds the bias, applies relu and the output
-// layer in fp32 and feeds the running per-user top-k lists (candidate scheme of score.cu: keys (score bits, ~item),
-// ties to the lower item index, result independent of insertion order).  Operand and accumulator are double buffered in
-// TMEM and the three stages run on their own warps (below).
+// layer in fp32 and feeds the running per-user top-k lists (the candidate lists of common.cuh, keyed on the logit).
+// Operand and accumulator are double buffered in TMEM and the three stages run on their own warps (below).
 #include "common.cuh"
 #include "tc05.cuh"
 
@@ -76,7 +75,7 @@ __global__ void __launch_bounds__(kS3WsThreads, 1) score_tf32x3_ws_kernel(const 
     static_assert(2 * NP + 4 * C1 <= 512, "TMEM budget");
     static_assert(E == 16 || E == 32, "a producer thread's slice is one 16- or 32-column TMEM store");
     constexpr int kThreads = kS3WsThreads;
-    const int cap = 2 * p.k + kS3TI;
+    const int cap = topk_list_cap(p.k);
     unsigned char *Wh = s3_smem;                     // [kAtoms][NP][128 B]
     unsigned char *Wl = Wh + kImage;
     float *Ps = reinterpret_cast<float *>(Wl + kImage);              // [TU][C1]
@@ -216,7 +215,7 @@ __global__ void __launch_bounds__(kS3WsThreads, 1) score_tf32x3_ws_kernel(const 
         for (int tile = 0; tile < n_tiles; ++tile) {
             // a user's list must have room for the 32 candidates one item tile can add
             for (int ul = quad; ul < kS3TU; ul += 4)   // user ul is only ever touched by warp 9 + ul % 4
-                if (cnt[ul] > cap - kS3TI) topk_compact(cand + ul * cap, cnt + ul, thr + ul, p.k, lane);
+                topk_make_room(cand, cnt, thr, cap, ul, p.k, lane);
 #pragma unroll 1
             for (int pass = 0; pass < kPasses; ++pass, ++step) {
                 const int buf = step & 1;
@@ -241,15 +240,9 @@ __global__ void __launch_bounds__(kS3WsThreads, 1) score_tf32x3_ws_kernel(const 
                 const int ul = pass * 4 + quad;
                 const int item = tile * kS3TI + lane;
                 const int64_t user = u0 + ul;
-                if (item < p.n_items && user < p.n_users) {
-                    // candidates are ranked by the logit (sigmoid is monotonic); the sigmoid is applied to the k winners
-                    const unsigned long long key = ((unsigned long long)orderable_f32(logit + b3) << 32) |
-                                                   (unsigned long long)(0xffffffffu - (uint32_t)item);
-                    if (key > thr[ul] && !(kExcl && excluded_item(p.excl_rowptr, p.excl_items, user, item))) {
-                        const int pos = atomicAdd(cnt + ul, 1);
-                        cand[ul * cap + pos] = key;
-                    }
-                }
+                // candidates are ranked by the logit (sigmoid is monotonic); the sigmoid is applied to the k winners
+                if (item < p.n_items && user < p.n_users)
+                    topk_offer<kExcl>(cand, cnt, thr, cap, ul, logit + b3, item, user, p.excl_rowptr, p.excl_items);
             }
         }
     }
@@ -259,41 +252,19 @@ __global__ void __launch_bounds__(kS3WsThreads, 1) score_tf32x3_ws_kernel(const 
         tc::tc_fence_after_sync();
         tc::tmem_dealloc(tmem_base, kCols);
     }
-    for (int ul = warp; ul < kS3TU; ul += kThreads / 32) {
-        topk_compact(cand + ul * cap, cnt + ul, thr + ul, p.k, lane);
-        const int64_t user = u0 + ul;
-        if (user >= p.n_users) continue;
-        const int n = cnt[ul];
-        for (int r = lane; r < p.k; r += 32) {
-            const int64_t o = user * p.k + r;
-            if (r < n) {
-                const unsigned long long key = cand[ul * cap + r];
-                p.ids_out[o] = (int32_t)(0xffffffffu - (uint32_t)(key & 0xffffffffull));
-                p.scores_out[o] = 1.f / (1.f + expf(-from_orderable_f32((uint32_t)(key >> 32))));
-            } else {
-                p.ids_out[o] = -1;
-                p.scores_out[o] = -INFINITY;
-            }
-        }
-    }
+    for (int ul = warp; ul < kS3TU; ul += kThreads / 32)
+        topk_write<true>(cand, cnt, thr, cap, ul, p.k, lane, u0 + ul, p.n_users, p.ids_out, p.scores_out);
 }
 
 static size_t s3_smem_bytes(int c1, int np, int k) {
-    const int cap = 2 * k + kS3TI;
-    return 2 * (size_t)(c1 / 32) * np * 128 + (size_t)kS3TU * c1 * 4 + (size_t)np * 8 + (size_t)kS3TU * cap * 8 + kS3TU * 8 + 8 * 8 +
-           kS3TU * 4 + 16;
+    return 2 * (size_t)(c1 / 32) * np * 128 + (size_t)kS3TU * c1 * 4 + (size_t)np * 8 + topk_lists_smem_bytes(kS3TU, k) + 8 * 8 + 16;
 }
 
 template <int C1, int NP>
 static int s3_launch_ws(const ScoreT3Params &p, cudaStream_t s) {
-    const size_t smem = s3_smem_bytes(C1, NP, p.k);
-    CBRS_REQUIRE(smem <= 200 * 1024, CBRS_E_UNSUPPORTED, "score_catalog_tf32x3: needs %zu bytes of shared memory", smem);
-    auto kernel = p.excl_rowptr ? score_tf32x3_ws_kernel<C1, NP, true> : score_tf32x3_ws_kernel<C1, NP, false>;
-    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    CBRS_REQUIRE(e == cudaSuccess, CBRS_E_CUDA, "score_catalog_tf32x3: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    kernel<<<(unsigned)cdiv(p.n_users, kS3TU), kS3WsThreads, smem, s>>>(p);
-    CBRS_CHECK_LAUNCH("score_catalog_tf32x3");
-    return CBRS_OK;
+    return launch_catalog_scorer(score_tf32x3_ws_kernel<C1, NP, false>, score_tf32x3_ws_kernel<C1, NP, true>, p,
+                                 (unsigned)cdiv(p.n_users, kS3TU), kS3WsThreads, s3_smem_bytes(C1, NP, p.k), 200 * 1024, s,
+                                 "score_catalog_tf32x3", "score_catalog_tf32x3");
 }
 
 }  // namespace cbrs
@@ -323,10 +294,8 @@ extern "C" int cbrs_score_catalog_topk_tf32x3_ex(const float *P, int64_t ldp, co
                                                  float *scores_out, const int64_t *excl_rowptr, const int32_t *excl_items,
                                                  void *workspace, size_t workspace_bytes, void *stream) {
     CBRS_REQUIRE(P && Q && w2 && b2 && w3 && b3 && ids_out && scores_out, CBRS_E_INVALID, "score_catalog_tf32x3: null argument");
-    CBRS_REQUIRE(!excl_rowptr == !excl_items, CBRS_E_INVALID, "score_catalog_tf32x3: %s is null but %s is not",
-                 excl_rowptr ? "excl_items" : "excl_rowptr", excl_rowptr ? "excl_rowptr" : "excl_items");
-    CBRS_REQUIRE(n_users >= 0 && n_items > 0 && k > 0 && k <= 128, CBRS_E_INVALID, "score_catalog_tf32x3: n_users=%lld n_items=%d k=%d",
-                 (long long)n_users, n_items, k);
+    const int rc = check_catalog_args("score_catalog_tf32x3", excl_rowptr, excl_items, n_users, n_items, k);
+    if (rc != CBRS_OK) return rc;
     CBRS_REQUIRE(cbrs_score_catalog_topk_tf32x3_eligible(c1, c2), CBRS_E_UNSUPPORTED,
                  "score_catalog_tf32x3: classifier widths c1=%d (32 or 64), c2=%d (<= 64); use cbrs_score_catalog_topk", c1, c2);
     CBRS_REQUIRE(ldp >= c1 && ldq >= c1 && ldq % 4 == 0 && ((uintptr_t)Q % 16) == 0, CBRS_E_INVALID,
@@ -348,8 +317,8 @@ extern "C" int cbrs_score_catalog_topk_tf32x3_ex(const float *P, int64_t ldp, co
         CBRS_REQUIRE(e == cudaSuccess, CBRS_E_CUDA, "score_catalog_tf32x3: padding W2: %s", cudaGetErrorString(e));
         w_src = w_pad;
     }
-    int rc = cbrs_dense_tf32x3_prepare(w_src, c1, np, image, stream);
-    if (rc != CBRS_OK) return rc;
+    const int rc_prep = cbrs_dense_tf32x3_prepare(w_src, c1, np, image, stream);
+    if (rc_prep != CBRS_OK) return rc_prep;
     ScoreT3Params p{P, ldp, Q, ldq, n_users, n_items, c1, c2, image, b2, w3, b3, k, ids_out, scores_out, excl_rowptr, excl_items};
     if (c1 == 64) return np == 64 ? s3_launch_ws<64, 64>(p, s) : s3_launch_ws<64, 32>(p, s);
     return np == 64 ? s3_launch_ws<32, 64>(p, s) : s3_launch_ws<32, 32>(p, s);

@@ -9,15 +9,6 @@
 
 namespace cbrs {
 
-// order-preserving map float -> uint32 (ascending)
-__device__ __forceinline__ uint32_t orderable(float f) {
-    const uint32_t u = __float_as_uint(f);
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float from_orderable(uint32_t o) {
-    return __uint_as_float((o & 0x80000000u) ? (o & 0x7fffffffu) : ~o);
-}
-
 constexpr int kTopkThreads = 256;
 
 // One CTA per user.  Candidates are 64-bit keys (score bits high, ~item low) so "better"
@@ -32,10 +23,9 @@ __global__ void __launch_bounds__(kTopkThreads) topk_rows_kernel(const float *__
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     unsigned long long bound = ~0ull;  // exclusive upper bound
     for (int r = 0; r < k; ++r) {
-        unsigned long long best = 0ull;  // 0 is below every real key (orderable(-inf) > 0)
+        unsigned long long best = 0ull;  // 0 is below every real key
         for (int i = threadIdx.x; i < n_items; i += kTopkThreads) {
-            const unsigned long long key =
-                ((unsigned long long)orderable(row[i]) << 32) | (unsigned long long)(0xffffffffu - (uint32_t)i);
+            const unsigned long long key = topk_key(row[i], (uint32_t)i);
             if (key < bound && key > best) best = key;
         }
 #pragma unroll
@@ -51,13 +41,7 @@ __global__ void __launch_bounds__(kTopkThreads) topk_rows_kernel(const float *__
             for (int w = 1; w < kTopkThreads / 32; ++w) b = warp_best[w] > b ? warp_best[w] : b;
             winner = b;
             const int64_t o = (int64_t)blockIdx.x * k + r;
-            if (b == 0ull) {  // fewer than k items
-                ids_out[o] = -1;
-                vals_out[o] = -INFINITY;
-            } else {
-                ids_out[o] = (int32_t)(0xffffffffu - (uint32_t)(b & 0xffffffffull));
-                vals_out[o] = from_orderable((uint32_t)(b >> 32));
-            }
+            topk_store<false>(b, ids_out + o, vals_out + o);   // b = 0: fewer than k items
         }
         __syncthreads();
         bound = winner;
@@ -70,7 +54,7 @@ __global__ void pair_keys_kernel(const int64_t *__restrict__ users, const float 
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     // ascending key == (user asc, score desc); the stable sort keeps input order on ties
-    keys[i] = ((uint64_t)users[i] << 32) | (uint64_t)(~orderable(scores[i]));
+    keys[i] = ((uint64_t)users[i] << 32) | (uint64_t)(~orderable_f32(scores[i]));
     payload[i] = (uint32_t)i;
 }
 

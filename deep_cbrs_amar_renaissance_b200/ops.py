@@ -697,92 +697,70 @@ def score_catalog_topk(P, Q, w2, b2, w3, b3, k, precision="fp32", exclude=None):
     exclude = (rowptr, items): per-row lists of catalog items kept out of row r's top-k (row r = row r of P)."""
     lib = L.load()
     rp, it = _exclusion(exclude, P.shape[0])
-    if precision == "fp32" and lib.cbrs_score_catalog_topk_tf32x3_eligible(P.shape[1], w2.shape[1]):
-        P, ldp = _rowmajor(P)
-        Q, ldq = _rowmajor(Q)
-        n_users, c1 = P.shape
-        c2 = w2.shape[1]
-        ids = torch.empty(n_users, k, dtype=torch.int32, device=P.device)
-        vals = torch.empty(n_users, k, dtype=torch.float32, device=P.device)
-        ws = _ws(lib.cbrs_score_catalog_topk_tf32x3_workspace_bytes(c1, c2), P.device)
-        L.check(lib.cbrs_score_catalog_topk_tf32x3_ex(_ptr(P), ldp, _ptr(Q), ldq, n_users, Q.shape[0], c1,
-                                                      _ptr(w2, torch.float32), _ptr(b2, torch.float32), c2,
-                                                      _ptr(w3, torch.float32), _ptr(b3, torch.float32), k, _ptr(ids),
-                                                      _ptr(vals), rp, it, _ptr(ws), ws.numel(), _stream()),
-                "cbrs_score_catalog_topk_tf32x3")
-        _count(2)
-        return ids, vals
     if precision not in ("fp32", "fp32-ffma", "bf16"):
         raise L.CbrsError("score_catalog_topk: precision must be 'fp32', 'fp32-ffma' or 'bf16'")
-    if precision == "bf16":
-        P, ldp = _rowmajor(P)
-        Q, ldq = _rowmajor(Q)
-        n_users, c1 = P.shape
-        c2 = w2.shape[1]
-        ids = torch.empty(n_users, k, dtype=torch.int32, device=P.device)
-        vals = torch.empty(n_users, k, dtype=torch.float32, device=P.device)
-        ws = _ws(lib.cbrs_score_catalog_topk_bf16_workspace_bytes(Q.shape[0], c1, c2), P.device)
-        L.check(lib.cbrs_score_catalog_topk_bf16_ex(_ptr(P), ldp, _ptr(Q), ldq, n_users, Q.shape[0], c1,
-                                                    _ptr(w2, torch.float32), _ptr(b2, torch.float32), c2,
-                                                    _ptr(w3, torch.float32), _ptr(b3, torch.float32), k, _ptr(ids),
-                                                    _ptr(vals), rp, it, _ptr(ws), ws.numel(), _stream()),
-                "cbrs_score_catalog_topk_bf16")
-        _count(4 if (c1 <= 64 and c2 <= 64) else (3 if c1 <= 64 and c2 <= 128 else 2))
-        return ids, vals
     P, ldp = _rowmajor(P)
     Q, ldq = _rowmajor(Q)
     n_users, c1 = P.shape
     n_items = Q.shape[0]
     c2 = w2.shape[1]
+    # entry point, workspace bytes (None: takes no workspace), launches
+    if precision == "fp32" and lib.cbrs_score_catalog_topk_tf32x3_eligible(c1, c2):
+        name, ws_bytes, launches = "cbrs_score_catalog_topk_tf32x3", lib.cbrs_score_catalog_topk_tf32x3_workspace_bytes(c1, c2), 2
+    elif precision == "bf16":
+        name, ws_bytes, launches = ("cbrs_score_catalog_topk_bf16",
+                                    lib.cbrs_score_catalog_topk_bf16_workspace_bytes(n_items, c1, c2),
+                                    4 if (c1 <= 64 and c2 <= 64) else (3 if c1 <= 64 and c2 <= 128 else 2))
+    else:
+        name, ws_bytes, launches = "cbrs_score_catalog_topk", None, 1
     ids = torch.empty(n_users, k, dtype=torch.int32, device=P.device)
     vals = torch.empty(n_users, k, dtype=torch.float32, device=P.device)
-    L.check(lib.cbrs_score_catalog_topk_ex(_ptr(P), ldp, _ptr(Q), ldq, n_users, n_items, c1, _ptr(w2, torch.float32),
-                                           _ptr(b2, torch.float32), c2, _ptr(w3, torch.float32), _ptr(b3, torch.float32),
-                                           k, _ptr(ids), _ptr(vals), rp, it, _stream()), "cbrs_score_catalog_topk")
-    _count(1)
+    args = [_ptr(P), ldp, _ptr(Q), ldq, n_users, n_items, c1, _ptr(w2, torch.float32), _ptr(b2, torch.float32), c2,
+            _ptr(w3, torch.float32), _ptr(b3, torch.float32), k, _ptr(ids), _ptr(vals), rp, it]
+    if ws_bytes is not None:
+        ws = _ws(ws_bytes, P.device)
+        args += [_ptr(ws), ws.numel()]
+    L.check(getattr(lib, name + "_ex")(*args, _stream()), name)
+    _count(launches)
     return ids, vals
 
 
 # ------------------------------------------------------------------ misc
-def score_hybrid_topk_bf16(P1, Q1, P2, Q2, w3a2, b3a2, w3b2, b3b2, wc1, bc1, wc2, bc2, wc3, bc3, k, exclude=None):
-    """Feature-based hybrid scorer over the whole catalog + per-user top-k, chained tcgen05 kernel
-    (cbrs_score_hybrid_topk_bf16).  Returns (item index int32 [U, k], score float32 [U, k]).
-    exclude = (rowptr, items) as in score_catalog_topk."""
-    lib = L.load()
-    ts = [t.contiguous() for t in (P1, Q1, P2, Q2, w3a2, b3a2, w3b2, b3b2, wc1, bc1, wc2, bc2, wc3, bc3)]
+def _score_hybrid_topk(fn, name, ws_bytes, launches, tensors, k, exclude):
+    """Body of the two hybrid catalog scorers: entry point fn (reported as name), its workspace bytes and launch count;
+    tensors = (P1, Q1, P2, Q2, w3a2, ..., bc3) as in score_hybrid_topk_bf16."""
+    ts = [t.contiguous() for t in tensors]
     n_users, c = ts[0].shape
     rp, it = _exclusion(exclude, n_users)
     n_items = ts[1].shape[0]
     dev = ts[0].device
     ids = torch.empty(n_users, k, dtype=torch.int32, device=dev)
     vals = torch.empty(n_users, k, dtype=torch.float32, device=dev)
-    ws = _ws(lib.cbrs_score_hybrid_topk_bf16_workspace_bytes(), dev)
-    L.check(lib.cbrs_score_hybrid_topk_bf16_ex(_ptr(ts[0], torch.float32), _ptr(ts[1], torch.float32),
-                                               _ptr(ts[2], torch.float32), _ptr(ts[3], torch.float32), n_users, n_items, c,
-                                               *[_ptr(t, torch.float32) for t in ts[4:]], k, _ptr(ids), _ptr(vals), rp, it,
-                                               _ptr(ws), ws.numel(), _stream()), "cbrs_score_hybrid_topk_bf16")
-    _count(2)
+    ws = _ws(ws_bytes, dev)
+    L.check(fn(_ptr(ts[0], torch.float32), _ptr(ts[1], torch.float32), _ptr(ts[2], torch.float32), _ptr(ts[3], torch.float32),
+               n_users, n_items, c, *[_ptr(t, torch.float32) for t in ts[4:]], k, _ptr(ids), _ptr(vals), rp, it, _ptr(ws),
+               ws.numel(), _stream()), name)
+    _count(launches)
     return ids, vals
+
+
+def score_hybrid_topk_bf16(P1, Q1, P2, Q2, w3a2, b3a2, w3b2, b3b2, wc1, bc1, wc2, bc2, wc3, bc3, k, exclude=None):
+    """Feature-based hybrid scorer over the whole catalog + per-user top-k, chained tcgen05 kernel
+    (cbrs_score_hybrid_topk_bf16).  Returns (item index int32 [U, k], score float32 [U, k]).
+    exclude = (rowptr, items) as in score_catalog_topk."""
+    lib = L.load()
+    return _score_hybrid_topk(lib.cbrs_score_hybrid_topk_bf16_ex, "cbrs_score_hybrid_topk_bf16",
+                              lib.cbrs_score_hybrid_topk_bf16_workspace_bytes(), 2,
+                              (P1, Q1, P2, Q2, w3a2, b3a2, w3b2, b3b2, wc1, bc1, wc2, bc2, wc3, bc3), k, exclude)
 
 
 def score_hybrid_topk_tf32x3(P1, Q1, P2, Q2, w3a2, b3a2, w3b2, b3b2, wc1, bc1, wc2, bc2, wc3, bc3, k, exclude=None):
     """The scorer of score_hybrid_topk_bf16 at fp32 accuracy (1e-5): the five 64 x 64 products as 3xTF32 on the tensor
     cores (cbrs_score_hybrid_topk_tf32x3).  Same arguments and return value as score_hybrid_topk_bf16."""
     lib = L.load()
-    ts = [t.contiguous() for t in (P1, Q1, P2, Q2, w3a2, b3a2, w3b2, b3b2, wc1, bc1, wc2, bc2, wc3, bc3)]
-    n_users, c = ts[0].shape
-    rp, it = _exclusion(exclude, n_users)
-    n_items = ts[1].shape[0]
-    dev = ts[0].device
-    ids = torch.empty(n_users, k, dtype=torch.int32, device=dev)
-    vals = torch.empty(n_users, k, dtype=torch.float32, device=dev)
-    ws = _ws(lib.cbrs_score_hybrid_topk_tf32x3_workspace_bytes(), dev)
-    L.check(lib.cbrs_score_hybrid_topk_tf32x3(_ptr(ts[0], torch.float32), _ptr(ts[1], torch.float32),
-                                              _ptr(ts[2], torch.float32), _ptr(ts[3], torch.float32), n_users, n_items, c,
-                                              *[_ptr(t, torch.float32) for t in ts[4:]], k, _ptr(ids), _ptr(vals), rp, it,
-                                              _ptr(ws), ws.numel(), _stream()), "cbrs_score_hybrid_topk_tf32x3")
-    _count(6)
-    return ids, vals
+    return _score_hybrid_topk(lib.cbrs_score_hybrid_topk_tf32x3, "cbrs_score_hybrid_topk_tf32x3",
+                              lib.cbrs_score_hybrid_topk_tf32x3_workspace_bytes(), 6,
+                              (P1, Q1, P2, Q2, w3a2, b3a2, w3b2, b3b2, wc1, bc1, wc2, bc2, wc3, bc3), k, exclude)
 
 
 def synth_bipartite(n_users, n_items, n_edges, seed, device, scatter_items=True):
