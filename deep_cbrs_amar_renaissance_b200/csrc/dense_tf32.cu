@@ -30,6 +30,11 @@
 //             t+1's MMAs run under tile t's epilogue), bias, activation, 256-bit global stores (a full 32-byte sector per
 //             lane), optionally also into the peer-mapped copies of the other GPUs (multi-GPU all-gather from the
 //             producing kernel).
+// Deep contractions (k >= kT3SplitK): the error of the fp32 accumulator grows linearly with the 3 k / 8 MMAs a tile
+// issues into it (measured on a B200: 1.5e-5 of a tile's max |out| at k = 1536, n = 16; 0.56e-5 split).  From
+// kT3SplitK on the two cross terms Xl Wh + Xh Wl go to an accumulator of their own, n TMEM columns after the main one,
+// which then takes k / 8 MMAs; the epilogue adds the two.  The cross terms are 2^-11 of the product, so their own
+// rounding does not count.  Below kT3SplitK the single accumulator stays (and keeps its bits).
 // HBM traffic = X once + out once: the kernel's roofline is the copy bandwidth (1.7 ms at config 5).
 // Row results do not depend on the row's position in its tile (each accumulator element is an independent dot
 // product over K), so a row partition produces the same bits as the full run.
@@ -45,6 +50,7 @@ constexpr int kT3Atom = 32;      // fp32 elements per 128-byte swizzle row
 constexpr int kT3AtomBytes = kT3Rows * 128;   // one operand atom tile: 128 rows x 128 B
 constexpr int kT3MaxRaw = 8;     // at most this many landing slots for the TMA loads (16 KB each)
 constexpr int kT3Threads = 320;  // 4 split warps, 4 epilogue warps, producer warp, MMA warp
+constexpr int kT3SplitK = 384;   // from this k on the cross terms accumulate apart (eligible shapes there have n <= 64)
 
 struct T3Params {
     const uint8_t *w_image;  // [2 (hi, lo)][k_atoms][n][128 B], SWIZZLE_128B, K-major
@@ -61,7 +67,8 @@ struct T3Params {
     const float *addend; int64_t ld_add;   // optional [m, n] matrix added to the product before bias / row-op (cbrs_dense_tf32x3_ex)
     int32_t l2norm;     // CBRS_ROWOP_L2NORM: v / sqrt(max(sum v^2, 1e-12)) before the activation (GraphSageConv)
     int32_t n_raw;      // landing slots (2 .. kT3MaxRaw)
-    int32_t acc_bufs;   // accumulators in TMEM (2 when 2 n + 128 <= 512 columns, else 1)
+    int32_t acc_bufs;   // accumulators in TMEM (2 when 2 acc_cols + 128 <= 512 columns, else 1)
+    int32_t split_acc;  // k >= kT3SplitK: each accumulator is n main + n cross-term columns (acc_cols = 2 n, else n)
     // GAT row-op (cbrs_dense_tf32x3_attn): p[m] = out[m,:] . a_self, q[m] = out[m,:] . a_neigh (GATConv's attention logits)
     const float *a_self, *a_neigh;
     float *p_out, *q_out;
@@ -189,12 +196,14 @@ __global__ void __launch_bounds__(kT3Threads, 1)
     uint64_t *acc_full = op_empty + 2, *acc_empty = acc_full + 2, *w_full = acc_empty + 2;
     uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(w_full + 1);
     float *bias_s = reinterpret_cast<float *>(tmem_slot + 2);
-    // TMEM columns: accumulators [0, acc_bufs n), then the split operand, double buffered: (hi 32 | lo 32) x 2
-    const uint32_t col_a = (uint32_t)(p.acc_bufs * p.n);
+    // TMEM columns: accumulators [0, acc_bufs acc_cols) (each: n main columns, then n cross-term columns when split),
+    // then the split operand, double buffered: (hi 32 | lo 32) x 2
+    const uint32_t acc_cols = (uint32_t)(p.n << p.split_acc);
+    const uint32_t col_a = (uint32_t)p.acc_bufs * acc_cols;
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     uint32_t tmem_cols = 32;
-    while ((int)tmem_cols < p.acc_bufs * p.n + 128) tmem_cols <<= 1;
+    while (tmem_cols < col_a + 128) tmem_cols <<= 1;
     if ((tc::smem_u32(t3_smem) & 1023u) != 0u) __trap();  // SWIZZLE_128B tiles need the declared alignment
 
     if (warp == 0) tc::tmem_alloc(tmem_slot, tmem_cols);
@@ -258,7 +267,8 @@ __global__ void __launch_bounds__(kT3Threads, 1)
                 const int64_t acc_use = lt / p.acc_bufs;
                 if (acc_use > 0) tc::mbar_wait(acc_empty + acc, (uint32_t)(acc_use - 1) & 1u);
                 tc::tc_fence_after_sync();
-                const uint32_t d = tmem_base + (uint32_t)(acc * p.n);
+                const uint32_t d = tmem_base + (uint32_t)acc * acc_cols;
+                const uint32_t dx = p.split_acc ? d + (uint32_t)p.n : d;   // where the cross terms accumulate
                 for (int a = 0; a < k_atoms; ++a, ++it) {
                     const int o = (int)(it & 1);
                     tc::mbar_wait(op_ready + o, (uint32_t)(it >> 1) & 1u);
@@ -268,9 +278,10 @@ __global__ void __launch_bounds__(kT3Threads, 1)
 #pragma unroll
                     for (int ks = 0; ks < 4; ++ks) {   // 4 x K=8 inside the 32-wide atom; small terms first
                         const uint32_t koff = (uint32_t)ks * 32;
-                        t3_mma_ts(d, al + (uint32_t)ks * 8, tc::smem_desc_sw128(bh + koff), idesc, (a > 0 || ks > 0) ? 1u : 0u);
-                        t3_mma_ts(d, ah + (uint32_t)ks * 8, tc::smem_desc_sw128(bl + koff), idesc, 1u);
-                        t3_mma_ts(d, ah + (uint32_t)ks * 8, tc::smem_desc_sw128(bh + koff), idesc, 1u);
+                        const uint32_t more = (a > 0 || ks > 0) ? 1u : 0u;
+                        t3_mma_ts(dx, al + (uint32_t)ks * 8, tc::smem_desc_sw128(bh + koff), idesc, more);
+                        t3_mma_ts(dx, ah + (uint32_t)ks * 8, tc::smem_desc_sw128(bl + koff), idesc, 1u);
+                        t3_mma_ts(d, ah + (uint32_t)ks * 8, tc::smem_desc_sw128(bh + koff), idesc, p.split_acc ? more : 1u);
                     }
                     tc::mma_commit(op_empty + o);       // operand buffer reusable once these MMAs have read it
                 }
@@ -329,7 +340,20 @@ __global__ void __launch_bounds__(kT3Threads, 1)
             tc::mbar_wait(acc_full + acc, (uint32_t)(lt / p.acc_bufs) & 1u);
             tc::tc_fence_after_sync();
             const int64_t row = tile * kT3Rows + quad * 32 + lane;
-            const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(acc * p.n);
+            const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)acc * acc_cols;
+            // columns cb..cb+15 of the accumulator (warp-collective); cross: add the split-off cross terms
+            auto ld_acc = [&](int cb, uint32_t (&v)[16], bool cross) {
+                tc::tmem_ld16(taddr + (uint32_t)cb, v);
+                if (cross) {
+                    uint32_t c[16];
+                    tc::tmem_ld16(taddr + (uint32_t)(p.n + cb), c);
+                    tc::tmem_ld_wait();
+#pragma unroll
+                    for (int j = 0; j < 16; ++j) v[j] = __float_as_uint(__uint_as_float(v[j]) + __uint_as_float(c[j]));
+                } else {
+                    tc::tmem_ld_wait();
+                }
+            };
             float ps = 0.f, qs = 0.f;
             float scale = 1.f;
             const float *arow = (!kPlain && p.addend && row < p.m) ? p.addend + row * p.ld_add : nullptr;
@@ -348,8 +372,7 @@ __global__ void __launch_bounds__(kT3Threads, 1)
                 for (int cb = 0; cb < p.n; cb += 16) {
                     if (cb + 16 < p.n) load_add(cb + 16, a_nxt);
                     uint32_t v[16];
-                    tc::tmem_ld16(taddr + (uint32_t)cb, v);   // warp-collective
-                    tc::tmem_ld_wait();
+                    ld_acc(cb, v, p.split_acc);
 #pragma unroll
                     for (int q = 0; q < 4; ++q) {
                         const float4 bb = *reinterpret_cast<const float4 *>(bias_s + cb + 4 * q);
@@ -369,8 +392,7 @@ __global__ void __launch_bounds__(kT3Threads, 1)
             }
             for (int cb = 0; cb < p.n; cb += 16) {
                 uint32_t v[16];
-                tc::tmem_ld16(taddr + (uint32_t)cb, v);   // warp-collective
-                tc::tmem_ld_wait();
+                ld_acc(cb, v, p.split_acc && !folded);   // a folded accumulator already holds the cross terms
                 if (row < p.m) {
                     float o[2][8];
 #pragma unroll
@@ -536,7 +558,8 @@ static int t3_impl(const float *x, int64_t ldx, const void *w_image, const float
     p.addend = addend; p.ld_add = ld_add; p.l2norm = rowop == CBRS_ROWOP_L2NORM;
     p.n_tiles = cdiv(m, kT3Rows);
     p.n_raw = t3_raw_slots(k, n);
-    p.acc_bufs = (2 * n + 128 <= 512) ? 2 : 1;
+    p.split_acc = k >= kT3SplitK ? 1 : 0;
+    p.acc_bufs = (2 * (n << p.split_acc) + 128 <= 512) ? 2 : 1;
     const size_t smem = t3_smem_bytes(k, n);
     static bool attr_set = false;
     if (!attr_set) {
