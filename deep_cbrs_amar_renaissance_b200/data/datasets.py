@@ -6,6 +6,8 @@ np.random.RandomState(seed) re-shuffling a fresh arange at every epoch end.
 """
 import numpy as np
 
+from .. import checkpoint
+
 
 class Sequence:
     """Stand-in for keras.utils.Sequence: indexable, sized, with an epoch hook."""
@@ -18,6 +20,14 @@ class Sequence:
 
     def on_epoch_end(self):
         pass
+
+    def get_state(self):
+        """{name: ndarray}: what decides the batches of the epochs to come (the row order and the RandomState that
+        reshuffles it), saved by keras_like.BackupAndRestore so that a resumed fit replays them."""
+        return {}
+
+    def set_state(self, state):
+        """Put back get_state()'s arrays (ndarrays or anything np.asarray reads)."""
 
     def __iter__(self):
         return (self[i] for i in range(len(self)))
@@ -46,6 +56,25 @@ class _RatingBatches(Sequence):
             self.random_state = np.random.RandomState(self.seed)
         self.indexes = np.arange(len(self.ratings))
         self.random_state.shuffle(self.indexes)
+
+    def get_state(self):
+        if not self.shuffle:
+            return {}
+        return dict(checkpoint.rng_arrays(self.random_state), indexes=self.indexes)
+
+    def set_state(self, state):
+        if self.shuffle:
+            checkpoint.set_rng(self.random_state, state)
+            self.indexes = np.array(state["indexes"], dtype=np.int64)
+
+
+def _sub_states(subs):
+    return {name + "/" + k: a for name, seq in subs for k, a in seq.get_state().items()}
+
+
+def _set_sub_states(subs, state):
+    for name, seq in subs:
+        seq.set_state({k[len(name) + 1:]: a for k, a in state.items() if k.startswith(name + "/")})
 
 
 class UserItemGraph(_RatingBatches):
@@ -93,6 +122,12 @@ class HybridUserItemEmbeddings(Sequence):
         self.graph_embeddings.on_epoch_end()
         self.bert_embeddings.on_epoch_end()
 
+    def get_state(self):
+        return _sub_states([("graph_embeddings", self.graph_embeddings), ("bert_embeddings", self.bert_embeddings)])
+
+    def set_state(self, state):
+        _set_sub_states([("graph_embeddings", self.graph_embeddings), ("bert_embeddings", self.bert_embeddings)], state)
+
 
 class UserItemGraphEmbeddings(Sequence):
     """((user_ids, item_ids, bert[user], bert[item]), ratings) (datasets.py:309-373).
@@ -122,3 +157,9 @@ class UserItemGraphEmbeddings(Sequence):
     def on_epoch_end(self):
         self.graph_ids.on_epoch_end()
         self.embeddings.on_epoch_end()
+
+    def get_state(self):
+        return _sub_states([("graph_ids", self.graph_ids), ("embeddings", self.embeddings)])
+
+    def set_state(self, state):
+        _set_sub_states([("graph_ids", self.graph_ids), ("embeddings", self.embeddings)], state)

@@ -13,6 +13,11 @@ What is added, off unless a config sets the top-level key `catalog_metrics: true
 (every item ranked for every user, the user's training items excluded) against the test ratings, reported as
 catalog_{precision,recall,f1}_at_{k}; `catalog_metrics: all` adds catalog_{ndcg,map,hit_rate,mrr}_at_{k}.  The metrics
 are computed on the device from the lists and the test ratings (utilities.metrics.catalog_ranking_metrics).
+Every run keeps its trained model, as the reference's MLflow autolog does: <run dir>/model/weights.npz
+(Model.save_weights; Model.load_weights reads it into a model built from the run's config.yaml).  The top-level key
+`backup_and_restore: true` trains with a keras_like.BackupAndRestore(<run dir>/backup): a run that stopped before the
+end of training leaves its last epoch's state there, and running the same grid again continues that run, in its
+directory, from the next epoch, bit for bit as if it had not stopped.
 What is replaced: MLflow run management by a directory per run holding config.yaml, log.txt, metrics.json;
 ruamel.yaml by PyYAML with the YAML-1.2 float forms the files use (`1e-4`); the Java evaluator by
 utilities.metrics.top_k_metrics.
@@ -32,7 +37,7 @@ import yaml
 
 from . import models  # noqa: F401  (model modules are looked up by name below)
 from .data import loaders
-from .keras_like import set_seed
+from .keras_like import BackupAndRestore, set_seed
 from .models.basic import BasicGNN, BasicKnowledgeGCN, BasicRS, BasicTSGNN, BasicTWGNN
 from .models.hybrid import HybridBertGNN, HybridCBRS
 from .training import Adam
@@ -46,6 +51,7 @@ EXPERIMENTS_PATH = 'experiments.yaml'
 RUNS_PATH = './runs'
 LOG_FREQUENCY = 100
 METRICS_TOP_KS = [5, 10]
+WEIGHTS_FILE = 'weights.npz'   # <run dir>/model/, written by Model.save_weights after training
 CATALOG_METRICS = ("precision", "recall", "f1")   # catalog_metrics: true; `all` reports every RANKING_METRICS entry
 
 
@@ -87,6 +93,20 @@ class Config(dict):
         return {k: v.plain() if isinstance(v, Config) else v for k, v in self.items()}
 
 
+def _unfinished_run(exp_path, exp_name, config):
+    """The run directory of an earlier run of the same experiment (same name after the time stamp, same config) that
+    left a training backup, or None."""
+    stem = exp_name.split('-', 2)[2]
+    pattern = re.compile(r'^\d\d_\d\d-\d\d_\d\d-' + re.escape(stem) + r'(\.\d+)?$')
+    for name in sorted(os.listdir(exp_path)):
+        run_dir = os.path.join(exp_path, name)
+        saved = os.path.join(run_dir, 'artifacts', 'config.yaml')
+        if pattern.match(name) and os.path.exists(os.path.join(run_dir, 'backup', BackupAndRestore.FILE)) \
+                and os.path.exists(saved) and load_yaml(saved) == config:
+            return run_dir
+    return None
+
+
 def _by_signature(fn, mapping):
     """the entries of `mapping` that `fn` takes (experiment.py:125-127,131-133)"""
     accepted = inspect.signature(fn).parameters.keys()
@@ -116,13 +136,17 @@ class Experimenter:
             self.exp_name += '-{}-{}'.format(self.config.model.l2_regularizer, self.config.model.final_node)
         if self.config.get('details'):
             self.exp_name += '-' + str(self.config.details)
-        run_dir, k = os.path.join(exp_path, self.exp_name), 1
-        while os.path.exists(run_dir):
-            k += 1
-            run_dir = os.path.join(exp_path, "{}.{}".format(self.exp_name, k))
+        self.backup_and_restore = bool(self.config.get('backup_and_restore'))
+        run_dir = _unfinished_run(exp_path, self.exp_name, config) if self.backup_and_restore else None
+        if run_dir is None:
+            run_dir, k = os.path.join(exp_path, self.exp_name), 1
+            while os.path.exists(run_dir):
+                k += 1
+                run_dir = os.path.join(exp_path, "{}.{}".format(self.exp_name, k))
+        self.run_dir = run_dir
         self.dest = os.path.join(run_dir, 'artifacts')
         self.predictions_dest = os.path.join(self.dest, "predictions")
-        os.makedirs(self.predictions_dest)
+        os.makedirs(self.predictions_dest, exist_ok=True)
         with open(os.path.join(self.dest, "config.yaml"), 'w') as fp:
             yaml.safe_dump(config, fp)
         self.logger = get_experiment_logger(self.dest)
@@ -162,10 +186,14 @@ class Experimenter:
         self.build_model()
         self.logger.info('Training:')
         self.callback = LogCallback(self.logger, LOG_FREQUENCY)
+        callbacks = [self.callback]
+        if self.backup_and_restore:
+            callbacks.append(BackupAndRestore(os.path.join(self.run_dir, "backup")))
         history = self.model.fit(self.trainset, epochs=self.parameters.epochs, workers=self.config.n_workers,
-                                 callbacks=[self.callback])
+                                 callbacks=callbacks)
         self.metrics.update(batch_time=self.callback.get_batch_time(), training_time=self.callback.training_time,
                             history=history.history)
+        self.model.save_weights(os.path.join(self.run_dir, "model", WEIGHTS_FILE))
 
     def evaluate(self):
         loss, accuracy = self.model.evaluate(self.testset)

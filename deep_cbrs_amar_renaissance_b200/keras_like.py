@@ -6,6 +6,7 @@ Keras (glorot_uniform / zeros / ones) and are drawn on the host from one seeded
 generator so a run is reproducible across devices.
 """
 import math
+import os
 from collections import OrderedDict
 
 import numpy as np
@@ -153,6 +154,107 @@ class History:
         self.epoch = []
 
 
+class _FitState:
+    """The loop state of a running `fit`: the sequence, the batch-order RandomState, the History and the next epoch."""
+
+    def __init__(self, sequence, rng, history, epoch):
+        self.sequence, self.rng, self.history, self.epoch = sequence, rng, history, epoch
+
+
+def _row_partition(model):
+    """The RowPartition attached to one of the model's GNN stacks, or None."""
+    from .models.gnn import SequentialGNN
+    gnn = getattr(model, "gnn", None)
+    for s in (vars(gnn).values() if gnn is not None else ()):
+        if isinstance(s, SequentialGNN) and s.partition is not None:
+            return s.partition
+    return None
+
+
+class BackupAndRestore:
+    """keras.callbacks.BackupAndRestore(backup_dir): lets a training run that stopped continue where it stopped.
+
+    At every epoch end the training state goes to <backup_dir>/training_state.npz, written under a temporary name
+    and renamed over the previous one (checkpoint.write), so a run killed mid-write leaves the previous epoch's file.
+    At train begin a state found there is restored and `fit` continues with the epoch after the saved one.  The
+    state: the weights, the Adam moments and iteration count, the epoch index, fit's batch-order RandomState, the
+    sequence's RandomState(s) and row order, and the History so far.  Every kernel of a step is deterministic, so the
+    resumed run computes the bits of the run that never stopped.  The file is deleted when training ends.
+
+    Under a RowPartition every rank holds the same weights and moments bit for bit: rank 0 writes, then the ranks
+    meet at a barrier, and every rank restores from the same file."""
+
+    FILE = "training_state.npz"
+
+    def __init__(self, backup_dir):
+        self.backup_dir = backup_dir
+        self.path = os.path.join(backup_dir, self.FILE)
+        self.model = None
+
+    def set_model(self, model):
+        self.model = model
+
+    def _rank_and_group(self):
+        part = _row_partition(self.model)
+        return (0, None) if part is None else (part.rank, part)
+
+    def _barrier(self, part):
+        if part is not None:
+            import torch.distributed as dist
+            dist.barrier(group=part.group)
+
+    def _sequence_state(self, st):
+        get = getattr(st.sequence, "get_state", None)
+        return get() if get is not None else {}
+
+    def on_train_begin(self, logs=None):
+        from . import checkpoint
+        if not os.path.exists(self.path):
+            return
+        m, st = self.model, self.model._fit_state
+        adam = m.adam()
+        with checkpoint.Reader(self.path, "training_state") as rd:
+            h = rd.header
+            m._check_weight_arrays(rd, rd.arrays("weights/"))
+            seq = rd.arrays("sequence/")
+            checkpoint.check_arrays(self.path + " (sequence state)",
+                                    checkpoint.spec(self._sequence_state(st).items()), seq)
+            checkpoint.check_arrays(self.path + " (fit batch order)",
+                                    checkpoint.spec(checkpoint.rng_arrays(st.rng).items()), rd.arrays("fit/"))
+            # checks the Adam hyper-parameters and moments before writing anything, so nothing is written on a refusal
+            adam.load_state_dict(m, dict(h["adam"], m=rd.arrays("adam/m/"), v=rd.arrays("adam/v/")))
+            m._copy_weights(rd.arrays("weights/"))
+            if seq:
+                st.sequence.set_state(seq)
+            checkpoint.set_rng(st.rng, rd.arrays("fit/"))
+            st.history.history = {k: list(v) for k, v in h["history"].items()}
+            st.history.epoch = list(h["history_epochs"])
+            st.epoch = int(h["epoch"]) + 1
+
+    def on_epoch_end(self, epoch, logs=None):
+        from . import checkpoint
+        rank, part = self._rank_and_group()
+        if rank == 0:
+            m, st = self.model, self.model._fit_state
+            adam = m.adam().state_dict(m)
+            arrays = [("weights/" + p, w) for p, w in m.named_weights()]
+            arrays += [("adam/m/" + p, t) for p, t in adam.pop("m").items()]
+            arrays += [("adam/v/" + p, t) for p, t in adam.pop("v").items()]
+            arrays += [("sequence/" + k, a) for k, a in self._sequence_state(st).items()]
+            arrays += [("fit/" + k, a) for k, a in checkpoint.rng_arrays(st.rng).items()]
+            header = {"kind": "training_state", "version": checkpoint.VERSION, "model": type(m).__name__,
+                      "epoch": int(epoch), "adam": adam, "history": st.history.history,
+                      "history_epochs": st.history.epoch}
+            checkpoint.write(self.path, header, arrays)
+        self._barrier(part)
+
+    def on_train_end(self, logs=None):
+        rank, part = self._rank_and_group()
+        self._barrier(part)
+        if rank == 0 and os.path.exists(self.path):
+            os.remove(self.path)
+
+
 class Model(Layer):
     """compile / fit / predict / evaluate / summary as the reference's Experimenter calls them
     (/root/reference/src/experiment.py:155-197)."""
@@ -167,19 +269,61 @@ class Model(Layer):
         self.loss, self.optimizer, self.metrics = loss, optimizer, metrics
         self._adam = None
 
-    def train_on_batch(self, x, y):
-        """One optimiser step; returns (loss incl. l2 penalty, #correct) as device scalars."""
+    def adam(self):
+        """The optimiser the training steps update (created from the compiled config at first use)."""
         from . import training
         if getattr(self, "_adam", None) is None:
             self._adam = training.Adam.from_config(self.optimizer)
-        return training.train_step(self, self._adam, x, y)
+        return self._adam
+
+    def train_on_batch(self, x, y):
+        """One optimiser step; returns (loss incl. l2 penalty, #correct) as device scalars."""
+        from . import training
+        return training.train_step(self, self.adam(), x, y)
 
     def make_graphed_train_step(self, batch_size, content_dim=None):
         """CUDA-graph replay of the whole optimiser step for a fixed batch size (training.GraphedTrainStep)."""
         from . import training
-        if getattr(self, "_adam", None) is None:
-            self._adam = training.Adam.from_config(self.optimizer)
-        return training.GraphedTrainStep(self, self._adam, batch_size, content_dim)
+        return training.GraphedTrainStep(self, self.adam(), batch_size, content_dim)
+
+    # -- weight files ----------------------------------------------------
+    def build_from_shapes(self, shapes):
+        """Create the weights for a file whose arrays have `shapes` ({weight path: shape}).  The GNN models build
+        from their constructor arguments; the scorers and hybrids override this to read their input widths."""
+        self.build_weights()
+
+    def save_weights(self, path):
+        """Write every weight to `path` (a .npz, see checkpoint.py), keyed by its path in named_weights(), with a
+        header naming the model class and each path's shape and dtype.  Not saved, because they are data or settings
+        rather than weights: the content table (set_content_table), the scorer precision and the feature dtype."""
+        from . import checkpoint
+        named = self.named_weights()
+        checkpoint.write(path, {"kind": "weights", "version": checkpoint.VERSION, "model": type(self).__name__,
+                                "weights": checkpoint.spec(named)}, named)
+
+    def load_weights(self, path):
+        """Read a file of save_weights into this model, building its weights first if needed.  Refuses, before any
+        weight is written, a file of another model class, and a missing path, an extra path or a shape or dtype
+        mismatch, naming the first offending path.  Copies in place: tensors captured by a GraphedTrainStep stay
+        valid."""
+        from . import checkpoint
+        with checkpoint.Reader(path, "weights") as rd:
+            self._check_weight_arrays(rd, rd.arrays())
+            self._copy_weights(rd.arrays())
+
+    def _check_weight_arrays(self, reader, arrays):
+        from . import checkpoint
+        if reader.header["model"] != type(self).__name__:
+            raise ValueError("{}: written by a {}, this model is a {}".format(reader.path, reader.header["model"],
+                                                                             type(self).__name__))
+        self.build_from_shapes({k: tuple(a.shape) for k, a in arrays.items()})
+        checkpoint.check_arrays(reader.path, checkpoint.spec(self.named_weights()), arrays)
+
+    def _copy_weights(self, arrays):
+        for name, w in self.named_weights():
+            w.copy_(torch.from_numpy(np.asarray(arrays[name])))
+        if hasattr(self, "invalidate"):
+            self.invalidate()
 
     def predict(self, sequence):
         outs = []
@@ -201,16 +345,28 @@ class Model(Layer):
             n += len(y)
         return [loss / max(n, 1), acc / max(n, 1)]
 
-    def fit(self, sequence, epochs=1, workers=1, callbacks=None, shuffle=True, verbose=0, cuda_graph=False):
+    def fit(self, sequence, epochs=1, workers=1, callbacks=None, shuffle=True, verbose=0, cuda_graph=False,
+            initial_epoch=0):
         """Keras `fit` over a `Sequence` (/root/reference/src/experiment.py:183-188): per epoch every batch
         once, in shuffled batch order, `sequence.on_epoch_end()` after the last one (the reference's
         datasets reshuffle their rows there, src/data/datasets.py:205-213); callbacks receive the Keras
         hooks the reference's own callbacks implement (src/utilities/keras.py:43-90).  `workers` is accepted
         and ignored (batches are index slices of an in-memory array).  cuda_graph=True replays full-size
         batches through one captured CUDA graph of the whole step (same kernels, same results); a short last
-        batch runs eagerly."""
+        batch runs eagerly.
+
+        initial_epoch: the epoch to start at (Keras): epochs initial_epoch .. epochs-1 run.  The batch order of an
+        epoch depends only on its index, so a model and sequences saved after epoch k-1 and trained on with
+        initial_epoch=k replay the batches of the run that never stopped.  A BackupAndRestore callback that finds a
+        saved state sets the start epoch itself."""
         callbacks = list(callbacks or [])
         hist = History()
+        rng = np.random.RandomState(self.shuffle_seed)
+        if shuffle:
+            for _ in range(int(initial_epoch)):
+                rng.permutation(len(sequence))
+        # what a BackupAndRestore callback saves and restores besides the weights and the optimiser
+        self._fit_state = _FitState(sequence, rng, hist, int(initial_epoch))
 
         def fire(name, *args):
             for cb in callbacks:
@@ -223,11 +379,10 @@ class Model(Layer):
                 cb.set_model(self)
             else:
                 cb.model = self
-        rng = np.random.RandomState(self.shuffle_seed)
         graphed = None
         fire("on_train_begin", {})
         logs = {}
-        for epoch in range(int(epochs)):
+        for epoch in range(self._fit_state.epoch, int(epochs)):
             fire("on_epoch_begin", epoch, {})
             order = rng.permutation(len(sequence)) if shuffle else np.arange(len(sequence))
             losses, corrects, sizes = [], [], []
@@ -258,8 +413,10 @@ class Model(Layer):
                 sequence.on_epoch_end()
             if verbose:
                 print("epoch {}: {}".format(epoch + 1, logs))
+            self._fit_state.epoch = epoch + 1
             fire("on_epoch_end", epoch, logs)
         fire("on_train_end", logs)
+        self._fit_state = None
         return hist
 
     def summary(self, print_fn=print, expand_nested=True):

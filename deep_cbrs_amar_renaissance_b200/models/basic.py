@@ -43,6 +43,12 @@ class BasicRS(Model):
         di = self.inet.build_for(d)
         self.clf.build_for(du + di)
 
+    def build_from_shapes(self, shapes):
+        """the input width from a weight file: the first tower kernel's rows (half the classifier's without towers)"""
+        key = "unet/layers.0/kernel" if self.unet.layers else "clf/layers.0/kernel"
+        if key in shapes:
+            self.build_for(shapes[key][0] if self.unet.layers else shapes[key][0] // 2)
+
     def call(self, inputs, **kwargs):
         """as a model of its own (config.yaml:6, experiment.py:152): inputs = the (user rows, item rows) batches of
         data.datasets.UserItemEmbeddings"""

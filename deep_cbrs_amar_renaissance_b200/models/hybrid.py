@@ -63,6 +63,12 @@ class HybridCBRS(Model):
         else:
             self.clf.build_for(x)
 
+    def build_from_shapes(self, shapes):
+        """the graph and content widths from a weight file: the rows of the first graph and content tower kernels"""
+        g, c = shapes.get("dense1a/layers.0/kernel"), shapes.get("dense2a/layers.0/kernel")
+        if g is not None and c is not None:
+            self.build_for(g[0], c[0])
+
     def call(self, inputs, **kwargs):
         ug, ig, ub, ib = inputs
         return self.call_sources((_rows(ug), None), (_rows(ig), None), (_rows(ub), None), (_rows(ib), None))
@@ -112,6 +118,12 @@ class HybridBertGNN(Model, abc.ABC):
         self.gnn.build_layers()
         self.rs.build_for(self.gnn.out_dim, content_dim)
         return self
+
+    def build_from_shapes(self, shapes):
+        """the content width from a weight file: the rows of the first content tower kernel"""
+        c = shapes.get("rs/dense2a/layers.0/kernel")
+        if c is not None:
+            self.build_weights(c[0])
 
     def set_content_table(self, table, dtype="fp32"):
         """Upload the [N, 768] content embeddings once (rows ordered like node ids).  dtype='bf16' keeps the table

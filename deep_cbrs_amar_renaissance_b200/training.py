@@ -14,6 +14,7 @@ of its output, accumulates the gradients of its inputs (`Node.grad`) and of its 
 """
 import math
 
+import numpy as np
 import torch
 
 from . import _lib as L
@@ -585,8 +586,51 @@ class Adam:
         get = lambda k, d: float(getattr(cfg, k, d))  # a keras-like optimizer object
         return cls(get("learning_rate", 1e-3), get("beta_1", 0.9), get("beta_2", 0.999), get("epsilon", 1e-7))
 
+    HYPER_PARAMETERS = ("learning_rate", "beta_1", "beta_2", "epsilon")
+
     def rate(self, t):
         return self.learning_rate * math.sqrt(1.0 - self.beta_2 ** t) / (1.0 - self.beta_1 ** t)
+
+    def state_dict(self, model):
+        """{'iterations', the hyper-parameters, 'm': {weight path: first moment}, 'v': {...: second moment}} for the
+        weights of `model` that have moments (a weight gets them at its first update).  The moments are the slot
+        tensors themselves, not copies."""
+        out = {"iterations": int(self.iterations), "m": {}, "v": {}}
+        out.update({k: getattr(self, k) for k in self.HYPER_PARAMETERS})
+        for path, w in model.named_weights():
+            st = self._state.get(id(w))
+            if st is not None:
+                out["m"][path], out["v"][path] = st
+        return out
+
+    def load_state_dict(self, model, state):
+        """Put back what state_dict returned (moments as tensors, ndarrays or anything np.asarray reads).  Refuses,
+        before any write, hyper-parameters that differ from this optimiser's and moments whose path, shape or dtype
+        does not match a weight of `model`.  Existing slots are filled in place (a captured GraphedTrainStep keeps
+        reading them); missing ones are created; a slot the state has no moments for is zeroed, as a weight that was
+        never updated."""
+        from . import checkpoint
+        for k in self.HYPER_PARAMETERS:
+            if float(state[k]) != getattr(self, k):
+                raise ValueError("Adam state: {} = {!r}, this optimiser has {!r}".format(k, float(state[k]),
+                                                                                           getattr(self, k)))
+        weights = dict(model.named_weights())
+        m, v = state["m"], state["v"]
+        want = [(p, tuple(w.shape), "float32") for p, w in model.named_weights() if p in m or p in v]
+        checkpoint.check_arrays("Adam first moments", want, m)
+        checkpoint.check_arrays("Adam second moments", want, v)
+        for path, w in weights.items():
+            st = self._state.get(id(w))
+            if path not in m:
+                if st is not None:
+                    st[0].zero_()
+                    st[1].zero_()
+                continue
+            if st is None:
+                st = self._state[id(w)] = (torch.empty_like(w), torch.empty_like(w))
+            for slot, a in zip(st, (m[path], v[path])):
+                slot.copy_(a if isinstance(a, torch.Tensor) else torch.from_numpy(np.asarray(a)))
+        self.iterations = int(state["iterations"])
 
     def apply(self, weights, grads, l2s, capturing=False):
         if not capturing:
