@@ -150,11 +150,13 @@ __global__ void __launch_bounds__(kSpmmThreads, MINB) spmm_chunk_kernel(const Sp
     const int64_t e = p.chunk_len ? b + p.chunk_len[gid] : ((b + p.chunk_edges < row_e) ? b + p.chunk_edges : row_e);
     const int32_t slot = p.chunk_slot[gid];
     const bool weighted = (p.agg == CBRS_AGG_WEIGHTED) && p.vals != nullptr;
+    // row stride in bytes as a 32-bit value (checked on the host): a row address is one IMAD.WIDE per edge
+    const int ldx_bytes = (int)(p.ldx * (int64_t)sizeof(XT));
 
     for (int c0 = 0; c0 < p.d; c0 += G * VEC) {
         const int col = c0 + lg * VEC;
         const bool col_ok = col < p.d;
-        const XT *xcol = reinterpret_cast<const XT *>(p.x) + (col_ok ? col : 0);
+        const char *xcol = reinterpret_cast<const char *>(reinterpret_cast<const XT *>(p.x) + (col_ok ? col : 0));
         Vec<VEC> acc;
         acc.zero();
         // (col,val) of the next G edges are fetched while the current G rows are in flight
@@ -193,7 +195,7 @@ __global__ void __launch_bounds__(kSpmmThreads, MINB) spmm_chunk_kernel(const Sp
 #pragma unroll
                     for (int u = 0; u < U; ++u)
                         if (col_ok && k0 + u < cnt)
-                            raw[u] = __ldg(reinterpret_cast<const uint2 *>(xcol + (int64_t)cc[u] * p.ldx));
+                            raw[u] = __ldg(reinterpret_cast<const uint2 *>(xcol + (int64_t)cc[u] * ldx_bytes));
 #pragma unroll
                     for (int u = 0; u < U; ++u)
                         if (col_ok && k0 + u < cnt) {
@@ -206,7 +208,7 @@ __global__ void __launch_bounds__(kSpmmThreads, MINB) spmm_chunk_kernel(const Sp
 #pragma unroll
                     for (int u = 0; u < U; ++u)
                         if (col_ok && k0 + u < cnt)
-                            raw[u] = __ldg(reinterpret_cast<const uint4 *>(xcol + (int64_t)cc[u] * p.ldx));
+                            raw[u] = __ldg(reinterpret_cast<const uint4 *>(xcol + (int64_t)cc[u] * ldx_bytes));
 #pragma unroll
                     for (int u = 0; u < U; ++u)
                         if (col_ok && k0 + u < cnt) {
@@ -216,7 +218,8 @@ __global__ void __launch_bounds__(kSpmmThreads, MINB) spmm_chunk_kernel(const Sp
                 } else {
 #pragma unroll
                     for (int u = 0; u < U; ++u)
-                        if (col_ok && k0 + u < cnt) xr[u].load(xcol + (int64_t)cc[u] * p.ldx);
+                        if (col_ok && k0 + u < cnt)
+                            xr[u].load(reinterpret_cast<const XT *>(xcol + (int64_t)cc[u] * ldx_bytes));
 #pragma unroll
                     for (int u = 0; u < U; ++u)
                         if (col_ok && k0 + u < cnt) acc.fma(vv[u], xr[u]);
@@ -312,6 +315,7 @@ static int spmm_impl(const cbrs_csr_t *g, const void *x, int64_t ldx, void *y, i
     CBRS_REQUIRE(dtype == CBRS_DTYPE_F32 || dtype == CBRS_DTYPE_BF16, CBRS_E_INVALID, "spmm: dtype=%d", dtype);
     CBRS_REQUIRE(d > 0 && ldx >= d && ldy >= d, CBRS_E_INVALID, "spmm: d=%d ldx=%lld ldy=%lld", d, (long long)ldx,
                  (long long)ldy);
+    CBRS_REQUIRE(ldx <= INT32_MAX / 4, CBRS_E_INVALID, "spmm: ldx=%lld (a row stride under 2^31 bytes)", (long long)ldx);
     CBRS_REQUIRE(agg >= CBRS_AGG_WEIGHTED && agg <= CBRS_AGG_MEAN, CBRS_E_INVALID, "spmm: agg=%d", agg);
     CBRS_REQUIRE(g->n_rows >= 0 && g->n_chunks >= 0 && g->chunk_edges > 0, CBRS_E_INVALID, "spmm: bad graph descriptor");
     if (g->n_rows == 0) return CBRS_OK;
