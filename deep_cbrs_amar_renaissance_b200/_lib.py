@@ -35,6 +35,12 @@ _SIGS = {
     "cbrs_graph_build_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int]),
     "cbrs_graph_build_csr": (c_int, [P, P, P, c_int64, c_int64, c_int, P, P, P, P, P, c_size_t, P]),
     "cbrs_graph_build_csr_rel": (c_int, [P, P, P, P, c_int64, c_int64, c_int32, c_int32, c_int, P, P, P, P, P, c_size_t, P]),
+    "cbrs_coo_row_histogram": (c_int, [P, c_int64, c_int64, P, P]),
+    "cbrs_coo_select_rows_workspace_bytes": (c_size_t, [c_int64]),
+    "cbrs_coo_select_rows": (c_int, [P, P, P, c_int64, c_int64, c_int64, c_int, P, P, P, P, c_int64, P, c_size_t, P]),
+    "cbrs_graph_build_block_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int]),
+    "cbrs_graph_build_block": (c_int, [P, P, P, c_int64, c_int64, c_int64, c_int64, c_int, P, P, P, P, P, P, c_size_t, P]),
+    "cbrs_graph_block_scale": (c_int, [P, P, P, c_int64, c_int64, c_int64, P, P]),
     "cbrs_chunks_workspace_bytes": (c_size_t, [c_int64]),
     "cbrs_chunks_count": (c_int, [P, c_int64, c_int32, P, P, c_size_t, P]),
     "cbrs_chunks_fill": (c_int, [P, c_int64, c_int32, P, P, P, P, P, P, c_size_t, P]),
@@ -157,6 +163,7 @@ _SIGS = {
                                      POINTER(c_int64), POINTER(c_float), c_float, P, c_float, c_float, c_float, P]),
     "cbrs_synth_bipartite": (c_int, [c_int64, c_int64, c_int64, c_uint64, P, P, P]),
     "cbrs_synth_bipartite_ex": (c_int, [c_int64, c_int64, c_int64, c_uint64, c_int, P, P, P]),
+    "cbrs_synth_bipartite_range": (c_int, [c_int64, c_int64, c_int64, c_uint64, c_int, c_int64, c_int64, P, P, P]),
     "cbrs_sort_workspace_bytes": (c_size_t, [c_int64]),
     "cbrs_sort_pairs_u64": (c_int, [P, P, c_int64, c_int, P, c_size_t, P]),
 }

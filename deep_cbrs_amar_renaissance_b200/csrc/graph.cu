@@ -31,20 +31,22 @@ struct KeyLayout {
     __device__ int64_t col(uint64_t k) const { return (int64_t)(k & ((1ull << col_bits) - 1)); }
 };
 
+// Rows [row_lo, row_lo + n_rows) of an n_cols-node graph (the whole build: row_lo = 0, n_rows = n_cols); keys carry
+// the row relative to row_lo, entries of other rows are invalid.
 __global__ void make_keys_kernel(const int32_t *__restrict__ row, const int32_t *__restrict__ col,
                                  const int32_t *__restrict__ rel, const float *__restrict__ val, int64_t nnz,
-                                 int64_t n_nodes, int64_t n_loops, int32_t self_rel, int drop_diag, KeyLayout kl,
-                                 uint64_t *__restrict__ keys, uint32_t *__restrict__ payload) {
+                                 int64_t row_lo, int64_t n_rows, int64_t n_cols, int64_t n_loops, int32_t self_rel,
+                                 int drop_diag, KeyLayout kl, uint64_t *__restrict__ keys, uint32_t *__restrict__ payload) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= nnz + n_loops) return;
     if (i < nnz) {
-        const int64_t r = row[i], c = col[i];
-        const bool bad = r < 0 || c < 0 || r >= n_nodes || c >= n_nodes || (drop_diag && r == c);
+        const int64_t r = (int64_t)row[i] - row_lo, c = col[i];
+        const bool bad = r < 0 || c < 0 || r >= n_rows || c >= n_cols || (drop_diag && r + row_lo == c);
         keys[i] = bad ? kl.invalid() : kl.pack(r, rel ? rel[i] : 0, c);
         payload[i] = val ? __float_as_uint(val[i]) : __float_as_uint(1.0f);
     } else {  // appended diagonal: M_ii += 1 falls out of the duplicate sum
         const int64_t d = i - nnz;
-        keys[i] = kl.pack(d, self_rel, d);
+        keys[i] = kl.pack(d, self_rel, row_lo + d);
         payload[i] = __float_as_uint(1.0f);
     }
 }
@@ -66,7 +68,7 @@ __global__ void head_flags_kernel(const uint64_t *__restrict__ keys, int64_t n, 
 // in sorted == input order); row boundaries fill the row-pointer gaps.
 __global__ void compact_kernel(const uint64_t *__restrict__ keys, const uint32_t *__restrict__ payload,
                                const uint32_t *__restrict__ pos, const uint32_t *__restrict__ total, int64_t n,
-                               int64_t n_nodes, KeyLayout kl, int dedup, int64_t *__restrict__ rowptr,
+                               int64_t n_rows, int64_t n_cols, KeyLayout kl, int dedup, int64_t *__restrict__ rowptr,
                                int32_t *__restrict__ colidx, float *__restrict__ vals, int64_t *__restrict__ nnz_out) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i == 0 && nnz_out) *nnz_out = (int64_t)*total;
@@ -78,7 +80,7 @@ __global__ void compact_kernel(const uint64_t *__restrict__ keys, const uint32_t
     const bool head = !dedup || i == 0 || keys[i - 1] != k;
     if (head) {
         const uint32_t o = pos[i];
-        colidx[o] = (int32_t)(kl.rel(k) * n_nodes + kl.col(k));
+        colidx[o] = (int32_t)(kl.rel(k) * n_cols + kl.col(k));
         float acc = __uint_as_float(payload[i]);
         if (dedup)
             for (int64_t j = i + 1; j < n && keys[j] == k; ++j) acc += __uint_as_float(payload[j]);
@@ -89,7 +91,7 @@ __global__ void compact_kernel(const uint64_t *__restrict__ keys, const uint32_t
     const bool last_valid = (i + 1 == n) || keys[i + 1] >= inv;
     if (last_valid) {
         const int64_t t = (int64_t)*total;
-        for (int64_t rr = r + 1; rr <= n_nodes; ++rr) rowptr[rr] = t;
+        for (int64_t rr = r + 1; rr <= n_rows; ++rr) rowptr[rr] = t;
     }
 }
 
@@ -112,15 +114,17 @@ __global__ void __launch_bounds__(kThreads) inv_sqrt_degree_kernel(const int64_t
     }
 }
 
+// d_i from dinv_rows[row] (the rows held here), d_j from dinv[column] (every node)
 __global__ void __launch_bounds__(kThreads) sym_scale_kernel(const int64_t *__restrict__ rowptr,
                                                              const int32_t *__restrict__ colidx,
+                                                             const float *__restrict__ dinv_rows,
                                                              const float *__restrict__ dinv, int64_t n_rows,
                                                              int64_t n_nodes, float *__restrict__ vals) {
     const int64_t row = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     if (row >= n_rows) return;
     const int64_t b = rowptr[row], e = rowptr[row + 1];
-    const float di = dinv[row];
+    const float di = dinv_rows[row];
     for (int64_t j = b + lane; j < e; j += 32) {
         const int64_t c = (int64_t)colidx[j] % n_nodes;  // strip the relation block
         vals[j] = __fmul_rn(__fmul_rn(di, vals[j]), dinv[c]);
@@ -136,23 +140,33 @@ static size_t graph_ws_bytes(int64_t nnz, int64_t n_nodes, int flags) {
            4096;
 }
 
+// Rows [row_lo, row_lo + n_rows) of the n_nodes-node graph (the whole graph: row_lo = 0, n_rows = n_nodes).  With
+// SYM_NORM: dinv_out == NULL scales the values here (the rows' own d serves every column: the whole graph only);
+// otherwise the rows' d goes to dinv_out and the values stay unscaled (cbrs_graph_block_scale finishes them).
 static int build(const int32_t *coo_row, const int32_t *coo_col, const int32_t *coo_rel, const float *coo_val,
-                 int64_t nnz, int64_t n_nodes, int32_t n_rel, int32_t self_rel, int flags, int64_t *rowptr,
-                 int32_t *colidx, float *vals, int64_t *nnz_out, void *ws, size_t ws_bytes, cudaStream_t s) {
+                 int64_t nnz, int64_t row_lo, int64_t n_rows, int64_t n_nodes, int32_t n_rel, int32_t self_rel,
+                 int flags, int64_t *rowptr, int32_t *colidx, float *vals, float *dinv_out, int64_t *nnz_out, void *ws,
+                 size_t ws_bytes, cudaStream_t s) {
     CBRS_REQUIRE(nnz >= 0 && n_nodes > 0 && n_rel >= 1, CBRS_E_INVALID, "graph_build: nnz=%lld n=%lld n_rel=%d",
                  (long long)nnz, (long long)n_nodes, n_rel);
+    CBRS_REQUIRE(row_lo >= 0 && n_rows > 0 && row_lo + n_rows <= n_nodes, CBRS_E_INVALID,
+                 "graph_build: rows [%lld, %lld) of %lld", (long long)row_lo, (long long)(row_lo + n_rows),
+                 (long long)n_nodes);
+    CBRS_REQUIRE(dinv_out || !(flags & CBRS_GRAPH_SYM_NORM) || (row_lo == 0 && n_rows == n_nodes), CBRS_E_INVALID,
+                 "graph_build: a row block needs dinv_out for SYM_NORM");
     CBRS_REQUIRE(rowptr && colidx && vals, CBRS_E_INVALID, "graph_build: null output");
     CBRS_REQUIRE(nnz == 0 || (coo_row && coo_col), CBRS_E_INVALID, "graph_build: null input");
     CBRS_REQUIRE(!(flags & CBRS_GRAPH_ADD_SELF_LOOPS) || (flags & CBRS_GRAPH_DEDUP_SUM), CBRS_E_INVALID,
                  "graph_build: ADD_SELF_LOOPS requires DEDUP_SUM");
     CBRS_REQUIRE((int64_t)n_rel * n_nodes < ((int64_t)1 << 31), CBRS_E_INVALID, "graph_build: n_rel*n_nodes overflows int32");
     CBRS_REQUIRE(self_rel >= 0 && self_rel < n_rel, CBRS_E_INVALID, "graph_build: self_rel=%d", self_rel);
-    const int64_t n_loops = (flags & CBRS_GRAPH_ADD_SELF_LOOPS) ? n_nodes : 0;
+    const int64_t n_loops = (flags & CBRS_GRAPH_ADD_SELF_LOOPS) ? n_rows : 0;
     const int64_t n_in = nnz + n_loops;
     CBRS_REQUIRE(n_in < (int64_t)0xfffffff0ll, CBRS_E_INVALID, "graph_build: %lld entries exceed the 32-bit position range",
                  (long long)n_in);
     KeyLayout kl;
-    kl.col_bits = kl.row_bits = bits_for(n_nodes);
+    kl.col_bits = bits_for(n_nodes);
+    kl.row_bits = bits_for(n_rows);
     kl.rel_bits = n_rel > 1 ? bits_for(n_rel) : 0;
     CBRS_REQUIRE(kl.key_bits() <= 64, CBRS_E_INVALID, "graph_build: key needs %d bits", kl.key_bits());
 
@@ -161,18 +175,18 @@ static int build(const int32_t *coo_row, const int32_t *coo_col, const int32_t *
     uint32_t *payload = a.take<uint32_t>((size_t)n_in);
     uint32_t *pos = a.take<uint32_t>((size_t)n_in);
     uint32_t *total = a.take<uint32_t>(1);
-    float *dinv = a.take<float>((size_t)n_nodes);
+    float *dinv = a.take<float>((size_t)n_rows);
     CBRS_REQUIRE(keys && payload && pos && total && dinv, CBRS_E_WORKSPACE, "graph_build: workspace too small");
     void *sub = (char *)ws + a.off;
     const size_t sub_bytes = ws_bytes - a.off;
 
-    cudaMemsetAsync(rowptr, 0, (size_t)(n_nodes + 1) * sizeof(int64_t), s);
+    cudaMemsetAsync(rowptr, 0, (size_t)(n_rows + 1) * sizeof(int64_t), s);
     cudaMemsetAsync(total, 0, sizeof(uint32_t), s);
     if (nnz_out) cudaMemsetAsync(nnz_out, 0, sizeof(int64_t), s);
     if (n_in == 0) return CBRS_OK;
     const unsigned gb = (unsigned)cdiv(n_in, kThreads);
-    make_keys_kernel<<<gb, kThreads, 0, s>>>(coo_row, coo_col, coo_rel, coo_val, nnz, n_nodes, n_loops, self_rel,
-                                             (flags & CBRS_GRAPH_DROP_DIAG) ? 1 : 0, kl, keys, payload);
+    make_keys_kernel<<<gb, kThreads, 0, s>>>(coo_row, coo_col, coo_rel, coo_val, nnz, row_lo, n_rows, n_nodes, n_loops,
+                                             self_rel, (flags & CBRS_GRAPH_DROP_DIAG) ? 1 : 0, kl, keys, payload);
     CBRS_CHECK_LAUNCH("make_keys");
     int rc = sort_pairs_u64(keys, payload, n_in, kl.key_bits(), sub, sub_bytes, s);
     if (rc) return rc;
@@ -181,17 +195,55 @@ static int build(const int32_t *coo_row, const int32_t *coo_col, const int32_t *
     CBRS_CHECK_LAUNCH("head_flags");
     rc = scan_u32_exclusive(pos, n_in, total, sub, sub_bytes, s);
     if (rc) return rc;
-    compact_kernel<<<gb, kThreads, 0, s>>>(keys, payload, pos, total, n_in, n_nodes, kl, dedup, rowptr, colidx, vals,
-                                           nnz_out);
+    compact_kernel<<<gb, kThreads, 0, s>>>(keys, payload, pos, total, n_in, n_rows, n_nodes, kl, dedup, rowptr, colidx,
+                                           vals, nnz_out);
     CBRS_CHECK_LAUNCH("compact");
     if (flags & CBRS_GRAPH_SYM_NORM) {
-        const unsigned gr = (unsigned)cdiv(n_nodes * 32, kThreads);
-        inv_sqrt_degree_kernel<<<gr, kThreads, 0, s>>>(rowptr, vals, n_nodes, dinv);
+        const unsigned gr = (unsigned)cdiv(n_rows * 32, kThreads);
+        inv_sqrt_degree_kernel<<<gr, kThreads, 0, s>>>(rowptr, vals, n_rows, dinv_out ? dinv_out : dinv);
         CBRS_CHECK_LAUNCH("inv_sqrt_degree");
-        sym_scale_kernel<<<gr, kThreads, 0, s>>>(rowptr, colidx, dinv, n_nodes, n_nodes, vals);
-        CBRS_CHECK_LAUNCH("sym_scale");
+        if (!dinv_out) {
+            sym_scale_kernel<<<gr, kThreads, 0, s>>>(rowptr, colidx, dinv, dinv, n_rows, n_nodes, vals);
+            CBRS_CHECK_LAUNCH("sym_scale");
+        }
     }
     return CBRS_OK;
+}
+
+// ------------------------------------------------------------------ row selection (partitioned build)
+__global__ void row_histogram_kernel(const int32_t *__restrict__ row, int64_t n, int64_t n_rows,
+                                     unsigned long long *__restrict__ counts) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int64_t r = row[i];
+    if (r >= 0 && r < n_rows) atomicAdd(counts + r, 1ull);
+}
+
+__global__ void select_flags_kernel(const int32_t *__restrict__ row, int64_t n, int64_t lo, int64_t hi,
+                                    uint32_t *__restrict__ flags) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) flags[i] = (row[i] >= lo && row[i] < hi) ? 1u : 0u;
+}
+
+// pos = exclusive scan of the flags: entry i goes to *cursor + pos[i], i.e. selected entries keep their input order
+__global__ void select_scatter_kernel(const int32_t *__restrict__ row, const int32_t *__restrict__ col,
+                                      const float *__restrict__ val, int64_t n, int64_t lo, int64_t hi, int rebase,
+                                      const uint32_t *__restrict__ pos, const int64_t *__restrict__ cursor,
+                                      int64_t capacity, int32_t *__restrict__ out_row, int32_t *__restrict__ out_col,
+                                      float *__restrict__ out_val) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int32_t r = row[i];
+    if (r < lo || r >= hi) return;
+    const int64_t o = *cursor + (int64_t)pos[i];
+    if (o >= capacity) return;
+    out_row[o] = rebase ? (int32_t)(r - lo) : r;
+    out_col[o] = col[i];
+    if (out_val) out_val[o] = val ? val[i] : 1.0f;
+}
+
+__global__ void select_advance_kernel(int64_t *__restrict__ cursor, const uint32_t *__restrict__ total) {
+    *cursor += (int64_t)*total;
 }
 
 // ------------------------------------------------------------------ chunks
@@ -364,8 +416,8 @@ extern "C" size_t cbrs_graph_build_workspace_bytes(int64_t nnz, int64_t n_nodes,
 extern "C" int cbrs_graph_build_csr(const int32_t *coo_row, const int32_t *coo_col, const float *coo_val, int64_t nnz,
                                     int64_t n_nodes, int flags, int64_t *rowptr, int32_t *colidx, float *vals,
                                     int64_t *nnz_out, void *workspace, size_t workspace_bytes, void *stream) {
-    return build(coo_row, coo_col, nullptr, coo_val, nnz, n_nodes, 1, 0, flags, rowptr, colidx, vals, nnz_out,
-                 workspace, workspace_bytes, (cudaStream_t)stream);
+    return build(coo_row, coo_col, nullptr, coo_val, nnz, 0, n_nodes, n_nodes, 1, 0, flags, rowptr, colidx, vals, nullptr,
+                 nnz_out, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 extern "C" int cbrs_graph_build_csr_rel(const int32_t *coo_row, const int32_t *coo_col, const int32_t *coo_rel,
@@ -373,8 +425,77 @@ extern "C" int cbrs_graph_build_csr_rel(const int32_t *coo_row, const int32_t *c
                                         int32_t self_rel, int flags, int64_t *rowptr, int32_t *colidx, float *vals,
                                         int64_t *nnz_out, void *workspace, size_t workspace_bytes, void *stream) {
     CBRS_REQUIRE(coo_rel || n_rel == 1, CBRS_E_INVALID, "graph_build_rel: null relation ids");
-    return build(coo_row, coo_col, coo_rel, coo_val, nnz, n_nodes, n_rel, self_rel, flags, rowptr, colidx, vals,
-                 nnz_out, workspace, workspace_bytes, (cudaStream_t)stream);
+    return build(coo_row, coo_col, coo_rel, coo_val, nnz, 0, n_nodes, n_nodes, n_rel, self_rel, flags, rowptr, colidx,
+                 vals, nullptr, nnz_out, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+// ---- partitioned build (include/cbrs_b200.h) -------------------------------------------------------------------
+extern "C" int cbrs_coo_row_histogram(const int32_t *coo_row, int64_t n, int64_t n_rows, int64_t *counts, void *stream) {
+    CBRS_REQUIRE(n >= 0 && n_rows > 0 && counts && (coo_row || n == 0), CBRS_E_INVALID, "coo_row_histogram: bad argument");
+    if (n == 0) return CBRS_OK;
+    row_histogram_kernel<<<(unsigned)cdiv(n, kThreads), kThreads, 0, (cudaStream_t)stream>>>(
+        coo_row, n, n_rows, (unsigned long long *)counts);
+    CBRS_CHECK_LAUNCH("row_histogram");
+    return CBRS_OK;
+}
+
+extern "C" size_t cbrs_coo_select_rows_workspace_bytes(int64_t n) {
+    return align_up((size_t)(n > 0 ? n : 1) * 4) + 256 + scan_u32_workspace_bytes(n > 0 ? n : 1) + 1024;
+}
+
+extern "C" int cbrs_coo_select_rows(const int32_t *coo_row, const int32_t *coo_col, const float *coo_val, int64_t n,
+                                    int64_t row_lo, int64_t row_hi, int rebase, int32_t *out_row, int32_t *out_col,
+                                    float *out_val, int64_t *cursor, int64_t capacity, void *workspace,
+                                    size_t workspace_bytes, void *stream) {
+    cudaStream_t s = (cudaStream_t)stream;
+    CBRS_REQUIRE(n >= 0 && (n == 0 || (coo_row && coo_col)) && out_row && out_col && cursor && capacity >= 0,
+                 CBRS_E_INVALID, "coo_select_rows: bad argument");
+    CBRS_REQUIRE(row_lo >= 0 && row_lo <= row_hi, CBRS_E_INVALID, "coo_select_rows: rows [%lld, %lld)", (long long)row_lo,
+                 (long long)row_hi);
+    CBRS_REQUIRE(n < (int64_t)0xfffffff0ll, CBRS_E_INVALID, "coo_select_rows: %lld entries exceed the 32-bit position range",
+                 (long long)n);
+    if (n == 0) return CBRS_OK;
+    Arena a(workspace, workspace_bytes);
+    uint32_t *pos = a.take<uint32_t>((size_t)n);
+    uint32_t *total = a.take<uint32_t>(1);
+    CBRS_REQUIRE(pos && total, CBRS_E_WORKSPACE, "coo_select_rows: workspace too small");
+    void *sub = (char *)workspace + a.off;
+    const size_t sub_bytes = workspace_bytes - a.off;
+    const unsigned g = (unsigned)cdiv(n, kThreads);
+    select_flags_kernel<<<g, kThreads, 0, s>>>(coo_row, n, row_lo, row_hi, pos);
+    CBRS_CHECK_LAUNCH("select_flags");
+    int rc = scan_u32_exclusive(pos, n, total, sub, sub_bytes, s);
+    if (rc) return rc;
+    select_scatter_kernel<<<g, kThreads, 0, s>>>(coo_row, coo_col, coo_val, n, row_lo, row_hi, rebase, pos, cursor, capacity,
+                                                 out_row, out_col, out_val);
+    CBRS_CHECK_LAUNCH("select_scatter");
+    select_advance_kernel<<<1, 1, 0, s>>>(cursor, total);   // after the scatter: it reads the cursor
+    CBRS_CHECK_LAUNCH("select_advance");
+    return CBRS_OK;
+}
+
+extern "C" size_t cbrs_graph_build_block_workspace_bytes(int64_t nnz, int64_t n_rows, int flags) {
+    return graph_ws_bytes(nnz, n_rows, flags);
+}
+
+extern "C" int cbrs_graph_build_block(const int32_t *coo_row, const int32_t *coo_col, const float *coo_val, int64_t nnz,
+                                      int64_t row_lo, int64_t row_hi, int64_t n_cols, int flags, int64_t *rowptr,
+                                      int32_t *colidx, float *vals, float *dinv_out, int64_t *nnz_out, void *workspace,
+                                      size_t workspace_bytes, void *stream) {
+    CBRS_REQUIRE(!(flags & CBRS_GRAPH_SYM_NORM) || dinv_out, CBRS_E_INVALID, "graph_build_block: SYM_NORM needs dinv_out");
+    return build(coo_row, coo_col, nullptr, coo_val, nnz, row_lo, row_hi - row_lo, n_cols, 1, 0, flags, rowptr, colidx,
+                 vals, (flags & CBRS_GRAPH_SYM_NORM) ? dinv_out : nullptr, nnz_out, workspace, workspace_bytes,
+                 (cudaStream_t)stream);
+}
+
+extern "C" int cbrs_graph_block_scale(const int64_t *rowptr, const int32_t *colidx, float *vals, int64_t n_rows,
+                                      int64_t row_lo, int64_t n_cols, const float *dinv, void *stream) {
+    CBRS_REQUIRE(rowptr && colidx && vals && dinv && n_rows > 0 && row_lo >= 0 && row_lo + n_rows <= n_cols,
+                 CBRS_E_INVALID, "graph_block_scale: bad argument");
+    const unsigned gr = (unsigned)cdiv(n_rows * 32, kThreads);
+    sym_scale_kernel<<<gr, kThreads, 0, (cudaStream_t)stream>>>(rowptr, colidx, dinv + row_lo, dinv, n_rows, n_cols, vals);
+    CBRS_CHECK_LAUNCH("sym_scale");
+    return CBRS_OK;
 }
 
 extern "C" size_t cbrs_chunks_workspace_bytes(int64_t n_rows) {

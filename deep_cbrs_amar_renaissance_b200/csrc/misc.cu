@@ -61,10 +61,13 @@ __host__ __device__ __forceinline__ uint64_t splitmix64(uint64_t x) {
 // piecewise-uniform Zipf(1): octave j covers ranks [c*(2^j-1), c*(2^(j+1)-1)) and every
 // octave carries the same mass, so the c hottest items each receive 1/(L*c) of the edges
 // ("capped" head).  Ranks are scattered over item ids by a multiplicative bijection.
-__global__ void synth_bipartite_kernel(int64_t n_users, int64_t n_items, int64_t n_edges, uint64_t seed, uint64_t c,
-                                       int levels, uint64_t mult, int32_t *__restrict__ row, int32_t *__restrict__ col) {
-    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= n_edges) return;
+// Edges [edge_lo, edge_lo + m): entry k (edge edge_lo + k) goes to row[k], its reverse to row[m + k].
+__global__ void synth_bipartite_kernel(int64_t n_users, int64_t n_items, int64_t edge_lo, int64_t m, uint64_t seed,
+                                       uint64_t c, int levels, uint64_t mult, int32_t *__restrict__ row,
+                                       int32_t *__restrict__ col) {
+    const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= m) return;
+    const int64_t e = edge_lo + k;
     const uint64_t h0 = splitmix64(seed ^ ((uint64_t)e * 0x2545F4914F6CDD1Dull));
     const uint64_t h1 = splitmix64(h0);
     const uint64_t h2 = splitmix64(h1);
@@ -73,10 +76,10 @@ __global__ void synth_bipartite_kernel(int64_t n_users, int64_t n_items, int64_t
     const uint64_t span = c << lvl;
     const uint64_t rank = (span - c + (h2 % span)) % (uint64_t)n_items;
     const int64_t it = (int64_t)((rank * mult) % (uint64_t)n_items);
-    row[e] = (int32_t)u;
-    col[e] = (int32_t)(n_users + it);
-    row[n_edges + e] = (int32_t)(n_users + it);
-    col[n_edges + e] = (int32_t)u;
+    row[k] = (int32_t)u;
+    col[k] = (int32_t)(n_users + it);
+    row[m + k] = (int32_t)(n_users + it);
+    col[m + k] = (int32_t)u;
 }
 
 static uint64_t gcd64(uint64_t a, uint64_t b) { while (b) { uint64_t t = a % b; a = b; b = t; } return a; }
@@ -139,9 +142,20 @@ extern "C" int cbrs_synth_bipartite(int64_t n_users, int64_t n_items, int64_t n_
 extern "C" int cbrs_synth_bipartite_ex(int64_t n_users, int64_t n_items, int64_t n_edges, uint64_t seed, int scatter_items,
                                        int32_t *coo_row, int32_t *coo_col, void *stream) {
     CBRS_REQUIRE(coo_row && coo_col, CBRS_E_INVALID, "synth_bipartite: null argument");
+    return cbrs_synth_bipartite_range(n_users, n_items, n_edges, seed, scatter_items, 0, n_edges, coo_row, coo_col, stream);
+}
+
+extern "C" int cbrs_synth_bipartite_range(int64_t n_users, int64_t n_items, int64_t n_edges, uint64_t seed,
+                                          int scatter_items, int64_t edge_lo, int64_t edge_hi, int32_t *coo_row,
+                                          int32_t *coo_col, void *stream) {
     CBRS_REQUIRE(n_users > 0 && n_items > 0 && n_edges >= 0 && n_users + n_items < ((int64_t)1 << 31), CBRS_E_INVALID,
                  "synth_bipartite: bad shape");
-    if (n_edges == 0) return CBRS_OK;
+    CBRS_REQUIRE(0 <= edge_lo && edge_lo <= edge_hi && edge_hi <= n_edges, CBRS_E_INVALID,
+                 "synth_bipartite: edge range [%lld, %lld) outside [0, %lld)", (long long)edge_lo, (long long)edge_hi,
+                 (long long)n_edges);
+    const int64_t m = edge_hi - edge_lo;
+    if (m == 0) return CBRS_OK;
+    CBRS_REQUIRE(coo_row && coo_col, CBRS_E_INVALID, "synth_bipartite: null argument");
     const uint64_t c = (uint64_t)(n_items / 1024 > 0 ? n_items / 1024 : 1);
     int levels = 1;
     while (c * ((1ull << levels) - 1) < (uint64_t)n_items) ++levels;
@@ -149,8 +163,8 @@ extern "C" int cbrs_synth_bipartite_ex(int64_t n_users, int64_t n_items, int64_t
     if (mult == 0) mult = 1;
     while (gcd64(mult, (uint64_t)n_items) != 1) ++mult;
     if (!scatter_items) mult = 1;  // item id = popularity rank: the hottest items are neighbours in id space
-    synth_bipartite_kernel<<<(unsigned)cdiv(n_edges, 256), 256, 0, (cudaStream_t)stream>>>(n_users, n_items, n_edges, seed, c,
-                                                                                         levels, mult, coo_row, coo_col);
+    synth_bipartite_kernel<<<(unsigned)cdiv(m, 256), 256, 0, (cudaStream_t)stream>>>(n_users, n_items, edge_lo, m, seed, c,
+                                                                                   levels, mult, coo_row, coo_col);
     CBRS_CHECK_LAUNCH("synth_bipartite");
     return CBRS_OK;
 }

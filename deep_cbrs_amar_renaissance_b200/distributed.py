@@ -115,6 +115,22 @@ def exchange_rows(x, ranges, group=None):
     return x
 
 
+def gather_degrees_dist(ranges, n_nodes, group=None):
+    """gather_degrees for graph.build_row_blocks in a real run: every rank contributes its blocks' degrees and gets the
+    whole vector (float32 [n_nodes]), one broadcast per block: the blocks are ragged, and gloo groups take it too."""
+    def gather(local):
+        d = torch.zeros(n_nodes, dtype=torch.float32, device=local[0][2].device if local else "cuda")
+        for a, b, v in local:
+            d[a:b].copy_(v)
+        for r, blocks in enumerate(ranges):
+            src = dist.get_global_rank(group, r) if group is not None else r
+            for a, b in blocks:
+                if b > a:
+                    dist.broadcast(d[a:b], src=src, group=group)
+        return d
+    return gather
+
+
 class SymmetricBuffer:
     """One allocation of a PeerHeap: the same number of bytes on every rank, all copies mapped here."""
 
@@ -369,6 +385,25 @@ class RowPartition:
             full = getattr(graph, view_name)
             self._slices[view_name] = [full.row_slice(a, b) for a, b in self.mine]
         return self._slices[view_name]
+
+    def build_graph(self, source, views=("norm",), gather_degrees=None, hist=None, chunk_edges=None):
+        """Partitioned build: this rank builds only its own row blocks of the graph `views` ("norm" for GCN / LightGCN,
+        "raw" for GraphSage / GAT) from `source` (graph.SyntheticSource, graph.CooSource or a scipy matrix), streamed
+        twice, and puts them in the csr_slices cache.  Each slice equals the whole build's row_slice bit for bit.
+        Returns a graph.PartitionedGraph for the model constructors (BasicGCN(graph, ...)); it has no whole-graph
+        views.  gather_degrees: graph.build_row_blocks; default gather_degrees_dist over this partition's group.
+        hist: graph.row_histogram(source) when the caller already has it (e.g. to cut the partition with
+        balance_rowptr=graph.estimated_rowptr(hist))."""
+        from . import graph as G
+        source = G.as_source(source)
+        n = sum(self.n_rows_by_type)
+        if source.n_nodes != n:
+            raise ValueError("partitioned build: the source has {} nodes, the partition {}".format(source.n_nodes, n))
+        chunk_edges = chunk_edges or G.DEFAULT_CHUNK_EDGES
+        gather = gather_degrees or gather_degrees_dist(self.ranges, n, self.group)
+        for view, slices in G.build_row_blocks(source, self.mine, gather, views, hist, chunk_edges).items():
+            self._slices[view] = slices
+        return G.PartitionedGraph(n, views, chunk_edges)
 
     def release_full_views(self, graph):
         """Keep only this rank's row slices in HBM."""

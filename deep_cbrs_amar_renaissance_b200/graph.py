@@ -251,3 +251,208 @@ class DeviceGraph:
             rowptr, colidx, vals = ops.graph_build_csr(row, col, val, n, L.GRAPH_DEDUP_SUM)  # (a + crosshop) + I
             self._views["dgcf"] = CsrSlice(rowptr, colidx.contiguous(), vals.contiguous(), n, self.chunk_edges)
         return self._views["dgcf"]
+
+
+# ------------------------------------------------------------------ partitioned build (one rank's row blocks only)
+# A rank of a row partition builds the CSR rows of its own blocks and never holds the other ranks' COO entries or the
+# whole graph's sort workspace (DESIGN.md section 3).  The COO is streamed twice from a source: pass 1 counts the
+# entries of every row (cuts, exact buffer sizes), pass 2 selects the rank's entries in their input order.  Each block
+# is then built by the kernels of the whole build with a row offset (cbrs_graph_build_block); the normalised view
+# needs every column's degree, so the blocks' degrees are gathered between its two phases (`gather_degrees`).  Every
+# slice equals DeviceGraph(...).<view>.row_slice(a, b) bit for bit: rowptr, colidx, vals and chunk decomposition.
+PIECE_EDGES = 1 << 25       # edges per generated piece of a synthetic source (2^26 entries, 512 MB of int32 pairs)
+PIECE_ENTRIES = 1 << 26     # entries per uploaded piece of a host COO source
+
+# view name -> (cbrs_graph_build flags, values kept): DeviceGraph.norm and DeviceGraph.raw
+BLOCK_VIEWS = {"norm": (L.GRAPH_DEDUP_SUM | L.GRAPH_ADD_SELF_LOOPS | L.GRAPH_SYM_NORM, True), "raw": (0, False)}
+
+
+class SyntheticSource:
+    """The graph ops.synth_bipartite(n_users, n_items, n_edges, seed, scatter_items) generates, produced in pieces of
+    `piece_edges` edges (cbrs_synth_bipartite_range) instead of all 2 * n_edges entries at once."""
+
+    def __init__(self, n_users, n_items, n_edges, seed, scatter_items=True, piece_edges=None):
+        self.n_users, self.n_items, self.n_edges = int(n_users), int(n_items), int(n_edges)
+        self.seed, self.scatter_items = int(seed), bool(scatter_items)
+        self.n_nodes = self.n_users + self.n_items
+        self.piece_edges = int(piece_edges or PIECE_EDGES)
+
+    def pieces(self, device):
+        """(row, col, val=None) pieces whose concatenation is the whole COO in its order: the forward entries of every
+        edge range, then their reverses.  A piece is valid until the next one is requested (stream order)."""
+        pe = min(self.piece_edges, max(self.n_edges, 1))
+        buf = (torch.empty(2 * pe, dtype=torch.int32, device=device), torch.empty(2 * pe, dtype=torch.int32, device=device))
+        for half in (0, 1):
+            for lo in range(0, self.n_edges, pe):
+                hi = min(lo + pe, self.n_edges)
+                m = hi - lo
+                row, col = ops.synth_bipartite_range(self.n_users, self.n_items, self.n_edges, self.seed, lo, hi, device,
+                                                     self.scatter_items, out=buf)
+                yield row[half * m:(half + 1) * m], col[half * m:(half + 1) * m], None
+
+
+class CooSource:
+    """A host COO matrix (scipy, any format; the COO entry order is kept, as DeviceGraph.from_scipy keeps it), uploaded
+    in pieces of `piece_entries` entries."""
+
+    def __init__(self, adj, piece_entries=None):
+        coo = adj.tocoo()
+        self.row = np.ascontiguousarray(coo.row, dtype=np.int32)
+        self.col = np.ascontiguousarray(coo.col, dtype=np.int32)
+        self.val = np.ascontiguousarray(coo.data, dtype=np.float32)
+        self.n_nodes = int(coo.shape[0])
+        self.piece_entries = int(piece_entries or PIECE_ENTRIES)
+
+    def pieces(self, device):
+        for lo in range(0, self.row.shape[0], self.piece_entries):
+            hi = min(lo + self.piece_entries, self.row.shape[0])
+            yield tuple(torch.from_numpy(a[lo:hi]).to(device) for a in (self.row, self.col, self.val))
+
+
+def as_source(src):
+    """a SyntheticSource / CooSource, or a scipy matrix wrapped as a CooSource"""
+    return src if hasattr(src, "pieces") else CooSource(src)
+
+
+def row_histogram(source, device):
+    """Pass 1: the number of COO entries of every row (int64 [n_nodes], on `device`)."""
+    source = as_source(source)
+    counts = torch.zeros(source.n_nodes, dtype=torch.int64, device=device)
+    for row, _, _ in source.pieces(device):
+        ops.coo_row_histogram(row, source.n_nodes, counts)
+    return counts
+
+
+def estimated_rowptr(hist, self_loops=True):
+    """[N+1] row pointer of the normalised view as far as the histogram tells it: every entry plus a self loop per row.
+    Duplicates make it an upper bound; RowPartition(balance_rowptr=...) cuts by it, and the cuts only have to be the
+    same on every rank (results do not depend on them)."""
+    lens = hist + 1 if self_loops else hist
+    return torch.cat([torch.zeros(1, dtype=torch.int64, device=hist.device), torch.cumsum(lens, 0)])
+
+
+def _select_blocks(source, blocks, hist, device):
+    """Pass 2: every block's COO entries (global row ids) in their input order, in exactly sized buffers."""
+    caps = [int(hist[a:b].sum().item()) for a, b in blocks]
+    sel = []
+    for cap in caps:
+        sel.append([torch.empty(cap, dtype=torch.int32, device=device), torch.empty(cap, dtype=torch.int32, device=device),
+                    None, torch.zeros(1, dtype=torch.int64, device=device)])
+    for row, col, val in source.pieces(device):
+        for (a, b), s in zip(blocks, sel):
+            if val is not None and s[2] is None:
+                s[2] = torch.empty(s[0].numel(), dtype=torch.float32, device=device)
+            ops.coo_select_rows(row, col, val, a, b, s[0], s[1], s[2], s[3])
+    got = [int(s[3].item()) for s in sel]
+    if got != caps:
+        raise L.CbrsError("partitioned build: selected {} entries where the histogram counted {}".format(got, caps))
+    return [(r, c, v) for r, c, v, _ in sel]
+
+
+def build_row_blocks(source, blocks, gather_degrees, views=("norm",), hist=None, chunk_edges=DEFAULT_CHUNK_EDGES,
+                     device=None):
+    """This rank's rows of the graph views `views` ("norm", "raw"): {view: [CsrSlice of rows [a, b) per block]}, each
+    equal to DeviceGraph(...).<view>.row_slice(a, b) bit for bit.
+
+    source: a SyntheticSource, CooSource or scipy matrix.  blocks: [(a, b)] non-empty row ranges.  hist: pass 1's
+    row_histogram when the caller already has it.  gather_degrees(local) -> full d: called once, for the normalised
+    view, with local = [(a, b, d of rows a..b)] of this rank; returns every node's degree (float32 [n_nodes] on the
+    device): an all-gather over the ranks (distributed.RowPartition.build_graph), or LoopbackDegrees in one process."""
+    source = as_source(source)
+    n = source.n_nodes
+    blocks = [(int(a), int(b)) for a, b in blocks]
+    if any(b <= a or a < 0 or b > n for a, b in blocks):
+        raise ValueError("partitioned build: row blocks {} of a {}-node graph (each non-empty)".format(blocks, n))
+    unknown = [v for v in views if v not in BLOCK_VIEWS]
+    if unknown:
+        raise ValueError("partitioned build: views {} (built: {})".format(unknown, sorted(BLOCK_VIEWS)))
+    device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+    if hist is None:
+        hist = row_histogram(source, device)
+    coo = _select_blocks(source, blocks, hist, device)
+    built = {}
+    for view in views:
+        flags, _ = BLOCK_VIEWS[view]
+        built[view] = [ops.graph_build_block(r, c, v if flags & L.GRAPH_DEDUP_SUM else None, a, b, n, flags)
+                       for (a, b), (r, c, v) in zip(blocks, coo)]
+    del coo
+    if "norm" in built:
+        d = gather_degrees([(a, b, blk[3]) for (a, b), blk in zip(blocks, built["norm"])])
+        for (a, _), (rowptr, colidx, vals, _) in zip(blocks, built["norm"]):
+            ops.graph_block_scale(rowptr, colidx, vals, a, n, d)
+        del d
+    blocking = blocking_policy(n)
+    return {view: [CsrSlice(rowptr, colidx.contiguous(), vals.contiguous() if BLOCK_VIEWS[view][1] else None, n,
+                            chunk_edges, row_offset=a, blocking=blocking)
+                   for (a, _), (rowptr, colidx, vals, _) in zip(blocks, built[view])]
+            for view in views}
+
+
+class LoopbackDegrees:
+    """gather_degrees for the ranks of a partition emulated one after the other in one process: the full degree vector
+    is assembled from every rank's blocks, each built in turn (phase 1 of the normalised view, only its degrees kept).
+    A call checks that the calling rank's own degrees are the ones assembled, bit for bit."""
+
+    def __init__(self, source, ranges, hist=None, device=None):
+        source = as_source(source)
+        device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        hist = row_histogram(source, device) if hist is None else hist
+        flags = BLOCK_VIEWS["norm"][0]
+        self.d = torch.empty(source.n_nodes, dtype=torch.float32, device=device)
+        for rank_blocks in ranges:
+            blocks = [(a, b) for a, b in rank_blocks if b > a]
+            for (a, b), (r, c, v) in zip(blocks, _select_blocks(source, blocks, hist, device)):
+                self.d[a:b].copy_(ops.graph_build_block(r, c, v, a, b, source.n_nodes, flags)[3])
+                del r, c, v
+
+    def __call__(self, local):
+        for a, b, d in local:
+            if not torch.equal(d, self.d[a:b]):
+                raise L.CbrsError("loopback degrees: rows [{}, {}) differ from the assembled vector".format(a, b))
+        return self.d
+
+
+class PartitionedGraph(DeviceGraph):
+    """What a model sees of a partitioned build (distributed.RowPartition.build_graph): the graph's shape and node
+    count only.  The rows exist on the ranks that own them, as the partition's csr_slices; whole-graph access raises,
+    so no code path can pick up a partial matrix in place of the whole one."""
+
+    def __init__(self, n_nodes, views, chunk_edges=DEFAULT_CHUNK_EDGES):
+        self.n_nodes, self.n_rel = int(n_nodes), 1
+        self.shape = (self.n_nodes, self.n_nodes)
+        self.views = tuple(views)
+        self.chunk_edges = chunk_edges
+        self.row = self.col = self.val = self.rel = None
+        self._views = {}
+
+    def _whole(self, what):
+        raise NotImplementedError(
+            "{} of a partitioned graph build: each rank holds only its own row blocks (views {}), as "
+            "RowPartition.csr_slices; build a DeviceGraph for whole-graph access".format(what, ", ".join(self.views)))
+
+    def _view(self, name, flags, keep_vals, self_rel=0):
+        self._whole("the '%s' view" % name)
+
+    @property
+    def symmetric(self):
+        self._whole("the symmetry test")
+
+    @property
+    def dgcf(self):
+        self._whole("the 'dgcf' view")
+
+    def transposed(self):
+        self._whole("the transpose")
+
+    def row_subset(self, ids):
+        self._whole("a row subset")
+
+    def release_coo(self):
+        pass
+
+
+def refuse_partitioned(graphs, what):
+    """NotImplementedError when one of `graphs` is a PartitionedGraph: `what` has no partitioned build."""
+    if any(isinstance(g, PartitionedGraph) for g in graphs):
+        raise NotImplementedError("{} on a partitioned graph build (it has no partitioned form; build a DeviceGraph)"
+                                  .format(what))

@@ -359,6 +359,8 @@ class Model(Layer):
         epoch depends only on its index, so a model and sequences saved after epoch k-1 and trained on with
         initial_epoch=k replay the batches of the run that never stopped.  A BackupAndRestore callback that finds a
         saved state sets the start epoch itself."""
+        from . import training
+        training.check_not_partitioned_build(self)
         callbacks = list(callbacks or [])
         hist = History()
         rng = np.random.RandomState(self.shuffle_seed)

@@ -32,6 +32,11 @@ class SequentialGNN(Model):
         self._finish_init(adj_matrix, seq_layers, final_node)
 
     def _finish_init(self, adj_matrix, seq_layers, final_node):
+        if type(self) is not SequentialGNN:
+            graph.refuse_partitioned([adj_matrix], "a Two-Step / Two-Way GNN stack")
+        for layer in seq_layers:
+            if not isinstance(layer, (GCNConv, LightGCNConv, GraphSageConv, GATConv)):
+                graph.refuse_partitioned([adj_matrix], type(layer).__name__)
         self.adj_matrix = convert_to_tensor(adj_matrix, device=default_device())
         self.n_nodes = int(adj_matrix.shape[0])
         self.dropout = None
@@ -265,6 +270,7 @@ class RGCN(GNN):
     with one relation - e.g. a plain scipy matrix - it equals GCN."""
 
     def __init__(self, adj_matrix, n_hiddens=(8, 8, 8), **kwargs):
+        graph.refuse_partitioned([adj_matrix], "RGCN")
         if not isinstance(adj_matrix, DeviceGraph):
             adj_matrix = DeviceGraph.from_scipy(adj_matrix, relational=True)   # keeps RelationalAdjacency's edge types
         self.n_hiddens = n_hiddens

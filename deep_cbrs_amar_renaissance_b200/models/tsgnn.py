@@ -6,6 +6,7 @@ puts in `trainset.adj_matrix`; constructor call as in experiment.py:142-146:
 cls(len(users), len(items), trainset.adj_matrix, **config.model)."""
 import abc
 
+from .. import graph
 from ..keras_like import L2, Model
 from ..layers import DGCFConv, GATConv, GCNConv, GraphSageConv, LightGCNConv
 from .gnn import HalfInputSequentialGNN, SequentialGNN
@@ -18,6 +19,7 @@ class TwoStepGNN(Model, abc.ABC):
         regularizer = L2(l2_regularizer) if l2_regularizer is not None else None
         if len(adj_matrices) != 2:
             raise ValueError('Exactly two adjacency matrix are needed!')
+        graph.refuse_partitioned(adj_matrices, type(self).__name__)
         adj_ui_matrix, adj_kg_matrix = adj_matrices
         step_one = [self.build_gnn_layer(i, regularizer=regularizer) for i in range(n_hops)]
         self.step_one_gnn_layers = SequentialGNN(adj_kg_matrix, step_one, embedding_dim=embedding_dim, final_node=item_node,

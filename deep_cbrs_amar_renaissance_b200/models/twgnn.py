@@ -9,6 +9,7 @@ import abc
 
 import torch
 
+from .. import graph
 from ..keras_like import L2, Model
 from ..layers import DGCFConv, GATConv, GCNConv, GraphSageConv, LightGCNConv
 from .gnn import FullInputSequentialGNN, SequentialGNN
@@ -21,6 +22,7 @@ class TwoWayGNN(Model, abc.ABC):
         regularizer = L2(l2_regularizer) if l2_regularizer is not None else None
         if len(adj_matrices) != 3:
             raise ValueError('Exactly three adjacency matrix are needed!')
+        graph.refuse_partitioned(adj_matrices, type(self).__name__)
         adj_ui_matrix, adj_ip_matrix, adj_up_matrix = adj_matrices
         way_one = [self.build_gnn_layer(i, regularizer=regularizer) for i in range(n_hops)]
         self.way_one_gnn_layers = SequentialGNN(adj_up_matrix, way_one, embedding_dim=embedding_dim, final_node=user_item_node,

@@ -77,6 +77,65 @@ def graph_build_csr(row, col, val, n_nodes, flags, rel=None, n_rel=1, self_rel=0
     return rowptr, colidx[:n_out], vals[:n_out]
 
 
+# ------------------------------------------------------------------ partitioned build (rows of one block only)
+def coo_row_histogram(row, n_rows, counts=None):
+    """counts[r] += number of entries of row r (int64 [n_rows], created zeroed when None); rows outside are ignored."""
+    lib = L.load()
+    if counts is None:
+        counts = torch.zeros(n_rows, dtype=torch.int64, device=row.device)
+    L.check(lib.cbrs_coo_row_histogram(_ptr(row, torch.int32), row.numel(), n_rows, _ptr(counts, torch.int64), _stream()),
+            "cbrs_coo_row_histogram")
+    return counts
+
+
+def coo_select_rows(row, col, val, row_lo, row_hi, out_row, out_col, out_val, cursor, rebase=False):
+    """Appends the entries of rows [row_lo, row_hi), in input order, to out_* at the device int64 `cursor`, which
+    advances by their number (cbrs_coo_select_rows).  Nothing is written past the outputs' length."""
+    lib = L.load()
+    n = row.numel()
+    if n == 0:
+        return cursor
+    ws = _ws(lib.cbrs_coo_select_rows_workspace_bytes(n), row.device)
+    L.check(lib.cbrs_coo_select_rows(_ptr(row, torch.int32), _ptr(col, torch.int32), _ptr(val, torch.float32), n,
+                                     int(row_lo), int(row_hi), 1 if rebase else 0, _ptr(out_row, torch.int32),
+                                     _ptr(out_col, torch.int32), _ptr(out_val, torch.float32), _ptr(cursor, torch.int64),
+                                     out_row.numel(), _ptr(ws), ws.numel(), _stream()), "cbrs_coo_select_rows")
+    return cursor
+
+
+def graph_build_block(row, col, val, row_lo, row_hi, n_nodes, flags):
+    """Phase 1 of a row block's build (cbrs_graph_build_block): COO entries of rows [row_lo, row_hi) (global ids) ->
+    (rowptr int64, colidx int32, vals float32, dinv float32 [row_hi - row_lo] or None).  With GRAPH_SYM_NORM the
+    values are left unscaled and dinv holds the block's degrees; graph_block_scale finishes them."""
+    lib = L.load()
+    dev = row.device
+    nnz, n_rows = row.numel(), int(row_hi) - int(row_lo)
+    cap = nnz + (n_rows if flags & L.GRAPH_ADD_SELF_LOOPS else 0)
+    rowptr = torch.empty(n_rows + 1, dtype=torch.int64, device=dev)
+    colidx = torch.empty(max(cap, 1), dtype=torch.int32, device=dev)
+    vals = torch.empty(max(cap, 1), dtype=torch.float32, device=dev)
+    dinv = torch.empty(n_rows, dtype=torch.float32, device=dev) if flags & L.GRAPH_SYM_NORM else None
+    ws = _ws(lib.cbrs_graph_build_block_workspace_bytes(nnz, n_rows, flags), dev)
+    L.check(lib.cbrs_graph_build_block(_ptr(row, torch.int32), _ptr(col, torch.int32), _ptr(val, torch.float32), nnz,
+                                       int(row_lo), int(row_hi), int(n_nodes), flags, _ptr(rowptr), _ptr(colidx),
+                                       _ptr(vals), _ptr(dinv), None, _ptr(ws), ws.numel(), _stream()),
+            "cbrs_graph_build_block")
+    del ws
+    n_out = int(rowptr[-1].item())
+    return rowptr, colidx[:n_out], vals[:n_out], dinv
+
+
+def graph_block_scale(rowptr, colidx, vals, row_lo, n_nodes, dinv):
+    """Phase 2: vals = fl32(fl32(d_i * m_ij) * d_j) in place, d = every node's degree (float32 [n_nodes])."""
+    lib = L.load()
+    if dinv.numel() != n_nodes:
+        raise L.CbrsError("graph_block_scale: {} degrees for {} nodes".format(dinv.numel(), n_nodes))
+    L.check(lib.cbrs_graph_block_scale(_ptr(rowptr, torch.int64), _ptr(colidx, torch.int32), _ptr(vals, torch.float32),
+                                       rowptr.numel() - 1, int(row_lo), int(n_nodes), _ptr(dinv, torch.float32),
+                                       _stream()), "cbrs_graph_block_scale")
+    return vals
+
+
 def build_chunks(rowptr, chunk_edges, colidx=None, n_cols=0, block_cols=0, block_min_len=0):
     """Chunk decomposition of a CSR row-pointer (see cbrs_csr_t).  With block_cols > 0 rows of at least
     block_min_len edges are cut at column-block borders and scheduled by (column block, row)
@@ -769,6 +828,21 @@ def synth_bipartite(n_users, n_items, n_edges, seed, device, scatter_items=True)
     col = torch.empty(2 * n_edges, dtype=torch.int32, device=device)
     L.check(lib.cbrs_synth_bipartite_ex(n_users, n_items, n_edges, seed, 1 if scatter_items else 0, _ptr(row), _ptr(col),
                                         _stream()), "cbrs_synth_bipartite_ex")
+    return row, col
+
+
+def synth_bipartite_range(n_users, n_items, n_edges, seed, edge_lo, edge_hi, device, scatter_items=True, out=None):
+    """The entries of edges [edge_lo, edge_hi) of synth_bipartite(n_users, n_items, n_edges, seed): (row, col) of
+    2 * (edge_hi - edge_lo) entries, the forward ones first, then their reverses.  out: (row, col) int32 buffers of
+    at least that length to write into (views of them are returned)."""
+    lib = L.load()
+    m = max(int(edge_hi) - int(edge_lo), 0)     # an inverted range is refused by the library
+    if out is None:
+        out = (torch.empty(2 * m, dtype=torch.int32, device=device), torch.empty(2 * m, dtype=torch.int32, device=device))
+    row, col = out[0][:2 * m], out[1][:2 * m]
+    L.check(lib.cbrs_synth_bipartite_range(n_users, n_items, n_edges, seed, 1 if scatter_items else 0, int(edge_lo),
+                                           int(edge_hi), _ptr(row, torch.int32), _ptr(col, torch.int32), _stream()),
+            "cbrs_synth_bipartite_range")
     return row, col
 
 

@@ -429,6 +429,19 @@ def concat_rows_train(tape, nodes):
 PARTITIONED_LAYERS = (GCNConv, RGCNConv, LightGCNConv, GraphSageConv, GATConv)
 
 
+def check_not_partitioned_build(model):
+    """Raises NotImplementedError, before any device work, when a GNN stack of `model` runs on a partitioned graph
+    build: the partitioned tape multiplies by row slices of the whole operator and of its transpose, which no rank of
+    such a build holds."""
+    from .graph import PartitionedGraph
+    from .models.gnn import SequentialGNN
+    gnn = getattr(model, "gnn", None)
+    for s in (vars(gnn).values() if gnn is not None else ()):
+        if isinstance(s, SequentialGNN) and isinstance(s.adj_matrix, PartitionedGraph):
+            raise NotImplementedError("training on a partitioned graph build (RowPartition.build_graph holds only each "
+                                      "rank's row blocks; train on a DeviceGraph)")
+
+
 def check_partitioned_training(seq):
     """Raises NotImplementedError, before any device work, for a partitioned stack the row-split tape does not cover."""
     for layer in seq.seq_layers:
@@ -710,6 +723,7 @@ def l2_coefficients(model):
 
 def train_step(model, optimizer, inputs, y, capturing=False):
     """One optimiser step on one batch.  Returns device scalars (loss incl. the l2 penalty, #correct)."""
+    check_not_partitioned_build(model)
     tape, loss, correct, _ = forward_backward(model, inputs, y)
     l2 = l2_coefficients(model)
     ws = [w for w in model.trainable_weights if id(w) in tape.wgrads]
@@ -733,6 +747,7 @@ class GraphedTrainStep:
     def __init__(self, model, optimizer, batch_size, content_dim=None):
         import numpy as np
         from .models.gnn import SequentialGNN
+        check_not_partitioned_build(model)
         gnn = getattr(model, "gnn", None)
         stacks = [s for s in vars(gnn).values() if isinstance(s, SequentialGNN)] if gnn is not None else []
         if any(s.partition is not None for s in stacks):

@@ -74,6 +74,39 @@ int cbrs_graph_build_csr_rel(const int32_t *coo_row, const int32_t *coo_col, con
                              int32_t self_rel, int flags, int64_t *rowptr, int32_t *colidx, float *vals,
                              int64_t *nnz_out, void *workspace, size_t workspace_bytes, void *stream);
 
+/* ---- partitioned build: the rows [row_lo, row_hi) of the graph cbrs_graph_build_csr builds -------------------
+ * A rank of a row partition builds only its own row blocks, bit for bit the rows the whole build gives them:
+ *   1. cbrs_coo_row_histogram over every piece of the COO -> exact entry counts per row (cuts, buffer sizes);
+ *   2. cbrs_coo_select_rows over every piece, in input order -> the block's entries, in their input order (the
+ *      duplicate sum adds them in that order);
+ *   3. cbrs_graph_build_block: sort, duplicate sum, self loops and row pointer for the block's rows only.  With
+ *      CBRS_GRAPH_SYM_NORM it writes the block's d_i = fl32(1/sqrt(double(rowsum_i))) to dinv_out and leaves the
+ *      values UNscaled: d_j of most columns belongs to other blocks;
+ *   4. cbrs_graph_block_scale once every block's d is known: vals = fl32(fl32(d_i*m_ij)*d_j), d = the full vector.
+ * Same kernels and rounding as cbrs_graph_build_csr, so rowptr / colidx / vals equal that build's rows row_lo..row_hi
+ * (rowptr rebased to 0, global column ids).  The workspace scales with the block's entries.                     */
+/* counts[r] += entries of row r, r in [0, n_rows) (int64, caller zeroes it; other rows are ignored) */
+int cbrs_coo_row_histogram(const int32_t *coo_row, int64_t n, int64_t n_rows, int64_t *counts, void *stream);
+size_t cbrs_coo_select_rows_workspace_bytes(int64_t n);
+/* Appends the entries with row_lo <= row < row_hi, in input order, at out[*cursor ..] and advances *cursor (device
+ * int64) by their number; rebase != 0 stores row - row_lo.  coo_val / out_val may be NULL.  Entries that would land
+ * at or past `capacity` are not written (the cursor still counts them: compare it with the capacity afterwards).  */
+int cbrs_coo_select_rows(const int32_t *coo_row, const int32_t *coo_col, const float *coo_val, int64_t n,
+                         int64_t row_lo, int64_t row_hi, int rebase, int32_t *out_row, int32_t *out_col,
+                         float *out_val, int64_t *cursor, int64_t capacity, void *workspace, size_t workspace_bytes,
+                         void *stream);
+/* nnz = the block's entries (global row ids); n_rows = row_hi - row_lo; n_cols = the graph's node count.
+ * Capacity of colidx / vals: nnz (+ n_rows with ADD_SELF_LOOPS).  rowptr [n_rows + 1].  dinv_out [n_rows] (needed
+ * with SYM_NORM).                                                                                              */
+size_t cbrs_graph_build_block_workspace_bytes(int64_t nnz, int64_t n_rows, int flags);
+int cbrs_graph_build_block(const int32_t *coo_row, const int32_t *coo_col, const float *coo_val, int64_t nnz,
+                           int64_t row_lo, int64_t row_hi, int64_t n_cols, int flags, int64_t *rowptr,
+                           int32_t *colidx, float *vals, float *dinv_out, int64_t *nnz_out, void *workspace,
+                           size_t workspace_bytes, void *stream);
+/* rows [row_lo, row_lo + n_rows) of a block built above; dinv: all n_cols degrees */
+int cbrs_graph_block_scale(const int64_t *rowptr, const int32_t *colidx, float *vals, int64_t n_rows, int64_t row_lo,
+                           int64_t n_cols, const float *dinv, void *stream);
+
 /* ---- work decomposition -------------------------------------------------
  * Rows are cut into chunks of at most chunk_edges edges so that power-law item
  * rows do not serialise on one warp.  A row with a single chunk is written by
@@ -439,6 +472,12 @@ int cbrs_synth_bipartite(int64_t n_users, int64_t n_items, int64_t n_edges, uint
  * catalogue that is sorted by popularity - the adversarial case for a row-count partition (SURVEY 8e).  1 = as above. */
 int cbrs_synth_bipartite_ex(int64_t n_users, int64_t n_items, int64_t n_edges, uint64_t seed, int scatter_items,
                             int32_t *coo_row, int32_t *coo_col, void *stream);
+/* The entries of edges [edge_lo, edge_hi) only, 2*(edge_hi - edge_lo) of them: the forward entries of those edges
+ * in [0, m) and their reverses in [m, 2m), m = edge_hi - edge_lo, each with the bits cbrs_synth_bipartite_ex writes
+ * for that edge.  The forward parts of consecutive ranges, then their reverse parts, make up the whole output:
+ * a graph can be streamed in fixed-size pieces instead of holding all 2*n_edges entries.                          */
+int cbrs_synth_bipartite_range(int64_t n_users, int64_t n_items, int64_t n_edges, uint64_t seed, int scatter_items,
+                               int64_t edge_lo, int64_t edge_hi, int32_t *coo_row, int32_t *coo_col, void *stream);
 
 /* ---- peer memory + producer kernels that store into every rank's copy (SURVEY 8e; multi-GPU) ---
  * One process per GPU.  Every rank allocates the same ("symmetric") buffers with
